@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: detection inference images/sec INCLUDING NMS (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4|5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4|5] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...      (N > 1, one rank per GPU)
 
 One "step" = one pass of the hot path (forward + DFL decode + batched NMS) over one batch of synthetic images per GPU.
@@ -15,6 +15,11 @@ One "step" = one pass of the hot path (forward + DFL decode + batched NMS) over 
 
 Images shard across ranks with no collective on the data path (SURVEY.md 8e); NCCL only gathers the timing.
 Prints ONE JSON line (rank 0).
+
+`--dump-outputs DIR` writes what the last timed step returned to its caller: one float32 [n, 6] array per image
+(x1, y1, x2, y2, score, class) as DIR/det_<image>.npy, <image> counting over all ranks.  Inputs and weights are seeded,
+so two builds run with the same arguments can be compared file for file.  Only runs of the same --impl compare: the
+reference arm times its own smaller sample, so its det_000000.npy is a different image from the GPU arm's.
 
   value      images/s, device-timed (CUDA events), inputs already resident in HBM, through the PUBLIC API:
              YOLO.forward + non_max_suppression_async(...).result() -- i.e. including the D2H of the per-image counts
@@ -155,6 +160,24 @@ def cpu_reference_step(nodes, nc, sd, x, conf, iou):
     return N.non_max_suppression(y.permute(0, 2, 1).contiguous(), conf, iou, MAX_DET)
 
 
+DUMP_BYTES = 64_000_000    # --dump-outputs budget over all ranks
+NPY_HEADER = 128           # bytes numpy writes ahead of the data of a small 2-D array
+
+
+def dump_detections(out_dir: Path, dets, first_image: int, world: int) -> None:
+    """One float32 [n, 6] .npy per image.  A batch whose worst case (MAX_DET rows per image) would exceed this rank's share
+    of DUMP_BYTES is represented by a fixed, seeded sample of its images."""
+    import numpy as np
+    out_dir.mkdir(parents=True, exist_ok=True)
+    fits = max(1, DUMP_BYTES // world // (MAX_DET * 6 * 4 + NPY_HEADER))
+    idx = range(len(dets))
+    if len(dets) > fits:
+        idx = sorted(torch.randperm(len(dets), generator=torch.Generator().manual_seed(0))[:fits].tolist())
+    for i in idx:
+        d = dets[i] if isinstance(dets[i], np.ndarray) else dets[i].cpu().numpy()
+        np.save(out_dir / f"det_{first_image + i:06d}.npy", d.astype(np.float32))
+
+
 def per_gpu_batch(cfg: dict, world: int, override: int) -> int:
     if override > 0:
         return override
@@ -181,8 +204,10 @@ def run_reference(args, cfg):
         cpu_reference_step(nodes, nc, sd, x, cfg["conf"], cfg["iou"])
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        cpu_reference_step(nodes, nc, sd, x, cfg["conf"], cfg["iou"])
+        dets = cpu_reference_step(nodes, nc, sd, x, cfg["conf"], cfg["iou"])
     dt = (time.perf_counter() - t0) / args.steps
+    if args.dump_outputs:
+        dump_detections(Path(args.dump_outputs), dets, 0, 1)
     v = sample / dt
     print(json.dumps({
         "impl": "reference", "metric": cfg["metric"], "value": v, "unit": "images/s",
@@ -210,7 +235,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--quick", action="store_true", help="skip the secondary measurements (fp32-input e2e, default-flags run)")
     ap.add_argument("--per-op", default="", help="write a per-launch CSV (kernel, shape, ms, TFLOP/s) to this path")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the detections of the last timed step to DIR/det_<image>.npy (float32 [n, 6])")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     cfg = CONFIGS[args.config]
 
@@ -314,6 +343,8 @@ def main():
     clocks = sampler.stop() if rank == 0 else None
     value = world * Bn * args.steps / (ms_max / 1e3)
     dets_per_img = sum(len(d) for d in dets) / max(1, len(dets))
+    if args.dump_outputs:
+        dump_detections(Path(args.dump_outputs), dets, rank * Bn, world)
 
     # the same steps with no host synchronisation (nms_raw): what the host-side tail of the public API costs
     sync_all()

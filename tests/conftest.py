@@ -1,4 +1,3 @@
-import os
 import sys
 from pathlib import Path
 
@@ -12,10 +11,6 @@ for p in (ROOT, ROOT / "yolo-re_b200"):
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    config.addinivalue_line("markers", "reference: needs the reference checkout at /root/reference")
-
-
-HAVE_REFERENCE = os.path.isdir("/root/reference/src/yolo")
 
 
 @pytest.fixture(scope="session")

@@ -100,7 +100,9 @@ class Plan:
         self.device, self.batch, self.prec = device, batch, prec
         self.dt = L.BF16 if prec == "bf16" else L.F32
         self.tdt = torch.bfloat16 if prec == "bf16" else torch.float32
-        self.engine = L.ENGINE_AUTO if prec == "bf16" else L.ENGINE_FFMA
+        # tcgen05 convs encode TMA descriptors of device buffers, so a dry (host-buffer) plan takes the FFMA engine even
+        # where a CUDA driver is present
+        self.engine = L.ENGINE_AUTO if prec == "bf16" and not self.dry else L.ENGINE_FFMA
         h = C.c_void_p()
         L.check(self.lib.yre_plan_create(C.byref(h)), "plan_create")
         self.h = h
