@@ -90,6 +90,12 @@ typedef struct yre_conv_desc {
     yre_view    xu;         /* xu.ptr == NULL: plain conv */
 } yre_conv_desc;
 int yre_conv(const yre_conv_desc* d, yre_stream_t s);
+/* Host-only query: the string yre_plan_op_variant reports for d on the tcgen05 engine of a device with num_sms SMs.  No
+ * device is touched and no pointer is dereferenced.  d is validated as yre_conv validates it; beyond that, of the
+ * pointers only whether res.ptr and xu.ptr are NULL changes the result (address alignment is not checked).
+ * YRE_EUNSUPPORTED, with the reason in yre_last_error(), when the engine does not take the shape or its tile does not fit
+ * shared memory. */
+int yre_conv_tc_describe(const yre_conv_desc* d, int32_t num_sms, char* out, int32_t cap);
 
 /* ---- K2: first conv straight from the image ------------------------------------------------------
  * Replaces layers.stem1 (Conv 3x3 s2 on the input image; configs/models/gelan-c.yaml stem1,

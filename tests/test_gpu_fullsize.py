@@ -19,6 +19,7 @@ from bench_data import make_inputs
 from oracle import nms_ref as N
 from tests import cpu_plan_exec as X
 from tests.conftest import ROOT
+from tests.test_cpu_conv_tc_select import tc_variant
 
 pytestmark = pytest.mark.gpu
 
@@ -165,8 +166,9 @@ def test_full_size_batch_permutation_and_nms(request):
 
 
 def test_kernel_selection_rules_at_config_2(request):
-    """The per-layer kernel selection (conv_tc_prepare, rules measured in profiles/r02_notes.md) is visible through
-    yre_plan_op_variant; pin what the full-size config-2 plan gets so that a rule change shows up here."""
+    """The per-layer kernel selection (conv_tc_select, rules measured in profiles/r02_notes.md) is visible through
+    yre_plan_op_variant; pin what the full-size config-2 plan gets so that a rule change shows up here.  The host-only
+    query yre_conv_tc_describe must report exactly what the plan prepared on the device."""
     name, img, Bn = CONFIGS[2]
     model = _model(name, request)
     x = make_inputs(Bn, img, seed=7).to(DEV)
@@ -174,6 +176,11 @@ def test_kernel_selection_rules_at_config_2(request):
         p = E.compile_model(model, x)
     rows = [(d, v) for (n, _), d, v in zip(p.op_table(), p.op_descriptions(), p.op_variants()) if n == "conv_tc"]
     assert len(rows) == p.num_tcgen05 and "conv_ffma" not in [n for n, _ in p.op_table()]
+    sms = torch.cuda.get_device_properties(x.device).multi_processor_count
+    convs = [(v, a) for (kind, a), v in zip(p.trace, p.op_variants()) if kind == "conv"]
+    assert len(convs) == len(rows)
+    for v, a in convs:
+        assert tc_variant(a, sms) == v
 
     def variants(prefix):
         got = {v.split(" thr=")[0] for d, v in rows if d.startswith(prefix)}

@@ -16,7 +16,8 @@
 //                             streamed through a second ring, optionally two patches per weight box; on maps that 8x16
 //                             patches do not tile, 8x8 patches of two images (TcParams::ybx).
 // conv_tc_kernel<.., CTA2>: clusters of two CTAs feed one 256-row cta_group::2 MMA (each stages half of the weight tile).
-// Which kernel / tile shape a layer gets is decided in conv_tc_prepare from rules measured per layer (profiles/r02_notes.md).
+// Which kernel / tile shape a layer gets is decided by conv_tc_select, a host-only function of the shapes and the SM count,
+// from rules measured per layer (profiles/r02_notes.md); yre_conv_tc_describe reports its choice without a device.
 // Operands land in 128B- (BLOCK_K=64) or 64B- (BLOCK_K=32) swizzled shared memory that the UMMA smem descriptors read
 // directly.  Accumulators live in a ring of TMEM buffers (6x64, 4x128, 3x160 or 2x256 columns), so the epilogue of
 // one tile overlaps the MMAs of the next ones.  All kernels are persistent (grid = min(work units, SMs)).
@@ -35,8 +36,10 @@
 // UTCHMMA/UTMALDG in a serialising ELECT loop.  Measurements behind the design choices: profiles/r01_notes.md.
 #include "yre_common.cuh"
 #include <cuda.h>
+#include <algorithm>
 #include <cstring>
 #include <cstdlib>
+#include <memory>
 
 struct ConvTcPlan;
 
@@ -1129,23 +1132,19 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
 EncodeTiledFn get_encode() {
-    static EncodeTiledFn fn = nullptr;
-    static bool tried = false;
-    if (!tried) {
-        tried = true;
+    static const EncodeTiledFn fn = [] {          // looked up once, thread-safe
         void* sym = nullptr;
         cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &sym, cudaEnableDefault, &qres) == cudaSuccess &&
-            qres == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<EncodeTiledFn>(sym);
-    }
+        const bool ok = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &sym, cudaEnableDefault, &qres) == cudaSuccess &&
+                        qres == cudaDriverEntryPointSuccess;
+        return ok ? reinterpret_cast<EncodeTiledFn>(sym) : nullptr;
+    }();
     return fn;
 }
 
 int* g_trace_buf = nullptr;
 
-// Tuning knobs (YRE_TC_*) exist only in builds made with -DYRE_TUNING (YRE_TUNING=1 python yolo-re_b200/build.py);
-// the product build reads no environment variables.
+// ---- knobs ----
 int env_int(const char* name, int dflt) {
 #ifdef YRE_TUNING
     const char* v = getenv(name);
@@ -1156,58 +1155,45 @@ int env_int(const char* name, int dflt) {
 #endif
 }
 
-}  // namespace
-
-struct ConvTcPlan {
-    CUtensorMap tmA, tmB, tmY, tmAu;
-    TcParams p;
-    int grid;
-    size_t smem;
+struct TcKnobs {
+    int pdl, sms, halo, halo_slack, halo_wide, halo_ybx, halo_pair, halo_pair64, halo_tps, prefer128, block_n, cta2, threads,
+        tgroups, split, stages, pipes, stage64, direct_store, f32_tma, l2promo_a, trace;
 };
 
-// output tensor map of the staged TMA store: one box = the 32 pixels of a TMEM lane quarter x 32 (64 with stage64) channels;
-// fp32 outputs use 128-byte rows (32 channels) in a 128B-swizzled tile.  Also used when an output buffer is re-bound.
-static CUresult encode_y(ConvTcPlan* pl, void* ptr) {
-    const auto& p = pl->p;
-    const cuuint64_t es = p.y_f32 ? 4 : 2, ct = (cuuint64_t)p.y_ctot;
-    cuuint64_t gdim[4] = {ct, (cuuint64_t)p.Wo, (cuuint64_t)p.Ho, (cuuint64_t)p.B};
-    cuuint64_t gstr[3] = {ct * es, (cuuint64_t)p.Wo * ct * es, (cuuint64_t)p.Ho * p.Wo * ct * es};
-    cuuint32_t box[4] = {p.stage64 ? 64u : 32u, (cuuint32_t)p.stw, (cuuint32_t)p.sth, (cuuint32_t)p.stb};
-    if (p.ybx) {                                                   // {C, W, B, H}, like the input map
-        gdim[2] = (cuuint64_t)p.B; gdim[3] = (cuuint64_t)p.Ho;
-        const cuuint64_t sh = gstr[1], sb = gstr[2];
-        gstr[1] = sb; gstr[2] = sh;
-        box[2] = (cuuint32_t)p.stb; box[3] = (cuuint32_t)p.sth;
-    }
-    cuuint32_t est[4] = {1, 1, 1, 1};
-    return get_encode()(&pl->tmY, p.y_f32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, ptr, gdim, gstr, box, est,
-                        CU_TENSOR_MAP_INTERLEAVE_NONE, (p.stage64 || p.y_f32) ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
-                        CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+// Tuning knobs (YRE_TC_*) are read only in builds made with -DYRE_TUNING (YRE_TUNING=1 python yolo-re_b200/build.py); the
+// product build reads no environment variables and runs with the defaults below.  A "forced" knob left at its default
+// leaves the rule in charge.  (YRE_TC_REV, the tile-walk order of a plan, is read in yre_capi.cu.)
+TcKnobs tc_knobs() {
+    TcKnobs k;
+    k.pdl          = env_int("YRE_TC_PDL", 1);            // programmatic dependent launch
+    k.sms          = env_int("YRE_TC_SMS", 0);            // > 0: persistent grids sized for that many SMs, not the device's
+    k.halo         = env_int("YRE_TC_HALO", 2);           // 0: no halo kernels, 1: the weight-stationary one only, 2: both
+    k.halo_slack   = env_int("YRE_TC_HALO_SLACK", 100);   // streamed halo while its tiles are <= this % of the generic tiles
+    k.halo_wide    = env_int("YRE_TC_HALO_WIDE", 0);      // 1: streamed halo also where Cout tiles into 256-wide N
+    k.halo_ybx     = env_int("YRE_TC_HALO_YBX", 1);       // 0: no two-image 8x8 halo tiles, 2: also for Cout % 128 == 0
+    k.halo_pair    = env_int("YRE_TC_HALO_PAIR", 1);      // 0: no patch pairs on the streamed halo kernel
+    k.halo_pair64  = env_int("YRE_TC_HALO_PAIR64", 1);    // 0: no patch pairs for a single 64-wide N tile
+    k.halo_tps     = env_int("YRE_TC_HALO_TPS", 0);       // 1 or 3: forced filter taps per weight slot (streamed halo)
+    k.prefer128    = env_int("YRE_TC_PREFER128", 1);      // 128-wide N tiles instead of the widths between 128 and 256
+    k.block_n      = env_int("YRE_TC_BLOCK_N", 0);        // forced N tile width
+    k.cta2         = env_int("YRE_TC_CTA2", -1);          // 0: no CTA pairs, 1: CTA pairs wherever legal
+    k.threads      = env_int("YRE_TC_THREADS", 0);        // forced threads per CTA (384 or 512)
+    k.tgroups      = env_int("YRE_TC_TGROUPS", 0);        // forced epilogue tile groups
+    k.split        = env_int("YRE_TC_SPLIT", 0);          // forced epilogue column split
+    k.stages       = env_int("YRE_TC_STAGES", 0);         // forced (shallower) operand ring
+    k.pipes        = env_int("YRE_TC_PIPES", 0);          // forced (producer, MMA) pair count
+    k.stage64      = env_int("YRE_TC_STAGE64", -1);       // 0: no 64-column output staging, 1: wherever legal
+    k.direct_store = env_int("YRE_TC_DIRECT_STORE", 0);   // 1: bf16 outputs without the staged TMA store
+    k.f32_tma      = env_int("YRE_TC_F32_TMA", 1);        // 0: fp32 outputs without the staged TMA store
+    k.l2promo_a    = env_int("YRE_TC_L2PROMO_A", (int)CU_TENSOR_MAP_L2_PROMOTION_L2_128B);   // L2 promotion of activation loads
+    k.trace        = env_int("YRE_TC_TRACE", 0);          // 1: per-role pipeline trace (yre_debug_read_trace)
+    return k;
 }
 
-template <typename K>
-static cudaError_t launch_tc(K kernel, int grid, int block, size_t smem, cudaStream_t s, const ConvTcPlan* pl) {
-    static const int pdl = env_int("YRE_TC_PDL", 1);
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3((unsigned)block); cfg.dynamicSmemBytes = smem; cfg.stream = s;
-    cudaLaunchAttribute at[2];
-    int n = 0;
-    if (pdl) {
-        at[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        at[n].val.programmaticStreamSerializationAllowed = 1;
-        ++n;
-    }
-    if (pl->p.cta2) {                     // CTA pairs: clusters of two (always on one TPC)
-        at[n].id = cudaLaunchAttributeClusterDimension;
-        at[n].val.clusterDim.x = 2; at[n].val.clusterDim.y = 1; at[n].val.clusterDim.z = 1;
-        ++n;
-    }
-    cfg.attrs = at; cfg.numAttrs = n;
-    return cudaLaunchKernelEx(&cfg, kernel, pl->tmA, pl->tmB, pl->tmY, pl->tmAu, pl->p);
-}
-
-int conv_tc_eligible(const yre_conv_desc& d, char* why, size_t n) {
+// ---- select ----
 #define NOPE(msg) do { if (why && n) snprintf(why, n, "%s", msg); return 0; } while (0)
+// what the kernels need of the dtypes, layouts, kernel size and channel windows -- all that conv_tc_select relies on
+int tc_shape_rules(const yre_conv_desc& d, char* why, size_t n) {
     if (d.x.dtype != YRE_BF16) NOPE("input must be bf16");
     if (d.y.layout != YRE_NHWC) NOPE("output must be NHWC");
     if (d.k != 1 && d.k != 3) NOPE("kernel must be 1x1 or 3x3");
@@ -1221,7 +1207,6 @@ int conv_tc_eligible(const yre_conv_desc& d, char* why, size_t n) {
         const int bk = ((d.x.C + d.xu.C) % 64 == 0) ? 64 : 32;
         if (d.xu.C % bk || d.x.C % bk) NOPE("upsampled source: both sources must be whole K chunks");
         if ((d.x.H & 1) || (d.x.W & 1)) NOPE("upsampled source: the map must have even extents");
-        if (reinterpret_cast<uintptr_t>(d.xu.ptr) & 127) NOPE("xu must be 128-byte aligned");
     }
     if (d.y.C % 16) NOPE("Cout must be a multiple of 16");
     const int yal = d.y.dtype == YRE_F32 ? 4 : 8;
@@ -1230,20 +1215,16 @@ int conv_tc_eligible(const yre_conv_desc& d, char* why, size_t n) {
         const int ral = d.res.dtype == YRE_F32 ? 4 : 8;
         if (d.res.layout != YRE_NHWC || d.res.c_off % ral || d.res.C_total % ral) NOPE("residual must be an aligned NHWC window");
     }
-    if ((reinterpret_cast<uintptr_t>(d.x.ptr) & 127) || (reinterpret_cast<uintptr_t>(d.w) & 127)) NOPE("x and w must be 128-byte aligned");
-    if (reinterpret_cast<uintptr_t>(d.y.ptr) & 127) NOPE("y must be 128-byte aligned");
-    if (d.bias && (reinterpret_cast<uintptr_t>(d.bias) & 15)) NOPE("bias must be 16-byte aligned");
-    if (!get_encode()) NOPE("cuTensorMapEncodeTiled unavailable");
     return 1;
-#undef NOPE
 }
 
-int conv_tc_prepare(const yre_conv_desc& d, ConvTcPlan** out) {
-    EncodeTiledFn enc = get_encode();
-    if (!enc) YRE_FAIL(YRE_EUNSUPPORTED, "conv_tc: cuTensorMapEncodeTiled unavailable");
-    ConvTcPlan* pl = new ConvTcPlan();
-    memset(pl, 0, sizeof(*pl));
-    TcParams& p = pl->p;
+// Kernel, tiling, pipeline depth, shared memory and grid of a conv that passes tc_shape_rules on a device with `sms` SMs.
+// A pure function: no CUDA call, no global state; pointers are copied into the parameters, never read.  The rules were
+// measured per layer (profiles/r02_notes.md).  Fails with YRE_EUNSUPPORTED when the tile does not fit shared memory.
+int conv_tc_select(const yre_conv_desc& d, int sms, const TcKnobs& kn, TcParams* out, int* grid, size_t* smem) {
+    if (kn.sms > 0) sms = kn.sms;              // tuning builds: persistent grids sized for a share of the machine
+    TcParams& p = *out;
+    p = TcParams{};
     const int Cu = d.xu.ptr ? d.xu.C : 0;
     const int Cin = d.x.C + Cu, Cout = d.y.C, Ho = d.y.H, Wo = d.y.W, B = d.y.B;
     p.Ho = Ho; p.Wo = Wo; p.B = B; p.Cin = Cin; p.Cout = Cout; p.x_coff = d.x.c_off;
@@ -1269,28 +1250,25 @@ int conv_tc_prepare(const yre_conv_desc& d, ConvTcPlan** out) {
     {
         const long long htiles = (long long)yre_cdiv(Wo, 8) * yre_cdiv(Ho, 16) * B;
         p.halo = d.k == 3 && d.stride == 1 && p.kchunks == 1 && (Cout == 64 || Cout == 32) &&
-                 htiles * 3 <= best * 4 && env_int("YRE_TC_HALO", 1) != 0;
+                 htiles * 3 <= best * 4 && kn.halo != 0;
         // larger layers: streamed weights; worth it while the 8x16 patches waste less than the halo saves.  Not for Cout that
         // tiles into 256-wide N: there the CTA-pair generic kernel (256 x 256 MMAs, half of the weight tile per SM) is
         // 11 % faster (3x3 256->256 @80x80 B64: 370 -> 327 us, 3x3 512->512 @80x80 B16: 332 -> 296 us)
         // (measured at batch 64: +5..8% on the 80x80 maps that tile exactly, a loss on 40x40 where a sixth of the
         //  patch rows is padding -- so by default only maps without patch waste take this path)
-        if (!p.halo && d.k == 3 && d.stride == 1 && p.block_k == 64 && htiles * 100 <= best * env_int("YRE_TC_HALO_SLACK", 100) &&
-            env_int("YRE_TC_HALO", 2) >= 2 && (Cout % 256 != 0 || env_int("YRE_TC_HALO_WIDE", 0))) p.halo = 2;
+        if (!p.halo && d.k == 3 && d.stride == 1 && p.block_k == 64 && htiles * 100 <= best * kn.halo_slack &&
+            kn.halo >= 2 && (Cout % 256 != 0 || kn.halo_wide)) p.halo = 2;
         if (p.halo) { btw = 8; bth = 16; btb = 1; best = htiles; }
         // maps that 8x16 patches do not tile but 8x8 ones do (40x40): the same kernel on 8 x 8 patches of TWO images (ybx)
         const long long htiles2 = (long long)yre_cdiv(Wo, 8) * yre_cdiv(Ho, 8) * yre_cdiv(B, 2);
         // (only where two patches can share every weight box -- the unpaired halo stream loses to the CTA-pair generic kernel)
-        int sms0 = 148, dev0 = 0;
-        cudaGetDevice(&dev0);
-        cudaDeviceGetAttribute(&sms0, cudaDevAttrMultiProcessorCount, dev0);
         // Measured at batch 64 on 40x40 maps: the single 64-wide N tile with a long K gains (3x3 512->64: 104 -> 81 us, the weight
         // matrix is re-streamed per patch PAIR instead of per tile), 128-wide tiles lose to the CTA-pair generic kernel
         // (3x3 128->128: 33.5 -> 40 us: 400 units are 2.7 rounds of long units) -- those need YRE_TC_HALO_YBX=2 (tuning builds)
-        const bool pairable = (Cout % 128 == 0 && ((htiles2 + 1) / 2) * (Cout / 128) >= sms0 && env_int("YRE_TC_HALO_YBX", 1) >= 2) ||
-                              (Cout == 64 && p.kchunks >= 2 && (htiles2 + 1) / 2 >= sms0);
+        const bool pairable = (Cout % 128 == 0 && ((htiles2 + 1) / 2) * (Cout / 128) >= sms && kn.halo_ybx >= 2) ||
+                              (Cout == 64 && p.kchunks >= 2 && (htiles2 + 1) / 2 >= sms);
         if (!p.halo && d.k == 3 && d.stride == 1 && p.block_k == 64 && B % 2 == 0 && htiles2 <= best && Cout % 256 != 0 && pairable &&
-            env_int("YRE_TC_HALO", 2) >= 2 && env_int("YRE_TC_HALO_YBX", 1)) {
+            kn.halo >= 2 && kn.halo_ybx) {
             p.halo = 2; p.ybx = 1; btw = 8; bth = 8; btb = 2; best = htiles2;
         }
     }
@@ -1299,28 +1277,22 @@ int conv_tc_prepare(const yre_conv_desc& d, ConvTcPlan** out) {
     const long long mtiles = best;
 
     // ---- N tiling ----
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    sms = env_int("YRE_TC_SMS", sms);          // tuning builds: persistent grids sized for a share of the machine
     int bn = 0;
     for (int c = 256; c >= 16; c -= 16) if (Cout % c == 0) { bn = c; break; }
     // 128-wide tiles beat the odd widths between 128 and 256 (3x3 512->640 @40x40: 5 x 128 runs in 118 us, 4 x 160 in 165 us:
     // four 128-column accumulators and CTA pairs against three unpaired 160-column ones)
-    if (bn > 128 && bn < 256 && Cout % 128 == 0 && env_int("YRE_TC_PREFER128", 1)) bn = 128;
+    if (bn > 128 && bn < 256 && Cout % 128 == 0 && kn.prefer128) bn = 128;
     // keep the machine busy: halve N tiles while there are fewer tiles than SMs
     while (bn >= 64 && bn % 32 == 0 && mtiles * (Cout / bn) < sms) bn /= 2;
-    const int force_bn = env_int("YRE_TC_BLOCK_N", 0);
-    if (force_bn >= 16 && force_bn <= 256 && force_bn % 16 == 0 && Cout % force_bn == 0) bn = force_bn;
+    if (kn.block_n >= 16 && kn.block_n <= 256 && kn.block_n % 16 == 0 && Cout % kn.block_n == 0) bn = kn.block_n;
     if (p.halo == 1) bn = Cout;
     p.npair = 1;
     if (p.halo == 2) {
         // two patches per weight box when a 128-wide N tile exists and there are enough pairs to fill the machine
-        const int want = env_int("YRE_TC_HALO_PAIR", 1);
-        if (want && Cout % 128 == 0 && ((mtiles + 1) / 2) * (Cout / 128) >= sms) { p.npair = 2; bn = 128; }
+        if (kn.halo_pair && Cout % 128 == 0 && ((mtiles + 1) / 2) * (Cout / 128) >= sms) { p.npair = 2; bn = 128; }
         // a single 64-wide N tile with a long K (head box tower, 3x3 256->64 @80x80): every patch re-streams the whole weight
         // matrix (295 KB against 92 KB of halo), so pairing halves what bounds it (L2 -> SM traffic)
-        else if (want >= 1 && env_int("YRE_TC_HALO_PAIR64", 1) && Cout == 64 && p.kchunks >= 2 && (mtiles + 1) / 2 >= sms) { p.npair = 2; bn = 64; }
+        else if (kn.halo_pair >= 1 && kn.halo_pair64 && Cout == 64 && p.kchunks >= 2 && (mtiles + 1) / 2 >= sms) { p.npair = 2; bn = 64; }
     }
     p.block_n = bn;
     p.tiles_n = Cout / bn;
@@ -1335,14 +1307,9 @@ int conv_tc_prepare(const yre_conv_desc& d, ConvTcPlan** out) {
     // also for launches of a single round of units, which an earlier rule excluded), and for K = 256 when the N tile is 256
     // wide (1x1 256->256 @160x160: 308 -> 286 us); K = 128 tiles are epilogue-bound and lose 3-10 % to the cross-CTA
     // accumulator hand-off.
-    {
-        const long long K_total = (long long)p.taps * Cin;
-        int want = (!p.halo && bn >= 128 && mtiles >= 2 && (K_total >= 512 || (K_total >= 256 && bn >= 256))) ? 1 : 0;
-        const int f = env_int("YRE_TC_CTA2", -1);          // tuning builds: 0 = never, 1 = whenever legal
-        if (f == 0) want = 0;
-        if (f == 1) want = (!p.halo && bn >= 128 && mtiles >= 2) ? 1 : 0;
-        p.cta2 = want;
-    }
+    const long long K_total = (long long)p.taps * Cin;
+    const bool cta2_legal = !p.halo && bn >= 128 && mtiles >= 2;
+    p.cta2 = kn.cta2 == 0 ? 0 : kn.cta2 == 1 ? cta2_legal : cta2_legal && (K_total >= 512 || (K_total >= 256 && bn >= 256));
     if (p.cta2) p.num_units = (int)((mtiles + 1) / 2) * p.tiles_n;
     p.a_bytes = (uint32_t)(BLOCK_M * p.block_k * 2);
     if (p.halo) {
@@ -1352,11 +1319,11 @@ int conv_tc_prepare(const yre_conv_desc& d, ConvTcPlan** out) {
     p.b_bytes = (uint32_t)((p.cta2 ? bn / 2 : bn) * p.block_k * 2);       // a pair's CTA stages half of the weight tile
     const uint32_t stage_bytes = p.a_bytes + p.b_bytes;
     // bf16 outputs leave through a swizzled staging tile + TMA store; fp32 outputs (raw head logits) store directly
-    p.tma_store = (d.y.dtype == YRE_BF16 && bn % 32 == 0 && env_int("YRE_TC_DIRECT_STORE", 0) == 0) ? 1 : 0;
+    p.tma_store = (d.y.dtype == YRE_BF16 && bn % 32 == 0 && kn.direct_store == 0) ? 1 : 0;
     // fp32 outputs (raw head logits): the full 32-column chunks of a tile go through a fp32 staging tile + TMA store on the
     // generic one-CTA kernel (a 16-column tail, Cout = 80, still stores directly): one 4 KB bulk store instead of eight
     // 16-byte stores per lane at a 576-byte pitch
-    const bool f32_tma = d.y.dtype == YRE_F32 && bn >= 32 && !p.halo && !p.cta2 && env_int("YRE_TC_F32_TMA", 1) != 0;
+    const bool f32_tma = d.y.dtype == YRE_F32 && bn >= 32 && !p.halo && !p.cta2 && kn.f32_tma != 0;
     if (f32_tma) p.tma_store = 1;
     p.stw = p.tw < 32 ? p.tw : 32;
     p.sth = (32 / p.stw) < p.th ? (32 / p.stw) : p.th;
@@ -1370,15 +1337,15 @@ int conv_tc_prepare(const yre_conv_desc& d, ConvTcPlan** out) {
     // With one buffer per tile-group the group idles while its buffer is refilled, so keep nacc >= 2 * tgroups;
     // where TMEM only holds 2-3 buffers, split the chunks of each tile over the warpgroups instead.
     p.nthreads = bn <= 64 ? NT_3WG : NT_2WG;
-    { const int f = env_int("YRE_TC_THREADS", 0); if ((f == NT_2WG || f == NT_3WG) && p.halo != 1) p.nthreads = f; }
+    if ((kn.threads == NT_2WG || kn.threads == NT_3WG) && p.halo != 1) p.nthreads = kn.threads;
     if (p.cta2) p.nthreads = NT_2WG;
     const int maxg = (p.nthreads / 32 - 4) / 4;
     if (bn <= 64)       { p.acc_stride = 64;  p.nacc = 6; p.tgroups = maxg; p.csplit = 1; }
     else if (bn <= 128) { p.acc_stride = 128; p.nacc = 4; p.tgroups = 2; p.csplit = 1; }
     else if (bn <= 160) { p.acc_stride = 160; p.nacc = 3; p.tgroups = 1; p.csplit = maxg; }
     else                { p.acc_stride = 256; p.nacc = 2; p.tgroups = 1; p.csplit = maxg; }
-    { const int f = env_int("YRE_TC_TGROUPS", 0); if (f >= 1 && f <= maxg && p.nacc % f == 0) { p.tgroups = f; if (p.tgroups * p.csplit > maxg) p.csplit = 1; } }
-    { const int f = env_int("YRE_TC_SPLIT", 0); if (f >= 1 && f * p.tgroups <= maxg) p.csplit = f; }
+    if (kn.tgroups >= 1 && kn.tgroups <= maxg && p.nacc % kn.tgroups == 0) { p.tgroups = kn.tgroups; if (p.tgroups * p.csplit > maxg) p.csplit = 1; }
+    if (kn.split >= 1 && kn.split * p.tgroups <= maxg) p.csplit = kn.split;
     if (p.npair == 2) { p.nthreads = NT_2WG; p.acc_stride = 128; p.nacc = 4; p.tgroups = 2; p.csplit = 1; }   // group h <-> patch h
     while (p.csplit > 1 && p.csplit > (bn + 31) / 32) --p.csplit;   // every warpgroup owns at least one chunk
     p.ngroups = p.tgroups * p.csplit;
@@ -1386,8 +1353,7 @@ int conv_tc_prepare(const yre_conv_desc& d, ConvTcPlan** out) {
     // 1x1 convs only: they are store/epilogue-bound and gain 25-35 % from the halved store count (1x1 128->128 @160x160:
     // 208 -> 135 us), while every 3x3 kernel (generic, CTA pair, halo stream) is main-loop bound and LOSES 8-25 % to the
     // 32 KB of operand ring the larger staging tiles take (3x3 256->256 @80x80: 366 -> 467 us) -- per-layer sweep, r02_notes.md
-    { const int f = env_int("YRE_TC_STAGE64", -1);
-      p.stage64 = (p.tma_store && p.nthreads == NT_2WG && bn % 64 == 0 && (f < 0 ? p.taps == 1 : f != 0)) ? 1 : 0; }
+    p.stage64 = (p.tma_store && p.nthreads == NT_2WG && bn % 64 == 0 && (kn.stage64 < 0 ? p.taps == 1 : kn.stage64 != 0)) ? 1 : 0;
     if (f32_tma) p.stage64 = 0;
     p.stage_out_bytes = p.tma_store ? ((p.stage64 || f32_tma) ? 4096u : 2048u) : 0u;      // 32 rows x 32 (or 64) bf16 / 32 fp32 channels per buffer
     const uint32_t n_stage_bufs = 8u * (uint32_t)p.ngroups;         // 4 warps x 2 buffers per group
@@ -1403,48 +1369,167 @@ int conv_tc_prepare(const yre_conv_desc& d, ConvTcPlan** out) {
         const uint32_t a_slot = (uint32_t)p.npair * p.a_bytes;
         int sa = 2;
         p.tps = ((room - 2u * a_slot) / (3u * p.b_bytes) >= (p.npair == 2 ? 2u : 3u)) ? 3 : 1;
-        { const int f = env_int("YRE_TC_HALO_TPS", 0); if (f == 1 || f == 3) p.tps = f; }
+        if (kn.halo_tps == 1 || kn.halo_tps == 3) p.tps = kn.halo_tps;
         int sb = (int)((room - 2u * a_slot) / ((uint32_t)p.tps * p.b_bytes));
         if (sb > (p.tps == 3 ? 4 : 8)) {           // room to spare: a third halo slot
             const int sb3 = (int)((room - 3u * a_slot) / ((uint32_t)p.tps * p.b_bytes));
             if (sb3 >= (p.tps == 3 ? 3 : 5)) { sa = 3; sb = sb3; }
         }
         if (sb > 8) sb = 8;
-        if (sb < 2) { delete pl; YRE_FAIL(YRE_EUNSUPPORTED, "conv_tc: halo tile does not fit shared memory"); }
+        if (sb < 2) YRE_FAIL(YRE_EUNSUPPORTED, "conv_tc: halo tile does not fit shared memory");
         stages = sa; p.stages_b = sb;
     }
-    const int force_st = env_int("YRE_TC_STAGES", 0);
-    if (force_st >= 2 && force_st <= stages) stages = force_st;
-    if (stages < 2) { delete pl; YRE_FAIL(YRE_EUNSUPPORTED, "conv_tc: tile does not fit shared memory"); }
+    if (kn.stages >= 2 && kn.stages <= stages) stages = kn.stages;
+    if (stages < 2) YRE_FAIL(YRE_EUNSUPPORTED, "conv_tc: tile does not fit shared memory");
     // two (producer, MMA) pairs when the ring gives each at least 3 stages
     p.npipes = (stages >= 6 && p.nacc % 2 == 0 && !p.halo) ? 2 : 1;
-    { const int f = env_int("YRE_TC_PIPES", 0); if (f >= 1 && f <= 2 && p.nacc % f == 0 && stages >= 2 * f) p.npipes = f; }
+    if (kn.pipes >= 1 && kn.pipes <= 2 && p.nacc % kn.pipes == 0 && stages >= 2 * kn.pipes) p.npipes = kn.pipes;
     if (p.npipes == 2 || p.halo == 1) stages &= ~1;
     p.stages = stages;
-    pl->smem = (size_t)stages * stage_bytes + n_stage_bufs * p.stage_out_bytes + 8 * (2 * stages + 16) + 32 + (size_t)Cout * 4 + align_slack;
-    if (p.halo == 2) pl->smem = (size_t)stages * p.npair * p.a_bytes + (size_t)p.stages_b * p.tps * p.b_bytes + n_stage_bufs * p.stage_out_bytes + 8 * (2 * stages + 2 * p.stages_b + 16) + 32 + (size_t)Cout * 4 + 1024;
-    else if (p.halo) pl->smem = 9 * (size_t)p.b_bytes + (size_t)stages * p.a_bytes + n_stage_bufs * p.stage_out_bytes + 8 * (2 * stages + 18) + 32 + (size_t)Cout * 4 + 1024;
+    // operand rings (the weight-stationary halo kernel keeps all nine weight taps resident), 8-byte mbarriers, 32 bytes of
+    // TMEM slot and flags, the epilogue's staging buffers, the bias copy and the alignment slack
+    const size_t rings = p.halo == 2 ? (size_t)stages * p.npair * p.a_bytes + (size_t)p.stages_b * p.tps * p.b_bytes
+                       : p.halo      ? (size_t)stages * p.a_bytes + 9 * (size_t)p.b_bytes
+                       :               (size_t)stages * stage_bytes;
+    *smem = rings + 8 * (2 * stages + 16 + (p.halo == 2 ? 2 * p.stages_b : p.halo ? 2 : 0)) + 32 + n_stage_bufs * p.stage_out_bytes +
+            (size_t)Cout * 4 + align_slack;
+    // persistent grids: one CTA (pair) per work unit, at most one per SM
+    *grid = p.cta2 ? 2 * std::min(p.num_units, sms / 2) : std::min(p.halo == 2 ? p.num_units : p.num_tiles, sms);
     p.idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(bn >> 3) << 17) | ((uint32_t)((p.cta2 ? 2 * BLOCK_M : BLOCK_M) >> 4) << 24);
     p.bias = d.bias; p.act = d.act;
     p.y = d.y.ptr; p.y_f32 = d.y.dtype == YRE_F32; p.y_ctot = d.y.C_total; p.y_coff = d.y.c_off;
     p.res = d.res.ptr; p.res_f32 = d.res.ptr ? d.res.dtype == YRE_F32 : 0;
     p.res_ctot = d.res.ptr ? d.res.C_total : 0; p.res_coff = d.res.ptr ? d.res.c_off : 0;
-    p.rev = 0;
-    p.dbg = nullptr;
-    if (env_int("YRE_TC_TRACE", 0)) {
-        static int* g_dbg = nullptr;
-        if (!g_dbg) { cudaMalloc(&g_dbg, 8192 * sizeof(int)); }
-        cudaMemset(g_dbg, 0, 8192 * sizeof(int));
-        p.dbg = g_dbg;
-        g_trace_buf = g_dbg;
+    return YRE_OK;
+}
+
+// ---- kernel table ----
+typedef void (*TcKernelFn)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, TcParams);
+
+// Every kernel instantiation with the TcParams values that select it.  The keys are exact (cout: Cout of the
+// weight-stationary halo kernel, 0 elsewhere; f32_tma: fp32 output through the staged TMA store), so no two entries match
+// the same parameters and the order of the rows does not matter.
+struct TcKernel {
+    TcKernelFn fn;
+    const char* name;                                    // for launch errors
+    int halo, block_k, cout, cta2, f32_tma, nthreads, stage64;
+};
+
+const TcKernel TC_KERNELS[] = {
+    //                                                                        halo  bk cout cta2 f32 nthreads s64
+    {conv_tc_kernel<4, NT_2WG, false, false>,       "conv_tc",                 0, 64,  0,  0,  0, NT_2WG, 0},
+    {conv_tc_kernel<2, NT_2WG, false, false>,       "conv_tc",                 0, 32,  0,  0,  0, NT_2WG, 0},
+    {conv_tc_kernel<4, NT_2WG, false, true>,        "conv_tc",                 0, 64,  0,  0,  0, NT_2WG, 1},
+    {conv_tc_kernel<2, NT_2WG, false, true>,        "conv_tc",                 0, 32,  0,  0,  0, NT_2WG, 1},
+    {conv_tc_kernel<4, NT_3WG, false, false>,       "conv_tc",                 0, 64,  0,  0,  0, NT_3WG, 0},
+    {conv_tc_kernel<2, NT_3WG, false, false>,       "conv_tc",                 0, 32,  0,  0,  0, NT_3WG, 0},
+    {conv_tc_kernel<4, NT_2WG, true, false>,        "conv_tc (CTA pair)",      0, 64,  0,  1,  0, NT_2WG, 0},
+    {conv_tc_kernel<2, NT_2WG, true, false>,        "conv_tc (CTA pair)",      0, 32,  0,  1,  0, NT_2WG, 0},
+    {conv_tc_kernel<4, NT_2WG, true, true>,         "conv_tc (CTA pair)",      0, 64,  0,  1,  0, NT_2WG, 1},
+    {conv_tc_kernel<2, NT_2WG, true, true>,         "conv_tc (CTA pair)",      0, 32,  0,  1,  0, NT_2WG, 1},
+    {conv_tc_kernel<4, NT_2WG, false, false, true>, "conv_tc (fp32 out)",      0, 64,  0,  0,  1, NT_2WG, 0},
+    {conv_tc_kernel<2, NT_2WG, false, false, true>, "conv_tc (fp32 out)",      0, 32,  0,  0,  1, NT_2WG, 0},
+    {conv_tc_kernel<4, NT_3WG, false, false, true>, "conv_tc (fp32 out)",      0, 64,  0,  0,  1, NT_3WG, 0},
+    {conv_tc_kernel<2, NT_3WG, false, false, true>, "conv_tc (fp32 out)",      0, 32,  0,  0,  1, NT_3WG, 0},
+    {conv3_halo_stream_kernel<NT_2WG, false>,       "conv3_halo_stream",       2, 64,  0,  0,  0, NT_2WG, 0},
+    {conv3_halo_stream_kernel<NT_2WG, true>,        "conv3_halo_stream",       2, 64,  0,  0,  0, NT_2WG, 1},
+    {conv3_halo_stream_kernel<NT_3WG, false>,       "conv3_halo_stream",       2, 64,  0,  0,  0, NT_3WG, 0},
+    {conv3_halo_kernel<4, 64>,                      "conv3_halo",              1, 64, 64,  0,  0, NT_3WG, 0},
+    {conv3_halo_kernel<4, 32>,                      "conv3_halo",              1, 64, 32,  0,  0, NT_3WG, 0},
+    {conv3_halo_kernel<2, 64>,                      "conv3_halo",              1, 32, 64,  0,  0, NT_3WG, 0},
+    {conv3_halo_kernel<2, 32>,                      "conv3_halo",              1, 32, 32,  0,  0, NT_3WG, 0},
+};
+
+}  // namespace
+
+struct ConvTcPlan {
+    CUtensorMap tmA, tmB, tmY, tmAu;
+    TcParams p;
+    int grid;
+    size_t smem;
+    const TcKernel* kernel;
+};
+
+// ---- describe ----
+// Human-readable kernel variant and tile shape of a conv: which of the tcgen05 kernels runs the layer and with which tiling,
+// so that the selection rules above are visible per layer (plan.op_table(), bench --per-op).
+static void tc_format(const TcParams& p, int grid, char* out, size_t n) {
+    const char* k = p.halo == 1 ? "halo-ws" : p.halo == 2 ? (p.ybx ? "halo-stream-ybx" : "halo-stream") : (p.cta2 ? "generic-cta2" : "generic");
+    snprintf(out, n, "%s M=%dx%dx%d N=%d K=%dx%d stages=%d%s%s%s thr=%d grid=%d", k, p.tb, p.th, p.tw, p.block_n, p.taps * p.kchunks, p.block_k,
+             p.stages, p.npair == 2 ? " pair" : "", p.stage64 ? " s64" : "", p.tma_store ? (p.y_f32 ? " tma-f32" : " tma") : " direct", p.nthreads, grid);
+}
+
+void conv_tc_describe(const ConvTcPlan* pl, char* out, size_t n) { tc_format(pl->p, pl->grid, out, n); }
+
+extern "C" int yre_conv_tc_describe(const yre_conv_desc* d, int32_t num_sms, char* out, int32_t cap) {
+    if (!out || cap <= 0 || num_sms <= 0) YRE_FAIL(YRE_EINVAL, "conv_tc_describe: null output or non-positive size / SM count");
+    if (int e = check_conv(d)) return e;
+    char why[256] = "";
+    if (!tc_shape_rules(*d, why, sizeof(why))) YRE_FAIL(YRE_EUNSUPPORTED, "conv_tc: %s", why);
+    TcParams p; int grid; size_t smem;
+    if (int e = conv_tc_select(*d, num_sms, tc_knobs(), &p, &grid, &smem)) return e;
+    tc_format(p, grid, out, (size_t)cap);
+    return YRE_OK;
+}
+
+// ---- prepare ----
+int conv_tc_eligible(const yre_conv_desc& d, char* why, size_t n) {
+    if (!tc_shape_rules(d, why, n)) return 0;
+    // address rules: what the tensor maps need
+    if (d.xu.ptr && (reinterpret_cast<uintptr_t>(d.xu.ptr) & 127)) NOPE("xu must be 128-byte aligned");
+    if ((reinterpret_cast<uintptr_t>(d.x.ptr) & 127) || (reinterpret_cast<uintptr_t>(d.w) & 127)) NOPE("x and w must be 128-byte aligned");
+    if (reinterpret_cast<uintptr_t>(d.y.ptr) & 127) NOPE("y must be 128-byte aligned");
+    if (d.bias && (reinterpret_cast<uintptr_t>(d.bias) & 15)) NOPE("bias must be 16-byte aligned");
+    if (!get_encode()) NOPE("cuTensorMapEncodeTiled unavailable");
+    return 1;
+}
+#undef NOPE
+
+// output tensor map of the staged TMA store: one box = the 32 pixels of a TMEM lane quarter x 32 (64 with stage64) channels;
+// fp32 outputs use 128-byte rows (32 channels) in a 128B-swizzled tile.  Also used when an output buffer is re-bound.
+static CUresult encode_y(ConvTcPlan* pl, void* ptr) {
+    const auto& p = pl->p;
+    const cuuint64_t es = p.y_f32 ? 4 : 2, ct = (cuuint64_t)p.y_ctot;
+    cuuint64_t gdim[4] = {ct, (cuuint64_t)p.Wo, (cuuint64_t)p.Ho, (cuuint64_t)p.B};
+    cuuint64_t gstr[3] = {ct * es, (cuuint64_t)p.Wo * ct * es, (cuuint64_t)p.Ho * p.Wo * ct * es};
+    cuuint32_t box[4] = {p.stage64 ? 64u : 32u, (cuuint32_t)p.stw, (cuuint32_t)p.sth, (cuuint32_t)p.stb};
+    if (p.ybx) {                                                   // {C, W, B, H}, like the input map
+        gdim[2] = (cuuint64_t)p.B; gdim[3] = (cuuint64_t)p.Ho;
+        const cuuint64_t sh = gstr[1], sb = gstr[2];
+        gstr[1] = sb; gstr[2] = sh;
+        box[2] = (cuuint32_t)p.stb; box[3] = (cuuint32_t)p.sth;
     }
-    pl->grid = p.num_tiles < sms ? p.num_tiles : sms;
-    if (p.halo == 2) pl->grid = p.num_units < sms ? p.num_units : sms;
-    if (p.cta2) pl->grid = 2 * (p.num_units < sms / 2 ? p.num_units : sms / 2);
+    cuuint32_t est[4] = {1, 1, 1, 1};
+    return get_encode()(&pl->tmY, p.y_f32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, ptr, gdim, gstr, box, est,
+                        CU_TENSOR_MAP_INTERLEAVE_NONE, (p.stage64 || p.y_f32) ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
+                        CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+}
+
+int conv_tc_prepare(const yre_conv_desc& d, ConvTcPlan** out) {
+    const EncodeTiledFn enc = get_encode();       // the address rules were checked by conv_tc_eligible
+    if (!enc) YRE_FAIL(YRE_EUNSUPPORTED, "conv_tc: cuTensorMapEncodeTiled unavailable");
+    int dev = 0, sms = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+    const TcKnobs kn = tc_knobs();
+    std::unique_ptr<ConvTcPlan> pl(new ConvTcPlan());
+    TcParams& p = pl->p;
+    if (int e = conv_tc_select(d, sms, kn, &p, &pl->grid, &pl->smem)) return e;
+    const int cout = p.halo == 1 ? p.Cout : 0, f32_tma = p.y_f32 && p.tma_store;
+    for (const TcKernel& k : TC_KERNELS)
+        if (k.halo == p.halo && k.block_k == p.block_k && k.cout == cout && k.cta2 == p.cta2 && k.f32_tma == f32_tma &&
+            k.nthreads == p.nthreads && k.stage64 == p.stage64) pl->kernel = &k;
+    if (!pl->kernel) YRE_FAIL(YRE_EUNSUPPORTED, "conv_tc: no kernel for halo %d, block_k %d, cta2 %d, %d threads, stage64 %d, "
+                              "fp32 TMA store %d", p.halo, p.block_k, p.cta2, p.nthreads, p.stage64, f32_tma);
+    if (kn.trace) {
+        if (!g_trace_buf) cudaMalloc(&g_trace_buf, 8192 * sizeof(int));
+        cudaMemset(g_trace_buf, 0, 8192 * sizeof(int));
+        p.dbg = g_trace_buf;
+    }
 
     // ---- tensor maps ----
     const CUtensorMapSwizzle swz = p.block_k == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B;
-    const CUtensorMapL2promotion promoA = (CUtensorMapL2promotion)env_int("YRE_TC_L2PROMO_A", (int)CU_TENSOR_MAP_L2_PROMOTION_L2_128B);
+    const CUtensorMapL2promotion promoA = (CUtensorMapL2promotion)kn.l2promo_a;
     CUresult r;
     if (!p.phase4) {
         cuuint64_t gdim[4] = {(cuuint64_t)d.x.C_total, (cuuint64_t)d.x.W, (cuuint64_t)d.x.H, (cuuint64_t)d.x.B};
@@ -1469,9 +1554,9 @@ int conv_tc_prepare(const yre_conv_desc& d, ConvTcPlan** out) {
         r = enc(&pl->tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, d.x.ptr, gdim, gstr, box, est, CU_TENSOR_MAP_INTERLEAVE_NONE, swz,
                 promoA, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     }
-    if (r != CUDA_SUCCESS) { delete pl; YRE_FAIL(YRE_ECUDA, "conv_tc: cuTensorMapEncodeTiled(A) failed with %d", (int)r); }
+    if (r != CUDA_SUCCESS) YRE_FAIL(YRE_ECUDA, "conv_tc: cuTensorMapEncodeTiled(A) failed with %d", (int)r);
     pl->tmAu = pl->tmA;   // unused unless an upsampled source is given
-    if (Cu) {
+    if (d.xu.ptr) {
         // {C, dup x, W/2, dup y, (H/2) * B}: the duplicated dimensions have stride 0 (accepted by the driver and the TMA
         // unit, scripts/ubench/tma_dup.cu), the images stack along the row dimension
         const cuuint64_t Ct = (cuuint64_t)d.xu.C_total, Wu = (cuuint64_t)d.xu.W, Hu = (cuuint64_t)d.xu.H;
@@ -1481,120 +1566,60 @@ int conv_tc_prepare(const yre_conv_desc& d, ConvTcPlan** out) {
         cuuint32_t est[5] = {1, 1, 1, 1, 1};
         r = enc(&pl->tmAu, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, d.xu.ptr, gdim, gstr, box, est, CU_TENSOR_MAP_INTERLEAVE_NONE, swz,
                 promoA, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (r != CUDA_SUCCESS) { delete pl; YRE_FAIL(YRE_ECUDA, "conv_tc: cuTensorMapEncodeTiled(upsampled A) failed with %d", (int)r); }
+        if (r != CUDA_SUCCESS) YRE_FAIL(YRE_ECUDA, "conv_tc: cuTensorMapEncodeTiled(upsampled A) failed with %d", (int)r);
     }
     {
-        const cuuint64_t K = (cuuint64_t)p.taps * Cin;
-        cuuint64_t gdim[2] = {K, (cuuint64_t)Cout};
+        const cuuint64_t K = (cuuint64_t)p.taps * p.Cin;
+        cuuint64_t gdim[2] = {K, (cuuint64_t)p.Cout};
         cuuint64_t gstr[1] = {K * 2};
-        cuuint32_t box[2] = {(cuuint32_t)p.block_k, (cuuint32_t)(p.cta2 ? bn / 2 : bn)};
+        cuuint32_t box[2] = {(cuuint32_t)p.block_k, (cuuint32_t)(p.cta2 ? p.block_n / 2 : p.block_n)};
         cuuint32_t est[2] = {1, 1};
         r = enc(&pl->tmB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(d.w), gdim, gstr, box, est, CU_TENSOR_MAP_INTERLEAVE_NONE, swz,
                 CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     }
-    if (r != CUDA_SUCCESS) { delete pl; YRE_FAIL(YRE_ECUDA, "conv_tc: cuTensorMapEncodeTiled(W) failed with %d", (int)r); }
+    if (r != CUDA_SUCCESS) YRE_FAIL(YRE_ECUDA, "conv_tc: cuTensorMapEncodeTiled(W) failed with %d", (int)r);
     if (p.tma_store) {
-        r = encode_y(pl, d.y.ptr);
-        if (r != CUDA_SUCCESS) { delete pl; YRE_FAIL(YRE_ECUDA, "conv_tc: cuTensorMapEncodeTiled(Y) failed with %d", (int)r); }
+        r = encode_y(pl.get(), d.y.ptr);
+        if (r != CUDA_SUCCESS) YRE_FAIL(YRE_ECUDA, "conv_tc: cuTensorMapEncodeTiled(Y) failed with %d", (int)r);
     } else {
         pl->tmY = pl->tmB;   // unused
     }
-    *out = pl;
+    *out = pl.release();
     return YRE_OK;
 }
 
-template <typename K> static int opt_in_smem(K kernel) {
-    YRE_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
-    return YRE_OK;
-}
-
+// ---- launch ----
 int conv_tc_launch(const ConvTcPlan* pl, cudaStream_t s) {
     static YrePerDeviceOnce once;
     if (int e = once.run([]() -> int {
-            if (int r = opt_in_smem(conv_tc_kernel<4, NT_2WG, false, false>)) return r;
-            if (int r = opt_in_smem(conv_tc_kernel<2, NT_2WG, false, false>)) return r;
-            if (int r = opt_in_smem(conv_tc_kernel<4, NT_2WG, false, true>)) return r;
-            if (int r = opt_in_smem(conv_tc_kernel<2, NT_2WG, false, true>)) return r;
-            if (int r = opt_in_smem(conv_tc_kernel<4, NT_3WG, false, false>)) return r;
-            if (int r = opt_in_smem(conv_tc_kernel<2, NT_3WG, false, false>)) return r;
-            if (int r = opt_in_smem(conv_tc_kernel<4, NT_2WG, true, false>)) return r;
-            if (int r = opt_in_smem(conv_tc_kernel<2, NT_2WG, true, false>)) return r;
-            if (int r = opt_in_smem(conv_tc_kernel<4, NT_2WG, true, true>)) return r;
-            if (int r = opt_in_smem(conv_tc_kernel<2, NT_2WG, true, true>)) return r;
-            if (int r = opt_in_smem(conv_tc_kernel<4, NT_2WG, false, false, true>)) return r;
-            if (int r = opt_in_smem(conv_tc_kernel<2, NT_2WG, false, false, true>)) return r;
-            if (int r = opt_in_smem(conv_tc_kernel<4, NT_3WG, false, false, true>)) return r;
-            if (int r = opt_in_smem(conv_tc_kernel<2, NT_3WG, false, false, true>)) return r;
-            if (int r = opt_in_smem(conv3_halo_stream_kernel<NT_2WG, false>)) return r;
-            if (int r = opt_in_smem(conv3_halo_stream_kernel<NT_2WG, true>)) return r;
-            if (int r = opt_in_smem(conv3_halo_stream_kernel<NT_3WG, false>)) return r;
-            if (int r = opt_in_smem(conv3_halo_kernel<4, 64>)) return r;
-            if (int r = opt_in_smem(conv3_halo_kernel<4, 32>)) return r;
-            if (int r = opt_in_smem(conv3_halo_kernel<2, 64>)) return r;
-            if (int r = opt_in_smem(conv3_halo_kernel<2, 32>)) return r;
+            for (const TcKernel& k : TC_KERNELS)
+                YRE_CUDA(cudaFuncSetAttribute(k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
             return YRE_OK;
         })) return e;
-    const bool k64 = pl->p.block_k == 64, s64 = pl->p.stage64 != 0;
-    if (pl->p.halo == 2) {
-        if (pl->p.nthreads == NT_3WG) YRE_CUDA(launch_tc(conv3_halo_stream_kernel<NT_3WG, false>, pl->grid, NT_3WG, pl->smem, s, pl));
-        else if (s64)                 YRE_CUDA(launch_tc(conv3_halo_stream_kernel<NT_2WG, true>, pl->grid, NT_2WG, pl->smem, s, pl));
-        else                          YRE_CUDA(launch_tc(conv3_halo_stream_kernel<NT_2WG, false>, pl->grid, NT_2WG, pl->smem, s, pl));
-        YRE_LAUNCH_CHECK("conv3_halo_stream");
-        return YRE_OK;
+    static const int pdl = tc_knobs().pdl;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)pl->grid); cfg.blockDim = dim3((unsigned)pl->p.nthreads); cfg.dynamicSmemBytes = pl->smem; cfg.stream = s;
+    cudaLaunchAttribute at[2];
+    int n = 0;
+    if (pdl) {
+        at[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+        at[n].val.programmaticStreamSerializationAllowed = 1;
+        ++n;
     }
-    if (pl->p.halo) {
-        const bool c64 = pl->p.Cout == 64;
-        if (k64) { if (c64) YRE_CUDA(launch_tc(conv3_halo_kernel<4, 64>, pl->grid, NT_3WG, pl->smem, s, pl));
-                   else     YRE_CUDA(launch_tc(conv3_halo_kernel<4, 32>, pl->grid, NT_3WG, pl->smem, s, pl)); }
-        else     { if (c64) YRE_CUDA(launch_tc(conv3_halo_kernel<2, 64>, pl->grid, NT_3WG, pl->smem, s, pl));
-                   else     YRE_CUDA(launch_tc(conv3_halo_kernel<2, 32>, pl->grid, NT_3WG, pl->smem, s, pl)); }
-        YRE_LAUNCH_CHECK("conv3_halo");
-        return YRE_OK;
+    if (pl->p.cta2) {                     // CTA pairs: clusters of two (always on one TPC)
+        at[n].id = cudaLaunchAttributeClusterDimension;
+        at[n].val.clusterDim.x = 2; at[n].val.clusterDim.y = 1; at[n].val.clusterDim.z = 1;
+        ++n;
     }
-    if (pl->p.cta2) {                     // N tiles >= 128 only, which always run the two-warpgroup epilogue
-        if (k64) { if (s64) YRE_CUDA(launch_tc(conv_tc_kernel<4, NT_2WG, true, true>, pl->grid, NT_2WG, pl->smem, s, pl));
-                   else     YRE_CUDA(launch_tc(conv_tc_kernel<4, NT_2WG, true, false>, pl->grid, NT_2WG, pl->smem, s, pl)); }
-        else     { if (s64) YRE_CUDA(launch_tc(conv_tc_kernel<2, NT_2WG, true, true>, pl->grid, NT_2WG, pl->smem, s, pl));
-                   else     YRE_CUDA(launch_tc(conv_tc_kernel<2, NT_2WG, true, false>, pl->grid, NT_2WG, pl->smem, s, pl)); }
-        YRE_LAUNCH_CHECK("conv_tc (CTA pair)");
-        return YRE_OK;
-    }
-    if (pl->p.y_f32 && pl->p.tma_store) {      // fp32 output through the staged TMA store
-        if (pl->p.nthreads == NT_3WG) {
-            if (k64) YRE_CUDA(launch_tc(conv_tc_kernel<4, NT_3WG, false, false, true>, pl->grid, NT_3WG, pl->smem, s, pl));
-            else     YRE_CUDA(launch_tc(conv_tc_kernel<2, NT_3WG, false, false, true>, pl->grid, NT_3WG, pl->smem, s, pl));
-        } else {
-            if (k64) YRE_CUDA(launch_tc(conv_tc_kernel<4, NT_2WG, false, false, true>, pl->grid, NT_2WG, pl->smem, s, pl));
-            else     YRE_CUDA(launch_tc(conv_tc_kernel<2, NT_2WG, false, false, true>, pl->grid, NT_2WG, pl->smem, s, pl));
-        }
-        YRE_LAUNCH_CHECK("conv_tc (fp32 out)");
-        return YRE_OK;
-    }
-    if (pl->p.nthreads == NT_3WG) {
-        if (k64) YRE_CUDA(launch_tc(conv_tc_kernel<4, NT_3WG, false, false>, pl->grid, NT_3WG, pl->smem, s, pl));
-        else     YRE_CUDA(launch_tc(conv_tc_kernel<2, NT_3WG, false, false>, pl->grid, NT_3WG, pl->smem, s, pl));
-    } else {
-        if (k64) { if (s64) YRE_CUDA(launch_tc(conv_tc_kernel<4, NT_2WG, false, true>, pl->grid, NT_2WG, pl->smem, s, pl));
-                   else     YRE_CUDA(launch_tc(conv_tc_kernel<4, NT_2WG, false, false>, pl->grid, NT_2WG, pl->smem, s, pl)); }
-        else     { if (s64) YRE_CUDA(launch_tc(conv_tc_kernel<2, NT_2WG, false, true>, pl->grid, NT_2WG, pl->smem, s, pl));
-                   else     YRE_CUDA(launch_tc(conv_tc_kernel<2, NT_2WG, false, false>, pl->grid, NT_2WG, pl->smem, s, pl)); }
-    }
-    YRE_LAUNCH_CHECK("conv_tc");
+    cfg.attrs = at; cfg.numAttrs = n;
+    YRE_CUDA(cudaLaunchKernelEx(&cfg, pl->kernel->fn, pl->tmA, pl->tmB, pl->tmY, pl->tmAu, pl->p));
+    YRE_LAUNCH_CHECK(pl->kernel->name);
     return YRE_OK;
 }
 
 void conv_tc_free(ConvTcPlan* p) { delete p; }
 
 void conv_tc_set_reverse(ConvTcPlan* pl, int rev) { pl->p.rev = rev ? 1 : 0; }
-
-// Human-readable kernel variant and tile shape of a prepared conv (yre_plan_op_variant): which of the tcgen05 kernels runs
-// the layer and with which tiling, so that the selection rules above are visible per layer (plan.op_table(), bench --per-op).
-void conv_tc_describe(const ConvTcPlan* pl, char* out, size_t n) {
-    const auto& p = pl->p;
-    const char* k = p.halo == 1 ? "halo-ws" : p.halo == 2 ? (p.ybx ? "halo-stream-ybx" : "halo-stream") : (p.cta2 ? "generic-cta2" : "generic");
-    snprintf(out, n, "%s M=%dx%dx%d N=%d K=%dx%d stages=%d%s%s%s thr=%d grid=%d", k, p.tb, p.th, p.tw, p.block_n, p.taps * p.kchunks, p.block_k,
-             p.stages, p.npair == 2 ? " pair" : "", p.stage64 ? " s64" : "", p.tma_store ? (p.y_f32 ? " tma-f32" : " tma") : " direct", p.nthreads, pl->grid);
-}
 
 int conv_tc_rebind(ConvTcPlan* pl, const void* old_ptr, void* new_ptr) {
     int n = 0;

@@ -66,6 +66,9 @@ const char* op_name(OpKind k) {
     return "?";
 }
 
+}  // namespace
+
+// validates a conv descriptor for the plan, yre_conv and yre_conv_tc_describe
 int check_conv(const yre_conv_desc* d) {
     if (!d || !d->w) YRE_FAIL(YRE_EINVAL, "conv: null descriptor/weights");
     if (yre_check_view(&d->x, "conv.x") || yre_check_view(&d->y, "conv.y")) return YRE_EINVAL;
@@ -90,6 +93,8 @@ int check_conv(const yre_conv_desc* d) {
     }
     return YRE_OK;
 }
+
+namespace {
 
 // decides the engine; fills op
 int make_conv_op(const yre_conv_desc* d, Op& o) {

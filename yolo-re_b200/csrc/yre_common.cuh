@@ -142,6 +142,7 @@ __device__ __forceinline__ float silu_tanh(float x) {
 // ---- op launchers implemented in the k_*.cu files (host side, used by the C API and the plan) -----
 struct ConvTcPlan;   // pre-encoded tensor maps + tile config of one tcgen05 conv (k_conv_tc.cu)
 
+int check_conv(const yre_conv_desc* d);                                     // descriptor validation shared by every conv entry point
 int launch_conv_ffma(const yre_conv_desc& d, cudaStream_t s);
 int conv_tc_eligible(const yre_conv_desc& d, char* why, size_t why_len);
 int conv_tc_prepare(const yre_conv_desc& d, ConvTcPlan** out);

@@ -66,6 +66,7 @@ SYMBOLS = {
     "yre_last_error": (C.c_char_p, []),
     "yre_device_check": (C.c_int, []),
     "yre_conv": (C.c_int, [C.POINTER(ConvDesc), C.c_void_p]),
+    "yre_conv_tc_describe": (C.c_int, [C.POINTER(ConvDesc), C.c_int32, C.c_char_p, C.c_int32]),
     "yre_stem_conv": (C.c_int, [C.POINTER(StemDesc), C.c_void_p]),
     "yre_adown_prepool": (C.c_int, [C.POINTER(View)] * 3 + [C.c_void_p]),
     "yre_spp_maxpool": (C.c_int, [C.POINTER(View)] * 4 + [C.c_void_p]),
