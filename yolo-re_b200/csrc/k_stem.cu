@@ -11,6 +11,7 @@
 //                         scalar gather; used for stride 1 or W % 4 != 0.
 //   stem_mma_s2v_kernel   the stride-2 product kernel: vectorised cp.async gather ring (see its comment).
 #include "yre_common.cuh"
+#include <algorithm>
 #include <cstdlib>
 
 namespace {
@@ -570,9 +571,43 @@ __global__ void __launch_bounds__(128, MINB) stem_mma_s2u8_kernel(const StemPara
     asm volatile("cp.async.wait_group 0;" ::: "memory");
 }
 
+// The stem kernels write output pixels only.  A parity-plane output of an odd extent also has cells without a source
+// pixel (the last row of the planes of odd rows when Ho is odd, the last column of the planes of odd columns when Wo is
+// odd), which a stride-2 conv reads at its last output row and column: they must hold zeros (include/yre.h).  One thread
+// per 8 channels of a cell on the last row or column of a plane.
+template <typename T>
+__global__ void __launch_bounds__(256) phase4_zero_edges_kernel(const DView y) {
+    const int groups = y.C / 8, cells = y.Hp + y.Wp;
+    const long long total = 4LL * y.B * cells * groups;
+    const float z[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+        const int g = (int)(i % groups);
+        long long r = i / groups;
+        const int cell = (int)(r % cells); r /= cells;
+        const int b = (int)(r % y.B), p = (int)(r / y.B);
+        const int py = 2 * (cell < y.Wp ? y.Hp - 1 : cell - y.Wp) + (p >> 1), px = 2 * (cell < y.Wp ? cell : y.Wp - 1) + (p & 1);
+        if (py >= y.H || px >= y.W) st8<T>(y.ptr, dview_pix(y, b, py, px) + g * 8, z);
+    }
+}
+
 }  // namespace
 
+static int launch_stem_pixels(const yre_stem_desc& d, cudaStream_t s);
+
 int launch_stem(const yre_stem_desc& d, cudaStream_t s) {
+    if (int e = launch_stem_pixels(d, s)) return e;
+    if (d.y.layout == YRE_PHASE4 && ((d.y.H | d.y.W) & 1)) {
+        const DView y = make_dview(d.y);
+        const long long total = 4LL * y.B * (y.Hp + y.Wp) * (y.C / 8);
+        const unsigned grid = (unsigned)std::min<long long>(yre_cdiv(total, 256), 1024);
+        if (d.y.dtype == YRE_F32) phase4_zero_edges_kernel<float><<<grid, 256, 0, s>>>(y);
+        else phase4_zero_edges_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(y);
+        YRE_LAUNCH_CHECK("stem_phase4_edges");
+    }
+    return YRE_OK;
+}
+
+static int launch_stem_pixels(const yre_stem_desc& d, cudaStream_t s) {
     const bool u8 = d.x_u8_hwc != nullptr;
     if ((!d.x_nchw && !u8) || !d.w) YRE_FAIL(YRE_EINVAL, "stem: null pointer");
     if (u8 && d.Cin != 3) YRE_FAIL(YRE_EUNSUPPORTED, "stem: uint8 HWC frames need Cin == 3 (got %d)", d.Cin);

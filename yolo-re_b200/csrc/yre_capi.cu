@@ -340,7 +340,8 @@ int yre_plan_num_ops(const yre_plan* p) { return p ? (int)p->ops.size() : 0; }
 int yre_plan_num_launches(const yre_plan* p) {
     if (!p) return 0;
     int n = 0;
-    for (auto& o : p->ops) n += (o.kind == OP_NMS) ? 3 : 1;
+    for (auto& o : p->ops)     // NMS: 3 kernels; a stem writing parity planes of an odd extent zeroes their edge cells
+        n += (o.kind == OP_NMS) ? 3 : (o.kind == OP_STEM && o.stem.y.layout == YRE_PHASE4 && ((o.stem.y.H | o.stem.y.W) & 1)) ? 2 : 1;
     return n;
 }
 int yre_plan_num_tcgen05(const yre_plan* p) {
