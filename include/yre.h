@@ -16,6 +16,11 @@
  * Data layout: activations are channels-last ("NHWC") with an explicit channel window so that
  * chunk()/cat() of the reference (blocks/gelan.py:59-62, blocks/csp.py:60, blocks/common.py:33)
  * become zero-copy views of one wider buffer.
+ *
+ * Activation types: YRE_BF16 (the default product precision), YRE_F16 (IEEE half: 3 more significant bits than bf16,
+ * but finite only up to +-65504 -- larger results are stored as +-inf, not saturated -- and normal only down to 2^-14)
+ * and YRE_F32 (the validation precision).  Every kernel accumulates in fp32 whichever 16-bit type it reads and writes.
+ * The two 16-bit types never mix within one call: an op whose 16-bit operands disagree fails with YRE_EUNSUPPORTED.
  */
 #ifndef YRE_H
 #define YRE_H
@@ -32,7 +37,7 @@ extern "C" {
 typedef void* yre_stream_t; /* cudaStream_t */
 
 enum { YRE_OK = 0, YRE_EINVAL = -1, YRE_ECUDA = -2, YRE_EUNSUPPORTED = -3, YRE_ENOMEM = -4 };
-enum { YRE_BF16 = 0, YRE_F32 = 1 };
+enum { YRE_BF16 = 0, YRE_F32 = 1, YRE_F16 = 2 };
 enum { YRE_ACT_NONE = 0, YRE_ACT_SILU = 1 };
 enum { YRE_NHWC = 0, YRE_PHASE4 = 1 };
 enum { YRE_ENGINE_AUTO = 0, YRE_ENGINE_FFMA = 1, YRE_ENGINE_TCGEN05 = 2 };
@@ -45,7 +50,7 @@ enum { YRE_ENGINE_AUTO = 0, YRE_ENGINE_FFMA = 1, YRE_ENGINE_TCGEN05 = 2 };
  *                that have no source pixel (odd H or W) hold zeros.                              */
 typedef struct yre_view {
     void*   ptr;
-    int32_t dtype;    /* YRE_BF16 | YRE_F32 */
+    int32_t dtype;    /* YRE_BF16 | YRE_F16 | YRE_F32 */
     int32_t layout;   /* YRE_NHWC | YRE_PHASE4 */
     int32_t B, H, W;  /* logical extent */
     int32_t C_total;  /* channels of the physical buffer (pixel pitch) */
@@ -69,8 +74,9 @@ int         yre_device_check(void);
  * grouped convs expanded to block-diagonal dense weights.
  *   y = [res +] act(conv(x, w) + bias),   kernel k in {1,3}, pad k/2, stride in {1,2}.
  * w: [Cout][k][k][Cin], same dtype as x.  bias: fp32 [Cout] (may be NULL).
+ * y and res are x's 16-bit type or fp32 (a bf16 x with an fp16 y or res, or the reverse, is YRE_EUNSUPPORTED).
  * engine: YRE_ENGINE_TCGEN05 = implicit-GEMM on tcgen05/TMEM with TMA-staged operands
- * (bf16 x/w, Cin%32==0, Cout%16==0, stride-2 needs a YRE_PHASE4 input);
+ * (x/w bf16 or fp16, of the same type; fp32 accumulation; Cin%32==0, Cout%16==0, stride-2 needs a YRE_PHASE4 input);
  * YRE_ENGINE_FFMA = fp32-accurate SIMT implicit GEMM (the fp32 validation mode and the
  * fallback for shapes tcgen05 does not take); YRE_ENGINE_AUTO picks tcgen05 when eligible.
  *
@@ -100,7 +106,8 @@ int yre_conv_tc_describe(const yre_conv_desc* d, int32_t num_sms, char* out, int
 /* ---- K2: first conv straight from the image ------------------------------------------------------
  * Replaces layers.stem1 (Conv 3x3 s2 on the input image; configs/models/gelan-c.yaml stem1,
  * src/yolo/blocks/conv.py:88-89).  x_nchw: fp32 [B][Cin<=4][H][W]; w: fp32 [Cout][3][3][Cin];
- * y may be YRE_NHWC or YRE_PHASE4, bf16 or fp32.
+ * y may be YRE_NHWC or YRE_PHASE4, bf16, fp16 or fp32 (a 16-bit y rounds image and weights to that type for the
+ * tensor-core kernels; the products are exact and accumulate in fp32).
  * x_u8_hwc (optional; when non-NULL it is the input and x_nchw is ignored): uint8 [B][H][W][3] frames in BGR
  * order (cv2.imread layout), Cin must be 3.  Fuses what the reference does on the host before model()
  * (scripts/detect.py:223-227): BGR->RGB, HWC->CHW, .float() / 255 (fp32 division, round to nearest). */
@@ -119,25 +126,29 @@ int yre_stem_conv(const yre_stem_desc* d, yre_stream_t s);
  * Replaces F.avg_pool2d(x,2,1,0) -> chunk(2,1) -> [ . | F.max_pool2d(.,3,2,1) ]
  *                                                        src/yolo/blocks/downsample.py:41-44
  * avg_lo: first C/2 channels of the (H-1)x(W-1) average map (YRE_PHASE4 or YRE_NHWC);
- * max_hi: max_pool(3,2,1) of the last C/2 channels of that map, NHWC [B,Ho,Wo,C/2]. */
+ * max_hi: max_pool(3,2,1) of the last C/2 channels of that map, NHWC [B,Ho,Wo,C/2].
+ * x, avg_lo and max_hi share one dtype (bf16, fp16 or fp32).  The 16-bit types average with packed 16-bit adds
+ * (three extra roundings to the storage type); fp32 sums in torch's order. */
 int yre_adown_prepool(const yre_view* x, const yre_view* avg_lo, const yre_view* max_hi, yre_stream_t s);
 
 /* ---- K4: SPPELAN pooling pyramid --------------------------------------------------------------
  * Replaces three chained nn.MaxPool2d(5,1,2)             src/yolo/blocks/sppelan.py:44-47
- * (== windows 5 / 9 / 13 of the same input). */
+ * (== windows 5 / 9 / 13 of the same input).  x and the outputs share one dtype (bf16, fp16 or fp32); exact. */
 int yre_spp_maxpool(const yre_view* x, const yre_view* y5, const yre_view* y9, const yre_view* y13, yre_stream_t s);
 
 /* ---- K5: nearest x2 upsample into a concat slice ----------------------------------------------
  * Replaces nn.Upsample(scale_factor=2, mode="nearest") + Concat
  *                                  src/yolo/model/parser.py:159-171, src/yolo/blocks/common.py:32-33 */
-int yre_upsample2x(const yre_view* x, const yre_view* y, yre_stream_t s);
+int yre_upsample2x(const yre_view* x, const yre_view* y, yre_stream_t s);   /* x, y: one dtype; exact */
 
 /* ---- K8: CBFuse (yolov9-c auxiliary branch) ----------------------------------------------------
  * Replaces CBFuse.forward: sum_i nearest_resize(src_i -> target size) + target
  *                                                        src/yolo/blocks/auxiliary.py:100-110 */
+/* all views share one dtype (bf16, fp16 or fp32); the sum runs in fp32 and is rounded once to y's type */
 int yre_cbfuse_sum(const yre_view* srcs, int32_t n_src, const yre_view* target, const yre_view* y, yre_stream_t s);
 
-/* ---- layout conversion at the API boundary ---------------------------------------------------- */
+/* ---- layout conversion at the API boundary ----------------------------------------------------
+ * the view may be bf16, fp16 or fp32: nchw_to_view rounds to nearest even (fp16 overflows to +-inf), view_to_nchw is exact */
 int yre_nchw_to_view(const float* x_nchw, const yre_view* y, yre_stream_t s);  /* fp32 NCHW -> view  */
 int yre_view_to_nchw(const yre_view* x, float* y_nchw, yre_stream_t s);        /* view -> fp32 NCHW  */
 

@@ -7,6 +7,7 @@
 // GEMM view: M = B*Ho*Wo output pixels, N = Cout, K = k*k*Cin; 64x64 tile, 16-deep K slices,
 // 256 threads x (4 pixels x 4 channels).
 #include "yre_common.cuh"
+#include <type_traits>
 
 namespace {
 
@@ -24,6 +25,8 @@ constexpr int TM = 64, TN = 64, TK = 16;
 
 template <typename TIn, typename TOut>
 __global__ void __launch_bounds__(256) conv_ffma_kernel(const FfmaParams p) {
+    // a 16-bit residual has x's type (fp16 with fp16 operands, bf16 otherwise)
+    using TRes16 = std::conditional_t<std::is_same_v<TIn, __half>, __half, __nv_bfloat16>;
     __shared__ __align__(16) float As[TK][TM + 4];
     __shared__ __align__(16) float Bs[TK][TN + 4];
 
@@ -106,7 +109,7 @@ __global__ void __launch_bounds__(256) conv_ffma_kernel(const FfmaParams p) {
         }
         if (p.has_res) {
             const float4 r = (p.res.dtype == YRE_F32) ? ld4<float>(p.res.ptr, dview_pix(p.res, b, oy, ox) + n)
-                                                      : ld4<__nv_bfloat16>(p.res.ptr, dview_pix(p.res, b, oy, ox) + n);
+                                                      : ld4<TRes16>(p.res.ptr, dview_pix(p.res, b, oy, ox) + n);
             v[0] += r.x; v[1] += r.y; v[2] += r.z; v[3] += r.w;
         }
         st4<TOut>(p.y.ptr, dview_pix(p.y, b, oy, ox) + n, make_float4(v[0], v[1], v[2], v[3]));
@@ -139,6 +142,8 @@ int launch_conv_ffma(const yre_conv_desc& d, cudaStream_t s) {
     if (d.x.dtype == YRE_F32 && d.y.dtype == YRE_F32) conv_ffma_kernel<float, float><<<grid, 256, 0, s>>>(p);
     else if (d.x.dtype == YRE_BF16 && d.y.dtype == YRE_BF16) conv_ffma_kernel<__nv_bfloat16, __nv_bfloat16><<<grid, 256, 0, s>>>(p);
     else if (d.x.dtype == YRE_BF16 && d.y.dtype == YRE_F32) conv_ffma_kernel<__nv_bfloat16, float><<<grid, 256, 0, s>>>(p);
+    else if (d.x.dtype == YRE_F16 && d.y.dtype == YRE_F16) conv_ffma_kernel<__half, __half><<<grid, 256, 0, s>>>(p);
+    else if (d.x.dtype == YRE_F16 && d.y.dtype == YRE_F32) conv_ffma_kernel<__half, float><<<grid, 256, 0, s>>>(p);
     else YRE_FAIL(YRE_EUNSUPPORTED, "conv_ffma: dtype combination x=%d y=%d", d.x.dtype, d.y.dtype);
     YRE_LAUNCH_CHECK("conv_ffma");
     return YRE_OK;

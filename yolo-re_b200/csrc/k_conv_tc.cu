@@ -67,7 +67,7 @@ struct TcParams {
     void* y; int y_f32; int y_ctot, y_coff;
     const void* res; int res_f32; int res_ctot, res_coff;
     int* dbg;                       // optional watchdog record (may be null)
-    int tma_store;                  // 1: bf16 output through the smem-staged TMA store
+    int tma_store;                  // 1: 16-bit (or fp32) output through the smem-staged TMA store
     int npipes;                     // 1 or 2 (producer, MMA) warp pairs
     int nthreads;                   // NT_2WG or NT_3WG
     int nacc, acc_stride;           // TMEM accumulator ring (2..6 buffers), columns per buffer
@@ -302,10 +302,24 @@ __device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr, uint32_t sbo1
     return d;
 }
 
+// f[0..8) += the eight 16-bit residual values in u (bf16: a shift or a mask per value; fp16: a conversion per pair)
+template <typename T16> __device__ __forceinline__ void add_res8(const uint4& u, float* f);
+template <> __device__ __forceinline__ void add_res8<__nv_bfloat16>(const uint4& u, float* f) {
+    f[0] += __uint_as_float(u.x << 16); f[1] += __uint_as_float(u.x & 0xffff0000u);
+    f[2] += __uint_as_float(u.y << 16); f[3] += __uint_as_float(u.y & 0xffff0000u);
+    f[4] += __uint_as_float(u.z << 16); f[5] += __uint_as_float(u.z & 0xffff0000u);
+    f[6] += __uint_as_float(u.w << 16); f[7] += __uint_as_float(u.w & 0xffff0000u);
+}
+template <> __device__ __forceinline__ void add_res8<__half>(const uint4& u, float* f) {
+    const float2 a = unpack_f16x2(u.x), b = unpack_f16x2(u.y), c = unpack_f16x2(u.z), d = unpack_f16x2(u.w);
+    f[0] += a.x; f[1] += a.y; f[2] += b.x; f[3] += b.y; f[4] += c.x; f[5] += c.y; f[6] += d.x; f[7] += d.y;
+}
+
 // epilogue math for NC accumulator columns [n, n+NC): +bias -> SiLU -> (+residual), result in f[].
 // `sbias` = shared-memory copy of the bias vector (whole Cout); packed fp32x2 ops (FADD2/FMUL2/FFMA2) halve
-// the FP issue slots, SiLU costs one MUFU.TANH per element.
-template <int NC>
+// the FP issue slots, SiLU costs one MUFU.TANH per element.  T16: the 16-bit activation type (bf16 or fp16) of a
+// 16-bit residual.
+template <int NC, typename T16>
 __device__ __forceinline__ void epilogue_math(const TcParams& p, const float* sbias, const uint32_t* v, float* f, bool valid, long long pix, int n,
                                               const uint4* rpre = nullptr) {
     float2 x2[NC / 2];
@@ -336,47 +350,45 @@ __device__ __forceinline__ void epilogue_math(const TcParams& p, const float* sb
                 f[i] += r4.x; f[i + 1] += r4.y; f[i + 2] += r4.z; f[i + 3] += r4.w;
             }
         } else {
-            const __nv_bfloat16* r = reinterpret_cast<const __nv_bfloat16*>(p.res) + pix * p.res_ctot + p.res_coff + n;
+            const T16* r = reinterpret_cast<const T16*>(p.res) + pix * p.res_ctot + p.res_coff + n;
 #pragma unroll
             for (int i = 0; i < NC; i += 8) {
                 const uint4 u = rpre ? rpre[i / 8] : *reinterpret_cast<const uint4*>(r + i);     // rpre: loaded a chunk ahead
-                f[i + 0] += __uint_as_float(u.x << 16); f[i + 1] += __uint_as_float(u.x & 0xffff0000u);
-                f[i + 2] += __uint_as_float(u.y << 16); f[i + 3] += __uint_as_float(u.y & 0xffff0000u);
-                f[i + 4] += __uint_as_float(u.z << 16); f[i + 5] += __uint_as_float(u.z & 0xffff0000u);
-                f[i + 6] += __uint_as_float(u.w << 16); f[i + 7] += __uint_as_float(u.w & 0xffff0000u);
+                add_res8<T16>(u, f + i);
             }
         }
     }
 }
 
-// direct global store of NC columns (fp32 or bf16 output)
-template <int NC>
+// direct global store of NC columns (fp32 or 16-bit output)
+template <int NC, typename T16>
 __device__ __forceinline__ void store_direct(const TcParams& p, const float* f, long long pix, int n) {
     if (p.y_f32) {
         float* o = reinterpret_cast<float*>(p.y) + pix * p.y_ctot + p.y_coff + n;
 #pragma unroll
         for (int i = 0; i < NC; i += 4) *reinterpret_cast<float4*>(o + i) = make_float4(f[i], f[i + 1], f[i + 2], f[i + 3]);
     } else {
-        __nv_bfloat16* o = reinterpret_cast<__nv_bfloat16*>(p.y) + pix * p.y_ctot + p.y_coff + n;
+        T16* o = reinterpret_cast<T16*>(p.y) + pix * p.y_ctot + p.y_coff + n;
 #pragma unroll
         for (int i = 0; i < NC; i += 8) {
             uint4 u;
-            u.x = pack_bf16x2(f[i], f[i + 1]); u.y = pack_bf16x2(f[i + 2], f[i + 3]);
-            u.z = pack_bf16x2(f[i + 4], f[i + 5]); u.w = pack_bf16x2(f[i + 6], f[i + 7]);
+            u.x = pack16x2<T16>(f[i], f[i + 1]); u.y = pack16x2<T16>(f[i + 2], f[i + 3]);
+            u.z = pack16x2<T16>(f[i + 4], f[i + 5]); u.w = pack16x2<T16>(f[i + 6], f[i + 7]);
             *reinterpret_cast<uint4*>(o + i) = u;
         }
     }
 }
 
-// 32 bf16 columns of one row into the swizzled staging tile.  `row_base` = smem address of the row,
+// 32 16-bit (T16) columns of one row into the swizzled staging tile.  `row_base` = smem address of the row,
 // `c16` = first 16-byte chunk inside the row, `sw` = XOR pattern of the row (matches the TMA swizzle).
+template <typename T16>
 __device__ __forceinline__ void store_staged32(const float* f, uint32_t row_base, uint32_t c16, uint32_t sw) {
 #pragma unroll
     for (int q = 0; q < 4; ++q) {
         const uint32_t a = row_base + (((c16 + q) ^ sw) << 4);
         asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(a),
-                     "r"(pack_bf16x2(f[q * 8 + 0], f[q * 8 + 1])), "r"(pack_bf16x2(f[q * 8 + 2], f[q * 8 + 3])),
-                     "r"(pack_bf16x2(f[q * 8 + 4], f[q * 8 + 5])), "r"(pack_bf16x2(f[q * 8 + 6], f[q * 8 + 7])) : "memory");
+                     "r"(pack16x2<T16>(f[q * 8 + 0], f[q * 8 + 1])), "r"(pack16x2<T16>(f[q * 8 + 2], f[q * 8 + 3])),
+                     "r"(pack16x2<T16>(f[q * 8 + 4], f[q * 8 + 5])), "r"(pack16x2<T16>(f[q * 8 + 6], f[q * 8 + 7])) : "memory");
     }
 }
 
@@ -401,7 +413,8 @@ __device__ __forceinline__ void store_staged32_f32(const float* f, uint32_t row_
 // ptxas spilled ~350 bytes in the chunk loop (16 with one path)
 // F32T: fp32 outputs (the raw head logits) leave through a 128B-swizzled fp32 staging tile + TMA store as well (generic
 // one-CTA kernel only); a template parameter for the same reason as S64
-template <bool PF, bool CTA2 = false, bool S64 = false, bool F32T = false>
+// T16: the 16-bit activation type (bf16 or fp16) of 16-bit outputs and residuals; a template parameter for the same reason
+template <typename T16, bool PF, bool CTA2 = false, bool S64 = false, bool F32T = false>
 __device__ __forceinline__ void epilogue_role(const TcParams& p, const CUtensorMap* tmY, const float* sbias, int warp, int lane,
                                               uint32_t tmem_base, uint32_t out_base, uint32_t tfull0, uint32_t tempty0) {
         // ================= epilogue (warp-local, no CTA barrier) =================
@@ -458,10 +471,10 @@ __device__ __forceinline__ void epilogue_role(const TcParams& p, const CUtensorM
             const int tc1 = x0 + sx0, tc2 = p.ybx ? b0 + sb0 : y0 + sy0, tc3 = p.ybx ? y0 + sy0 : b0 + sb0;
             const long long pix = ((long long)b * p.Ho + y) * p.Wo + x;
             const uint32_t tfull = tfull0 + 8u * acc, tempty = tempty0 + 8u * acc;
-            // bf16 residual of the chunk about to be processed: fetched before the accumulator wait / one chunk ahead,
+            // 16-bit residual of the chunk about to be processed: fetched before the accumulator wait / one chunk ahead,
             // so its global-memory latency hides behind the MMAs and the previous chunk's staging (it was the top stall)
             const bool res16 = p.res && !p.res_f32 && valid;
-            const __nv_bfloat16* rrow = reinterpret_cast<const __nv_bfloat16*>(p.res) + pix * p.res_ctot + p.res_coff + n0;
+            const T16* rrow = reinterpret_cast<const T16*>(p.res) + pix * p.res_ctot + p.res_coff + n0;
             uint4 rr[4];
             const int first_col = S64 ? cs * 64 : cs * 32;         // this warpgroup's first chunk of the tile
             if (res16 && first_col + 32 <= p.block_n) {
@@ -480,7 +493,7 @@ __device__ __forceinline__ void epilogue_role(const TcParams& p, const CUtensorM
 #ifdef YRE_TUNING
                 if (tracer) trace(p.dbg, 2, tn, 23);
 #endif
-                epilogue_math<32>(p, sbias, w, f, valid, pix, n0 + col, res16 ? rr : nullptr);
+                epilogue_math<32, T16>(p, sbias, w, f, valid, pix, n0 + col, res16 ? rr : nullptr);
 #ifdef YRE_TUNING
                 if (tracer) trace(p.dbg, 2, tn, 24);
 #endif
@@ -496,7 +509,7 @@ __device__ __forceinline__ void epilogue_role(const TcParams& p, const CUtensorM
 #endif
                     const uint32_t buf = stg + obuf * stage_out;
                     if (F32T) store_staged32_f32(f, buf + (uint32_t)lane * 128u, (uint32_t)(lane & 7));
-                    else store_staged32(f, buf + (uint32_t)lane * 64u, 0u, sw);
+                    else store_staged32<T16>(f, buf + (uint32_t)lane * 64u, 0u, sw);
                     fence_async_smem();
                     __syncwarp();
                     if (elect_one()) {
@@ -508,7 +521,7 @@ __device__ __forceinline__ void epilogue_role(const TcParams& p, const CUtensorM
 #endif
                     obuf ^= 1u;
                 } else if (valid) {
-                    store_direct<32>(p, f, pix, n0 + col);
+                    store_direct<32, T16>(p, f, pix, n0 + col);
                 }
             };
             auto tail16 = [&](int col) {                  // 16-column tail (block_n % 32 == 16, direct-store outputs only)
@@ -516,8 +529,8 @@ __device__ __forceinline__ void epilogue_role(const TcParams& p, const CUtensorM
                 float f[16];
                 TMEM_LD16(taddr + (uint32_t)col, w16);
                 tmem_ld_wait();
-                epilogue_math<16>(p, sbias, w16, f, valid, pix, n0 + col);
-                if (valid) store_direct<16>(p, f, pix, n0 + col);
+                epilogue_math<16, T16>(p, sbias, w16, f, valid, pix, n0 + col);
+                if (valid) store_direct<16, T16>(p, f, pix, n0 + col);
             };
             auto full_at = [&](int c) { return c < nchunks && c * 32 + 32 <= block_n; };
             if (S64) {
@@ -535,7 +548,7 @@ __device__ __forceinline__ void epilogue_role(const TcParams& p, const CUtensorM
                     float f[32];
                     tmem_ld_wait();
                     TMEM_LD32(taddr + (uint32_t)(col + 32), vb);
-                    epilogue_math<32>(p, sbias, va, f, valid, pix, n0 + col, res16 ? rr : nullptr);
+                    epilogue_math<32, T16>(p, sbias, va, f, valid, pix, n0 + col, res16 ? rr : nullptr);
                     if (res16) {
 #pragma unroll
                         for (int i = 0; i < 4; ++i) rr[i] = *reinterpret_cast<const uint4*>(rrow + col + 32 + 8 * i);
@@ -544,15 +557,15 @@ __device__ __forceinline__ void epilogue_role(const TcParams& p, const CUtensorM
                     __syncwarp();
                     const uint32_t buf = stg + obuf * stage_out;
                     const uint32_t rowb = buf + (uint32_t)lane * 128u;
-                    store_staged32(f, rowb, 0u, sw7);
+                    store_staged32<T16>(f, rowb, 0u, sw7);
                     tmem_ld_wait();
                     if (more) TMEM_LD32(taddr + (uint32_t)((u + CS) * 64), va);
-                    epilogue_math<32>(p, sbias, vb, f, valid, pix, n0 + col + 32, res16 ? rr : nullptr);
+                    epilogue_math<32, T16>(p, sbias, vb, f, valid, pix, n0 + col + 32, res16 ? rr : nullptr);
                     if (res16 && more) {
 #pragma unroll
                         for (int i = 0; i < 4; ++i) rr[i] = *reinterpret_cast<const uint4*>(rrow + (u + CS) * 64 + 8 * i);
                     }
-                    store_staged32(f, rowb, 4u, sw7);
+                    store_staged32<T16>(f, rowb, 4u, sw7);
                     fence_async_smem();
                     __syncwarp();
                     if (elect_one()) {
@@ -611,7 +624,7 @@ __device__ __forceinline__ void epilogue_role(const TcParams& p, const CUtensorM
 // CTA2: launched as clusters of two CTAs that feed one cta_group::2 MMA (see TcParams::cta2).  Per 256 x N x 16 MMA each
 // SM then reads 4 KB of A + 16 N bytes of B from its shared memory instead of 4 KB + 32 N, and the TMA writes shrink
 // alike -- the shared-memory port was what bounded the one-CTA kernel at N >= 128 (profiles/r01_notes.md).
-template <int KSTEPS, int NT, bool CTA2, bool S64, bool F32T = false>
+template <typename T16, int KSTEPS, int NT, bool CTA2, bool S64, bool F32T>
 __global__ void __launch_bounds__(NT, 1)
 conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                const __grid_constant__ CUtensorMap tmY, const __grid_constant__ CUtensorMap tmAu, const TcParams p) {
@@ -791,7 +804,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             while (acc >= NACC) { acc -= NACC; acc_phase ^= 1u; }
         }
     } else if (warp >= 4 && ((warp - 4) >> 2) < p.ngroups) {
-        epilogue_role<NT == NT_2WG, CTA2, S64, F32T>(p, &tmY, sbias, warp, lane, tmem_base, out_base, bar_base + 8u * (2u * S), bar_base + 8u * (2u * S + 8u));
+        epilogue_role<T16, NT == NT_2WG, CTA2, S64, F32T>(p, &tmY, sbias, warp, lane, tmem_base, out_base, bar_base + 8u * (2u * S), bar_base + 8u * (2u * S + 8u));
     }
 
     tc_fence_before();
@@ -828,7 +841,7 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 //     16-32 cycles such a small MMA occupies the tensor pipe, so TWO warps issue, each taking every other
 //     tile; Cout is a template parameter so that every descriptor offset is an immediate.
 // Warp roles: warp 0 TMA producer, warps 1 and 3 MMA issuers, warp 2 TMEM alloc, warps 4.. epilogue.
-template <int KSTEPS, int COUT>
+template <typename T16, int KSTEPS, int COUT>
 __global__ void __launch_bounds__(NT_3WG, 1)
 conv3_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                   const __grid_constant__ CUtensorMap tmY, const __grid_constant__ CUtensorMap /*tmAu: generic kernel only*/, const TcParams p) {
@@ -939,7 +952,7 @@ conv3_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
             acc += 2;   if (acc >= NACC) { acc -= NACC; acc_phase ^= 1u; }
         }
     } else if (warp >= 4 && ((warp - 4) >> 2) < p.ngroups) {
-        epilogue_role<false>(p, &tmY, sbias, warp, lane, tmem_base, out_base, bar_base + 8u * (2u * S), bar_base + 8u * (2u * S + 8u));
+        epilogue_role<T16, false>(p, &tmY, sbias, warp, lane, tmem_base, out_base, bar_base + 8u * (2u * S), bar_base + 8u * (2u * S + 8u));
     }
 
     tc_fence_before();
@@ -962,7 +975,7 @@ conv3_halo_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant
 // port with the UMMA operand reads and bounded the generic kernel at N = 128 (8 KB read + 8 KB written per
 // 64-cycle MMA) -- drops by the 4 KB of A per MMA.
 // Warp roles: warp 0 halo producer, warp 2 TMEM alloc + weight producer, warp 1 MMA issuer, warps 4.. epilogue.
-template <int NT, bool S64>
+template <typename T16, int NT, bool S64>
 __global__ void __launch_bounds__(NT, 1)
 conv3_halo_stream_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                          const __grid_constant__ CUtensorMap tmY, const __grid_constant__ CUtensorMap /*tmAu: generic kernel only*/, const TcParams p) {
@@ -1110,7 +1123,7 @@ conv3_halo_stream_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
             acc += NPAIR; if (acc >= NACC) { acc -= NACC; acc_phase ^= 1u; }
         }
     } else if (warp >= 4 && ((warp - 4) >> 2) < p.ngroups) {
-        epilogue_role<NT == NT_2WG, false, S64>(p, &tmY, sbias, warp, lane, tmem_base, out_base, bar_t, bar_t + 64u);
+        epilogue_role<T16, NT == NT_2WG, false, S64>(p, &tmY, sbias, warp, lane, tmem_base, out_base, bar_t, bar_t + 64u);
     }
 
     tc_fence_before();
@@ -1194,7 +1207,7 @@ TcKnobs tc_knobs() {
 #define NOPE(msg) do { if (why && n) snprintf(why, n, "%s", msg); return 0; } while (0)
 // what the kernels need of the dtypes, layouts, kernel size and channel windows -- all that conv_tc_select relies on
 int tc_shape_rules(const yre_conv_desc& d, char* why, size_t n) {
-    if (d.x.dtype != YRE_BF16) NOPE("input must be bf16");
+    if (d.x.dtype != YRE_BF16 && d.x.dtype != YRE_F16) NOPE("input must be bf16 or fp16");
     if (d.y.layout != YRE_NHWC) NOPE("output must be NHWC");
     if (d.k != 1 && d.k != 3) NOPE("kernel must be 1x1 or 3x3");
     if (d.stride == 2 && !(d.k == 3 && d.x.layout == YRE_PHASE4)) NOPE("stride-2 needs a 3x3 kernel on a PHASE4 input");
@@ -1202,7 +1215,7 @@ int tc_shape_rules(const yre_conv_desc& d, char* why, size_t n) {
     if (d.x.C % 32 || d.x.c_off % 8 || d.x.C_total % 8) NOPE("Cin must be a multiple of 32 (window 16-byte aligned)");
     if (d.xu.ptr) {
         if (d.k != 1 || d.stride != 1) NOPE("an upsampled source needs a 1x1 stride-1 conv");
-        if (d.xu.dtype != YRE_BF16 || d.xu.layout != YRE_NHWC) NOPE("upsampled source must be bf16 NHWC");
+        if (d.xu.dtype != d.x.dtype || d.xu.layout != YRE_NHWC) NOPE("upsampled source must be NHWC of x's dtype");
         if (d.xu.C % 32 || d.xu.c_off % 8 || d.xu.C_total % 8) NOPE("upsampled source: channels must be a multiple of 32 (window 16-byte aligned)");
         const int bk = ((d.x.C + d.xu.C) % 64 == 0) ? 64 : 32;
         if (d.xu.C % bk || d.x.C % bk) NOPE("upsampled source: both sources must be whole K chunks");
@@ -1318,8 +1331,8 @@ int conv_tc_select(const yre_conv_desc& d, int sms, const TcKnobs& kn, TcParams*
     }
     p.b_bytes = (uint32_t)((p.cta2 ? bn / 2 : bn) * p.block_k * 2);       // a pair's CTA stages half of the weight tile
     const uint32_t stage_bytes = p.a_bytes + p.b_bytes;
-    // bf16 outputs leave through a swizzled staging tile + TMA store; fp32 outputs (raw head logits) store directly
-    p.tma_store = (d.y.dtype == YRE_BF16 && bn % 32 == 0 && kn.direct_store == 0) ? 1 : 0;
+    // 16-bit outputs leave through a swizzled staging tile + TMA store; fp32 outputs (raw head logits) store directly
+    p.tma_store = (d.y.dtype != YRE_F32 && bn % 32 == 0 && kn.direct_store == 0) ? 1 : 0;
     // fp32 outputs (raw head logits): the full 32-column chunks of a tile go through a fp32 staging tile + TMA store on the
     // generic one-CTA kernel (a 16-column tail, Cout = 80, still stores directly): one 4 KB bulk store instead of eight
     // 16-byte stores per lane at a 576-byte pitch
@@ -1395,6 +1408,8 @@ int conv_tc_select(const yre_conv_desc& d, int sms, const TcKnobs& kn, TcParams*
             (size_t)Cout * 4 + align_slack;
     // persistent grids: one CTA (pair) per work unit, at most one per SM
     *grid = p.cta2 ? 2 * std::min(p.num_units, sms / 2) : std::min(p.halo == 2 ? p.num_units : p.num_tiles, sms);
+    // instruction descriptor: fp32 accumulator (bits 4-5), A and B bf16 (bits 7-9, 10-12; conv_tc_prepare clears them for
+    // fp16 operands -- the tiling is the same for both 16-bit types), N >> 3, M >> 4
     p.idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(bn >> 3) << 17) | ((uint32_t)((p.cta2 ? 2 * BLOCK_M : BLOCK_M) >> 4) << 24);
     p.bias = d.bias; p.act = d.act;
     p.y = d.y.ptr; p.y_f32 = d.y.dtype == YRE_F32; p.y_ctot = d.y.C_total; p.y_coff = d.y.c_off;
@@ -1406,38 +1421,47 @@ int conv_tc_select(const yre_conv_desc& d, int sms, const TcKnobs& kn, TcParams*
 // ---- kernel table ----
 typedef void (*TcKernelFn)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, TcParams);
 
-// Every kernel instantiation with the TcParams values that select it.  The keys are exact (cout: Cout of the
+// each kernel as the pair {bf16, fp16} of its instantiations for the two 16-bit activation types
+template <int KSTEPS, int NT, bool CTA2, bool S64, bool F32T = false>
+const TcKernelFn conv_tc_kernels[2] = {conv_tc_kernel<__nv_bfloat16, KSTEPS, NT, CTA2, S64, F32T>,
+                                       conv_tc_kernel<__half, KSTEPS, NT, CTA2, S64, F32T>};
+template <int KSTEPS, int COUT>
+const TcKernelFn conv3_halo_kernels[2] = {conv3_halo_kernel<__nv_bfloat16, KSTEPS, COUT>, conv3_halo_kernel<__half, KSTEPS, COUT>};
+template <int NT, bool S64>
+const TcKernelFn conv3_halo_stream_kernels[2] = {conv3_halo_stream_kernel<__nv_bfloat16, NT, S64>, conv3_halo_stream_kernel<__half, NT, S64>};
+
+// Every kernel (as its {bf16, fp16} pair of instantiations) with the TcParams values that select it.  The keys are exact (cout: Cout of the
 // weight-stationary halo kernel, 0 elsewhere; f32_tma: fp32 output through the staged TMA store), so no two entries match
 // the same parameters and the order of the rows does not matter.
 struct TcKernel {
-    TcKernelFn fn;
+    const TcKernelFn* fn;                                // [0]: bf16 activations, [1]: fp16
     const char* name;                                    // for launch errors
     int halo, block_k, cout, cta2, f32_tma, nthreads, stage64;
 };
 
 const TcKernel TC_KERNELS[] = {
     //                                                                        halo  bk cout cta2 f32 nthreads s64
-    {conv_tc_kernel<4, NT_2WG, false, false>,       "conv_tc",                 0, 64,  0,  0,  0, NT_2WG, 0},
-    {conv_tc_kernel<2, NT_2WG, false, false>,       "conv_tc",                 0, 32,  0,  0,  0, NT_2WG, 0},
-    {conv_tc_kernel<4, NT_2WG, false, true>,        "conv_tc",                 0, 64,  0,  0,  0, NT_2WG, 1},
-    {conv_tc_kernel<2, NT_2WG, false, true>,        "conv_tc",                 0, 32,  0,  0,  0, NT_2WG, 1},
-    {conv_tc_kernel<4, NT_3WG, false, false>,       "conv_tc",                 0, 64,  0,  0,  0, NT_3WG, 0},
-    {conv_tc_kernel<2, NT_3WG, false, false>,       "conv_tc",                 0, 32,  0,  0,  0, NT_3WG, 0},
-    {conv_tc_kernel<4, NT_2WG, true, false>,        "conv_tc (CTA pair)",      0, 64,  0,  1,  0, NT_2WG, 0},
-    {conv_tc_kernel<2, NT_2WG, true, false>,        "conv_tc (CTA pair)",      0, 32,  0,  1,  0, NT_2WG, 0},
-    {conv_tc_kernel<4, NT_2WG, true, true>,         "conv_tc (CTA pair)",      0, 64,  0,  1,  0, NT_2WG, 1},
-    {conv_tc_kernel<2, NT_2WG, true, true>,         "conv_tc (CTA pair)",      0, 32,  0,  1,  0, NT_2WG, 1},
-    {conv_tc_kernel<4, NT_2WG, false, false, true>, "conv_tc (fp32 out)",      0, 64,  0,  0,  1, NT_2WG, 0},
-    {conv_tc_kernel<2, NT_2WG, false, false, true>, "conv_tc (fp32 out)",      0, 32,  0,  0,  1, NT_2WG, 0},
-    {conv_tc_kernel<4, NT_3WG, false, false, true>, "conv_tc (fp32 out)",      0, 64,  0,  0,  1, NT_3WG, 0},
-    {conv_tc_kernel<2, NT_3WG, false, false, true>, "conv_tc (fp32 out)",      0, 32,  0,  0,  1, NT_3WG, 0},
-    {conv3_halo_stream_kernel<NT_2WG, false>,       "conv3_halo_stream",       2, 64,  0,  0,  0, NT_2WG, 0},
-    {conv3_halo_stream_kernel<NT_2WG, true>,        "conv3_halo_stream",       2, 64,  0,  0,  0, NT_2WG, 1},
-    {conv3_halo_stream_kernel<NT_3WG, false>,       "conv3_halo_stream",       2, 64,  0,  0,  0, NT_3WG, 0},
-    {conv3_halo_kernel<4, 64>,                      "conv3_halo",              1, 64, 64,  0,  0, NT_3WG, 0},
-    {conv3_halo_kernel<4, 32>,                      "conv3_halo",              1, 64, 32,  0,  0, NT_3WG, 0},
-    {conv3_halo_kernel<2, 64>,                      "conv3_halo",              1, 32, 64,  0,  0, NT_3WG, 0},
-    {conv3_halo_kernel<2, 32>,                      "conv3_halo",              1, 32, 32,  0,  0, NT_3WG, 0},
+    {conv_tc_kernels<4, NT_2WG, false, false>,        "conv_tc",               0, 64,  0,  0,  0, NT_2WG, 0},
+    {conv_tc_kernels<2, NT_2WG, false, false>,        "conv_tc",               0, 32,  0,  0,  0, NT_2WG, 0},
+    {conv_tc_kernels<4, NT_2WG, false, true>,         "conv_tc",               0, 64,  0,  0,  0, NT_2WG, 1},
+    {conv_tc_kernels<2, NT_2WG, false, true>,         "conv_tc",               0, 32,  0,  0,  0, NT_2WG, 1},
+    {conv_tc_kernels<4, NT_3WG, false, false>,        "conv_tc",               0, 64,  0,  0,  0, NT_3WG, 0},
+    {conv_tc_kernels<2, NT_3WG, false, false>,        "conv_tc",               0, 32,  0,  0,  0, NT_3WG, 0},
+    {conv_tc_kernels<4, NT_2WG, true, false>,         "conv_tc (CTA pair)",    0, 64,  0,  1,  0, NT_2WG, 0},
+    {conv_tc_kernels<2, NT_2WG, true, false>,         "conv_tc (CTA pair)",    0, 32,  0,  1,  0, NT_2WG, 0},
+    {conv_tc_kernels<4, NT_2WG, true, true>,          "conv_tc (CTA pair)",    0, 64,  0,  1,  0, NT_2WG, 1},
+    {conv_tc_kernels<2, NT_2WG, true, true>,          "conv_tc (CTA pair)",    0, 32,  0,  1,  0, NT_2WG, 1},
+    {conv_tc_kernels<4, NT_2WG, false, false, true>,  "conv_tc (fp32 out)",    0, 64,  0,  0,  1, NT_2WG, 0},
+    {conv_tc_kernels<2, NT_2WG, false, false, true>,  "conv_tc (fp32 out)",    0, 32,  0,  0,  1, NT_2WG, 0},
+    {conv_tc_kernels<4, NT_3WG, false, false, true>,  "conv_tc (fp32 out)",    0, 64,  0,  0,  1, NT_3WG, 0},
+    {conv_tc_kernels<2, NT_3WG, false, false, true>,  "conv_tc (fp32 out)",    0, 32,  0,  0,  1, NT_3WG, 0},
+    {conv3_halo_stream_kernels<NT_2WG, false>,        "conv3_halo_stream",     2, 64,  0,  0,  0, NT_2WG, 0},
+    {conv3_halo_stream_kernels<NT_2WG, true>,         "conv3_halo_stream",     2, 64,  0,  0,  0, NT_2WG, 1},
+    {conv3_halo_stream_kernels<NT_3WG, false>,        "conv3_halo_stream",     2, 64,  0,  0,  0, NT_3WG, 0},
+    {conv3_halo_kernels<4, 64>,                       "conv3_halo",            1, 64, 64,  0,  0, NT_3WG, 0},
+    {conv3_halo_kernels<4, 32>,                       "conv3_halo",            1, 64, 32,  0,  0, NT_3WG, 0},
+    {conv3_halo_kernels<2, 64>,                       "conv3_halo",            1, 32, 64,  0,  0, NT_3WG, 0},
+    {conv3_halo_kernels<2, 32>,                       "conv3_halo",            1, 32, 32,  0,  0, NT_3WG, 0},
 };
 
 }  // namespace
@@ -1448,6 +1472,7 @@ struct ConvTcPlan {
     int grid;
     size_t smem;
     const TcKernel* kernel;
+    int f16;                      // 1: fp16 activations and weights (kernel->fn[1]), 0: bf16
 };
 
 // ---- describe ----
@@ -1500,7 +1525,8 @@ static CUresult encode_y(ConvTcPlan* pl, void* ptr) {
         box[2] = (cuuint32_t)p.stb; box[3] = (cuuint32_t)p.sth;
     }
     cuuint32_t est[4] = {1, 1, 1, 1};
-    return get_encode()(&pl->tmY, p.y_f32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, ptr, gdim, gstr, box, est,
+    const CUtensorMapDataType dt = p.y_f32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : pl->f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+    return get_encode()(&pl->tmY, dt, 4, ptr, gdim, gstr, box, est,
                         CU_TENSOR_MAP_INTERLEAVE_NONE, (p.stage64 || p.y_f32) ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
                         CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
 }
@@ -1515,6 +1541,9 @@ int conv_tc_prepare(const yre_conv_desc& d, ConvTcPlan** out) {
     std::unique_ptr<ConvTcPlan> pl(new ConvTcPlan());
     TcParams& p = pl->p;
     if (int e = conv_tc_select(d, sms, kn, &p, &pl->grid, &pl->smem)) return e;
+    pl->f16 = d.x.dtype == YRE_F16;
+    if (pl->f16) p.idesc &= ~((7u << 7) | (7u << 10));      // A and B format 0 = F16
+    const CUtensorMapDataType dt16 = pl->f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
     const int cout = p.halo == 1 ? p.Cout : 0, f32_tma = p.y_f32 && p.tma_store;
     for (const TcKernel& k : TC_KERNELS)
         if (k.halo == p.halo && k.block_k == p.block_k && k.cout == cout && k.cta2 == p.cta2 && k.f32_tma == f32_tma &&
@@ -1543,7 +1572,7 @@ int conv_tc_prepare(const yre_conv_desc& d, ConvTcPlan** out) {
             box[2] = 2; box[3] = 10;
         }
         cuuint32_t est[4] = {1, 1, 1, 1};
-        r = enc(&pl->tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, d.x.ptr, gdim, gstr, box, est, CU_TENSOR_MAP_INTERLEAVE_NONE, swz,
+        r = enc(&pl->tmA, dt16, 4, d.x.ptr, gdim, gstr, box, est, CU_TENSOR_MAP_INTERLEAVE_NONE, swz,
                 promoA, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     } else {
         const cuuint64_t Hp = (cuuint64_t)(d.x.H + 1) / 2, Wp = (cuuint64_t)(d.x.W + 1) / 2, Ct = (cuuint64_t)d.x.C_total;
@@ -1551,7 +1580,7 @@ int conv_tc_prepare(const yre_conv_desc& d, ConvTcPlan** out) {
         cuuint64_t gstr[4] = {Ct * 2, Wp * Ct * 2, Hp * Wp * Ct * 2, (cuuint64_t)d.x.B * Hp * Wp * Ct * 2};
         cuuint32_t box[5] = {(cuuint32_t)p.block_k, (cuuint32_t)p.tw, (cuuint32_t)p.th, (cuuint32_t)p.tb, 1};
         cuuint32_t est[5] = {1, 1, 1, 1, 1};
-        r = enc(&pl->tmA, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, d.x.ptr, gdim, gstr, box, est, CU_TENSOR_MAP_INTERLEAVE_NONE, swz,
+        r = enc(&pl->tmA, dt16, 5, d.x.ptr, gdim, gstr, box, est, CU_TENSOR_MAP_INTERLEAVE_NONE, swz,
                 promoA, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     }
     if (r != CUDA_SUCCESS) YRE_FAIL(YRE_ECUDA, "conv_tc: cuTensorMapEncodeTiled(A) failed with %d", (int)r);
@@ -1564,7 +1593,7 @@ int conv_tc_prepare(const yre_conv_desc& d, ConvTcPlan** out) {
         cuuint64_t gstr[4] = {0, Ct * 2, 0, Wu * Ct * 2};
         cuuint32_t box[5] = {(cuuint32_t)p.block_k, 2, (cuuint32_t)(p.tw / 2), 2, (cuuint32_t)(p.th / 2)};
         cuuint32_t est[5] = {1, 1, 1, 1, 1};
-        r = enc(&pl->tmAu, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, d.xu.ptr, gdim, gstr, box, est, CU_TENSOR_MAP_INTERLEAVE_NONE, swz,
+        r = enc(&pl->tmAu, dt16, 5, d.xu.ptr, gdim, gstr, box, est, CU_TENSOR_MAP_INTERLEAVE_NONE, swz,
                 promoA, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
         if (r != CUDA_SUCCESS) YRE_FAIL(YRE_ECUDA, "conv_tc: cuTensorMapEncodeTiled(upsampled A) failed with %d", (int)r);
     }
@@ -1574,7 +1603,7 @@ int conv_tc_prepare(const yre_conv_desc& d, ConvTcPlan** out) {
         cuuint64_t gstr[1] = {K * 2};
         cuuint32_t box[2] = {(cuuint32_t)p.block_k, (cuuint32_t)(p.cta2 ? p.block_n / 2 : p.block_n)};
         cuuint32_t est[2] = {1, 1};
-        r = enc(&pl->tmB, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(d.w), gdim, gstr, box, est, CU_TENSOR_MAP_INTERLEAVE_NONE, swz,
+        r = enc(&pl->tmB, dt16, 2, const_cast<void*>(d.w), gdim, gstr, box, est, CU_TENSOR_MAP_INTERLEAVE_NONE, swz,
                 CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     }
     if (r != CUDA_SUCCESS) YRE_FAIL(YRE_ECUDA, "conv_tc: cuTensorMapEncodeTiled(W) failed with %d", (int)r);
@@ -1593,7 +1622,8 @@ int conv_tc_launch(const ConvTcPlan* pl, cudaStream_t s) {
     static YrePerDeviceOnce once;
     if (int e = once.run([]() -> int {
             for (const TcKernel& k : TC_KERNELS)
-                YRE_CUDA(cudaFuncSetAttribute(k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+                for (int t = 0; t < 2; ++t)
+                    YRE_CUDA(cudaFuncSetAttribute(k.fn[t], cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
             return YRE_OK;
         })) return e;
     static const int pdl = tc_knobs().pdl;
@@ -1612,7 +1642,7 @@ int conv_tc_launch(const ConvTcPlan* pl, cudaStream_t s) {
         ++n;
     }
     cfg.attrs = at; cfg.numAttrs = n;
-    YRE_CUDA(cudaLaunchKernelEx(&cfg, pl->kernel->fn, pl->tmA, pl->tmB, pl->tmY, pl->tmAu, pl->p));
+    YRE_CUDA(cudaLaunchKernelEx(&cfg, pl->kernel->fn[pl->f16], pl->tmA, pl->tmB, pl->tmY, pl->tmAu, pl->p));
     YRE_LAUNCH_CHECK(pl->kernel->name);
     return YRE_OK;
 }

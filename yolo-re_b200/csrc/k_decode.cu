@@ -181,6 +181,7 @@ int launch_decode(const yre_decode_desc& d, cudaStream_t s) {
     for (int l = 0; l < d.levels; ++l) {
         const yre_view& v = d.raw[l];
         if (yre_check_view(&v, "decode.raw")) return YRE_EINVAL;
+        if (v.dtype == YRE_F16) YRE_FAIL(YRE_EUNSUPPORTED, "decode: raw logits must be fp32 or bf16 (level %d is fp16)", l);
         // rows are read as 16-byte chunks: the pixel pitch must be a multiple of 4 and, when nc % 4 != 0, leave room for the
         // last partial chunk (the host pads the raw buffer's channel count, engine.towers)
         if (v.layout != YRE_NHWC || v.C != 64 + d.nc || v.c_off % 4 || v.C_total % 4 || v.c_off + (64 + d.nc + 3) / 4 * 4 > v.C_total ||

@@ -1,6 +1,6 @@
 // K3 (ADown pre-pool), K4 (SPPELAN pyramid), K5 (nearest x2 upsample), K8 (CBFuse sum) and the
 // NCHW<->channels-last conversions at the API boundary.  All are HBM-bound: one thread moves
-// 8 consecutive channels (16 B of bf16 / 32 B of fp32) so that a warp touches whole 128 B lines.
+// 8 consecutive channels (16 B of bf16 or fp16 / 32 B of fp32) so that a warp touches whole 128 B lines.
 #include "yre_common.cuh"
 #include <float.h>
 
@@ -127,6 +127,14 @@ template <> struct SmemPix<__nv_bfloat16> {
         o[6] = __uint_as_float(u.w << 16); o[7] = __uint_as_float(u.w & 0xffff0000u);
     }
 };
+template <> struct SmemPix<__half> {
+    static constexpr int CHN = 64;
+    static __device__ __forceinline__ void ld(const uint4* px, int g, float* o) {
+        const uint4 u = px[g];
+        const float2 a = unpack_f16x2(u.x), b = unpack_f16x2(u.y), c = unpack_f16x2(u.z), d = unpack_f16x2(u.w);
+        o[0] = a.x; o[1] = a.y; o[2] = b.x; o[3] = b.y; o[4] = c.x; o[5] = c.y; o[6] = d.x; o[7] = d.y;
+    }
+};
 template <> struct SmemPix<float> {
     static constexpr int CHN = 32;
     static __device__ __forceinline__ void ld(const uint4* px, int g, float* o) {
@@ -162,6 +170,37 @@ __device__ __forceinline__ uint4 bf8_quarter(uint4 a) {
 __device__ __forceinline__ uint4 bf8_max(uint4 a, uint4 b) {
     return make_uint4(bf2_max(a.x, b.x), bf2_max(a.y, b.y), bf2_max(a.z, b.z), bf2_max(a.w, b.w));
 }
+// the same with packed fp16 (HADD2 / HMUL2 / HMNMX2): each sum rounds to fp16, <= 3 * 2^-12 relative
+__device__ __forceinline__ uint32_t h2_add(uint32_t a, uint32_t b) {
+    __half2 r = __hadd2(*reinterpret_cast<__half2*>(&a), *reinterpret_cast<__half2*>(&b));
+    return *reinterpret_cast<uint32_t*>(&r);
+}
+__device__ __forceinline__ uint32_t h2_quarter(uint32_t a) {
+    __half2 r = __hmul2(*reinterpret_cast<__half2*>(&a), __floats2half2_rn(0.25f, 0.25f));
+    return *reinterpret_cast<uint32_t*>(&r);
+}
+__device__ __forceinline__ uint32_t h2_max(uint32_t a, uint32_t b) {
+    __half2 r = __hmax2(*reinterpret_cast<__half2*>(&a), *reinterpret_cast<__half2*>(&b));
+    return *reinterpret_cast<uint32_t*>(&r);
+}
+// eight packed 16-bit channels of type T: add, x0.25, max and the -inf pair
+template <typename T> struct Pk8;
+template <> struct Pk8<__nv_bfloat16> {
+    static constexpr uint32_t NEG_INF2 = 0xff80ff80u;
+    static __device__ __forceinline__ uint4 add(uint4 a, uint4 b) { return bf8_add(a, b); }
+    static __device__ __forceinline__ uint4 quarter(uint4 a) { return bf8_quarter(a); }
+    static __device__ __forceinline__ uint4 max(uint4 a, uint4 b) { return bf8_max(a, b); }
+};
+template <> struct Pk8<__half> {
+    static constexpr uint32_t NEG_INF2 = 0xfc00fc00u;
+    static __device__ __forceinline__ uint4 add(uint4 a, uint4 b) {
+        return make_uint4(h2_add(a.x, b.x), h2_add(a.y, b.y), h2_add(a.z, b.z), h2_add(a.w, b.w));
+    }
+    static __device__ __forceinline__ uint4 quarter(uint4 a) { return make_uint4(h2_quarter(a.x), h2_quarter(a.y), h2_quarter(a.z), h2_quarter(a.w)); }
+    static __device__ __forceinline__ uint4 max(uint4 a, uint4 b) {
+        return make_uint4(h2_max(a.x, b.x), h2_max(a.y, b.y), h2_max(a.z, b.z), h2_max(a.w, b.w));
+    }
+};
 
 template <typename T>
 __global__ void __launch_bounds__(256, sizeof(T) == 2 ? 4 : 3) adown_tiled_kernel(DView x, DView lo, DView hi, int half, int tiles_x, int tiles_y) {
@@ -233,8 +272,9 @@ __global__ void __launch_bounds__(256, sizeof(T) == 2 ? 4 : 3) adown_tiled_kerne
     __syncthreads();
 
     if constexpr (sizeof(T) == 2) {
-        __nv_bfloat16* lop = reinterpret_cast<__nv_bfloat16*>(lo.ptr);
-        __nv_bfloat16* hip = reinterpret_cast<__nv_bfloat16*>(hi.ptr);
+        using P = Pk8<T>;
+        T* lop = reinterpret_cast<T*>(lo.ptr);
+        T* hip = reinterpret_cast<T*>(hi.ptr);
         if (c0 < half) {
             // item k of a thread = average pixel (ayl = k, axl = tid / 8), channel group g = tid % 8: the output address is
             // one base per row parity plus a constant row stride
@@ -254,14 +294,14 @@ __global__ void __launch_bounds__(256, sizeof(T) == 2 ? 4 : 3) adown_tiled_kerne
             }
             const bool xok = ax < Wa, xst = ph4 ? (ax >> 1) < lo.Wp : xok;
             // horizontal pair sums are shared by vertically adjacent averages: avg[k] = (h[k+1] + h[k+2]) / 4
-            uint4 hprev = bf8_add(tile[1][axl + 1][g], tile[1][axl + 2][g]);
+            uint4 hprev = P::add(tile[1][axl + 1][g], tile[1][axl + 2][g]);
 #pragma unroll
             for (int k = 0; k < 2 * AD_TY; ++k) {
                 const int ay = 2 * oy0 + k;
                 const bool ok = xok && ay < Ha;
-                const uint4 hcur = bf8_add(tile[k + 2][axl + 1][g], tile[k + 2][axl + 2][g]);
+                const uint4 hcur = P::add(tile[k + 2][axl + 1][g], tile[k + 2][axl + 2][g]);
                 uint4 o = make_uint4(0u, 0u, 0u, 0u);
-                if (ok) o = bf8_quarter(bf8_add(hprev, hcur));
+                if (ok) o = P::quarter(P::add(hprev, hcur));
                 hprev = hcur;
                 const bool st = ph4 ? (xst && (ay >> 1) < lo.Hp) : ok;       // parity planes: cells without a source pixel hold zeros
                 if (st) *reinterpret_cast<uint4*>(lop + base[k & 1] + (k >> 1) * rstep) = o;
@@ -274,29 +314,29 @@ __global__ void __launch_bounds__(256, sizeof(T) == 2 ? 4 : 3) adown_tiled_kerne
                 if (oy >= hi.H || ox >= hi.W) continue;
                 // max over the 3x3 window of 2x2 averages: horizontal pair sums h[r][q] are shared by the two average rows
                 // that use them, and the exact x0.25 is applied once after the max (monotonic, power of two)
-                uint4 m = make_uint4(0xff80ff80u, 0xff80ff80u, 0xff80ff80u, 0xff80ff80u);      // -inf pairs
+                uint4 m = make_uint4(P::NEG_INF2, P::NEG_INF2, P::NEG_INF2, P::NEG_INF2);      // -inf pairs
                 uint4 hp[3], hc[3];
                 {
                     const uint4 t0 = tile[2 * oyl][2 * oxl][g], t1 = tile[2 * oyl][2 * oxl + 1][g], t2 = tile[2 * oyl][2 * oxl + 2][g], t3 = tile[2 * oyl][2 * oxl + 3][g];
-                    hp[0] = bf8_add(t0, t1); hp[1] = bf8_add(t1, t2); hp[2] = bf8_add(t2, t3);
+                    hp[0] = P::add(t0, t1); hp[1] = P::add(t1, t2); hp[2] = P::add(t2, t3);
                 }
 #pragma unroll
                 for (int j = 0; j < 3; ++j) {
                     const uint4 t0 = tile[2 * oyl + j + 1][2 * oxl][g], t1 = tile[2 * oyl + j + 1][2 * oxl + 1][g],
                                 t2 = tile[2 * oyl + j + 1][2 * oxl + 2][g], t3 = tile[2 * oyl + j + 1][2 * oxl + 3][g];
-                    hc[0] = bf8_add(t0, t1); hc[1] = bf8_add(t1, t2); hc[2] = bf8_add(t2, t3);
+                    hc[0] = P::add(t0, t1); hc[1] = P::add(t1, t2); hc[2] = P::add(t2, t3);
                     const int ay = 2 * oy - 1 + j;
                     if (ay >= 0 && ay < Ha) {
 #pragma unroll
                         for (int q = 0; q < 3; ++q) {
                             const int ax = 2 * ox - 1 + q;
-                            if (ax >= 0 && ax < Wa) m = bf8_max(m, bf8_add(hp[q], hc[q]));
+                            if (ax >= 0 && ax < Wa) m = P::max(m, P::add(hp[q], hc[q]));
                         }
                     }
 #pragma unroll
                     for (int q = 0; q < 3; ++q) hp[q] = hc[q];
                 }
-                m = bf8_quarter(m);
+                m = P::quarter(m);
                 *reinterpret_cast<uint4*>(hip + dview_pix(hi, b, oy, ox) + (c0 - half) + g * 8) = m;
             }
         }
@@ -472,7 +512,9 @@ __global__ void __launch_bounds__(256) spp_plane_kernel(DView x, DView y5, DView
 // with packed HMNMX2 -- max() of bf16 values is exact, so the result equals the fp32-staged kernel's bit for bit -- and the
 // column pass stores its result straight to the output slice.  A CTA owns CHK channels of one image; with CHK = 64 a
 // pixel is one full 128-byte line on both the load and the three store sides.
-__device__ __forceinline__ uint4 hmax8(const uint4 a, const uint4 b) {
+// The fp16 instantiation is the same kernel with max.f16x2 (exact as well).
+template <typename T> __device__ __forceinline__ uint4 hmax8(const uint4 a, const uint4 b);
+template <> __device__ __forceinline__ uint4 hmax8<__nv_bfloat16>(const uint4 a, const uint4 b) {
     uint4 r;
     asm("max.bf16x2 %0, %1, %2;" : "=r"(r.x) : "r"(a.x), "r"(b.x));
     asm("max.bf16x2 %0, %1, %2;" : "=r"(r.y) : "r"(a.y), "r"(b.y));
@@ -480,15 +522,23 @@ __device__ __forceinline__ uint4 hmax8(const uint4 a, const uint4 b) {
     asm("max.bf16x2 %0, %1, %2;" : "=r"(r.w) : "r"(a.w), "r"(b.w));
     return r;
 }
+template <> __device__ __forceinline__ uint4 hmax8<__half>(const uint4 a, const uint4 b) {
+    uint4 r;
+    asm("max.f16x2 %0, %1, %2;" : "=r"(r.x) : "r"(a.x), "r"(b.x));
+    asm("max.f16x2 %0, %1, %2;" : "=r"(r.y) : "r"(a.y), "r"(b.y));
+    asm("max.f16x2 %0, %1, %2;" : "=r"(r.z) : "r"(a.z), "r"(b.z));
+    asm("max.f16x2 %0, %1, %2;" : "=r"(r.w) : "r"(a.w), "r"(b.w));
+    return r;
+}
 
-template <int G>      // G = CHK / 8 sixteen-byte words per pixel
-__global__ void __launch_bounds__(1024) spp_plane_bf16_kernel(DView x, DView y5, DView y9, DView y13) {
+template <typename T, int G>      // T: bf16 or fp16; G = CHK / 8 sixteen-byte words per pixel
+__global__ void __launch_bounds__(1024) spp_plane16_kernel(DView x, DView y5, DView y9, DView y13) {
     extern __shared__ __align__(16) uint4 sq[];
     const int H = x.H, W = x.W, items = H * W * G;
     uint4* A = sq;
     uint4* Bf = sq + items;
     const int b = blockIdx.x, c0 = blockIdx.y * (G * 8);
-    const __nv_bfloat16* xp = reinterpret_cast<const __nv_bfloat16*>(x.ptr);
+    const T* xp = reinterpret_cast<const T*>(x.ptr);
     for (int i = threadIdx.x; i < items; i += blockDim.x) {
         const int g = i % G, pix = i / G;
         A[i] = *reinterpret_cast<const uint4*>(xp + dview_pix(x, b, pix / W, pix % W) + c0 + g * 8);
@@ -502,19 +552,19 @@ __global__ void __launch_bounds__(1024) spp_plane_bf16_kernel(DView x, DView y5,
 #pragma unroll
             for (int d = -2; d <= 2; ++d) {
                 if (d == 0 || px + d < 0 || px + d >= W) continue;
-                m = hmax8(m, A[i + d * G]);
+                m = hmax8<T>(m, A[i + d * G]);
             }
             Bf[i] = m;
         }
         __syncthreads();
-        __nv_bfloat16* op = reinterpret_cast<__nv_bfloat16*>(outs[lvl].ptr);
+        T* op = reinterpret_cast<T*>(outs[lvl].ptr);
         for (int i = threadIdx.x; i < items; i += blockDim.x) {          // column pass Bf -> A and the output slice
             const int g = i % G, pix = i / G, py = pix / W;
             uint4 m = Bf[i];
 #pragma unroll
             for (int d = -2; d <= 2; ++d) {
                 if (d == 0 || py + d < 0 || py + d >= H) continue;
-                m = hmax8(m, Bf[i + d * W * G]);
+                m = hmax8<T>(m, Bf[i + d * W * G]);
             }
             A[i] = m;
             *reinterpret_cast<uint4*>(op + dview_pix(outs[lvl], b, py, pix % W) + c0 + g * 8) = m;
@@ -667,8 +717,10 @@ int launch_adown_prepool(const yre_view& x, const yre_view& lo, const yre_view& 
         const int tiles_x = yre_cdiv(Gx, AD_TX), tiles_y = yre_cdiv(Gy, AD_TY);
         dim3 tg((unsigned)(tiles_x * tiles_y * x.B), (unsigned)(x.C / chn));
         if (x.dtype == YRE_F32) adown_tiled_kernel<float><<<tg, 256, 0, s>>>(make_dview(x), make_dview(lo), make_dview(hi), half, tiles_x, tiles_y);
+        else if (x.dtype == YRE_F16) adown_tiled_kernel<__half><<<tg, 256, 0, s>>>(make_dview(x), make_dview(lo), make_dview(hi), half, tiles_x, tiles_y);
         else adown_tiled_kernel<__nv_bfloat16><<<tg, 256, 0, s>>>(make_dview(x), make_dview(lo), make_dview(hi), half, tiles_x, tiles_y);
     } else if (x.dtype == YRE_F32) adown_prepool_kernel<float><<<grid, 256, 0, s>>>(make_dview(x), make_dview(lo), make_dview(hi), Gy, Gx, half);
+    else if (x.dtype == YRE_F16) adown_prepool_kernel<__half><<<grid, 256, 0, s>>>(make_dview(x), make_dview(lo), make_dview(hi), Gy, Gx, half);
     else adown_prepool_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(make_dview(x), make_dview(lo), make_dview(hi), Gy, Gx, half);
     YRE_LAUNCH_CHECK("adown_prepool");
     return YRE_OK;
@@ -681,27 +733,28 @@ int launch_spp_maxpool(const yre_view& x, const yre_view& y5, const yre_view& y9
         if (y->B != x.B || y->H != x.H || y->W != x.W || y->C != x.C || y->dtype != x.dtype || y->layout != YRE_NHWC)
             YRE_FAIL(YRE_EINVAL, "spp: output views must match the input");
     if (x.layout != YRE_NHWC) YRE_FAIL(YRE_EUNSUPPORTED, "spp: NHWC only");
-    // bf16: plane-resident kernel on 16-byte words, 64 (or 32) channels per CTA when the two bf16 planes fit in shared memory
-    if (x.dtype == YRE_BF16) {
+    // bf16 / fp16: plane-resident kernel on 16-byte words, 64 (or 32) channels per CTA when the two 16-bit planes fit in
+    // shared memory
+    if (x.dtype == YRE_BF16 || x.dtype == YRE_F16) {
         int chk = 0;
         for (int c : {64, 32, 16, 8})        // 20x20 planes: 64 channels per CTA; 40x40 (1280x1280 input): 16
             if (x.C % c == 0 && (size_t)2 * x.H * x.W * c * 2 <= 112 * 1024) { chk = c; break; }
         if (chk) {
             const size_t smem = (size_t)2 * x.H * x.W * chk * 2;
+            typedef void (*SppFn)(DView, DView, DView, DView);
+            static const SppFn fns[2][4] = {
+                {spp_plane16_kernel<__nv_bfloat16, 8>, spp_plane16_kernel<__nv_bfloat16, 4>, spp_plane16_kernel<__nv_bfloat16, 2>, spp_plane16_kernel<__nv_bfloat16, 1>},
+                {spp_plane16_kernel<__half, 8>, spp_plane16_kernel<__half, 4>, spp_plane16_kernel<__half, 2>, spp_plane16_kernel<__half, 1>}};
             static YrePerDeviceOnce once16;
             if (int e = once16.run([]() -> int {
-                    YRE_CUDA(cudaFuncSetAttribute(spp_plane_bf16_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024));
-                    YRE_CUDA(cudaFuncSetAttribute(spp_plane_bf16_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024));
-                    YRE_CUDA(cudaFuncSetAttribute(spp_plane_bf16_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024));
-                    YRE_CUDA(cudaFuncSetAttribute(spp_plane_bf16_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024));
+                    for (const auto& row : fns)
+                        for (SppFn f : row) YRE_CUDA(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024));
                     return YRE_OK;
                 })) return e;
             dim3 pg((unsigned)x.B, (unsigned)(x.C / chk));
-            if (chk == 64) spp_plane_bf16_kernel<8><<<pg, 1024, smem, s>>>(make_dview(x), make_dview(y5), make_dview(y9), make_dview(y13));
-            else if (chk == 32) spp_plane_bf16_kernel<4><<<pg, 1024, smem, s>>>(make_dview(x), make_dview(y5), make_dview(y9), make_dview(y13));
-            else if (chk == 16) spp_plane_bf16_kernel<2><<<pg, 1024, smem, s>>>(make_dview(x), make_dview(y5), make_dview(y9), make_dview(y13));
-            else                spp_plane_bf16_kernel<1><<<pg, 1024, smem, s>>>(make_dview(x), make_dview(y5), make_dview(y9), make_dview(y13));
-            YRE_LAUNCH_CHECK("spp_plane_bf16");
+            const SppFn f = fns[x.dtype == YRE_F16][chk == 64 ? 0 : chk == 32 ? 1 : chk == 16 ? 2 : 3];
+            f<<<pg, 1024, smem, s>>>(make_dview(x), make_dview(y5), make_dview(y9), make_dview(y13));
+            YRE_LAUNCH_CHECK("spp_plane16");
             return YRE_OK;
         }
     }
@@ -715,10 +768,12 @@ int launch_spp_maxpool(const yre_view& x, const yre_view& y5, const yre_view& y9
         if (int e = once.run([]() -> int {
                 YRE_CUDA(cudaFuncSetAttribute(spp_plane_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
                 YRE_CUDA(cudaFuncSetAttribute(spp_plane_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
+                YRE_CUDA(cudaFuncSetAttribute(spp_plane_kernel<__half>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
                 return YRE_OK;
             })) return e;
         dim3 pg((unsigned)x.B, (unsigned)(x.C / chk));
         if (x.dtype == YRE_F32) spp_plane_kernel<float><<<pg, 256, smem, s>>>(make_dview(x), make_dview(y5), make_dview(y9), make_dview(y13), chk);
+        else if (x.dtype == YRE_F16) spp_plane_kernel<__half><<<pg, 256, smem, s>>>(make_dview(x), make_dview(y5), make_dview(y9), make_dview(y13), chk);
         else spp_plane_kernel<__nv_bfloat16><<<pg, 256, smem, s>>>(make_dview(x), make_dview(y5), make_dview(y9), make_dview(y13), chk);
         YRE_LAUNCH_CHECK("spp_plane");
         return YRE_OK;
@@ -726,6 +781,7 @@ int launch_spp_maxpool(const yre_view& x, const yre_view& y5, const yre_view& y9
     const long long total = (long long)x.B * x.H * x.W * (x.C / 8);
     dim3 grid(yre_cdiv(total, 256));
     if (x.dtype == YRE_F32) spp_kernel<float><<<grid, 256, 0, s>>>(make_dview(x), make_dview(y5), make_dview(y9), make_dview(y13));
+    else if (x.dtype == YRE_F16) spp_kernel<__half><<<grid, 256, 0, s>>>(make_dview(x), make_dview(y5), make_dview(y9), make_dview(y13));
     else spp_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(make_dview(x), make_dview(y5), make_dview(y9), make_dview(y13));
     YRE_LAUNCH_CHECK("spp_maxpool");
     return YRE_OK;
@@ -738,6 +794,7 @@ int launch_upsample2x(const yre_view& x, const yre_view& y, cudaStream_t s) {
     const long long total = (long long)x.B * x.H * x.W * (x.C / 8);
     dim3 grid(yre_cdiv(total, 256));
     if (x.dtype == YRE_F32) upsample2x_kernel<float><<<grid, 256, 0, s>>>(make_dview(x), make_dview(y));
+    else if (x.dtype == YRE_F16) upsample2x_kernel<__half><<<grid, 256, 0, s>>>(make_dview(x), make_dview(y));
     else upsample2x_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(make_dview(x), make_dview(y));
     YRE_LAUNCH_CHECK("upsample2x");
     return YRE_OK;
@@ -756,6 +813,7 @@ int launch_cbfuse_sum(const yre_view* srcs, int n, const yre_view& tgt, const yr
     const long long total = (long long)y.B * y.H * y.W * (y.C / 8);
     dim3 grid(yre_cdiv(total, 256));
     if (y.dtype == YRE_F32) cbfuse_kernel<float><<<grid, 256, 0, s>>>(fs, make_dview(tgt), make_dview(y));
+    else if (y.dtype == YRE_F16) cbfuse_kernel<__half><<<grid, 256, 0, s>>>(fs, make_dview(tgt), make_dview(y));
     else cbfuse_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(fs, make_dview(tgt), make_dview(y));
     YRE_LAUNCH_CHECK("cbfuse_sum");
     return YRE_OK;
@@ -766,6 +824,7 @@ int launch_nchw_to_view(const float* x, const yre_view& y, cudaStream_t s) {
     if (yre_check_view(&y, "nchw_to_view.y")) return YRE_EINVAL;
     dim3 grid(yre_cdiv((long long)y.H * y.W, 32), yre_cdiv(y.C, 32), y.B);
     if (y.dtype == YRE_F32) nchw_to_view_kernel<float><<<grid, 256, 0, s>>>(x, make_dview(y));
+    else if (y.dtype == YRE_F16) nchw_to_view_kernel<__half><<<grid, 256, 0, s>>>(x, make_dview(y));
     else nchw_to_view_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(x, make_dview(y));
     YRE_LAUNCH_CHECK("nchw_to_view");
     return YRE_OK;
@@ -776,6 +835,7 @@ int launch_view_to_nchw(const yre_view& x, float* y, cudaStream_t s) {
     if (yre_check_view(&x, "view_to_nchw.x")) return YRE_EINVAL;
     dim3 grid(yre_cdiv((long long)x.H * x.W, 32), yre_cdiv(x.C, 32), x.B);
     if (x.dtype == YRE_F32) view_to_nchw_kernel<float><<<grid, 256, 0, s>>>(make_dview(x), y);
+    else if (x.dtype == YRE_F16) view_to_nchw_kernel<__half><<<grid, 256, 0, s>>>(make_dview(x), y);
     else view_to_nchw_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(make_dview(x), y);
     YRE_LAUNCH_CHECK("view_to_nchw");
     return YRE_OK;

@@ -7,9 +7,11 @@
 //   stem_kernel           fp32 FMA (validation mode, any Cin <= 4 / Cout): one thread owns 4 consecutive output pixels,
 //                         keeps their input patch in registers and walks the output channels 16 at a time with the
 //                         folded weights broadcast from shared memory.
-//   stem_mma_kernel       bf16 product path, mma.sync m16n8k16 with K = 9*Cin padded to 32 (too thin for tcgen05),
-//                         scalar gather; used for stride 1 or W % 4 != 0.
+//   stem_mma_kernel       16-bit product path (bf16 or fp16 operands, fp32 accumulation), mma.sync m16n8k16 with
+//                         K = 9*Cin padded to 32 (too thin for tcgen05), scalar gather; used for stride 1 or W % 4 != 0.
 //   stem_mma_s2v_kernel   the stride-2 product kernel: vectorised cp.async gather ring (see its comment).
+// The mma.sync kernels take the 16-bit type T16 as a template parameter: the image and the weights are rounded to it,
+// the products are exact in fp32 for both types, and the output is written in it.
 #include "yre_common.cuh"
 #include <algorithm>
 #include <cstdlib>
@@ -118,8 +120,14 @@ __global__ void __launch_bounds__(128) stem_kernel(const StemParams p) {
 // writes its 16 x 64 bf16 tile through shared memory as full 16-byte, pixel-contiguous stores.
 constexpr int SM_PX = 16;       // output pixels per warp tile (one m16 MMA tile)
 
-__device__ __forceinline__ void mma_bf16_16816(float* c, const uint32_t* a, const uint32_t* b) {
+template <typename T16> __device__ __forceinline__ void mma_16816(float* c, const uint32_t* a, const uint32_t* b);
+template <> __device__ __forceinline__ void mma_16816<__nv_bfloat16>(float* c, const uint32_t* a, const uint32_t* b) {
     asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
+                 : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
+                 : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b[0]), "r"(b[1]));
+}
+template <> __device__ __forceinline__ void mma_16816<__half>(float* c, const uint32_t* a, const uint32_t* b) {
+    asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
                  : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
                  : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b[0]), "r"(b[1]));
 }
@@ -127,16 +135,16 @@ __device__ __forceinline__ void mma_bf16_16816(float* c, const uint32_t* a, cons
 // Warps are independent (no block barrier): each walks its own sequence of 16-pixel row segments,
 // and the global loads of segment n+1 are issued into registers before segment n is computed, so
 // the HBM latency hides behind the MMA + store work of the current segment.
-template <int STRIDE>
+template <typename T16, int STRIDE>
 __global__ void __launch_bounds__(128, 3) stem_mma_kernel(const StemParams p, int segs, long long total_tiles) {
     constexpr int NCOLS = SM_PX * STRIDE + 2;                    // input columns one segment needs
     constexpr int PITCH = NCOLS + 1;
     constexpr int NLD = (9 * NCOLS + 31) / 32;                   // loads per lane (Cin <= 3 -> 9 smem rows)
     __shared__ float sin_all[4][9 * PITCH];                      // per warp: [ci*3+dy][input col]
-    __shared__ __align__(16) __nv_bfloat16 sout_all[4][16][64 + 8];  // per-warp output tile, 144-byte pitch
+    __shared__ __align__(16) T16 sout_all[4][16][64 + 8];            // per-warp output tile, 144-byte pitch
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
     float* sin = sin_all[warp];
-    __nv_bfloat16 (*sout)[72] = sout_all[warp];
+    T16 (*sout)[72] = sout_all[warp];
     const int K = 9 * p.Cin;                                     // <= 27
     const int nrows = 3 * p.Cin;
 
@@ -151,7 +159,7 @@ __global__ void __launch_bounds__(128, 3) stem_mma_kernel(const StemParams p, in
             for (int h = 0; h < 2; ++h) {
                 const int n = j * 8 + g, k0 = ks * 16 + 2 * t + 8 * h;
                 const float w0 = k0 < K ? p.w[n * K + k0] : 0.f, w1 = (k0 + 1) < K ? p.w[n * K + k0 + 1] : 0.f;
-                bfrag[ks][j][h] = pack_bf16x2(w0, w1);
+                bfrag[ks][j][h] = pack16x2<T16>(w0, w1);
             }
 #pragma unroll
     for (int j = 0; j < 8; ++j) {
@@ -235,11 +243,11 @@ __global__ void __launch_bounds__(128, 3) stem_mma_kernel(const StemParams p, in
                 const int o0 = aoff[ks][h][0], o1 = aoff[ks][h][1];
                 const float v00 = o0 >= 0 ? sin[o0 + m0] : 0.f, v01 = o1 >= 0 ? sin[o1 + m0] : 0.f;
                 const float v10 = o0 >= 0 ? sin[o0 + m1] : 0.f, v11 = o1 >= 0 ? sin[o1 + m1] : 0.f;
-                a[2 * h + 0] = pack_bf16x2(v00, v01);            // row g
-                a[2 * h + 1] = pack_bf16x2(v10, v11);            // row g + 8
+                a[2 * h + 0] = pack16x2<T16>(v00, v01);            // row g
+                a[2 * h + 1] = pack16x2<T16>(v10, v11);            // row g + 8
             }
 #pragma unroll
-            for (int j = 0; j < 8; ++j) mma_bf16_16816(acc[j], a, bfrag[ks][j]);
+            for (int j = 0; j < 8; ++j) mma_16816<T16>(acc[j], a, bfrag[ks][j]);
         }
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
@@ -247,8 +255,8 @@ __global__ void __launch_bounds__(128, 3) stem_mma_kernel(const StemParams p, in
 #pragma unroll
                 for (int q = 0; q < 4; ++q) acc[j][q] = silu_tanh(acc[j][q]);
             }
-            *reinterpret_cast<uint32_t*>(&sout[g][j * 8 + 2 * t]) = pack_bf16x2(acc[j][0], acc[j][1]);
-            *reinterpret_cast<uint32_t*>(&sout[g + 8][j * 8 + 2 * t]) = pack_bf16x2(acc[j][2], acc[j][3]);
+            *reinterpret_cast<uint32_t*>(&sout[g][j * 8 + 2 * t]) = pack16x2<T16>(acc[j][0], acc[j][1]);
+            *reinterpret_cast<uint32_t*>(&sout[g + 8][j * 8 + 2 * t]) = pack16x2<T16>(acc[j][2], acc[j][3]);
         }
         __syncwarp();
 #pragma unroll
@@ -257,7 +265,7 @@ __global__ void __launch_bounds__(128, 3) stem_mma_kernel(const StemParams p, in
             const int ox = ox0 + px;
             if (ox < p.Wo) {
                 const uint4 v = *reinterpret_cast<const uint4*>(&sout[px][c16 * 8]);
-                *reinterpret_cast<uint4*>(reinterpret_cast<__nv_bfloat16*>(p.y.ptr) + dview_pix(p.y, cb, coy, ox) + c16 * 8) = v;
+                *reinterpret_cast<uint4*>(reinterpret_cast<T16*>(p.y.ptr) + dview_pix(p.y, cb, coy, ox) + c16 * 8) = v;
             }
         }
     }
@@ -270,14 +278,14 @@ __global__ void __launch_bounds__(128, 3) stem_mma_kernel(const StemParams p, in
 // per-lane offset is a kernel-lifetime constant, K padding reads a zero word instead of a predicate, the epilogue
 // uses packed fp32x2 math and the output address is one base per segment plus constant per-lane offsets.  The
 // copies are cp.async (zero-fill = conv padding) into a per-warp ring of NST stages, NST-1 segments ahead.
-template <int NST, int MINB>
+template <typename T16, int NST, int MINB>
 __global__ void __launch_bounds__(128, MINB) stem_mma_s2v_kernel(const StemParams p, int segs, long long total_tiles) {
     constexpr int NC4 = 10, PITCH = 44, ZERO = 9 * PITCH, STAGE = 9 * PITCH + 4, NLD = 3;
     __shared__ __align__(16) float sin_all[4][NST * STAGE];                // per warp: ring of NST input stages
-    __shared__ __align__(16) __nv_bfloat16 sout_all[4][16][64 + 8];
+    __shared__ __align__(16) T16 sout_all[4][16][64 + 8];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
     float* sin = sin_all[warp];
-    __nv_bfloat16 (*sout)[72] = sout_all[warp];
+    T16 (*sout)[72] = sout_all[warp];
     const int K = 9 * p.Cin, nrows = 3 * p.Cin;
     for (int i = lane; i < NST * STAGE; i += 32) sin[i] = 0.f;            // rows of absent channels and the zero words
 
@@ -291,7 +299,7 @@ __global__ void __launch_bounds__(128, MINB) stem_mma_s2v_kernel(const StemParam
             for (int h = 0; h < 2; ++h) {
                 const int n = j * 8 + g, k0 = ks * 16 + 2 * t + 8 * h;
                 const float w0 = k0 < K ? p.w[n * K + k0] : 0.f, w1 = (k0 + 1) < K ? p.w[n * K + k0 + 1] : 0.f;
-                bfrag[ks][j][h] = pack_bf16x2(w0, w1);
+                bfrag[ks][j][h] = pack16x2<T16>(w0, w1);
             }
 #pragma unroll
     for (int j = 0; j < 8; ++j)
@@ -384,11 +392,11 @@ __global__ void __launch_bounds__(128, MINB) stem_mma_s2v_kernel(const StemParam
             uint32_t a[4];
 #pragma unroll
             for (int h = 0; h < 2; ++h) {
-                a[2 * h + 0] = pack_bf16x2(st[ao[ks][h][0][0]], st[ao[ks][h][1][0]]);     // row g
-                a[2 * h + 1] = pack_bf16x2(st[ao[ks][h][0][1]], st[ao[ks][h][1][1]]);     // row g + 8
+                a[2 * h + 0] = pack16x2<T16>(st[ao[ks][h][0][0]], st[ao[ks][h][1][0]]);     // row g
+                a[2 * h + 1] = pack16x2<T16>(st[ao[ks][h][0][1]], st[ao[ks][h][1][1]]);     // row g + 8
             }
 #pragma unroll
-            for (int j = 0; j < 8; ++j) mma_bf16_16816(acc[j], a, bfrag[ks][j]);
+            for (int j = 0; j < 8; ++j) mma_16816<T16>(acc[j], a, bfrag[ks][j]);
         }
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
@@ -402,14 +410,14 @@ __global__ void __launch_bounds__(128, MINB) stem_mma_s2v_kernel(const StemParam
                 asm("tanh.approx.f32 %0, %1;" : "=f"(th.y) : "f"(hh.y));
                 lo = __ffma2_rn(hl, tl, hl); hi = __ffma2_rn(hh, th, hh);
             }
-            *reinterpret_cast<uint32_t*>(&sout[g][j * 8 + 2 * t]) = pack_bf16x2(lo.x, lo.y);
-            *reinterpret_cast<uint32_t*>(&sout[g + 8][j * 8 + 2 * t]) = pack_bf16x2(hi.x, hi.y);
+            *reinterpret_cast<uint32_t*>(&sout[g][j * 8 + 2 * t]) = pack16x2<T16>(lo.x, lo.y);
+            *reinterpret_cast<uint32_t*>(&sout[g + 8][j * 8 + 2 * t]) = pack16x2<T16>(hi.x, hi.y);
         }
         __syncwarp();                                             // sout complete; all lanes are done reading stage cstage
         const long long ybase = ph4
             ? ((((long long)((coy & 1) * 2) * p.y.B + cb) * p.y.Hp + (coy >> 1)) * p.y.Wp + (ox0 >> 1)) * p.y.C_total + p.y.c_off
             : (((long long)cb * p.y.H + coy) * p.y.W + ox0) * p.y.C_total + p.y.c_off;
-        __nv_bfloat16* yb = reinterpret_cast<__nv_bfloat16*>(p.y.ptr) + ybase;
+        T16* yb = reinterpret_cast<T16*>(p.y.ptr) + ybase;
 #pragma unroll
         for (int q = 0; q < 4; ++q) {
             const int i = lane + 32 * q, px = i >> 3, c16 = i & 7;
@@ -428,17 +436,18 @@ __global__ void __launch_bounds__(128, MINB) stem_mma_s2v_kernel(const StemParam
 // A segment's three input rows are three 128-byte windows [96 seg - 16, 96 seg + 112) of the frame rows: 24 aligned
 // 16-byte cp.async copies per segment instead of 90 (chunks outside the row are zero-filled = conv padding, the value
 // of a padded pixel being 0 after the division as well).  im2col element (pixel m, tap (dy,dx), model channel ci) is
-// byte dy*128 + 6m + 3dx + (2 - ci) + 13 of the stage.  bf16(float(v) * (1/255)) equals bf16(float(v) / 255) for all
-// 256 byte values (checked exhaustively, tests/test_cpu_host.py), so the A fragments are bit-identical to the ones the
-// fp32-tensor path builds and so is the output.  float(v) is built as (0x4B000000 | v) - 2^23: no I2F on the MUFU pipe.
-template <int NST, int MINB>
+// byte dy*128 + 6m + 3dx + (2 - ci) + 13 of the stage.  bf16(float(v) * (1/255)) equals bf16(float(v) / 255), and
+// fp16(float(v) * (1/255)) equals fp16(float(v) / 255), for all 256 byte values (checked exhaustively,
+// tests/test_cpu_host.py and tests/test_cpu_fp16.py), so the A fragments are bit-identical to the ones the fp32-tensor
+// path builds and so is the output.  float(v) is built as (0x4B000000 | v) - 2^23: no I2F on the MUFU pipe.
+template <typename T16, int NST, int MINB>
 __global__ void __launch_bounds__(128, MINB) stem_mma_s2u8_kernel(const StemParams p, int segs, long long total_tiles) {
     constexpr int ROWB = 128, ZERO = 3 * ROWB, STAGE = 3 * ROWB + 16;     // bytes; the 16 bytes at ZERO stay 0 (K padding)
     __shared__ __align__(16) uint8_t sin_all[4][NST * STAGE];
-    __shared__ __align__(16) __nv_bfloat16 sout_all[4][16][64 + 8];
+    __shared__ __align__(16) T16 sout_all[4][16][64 + 8];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, g = lane >> 2, t = lane & 3;
     uint8_t* sin = sin_all[warp];
-    __nv_bfloat16 (*sout)[72] = sout_all[warp];
+    T16 (*sout)[72] = sout_all[warp];
     constexpr int K = 27;
     for (int i = lane; i < NST * STAGE / 4; i += 32) reinterpret_cast<uint32_t*>(sin)[i] = 0u;
 
@@ -452,7 +461,7 @@ __global__ void __launch_bounds__(128, MINB) stem_mma_s2u8_kernel(const StemPara
             for (int h = 0; h < 2; ++h) {
                 const int n = j * 8 + g, k0 = ks * 16 + 2 * t + 8 * h;
                 const float w0 = k0 < K ? p.w[n * K + k0] : 0.f, w1 = (k0 + 1) < K ? p.w[n * K + k0 + 1] : 0.f;
-                bfrag[ks][j][h] = pack_bf16x2(w0, w1);
+                bfrag[ks][j][h] = pack16x2<T16>(w0, w1);
             }
 #pragma unroll
     for (int j = 0; j < 8; ++j)
@@ -534,11 +543,11 @@ __global__ void __launch_bounds__(128, MINB) stem_mma_s2u8_kernel(const StemPara
             uint32_t a[4];
 #pragma unroll
             for (int h = 0; h < 2; ++h) {
-                a[2 * h + 0] = pack_bf16x2(cvt(st[ao[ks][h][0][0]]), cvt(st[ao[ks][h][1][0]]));     // row g
-                a[2 * h + 1] = pack_bf16x2(cvt(st[ao[ks][h][0][1]]), cvt(st[ao[ks][h][1][1]]));     // row g + 8
+                a[2 * h + 0] = pack16x2<T16>(cvt(st[ao[ks][h][0][0]]), cvt(st[ao[ks][h][1][0]]));     // row g
+                a[2 * h + 1] = pack16x2<T16>(cvt(st[ao[ks][h][0][1]]), cvt(st[ao[ks][h][1][1]]));     // row g + 8
             }
 #pragma unroll
-            for (int j = 0; j < 8; ++j) mma_bf16_16816(acc[j], a, bfrag[ks][j]);
+            for (int j = 0; j < 8; ++j) mma_16816<T16>(acc[j], a, bfrag[ks][j]);
         }
 #pragma unroll
         for (int j = 0; j < 8; ++j) {
@@ -552,14 +561,14 @@ __global__ void __launch_bounds__(128, MINB) stem_mma_s2u8_kernel(const StemPara
                 asm("tanh.approx.f32 %0, %1;" : "=f"(th.y) : "f"(hh.y));
                 lo = __ffma2_rn(hl, tl, hl); hi = __ffma2_rn(hh, th, hh);
             }
-            *reinterpret_cast<uint32_t*>(&sout[g][j * 8 + 2 * t]) = pack_bf16x2(lo.x, lo.y);
-            *reinterpret_cast<uint32_t*>(&sout[g + 8][j * 8 + 2 * t]) = pack_bf16x2(hi.x, hi.y);
+            *reinterpret_cast<uint32_t*>(&sout[g][j * 8 + 2 * t]) = pack16x2<T16>(lo.x, lo.y);
+            *reinterpret_cast<uint32_t*>(&sout[g + 8][j * 8 + 2 * t]) = pack16x2<T16>(hi.x, hi.y);
         }
         __syncwarp();
         const long long ybase = ph4
             ? ((((long long)((coy & 1) * 2) * p.y.B + cb) * p.y.Hp + (coy >> 1)) * p.y.Wp + (ox0 >> 1)) * p.y.C_total + p.y.c_off
             : (((long long)cb * p.y.H + coy) * p.y.W + ox0) * p.y.C_total + p.y.c_off;
-        __nv_bfloat16* yb = reinterpret_cast<__nv_bfloat16*>(p.y.ptr) + ybase;
+        T16* yb = reinterpret_cast<T16*>(p.y.ptr) + ybase;
 #pragma unroll
         for (int q = 0; q < 4; ++q) {
             const int i = lane + 32 * q, px = i >> 3, c16 = i & 7;
@@ -601,6 +610,7 @@ int launch_stem(const yre_stem_desc& d, cudaStream_t s) {
         const long long total = 4LL * y.B * (y.Hp + y.Wp) * (y.C / 8);
         const unsigned grid = (unsigned)std::min<long long>(yre_cdiv(total, 256), 1024);
         if (d.y.dtype == YRE_F32) phase4_zero_edges_kernel<float><<<grid, 256, 0, s>>>(y);
+        else if (d.y.dtype == YRE_F16) phase4_zero_edges_kernel<__half><<<grid, 256, 0, s>>>(y);
         else phase4_zero_edges_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(y);
         YRE_LAUNCH_CHECK("stem_phase4_edges");
     }
@@ -620,7 +630,8 @@ static int launch_stem_pixels(const yre_stem_desc& d, cudaStream_t s) {
     StemParams p;
     p.x = d.x_nchw; p.xu8 = d.x_u8_hwc; p.y = make_dview(d.y); p.w = d.w; p.bias = d.bias;
     p.B = d.B; p.Cin = d.Cin; p.H = d.H; p.W = d.W; p.Ho = Ho; p.Wo = Wo; p.Cout = d.y.C; p.stride = d.stride; p.act = d.act;
-    if (u8 && d.y.dtype == YRE_BF16 && d.y.C == 64 && d.stride == 2 && d.W % 16 == 0 &&
+    const bool f16 = d.y.dtype == YRE_F16;
+    if (u8 && d.y.dtype != YRE_F32 && d.y.C == 64 && d.stride == 2 && d.W % 16 == 0 &&
         (reinterpret_cast<uintptr_t>(d.y.ptr) & 15) == 0 && (reinterpret_cast<uintptr_t>(d.x_u8_hwc) & 15) == 0) {
         const int segs = yre_cdiv(Wo, SM_PX);
         const long long tiles = (long long)d.B * Ho * segs;
@@ -629,11 +640,12 @@ static int launch_stem_pixels(const yre_stem_desc& d, cudaStream_t s) {
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
         const long long want = (tiles + 3) / 4;
         const unsigned grid = (unsigned)(want < (long long)sms * 4 ? want : (long long)sms * 4);
-        stem_mma_s2u8_kernel<3, 3><<<grid, 128, 0, s>>>(p, segs, tiles);
+        if (f16) stem_mma_s2u8_kernel<__half, 3, 3><<<grid, 128, 0, s>>>(p, segs, tiles);
+        else stem_mma_s2u8_kernel<__nv_bfloat16, 3, 3><<<grid, 128, 0, s>>>(p, segs, tiles);
         YRE_LAUNCH_CHECK("stem_mma_u8");
         return YRE_OK;
     }
-    if (!u8 && d.y.dtype == YRE_BF16 && d.Cin <= 3 && d.y.C == 64 && (reinterpret_cast<uintptr_t>(d.y.ptr) & 15) == 0) {
+    if (!u8 && d.y.dtype != YRE_F32 && d.Cin <= 3 && d.y.C == 64 && (reinterpret_cast<uintptr_t>(d.y.ptr) & 15) == 0) {
         const int segs = yre_cdiv(Wo, SM_PX);
         const long long tiles = (long long)d.B * Ho * segs;
         int dev = 0, sms = 148;
@@ -645,9 +657,13 @@ static int launch_stem_pixels(const yre_stem_desc& d, cudaStream_t s) {
 #ifdef YRE_TUNING
         if (getenv("YRE_STEM_VEC") && atoi(getenv("YRE_STEM_VEC")) == 0) vec = false;
 #endif
-        if (vec) stem_mma_s2v_kernel<3, 3><<<grid, 128, 0, s>>>(p, segs, tiles);   // 4 stages or 4 CTAs/SM (128 regs, spills) measured no better
-        else if (d.stride == 2) stem_mma_kernel<2><<<grid, 128, 0, s>>>(p, segs, tiles);
-        else stem_mma_kernel<1><<<grid, 128, 0, s>>>(p, segs, tiles);
+        // vec: 4 stages or 4 CTAs/SM (128 regs, spills) measured no better
+        if (vec && f16) stem_mma_s2v_kernel<__half, 3, 3><<<grid, 128, 0, s>>>(p, segs, tiles);
+        else if (vec) stem_mma_s2v_kernel<__nv_bfloat16, 3, 3><<<grid, 128, 0, s>>>(p, segs, tiles);
+        else if (d.stride == 2 && f16) stem_mma_kernel<__half, 2><<<grid, 128, 0, s>>>(p, segs, tiles);
+        else if (d.stride == 2) stem_mma_kernel<__nv_bfloat16, 2><<<grid, 128, 0, s>>>(p, segs, tiles);
+        else if (f16) stem_mma_kernel<__half, 1><<<grid, 128, 0, s>>>(p, segs, tiles);
+        else stem_mma_kernel<__nv_bfloat16, 1><<<grid, 128, 0, s>>>(p, segs, tiles);
         YRE_LAUNCH_CHECK("stem_mma");
         return YRE_OK;
     }
@@ -658,8 +674,8 @@ static int launch_stem_pixels(const yre_stem_desc& d, cudaStream_t s) {
 #define STEM_GO(T, C) do { if (d.stride == 2) stem_kernel<T, C, 2><<<grid, 128, smem, s>>>(p); else stem_kernel<T, C, 1><<<grid, 128, smem, s>>>(p); } while (0)
 #define STEM_T(T) switch (d.Cin) { case 1: STEM_GO(T, 1); break; case 2: STEM_GO(T, 2); break; case 3: STEM_GO(T, 3); break; default: STEM_GO(T, 4); }
 #define STEM_U8(T) do { if (d.stride == 2) stem_kernel<T, 3, 2, true><<<grid, 128, smem, s>>>(p); else stem_kernel<T, 3, 1, true><<<grid, 128, smem, s>>>(p); } while (0)
-    if (u8) { if (d.y.dtype == YRE_F32) STEM_U8(float); else STEM_U8(__nv_bfloat16); }
-    else if (d.y.dtype == YRE_F32) { STEM_T(float) } else { STEM_T(__nv_bfloat16) }
+    if (u8) { if (d.y.dtype == YRE_F32) STEM_U8(float); else if (f16) STEM_U8(__half); else STEM_U8(__nv_bfloat16); }
+    else if (d.y.dtype == YRE_F32) { STEM_T(float) } else if (f16) { STEM_T(__half) } else { STEM_T(__nv_bfloat16) }
 #undef STEM_U8
 #undef STEM_T
 #undef STEM_GO

@@ -73,6 +73,12 @@ int check_conv(const yre_conv_desc* d) {
     if (!d || !d->w) YRE_FAIL(YRE_EINVAL, "conv: null descriptor/weights");
     if (yre_check_view(&d->x, "conv.x") || yre_check_view(&d->y, "conv.y")) return YRE_EINVAL;
     if (d->res.ptr && yre_check_view(&d->res, "conv.res")) return YRE_EINVAL;
+    // bf16 and fp16 never mix: w has x's type, and a 16-bit y or residual must have the same one
+    for (const yre_view* v : {&d->x, &d->y, &d->res})
+        for (const yre_view* u : {&d->x, &d->y, &d->res})
+            if (v->ptr && u->ptr && v->dtype != YRE_F32 && u->dtype != YRE_F32 && v->dtype != u->dtype)
+                YRE_FAIL(YRE_EUNSUPPORTED, "conv: bf16 and fp16 operands mixed (x %d, y %d, res %d)", d->x.dtype, d->y.dtype,
+                         d->res.ptr ? d->res.dtype : -1);
     if (d->k != 1 && d->k != 3) YRE_FAIL(YRE_EUNSUPPORTED, "conv: kernel size %d (1 or 3)", d->k);
     if (d->stride != 1 && d->stride != 2) YRE_FAIL(YRE_EUNSUPPORTED, "conv: stride %d (1 or 2)", d->stride);
     if (d->act != YRE_ACT_NONE && d->act != YRE_ACT_SILU) YRE_FAIL(YRE_EUNSUPPORTED, "conv: activation %d", d->act);

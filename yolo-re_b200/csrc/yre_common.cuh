@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <stdarg.h>
@@ -23,7 +24,7 @@ void yre_set_error(const char* fmt, ...);
 
 static inline int yre_check_view(const yre_view* v, const char* what) {
     if (!v || !v->ptr) YRE_FAIL(YRE_EINVAL, "%s: null view", what);
-    if (v->dtype != YRE_BF16 && v->dtype != YRE_F32) YRE_FAIL(YRE_EINVAL, "%s: bad dtype %d", what, v->dtype);
+    if (v->dtype != YRE_BF16 && v->dtype != YRE_F32 && v->dtype != YRE_F16) YRE_FAIL(YRE_EINVAL, "%s: bad dtype %d", what, v->dtype);
     if (v->layout != YRE_NHWC && v->layout != YRE_PHASE4) YRE_FAIL(YRE_EINVAL, "%s: bad layout %d", what, v->layout);
     if (v->B <= 0 || v->H <= 0 || v->W <= 0 || v->C <= 0 || v->c_off < 0 || v->c_off + v->C > v->C_total)
         YRE_FAIL(YRE_EINVAL, "%s: bad extent B%d H%d W%d C%d off%d tot%d", what, v->B, v->H, v->W, v->C, v->c_off, v->C_total);
@@ -79,6 +80,10 @@ template <> struct Elt<__nv_bfloat16> {
     static __device__ __forceinline__ float ld(const void* p, long long i) { return __bfloat162float(((const __nv_bfloat16*)p)[i]); }
     static __device__ __forceinline__ void st(void* p, long long i, float v) { ((__nv_bfloat16*)p)[i] = __float2bfloat16_rn(v); }
 };
+template <> struct Elt<__half> {
+    static __device__ __forceinline__ float ld(const void* p, long long i) { return __half2float(((const __half*)p)[i]); }
+    static __device__ __forceinline__ void st(void* p, long long i, float v) { ((__half*)p)[i] = __float2half_rn(v); }
+};
 
 // 4 consecutive channels (index i multiple of 4 elements => 8/16-byte aligned)
 template <typename T> __device__ __forceinline__ float4 ld4(const void* p, long long i);
@@ -96,6 +101,22 @@ __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
     __nv_bfloat162 h = __floats2bfloat162_rn(lo, hi);
     return *reinterpret_cast<uint32_t*>(&h);
 }
+// fp16 pair, round to nearest even (cvt.rn.f16x2.f32): values beyond +-65504 become +-inf, they are not saturated
+__device__ __forceinline__ uint32_t pack_f16x2(float lo, float hi) {
+    uint32_t r;
+    asm("cvt.rn.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
+    return r;
+}
+__device__ __forceinline__ float2 unpack_f16x2(uint32_t u) { return __half22float2(*reinterpret_cast<const __half2*>(&u)); }
+// the 16-bit pack of T (bf16 or fp16): lets one kernel body serve both activation types
+template <typename T> __device__ __forceinline__ uint32_t pack16x2(float lo, float hi);
+template <> __device__ __forceinline__ uint32_t pack16x2<__nv_bfloat16>(float lo, float hi) { return pack_bf16x2(lo, hi); }
+template <> __device__ __forceinline__ uint32_t pack16x2<__half>(float lo, float hi) { return pack_f16x2(lo, hi); }
+template <> __device__ __forceinline__ float4 ld4<__half>(const void* p, long long i) {
+    const uint2 u = *reinterpret_cast<const uint2*>((const __half*)p + i);
+    const float2 a = unpack_f16x2(u.x), b = unpack_f16x2(u.y);
+    return make_float4(a.x, a.y, b.x, b.y);
+}
 template <typename T> __device__ __forceinline__ void st4(void* p, long long i, float4 v);
 template <> __device__ __forceinline__ void st4<float>(void* p, long long i, float4 v) {
     *reinterpret_cast<float4*>((float*)p + i) = v;
@@ -103,6 +124,10 @@ template <> __device__ __forceinline__ void st4<float>(void* p, long long i, flo
 template <> __device__ __forceinline__ void st4<__nv_bfloat16>(void* p, long long i, float4 v) {
     uint2 u; u.x = pack_bf16x2(v.x, v.y); u.y = pack_bf16x2(v.z, v.w);
     *reinterpret_cast<uint2*>((__nv_bfloat16*)p + i) = u;
+}
+template <> __device__ __forceinline__ void st4<__half>(void* p, long long i, float4 v) {
+    uint2 u; u.x = pack_f16x2(v.x, v.y); u.y = pack_f16x2(v.z, v.w);
+    *reinterpret_cast<uint2*>((__half*)p + i) = u;
 }
 
 // 8 consecutive channels as fp32 (index i multiple of 8 elements: one 16-byte access for bf16, two for fp32)
@@ -118,6 +143,11 @@ template <> __device__ __forceinline__ void ld8<__nv_bfloat16>(const void* p, lo
     o[4] = __uint_as_float(u.z << 16); o[5] = __uint_as_float(u.z & 0xffff0000u);
     o[6] = __uint_as_float(u.w << 16); o[7] = __uint_as_float(u.w & 0xffff0000u);
 }
+template <> __device__ __forceinline__ void ld8<__half>(const void* p, long long i, float* o) {
+    const uint4 u = *reinterpret_cast<const uint4*>((const __half*)p + i);
+    const float2 a = unpack_f16x2(u.x), b = unpack_f16x2(u.y), c = unpack_f16x2(u.z), d = unpack_f16x2(u.w);
+    o[0] = a.x; o[1] = a.y; o[2] = b.x; o[3] = b.y; o[4] = c.x; o[5] = c.y; o[6] = d.x; o[7] = d.y;
+}
 template <typename T> __device__ __forceinline__ void st8(void* p, long long i, const float* o);
 template <> __device__ __forceinline__ void st8<float>(void* p, long long i, const float* o) {
     *reinterpret_cast<float4*>((float*)p + i) = make_float4(o[0], o[1], o[2], o[3]);
@@ -127,6 +157,11 @@ template <> __device__ __forceinline__ void st8<__nv_bfloat16>(void* p, long lon
     uint4 u;
     u.x = pack_bf16x2(o[0], o[1]); u.y = pack_bf16x2(o[2], o[3]); u.z = pack_bf16x2(o[4], o[5]); u.w = pack_bf16x2(o[6], o[7]);
     *reinterpret_cast<uint4*>((__nv_bfloat16*)p + i) = u;
+}
+template <> __device__ __forceinline__ void st8<__half>(void* p, long long i, const float* o) {
+    uint4 u;
+    u.x = pack_f16x2(o[0], o[1]); u.y = pack_f16x2(o[2], o[3]); u.z = pack_f16x2(o[4], o[5]); u.w = pack_f16x2(o[6], o[7]);
+    *reinterpret_cast<uint4*>((__half*)p + i) = u;
 }
 
 __device__ __forceinline__ float silu_f(float v) { return v / (1.0f + __expf(-v)); }

@@ -11,7 +11,7 @@ from pathlib import Path
 _HERE = Path(__file__).resolve().parent
 LIB_PATH = _HERE / "libyre.so"
 
-BF16, F32 = 0, 1
+BF16, F32, F16 = 0, 1, 2
 ACT_NONE, ACT_SILU = 0, 1
 NHWC, PHASE4 = 0, 1
 ENGINE_AUTO, ENGINE_FFMA, ENGINE_TCGEN05 = 0, 1, 2

@@ -4,7 +4,8 @@ of libyre launches -- the replacement for the reference's per-forward interprete
 
 What the compiler does (SURVEY.md section 7.1):
   * folds BatchNorm into the conv weights/bias in fp64 (w' = w*g/sqrt(var+eps), b' = beta - mu*g/sqrt(var+eps),
-    eps = 1e-3, src/yolo/blocks/conv.py:85), then casts to bf16 (product) or fp32 (validation);
+    eps = 1e-3, src/yolo/blocks/conv.py:85), then casts the weights to bf16 (product), fp16 (opt-in) or fp32 (validation);
+    the bias stays fp32;
   * folds RepConv's 1x1 branch into the 3x3 centre tap (conv.py:140-141);
   * merges sibling convs that share an input: RepNCSP conv1||conv2 (csp.py:59-60) and the detect
     towers' first 3x3s (heads/detect.py:48-64);
@@ -28,6 +29,18 @@ from . import blocks as B
 from .heads import REG_MAX, DetectDFL, DualDetectDFL
 
 _DEFAULT_PRECISION = "bf16"
+# per precision: (libyre activation dtype, torch dtype)
+_DTYPES = {"bf16": (L.BF16, torch.bfloat16), "fp16": (L.F16, torch.float16), "fp32": (L.F32, torch.float32)}
+_TORCH_DT = {L.BF16: torch.bfloat16, L.F16: torch.float16, L.F32: torch.float32}
+F16_MAX = 65504.0         # largest finite fp16
+
+
+def _check_f16_range(w: torch.Tensor, name: str) -> None:
+    """fp16 weights: a folded weight beyond +-65504 would become +-inf, so the compile fails instead, naming the layer."""
+    m = float(w.abs().max()) if w.numel() else 0.0
+    if not m <= F16_MAX:
+        raise L.YreError(f"fp16 precision: layer '{name}' has a folded weight of magnitude {m:.6g} > {F16_MAX:g} "
+                         "(largest finite fp16); run it in bf16 or fp32")
 # Test hook: with a CPU device a plan can be *compiled* (buffers on the host, every op recorded in
 # Plan.trace and in the C plan) but never run -- tests/ replays the trace with a CPU interpreter to
 # check the graph wiring without a GPU.  The product path never sets this.
@@ -36,7 +49,9 @@ _ALLOW_CPU_DRY_RUN = False
 
 @contextmanager
 def precision(p: str):
-    """Precision used when a *block* (not a whole YOLO) is called directly."""
+    """Precision ("bf16", "fp16" or "fp32") used when a *block* (not a whole YOLO) is called directly."""
+    if p not in _DTYPES:
+        raise ValueError("precision must be 'bf16', 'fp16' or 'fp32'")
     global _DEFAULT_PRECISION
     old, _DEFAULT_PRECISION = _DEFAULT_PRECISION, p
     try:
@@ -98,11 +113,11 @@ class Plan:
                 L.check(self.lib.yre_device_check(), "device_check")
         self.trace: list[tuple] = []
         self.device, self.batch, self.prec = device, batch, prec
-        self.dt = L.BF16 if prec == "bf16" else L.F32
-        self.tdt = torch.bfloat16 if prec == "bf16" else torch.float32
+        self.dt, self.tdt = _DTYPES[prec]
         # tcgen05 convs encode TMA descriptors of device buffers, so a dry (host-buffer) plan takes the FFMA engine even
         # where a CUDA driver is present
-        self.engine = L.ENGINE_AUTO if prec == "bf16" and not self.dry else L.ENGINE_FFMA
+        self.engine = L.ENGINE_AUTO if prec in ("bf16", "fp16") and not self.dry else L.ENGINE_FFMA
+        self.names: dict[int, str] = {}          # id(module) -> qualified name, for error messages
         h = C.c_void_p()
         L.check(self.lib.yre_plan_create(C.byref(h)), "plan_create")
         self.h = h
@@ -124,7 +139,7 @@ class Plan:
     # -- memory ---------------------------------------------------------------------------------------
     def alloc(self, H: int, W: int, Cn: int, dtype=None, layout=L.NHWC) -> V:
         dtype = self.dt if dtype is None else dtype
-        tdt = torch.bfloat16 if dtype == L.BF16 else torch.float32
+        tdt = _TORCH_DT[dtype]
         if layout == L.PHASE4:
             shape = (4, self.batch, (H + 1) // 2, (W + 1) // 2, Cn)
             t = torch.zeros(shape, dtype=tdt, device=self.device)   # cells without a source pixel stay 0
@@ -181,8 +196,14 @@ class Plan:
         raise L.YreError(f"cannot fold {type(m).__name__}")
 
     # -- op emission -------------------------------------------------------------------------------------
-    def conv(self, x: V | VCat, w, b, k, stride, silu, out: V | None = None, res: V | None = None, out_dtype=None) -> V:
+    def name_of(self, m) -> str:
+        return self.names.get(id(m), type(m).__name__)
+
+    def conv(self, x: V | VCat, w, b, k, stride, silu, out: V | None = None, res: V | None = None, out_dtype=None,
+             name: str = "conv") -> V:
         cout, cin = w.shape[0], w.shape[1]
+        if self.prec == "fp16":
+            _check_f16_range(w, name)
         assert cin == x.C, (cin, x.C)
         xu = None
         if isinstance(x, VCat):
@@ -203,18 +224,21 @@ class Plan:
 
     def conv_m(self, m, x: V, out: V | None = None, res: V | None = None, out_dtype=None) -> V:
         w, b, k, s, silu = self.fold(m)
-        return self.conv(x, w, b, k, s, silu, out, res, out_dtype)
+        return self.conv(x, w, b, k, s, silu, out, res, out_dtype, name=self.name_of(m))
 
     def conv_merged(self, ms, x: V, out: V | None = None) -> V:
         """Sibling convs on one input -> one GEMM with concatenated output channels."""
         fs = [self.fold(m) for m in ms]
         assert len({(f[2], f[3], f[4]) for f in fs}) == 1
-        return self.conv(x, torch.cat([f[0] for f in fs]), torch.cat([f[1] for f in fs]), fs[0][2], fs[0][3], fs[0][4], out)
+        return self.conv(x, torch.cat([f[0] for f in fs]), torch.cat([f[1] for f in fs]), fs[0][2], fs[0][3], fs[0][4], out,
+                         name=" + ".join(self.name_of(m) for m in ms))
 
     def stem(self, m: B.Conv, x: torch.Tensor, phase4: bool) -> V:
         """x: the fp32 NCHW image batch, or uint8 [B,H,W,3] BGR frames (BGR->RGB, HWC->CHW and /255 of
         scripts/detect.py:223-227 are then fused into the kernel's gather)."""
         w, b, k, s, silu = self.fold(m)
+        if self.prec == "fp16":                 # the tensor-core stem rounds its weights to fp16
+            _check_f16_range(w, self.name_of(m))
         u8 = x.dtype == torch.uint8
         if u8:
             Bn, H, W, Cin = x.shape
@@ -345,7 +369,7 @@ class Plan:
             if ncp != nc:
                 wc = torch.cat([wc, wc.new_zeros((ncp - nc,) + tuple(wc.shape[1:]))])
                 bc = torch.cat([bc, bc.new_zeros(ncp - nc)])
-            self.conv(hc, wc, bc, kc, sc, silu_c, out=raw_full.sl(4 * REG_MAX, ncp))
+            self.conv(hc, wc, bc, kc, sc, silu_c, out=raw_full.sl(4 * REG_MAX, ncp), name=self.name_of(cls[i][2]))
             raws.append(raw)
         A = sum(r.H * r.W for r in raws)
         y = torch.empty((self.batch, A, 4 + nc), dtype=torch.float32, device=self.device)
@@ -506,6 +530,7 @@ def compile_model(model, x: torch.Tensor) -> Plan:
     else:
         Bn, Cin, H, W = x.shape
     p = Plan(x.device, Bn, model.precision)
+    p.names = {id(m): n for n, m in model.named_modules()}
     names = list(model.layers.keys())
     conn = model.connections
     srcs = {n: ([conn[n]] if isinstance(conn[n], str) else list(conn[n])) for n in names}
@@ -582,7 +607,7 @@ def compile_model(model, x: torch.Tensor) -> Plan:
                 raise L.YreError(f"layer '{n}' reads the image but is not a 3x3 Conv (unsupported stem)")
             cons = consumers.get(n, [])
             ph = (len(cons) == 1 and isinstance(model.layers[cons[0]], B.Conv) and model.layers[cons[0]].conv.stride[0] == 2
-                  and model.layers[cons[0]].conv.kernel_size[0] == 3 and n not in dest and p.prec == "bf16")
+                  and model.layers[cons[0]].conv.kernel_size[0] == 3 and n not in dest and p.prec in ("bf16", "fp16"))
             vals[n] = p.stem(m, x, ph)
             continue
         a = ins[0] if single else ins
@@ -735,6 +760,7 @@ def compile_module(m: nn.Module, x, prec: str | None = None):
     (NCHW fp32 tensors, same nesting as the reference module returns) are filled by plan.run()."""
     t0 = _first_tensor(x)
     p = Plan(t0.device, t0.shape[0], prec or _DEFAULT_PRECISION)
+    p.names = {id(mm): n or type(m).__name__ for n, mm in m.named_modules()}
     if isinstance(m, B.Conv) and isinstance(x, torch.Tensor) and x.shape[1] <= 4 and m.conv.kernel_size[0] == 3:
         xin = x.contiguous().float()
         p.keep.append(xin)

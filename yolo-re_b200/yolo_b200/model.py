@@ -115,7 +115,7 @@ class YOLO(nn.Module):
         self.detect_inputs = detect_inputs
         self._stride_initialized = False
         # engine state (not part of the state_dict)
-        self.precision = "bf16"          # "bf16" (tcgen05) | "fp32" (FFMA validation mode)
+        self.precision = "bf16"          # "bf16" | "fp16" (tcgen05, fp32 accumulation) | "fp32" (FFMA validation mode)
         self.fresh_outputs = True        # False: return the plan's static output buffers (no allocation)
         self.check_weights = True        # re-fold when a parameter was modified in place
         self.use_cuda_graph = False      # with fresh_outputs=False: capture the launch list once per input buffer and replay it
@@ -131,8 +131,13 @@ class YOLO(nn.Module):
         self.__dict__.pop("_wt_tensors", None)
 
     def set_precision(self, precision: str) -> "YOLO":
-        if precision not in ("bf16", "fp32"):
-            raise ValueError("precision must be 'bf16' or 'fp32'")
+        """"bf16" (default): tcgen05 convolutions on bf16 activations and weights.  "fp16": the same kernels on IEEE half
+        operands -- 8x smaller rounding than bf16 at the same speed, but finite only up to +-65504: a folded conv weight
+        beyond that fails the compile with YreError, activations beyond it become +-inf (they are not saturated), and
+        weights below 2^-24 in magnitude become zero.  "fp32": the fp32-FMA validation engine.  Accumulation is fp32 in
+        every mode; the raw head logits and y stay fp32."""
+        if precision not in ("bf16", "fp16", "fp32"):
+            raise ValueError("precision must be 'bf16', 'fp16' or 'fp32'")
         if precision != self.precision:
             self.precision = precision
             self.invalidate()
