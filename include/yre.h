@@ -208,10 +208,12 @@ int    yre_nms_filter_only(const yre_nms_desc* d, yre_stream_t s);
  *             cv2.resize(INTER_LINEAR) on uint8          (OpenCV; 8-bit fixed point, bit-exact restatement)
  *             BGR->RGB, HWC->CHW, .float() / 255         scripts/detect.py:223-227
  * src: uint8 [h][w][3] (cv2.imread layout, rows `row_pitch` bytes apart) on the DEVICE.
- * out_mode YRE_LB_F32_CHW: dst = float [3][S][S], channel order reversed (RGB), value / 255 -- the tensor the
- *                          reference feeds to model(); YRE_LB_U8_HWC: dst = uint8 [S][S][3], what letterbox() returns.
- * The geometry (un-padded size, padding) comes from yre_letterbox_geometry, which mirrors the reference's
- * Python arithmetic including round-half-to-even. */
+ * The destination is an out_h x out_w rectangle (S x S when out_h = out_w = 0, the square letterbox):
+ * out_mode YRE_LB_F32_CHW: dst = float [3][out_h][out_w], channel order reversed (RGB), value / 255 -- the tensor the
+ *                          reference feeds to model(); YRE_LB_U8_HWC: dst = uint8 [out_h][out_w][3], what letterbox()
+ *                          returns.
+ * The geometry (un-padded size, padding, destination extent) comes from yre_letterbox_geometry_rect, which mirrors
+ * the reference's Python arithmetic including round-half-to-even. */
 enum { YRE_LB_F32_CHW = 0, YRE_LB_U8_HWC = 1 };
 typedef struct yre_letterbox_desc {
     const uint8_t* src;
@@ -223,12 +225,21 @@ typedef struct yre_letterbox_desc {
     uint8_t        color[4];         /* pad colour in SOURCE channel order (114,114,114), 4th byte unused */
     int32_t        out_mode;
     void*          dst;
+    int32_t        out_h, out_w;     /* destination extent; 0, 0 = new_shape x new_shape */
 } yre_letterbox_desc;
-/* host helper: fills new_w/new_h/top/left of *d from (h, w, new_shape); ratio and the (pad_w, pad_h) pair the
- * reference returns go to the optional outputs.  Fails with YRE_EINVAL when the padded size is not S x S. */
+/* host helper: letterbox geometry for a target (new_h, new_w) from the source (d->h, d->w).
+ *   r = min(new_h / h, new_w / w); the resized size is round(w r) x round(h r), half to even;
+ *   stride > 0 ("auto") reduces each axis' padding modulo stride: the smallest stride-multiple rectangle;
+ *   each padding d/2 is split round(d/2 - 0.1) before, round(d/2 + 0.1) after.
+ * Fills new_w/new_h/top/left/out_h/out_w of *d; ratio and the (pad_w, pad_h) pair the reference returns (int(d/2),
+ * truncated) go to the optional outputs.  Fails with YRE_EINVAL when the resized image is empty. */
+int yre_letterbox_geometry_rect(yre_letterbox_desc* d, int32_t new_h, int32_t new_w, int32_t stride, double* ratio,
+                                int32_t* pad_w, int32_t* pad_h);
+/* yre_letterbox_geometry_rect(d, d->new_shape, d->new_shape, 0, ...): the square letterbox */
 int yre_letterbox_geometry(yre_letterbox_desc* d, double* ratio, int32_t* pad_w, int32_t* pad_h);
 int yre_letterbox_u8(const yre_letterbox_desc* d, yre_stream_t s);
-/* n images sharing new_shape and out_mode in as few launches as possible (32 images per launch) */
+/* n images sharing the destination extent and out_mode in as few launches as possible (32 images per launch); their
+ * resized sizes and offsets inside the destination may differ */
 int yre_letterbox_u8_batch(const yre_letterbox_desc* d, int32_t n, yre_stream_t s);
 /* K9 replaces scale_boxes                                scripts/detect.py:74-109
  * boxes: n rows of xyxy fp32, `row_stride` floats apart (6 for detection rows), updated in place:

@@ -1,7 +1,7 @@
 // K8 / K9: letterbox pre-processing and box rescaling -- the steps either side of the detection path.
 //   letterbox + cv2.resize(INTER_LINEAR, uint8) + BGR->RGB + HWC->CHW + /255     reference scripts/detect.py:40-71, 223-227
 //   scale_boxes                                                                  reference scripts/detect.py:74-109
-// Byte / integer work, HBM-bound on the fp32 output (4 S^2 x 3 bytes written per image against <= 3 h w read):
+// Byte / integer work, HBM-bound on the fp32 output (4 x 3 bytes written per destination pixel against <= 3 h w read):
 // one thread per output pixel, 32 x 8 thread tiles so that the three channel planes are written in full 128-byte
 // rows and the source bytes of a tile sit in a handful of adjacent lines.
 // The resize restates OpenCV's 8-bit fixed-point bilinear kernel bit for bit (oracle/preproc_ref.py has the
@@ -15,7 +15,8 @@ struct LbParams {
     const uint8_t* src;
     int h, w;
     long long pitch;
-    int S, nw, nh, top, left;
+    int oh, ow;              // destination extent
+    int nw, nh, top, left;
     int c0, c1, c2;          // pad colour, source channel order
     int mode;                // 0 bilinear, 1 copy, 2 exact 2x area
     double sx, sy;           // src / dst scale
@@ -46,7 +47,7 @@ template <int OUT_U8>
 __global__ void __launch_bounds__(256) letterbox_kernel(const __grid_constant__ LbBatch batch) {
     const LbParams& p = batch.p[blockIdx.z];
     const int X = blockIdx.x * 32 + (threadIdx.x & 31), Y = blockIdx.y * 8 + (threadIdx.x >> 5);
-    if (X >= p.S || Y >= p.S) return;
+    if (X >= p.ow || Y >= p.oh) return;
     int v0 = p.c0, v1 = p.c1, v2 = p.c2;
     const int dx = X - p.left, dy = Y - p.top;
     if (dx >= 0 && dx < p.nw && dy >= 0 && dy < p.nh) {
@@ -77,11 +78,11 @@ __global__ void __launch_bounds__(256) letterbox_kernel(const __grid_constant__ 
         }
     }
     if (OUT_U8) {
-        uint8_t* o = reinterpret_cast<uint8_t*>(p.dst) + ((long long)Y * p.S + X) * 3;
+        uint8_t* o = reinterpret_cast<uint8_t*>(p.dst) + ((long long)Y * p.ow + X) * 3;
         o[0] = (uint8_t)v0; o[1] = (uint8_t)v1; o[2] = (uint8_t)v2;
     } else {
-        float* o = reinterpret_cast<float*>(p.dst) + (long long)Y * p.S + X;
-        const long long plane = (long long)p.S * p.S;
+        float* o = reinterpret_cast<float*>(p.dst) + (long long)Y * p.ow + X;
+        const long long plane = (long long)p.oh * p.ow;
         o[0] = __fdiv_rn((float)v2, 255.f);              // BGR -> RGB: plane 0 is the source's channel 2
         o[plane] = __fdiv_rn((float)v1, 255.f);
         o[2 * plane] = __fdiv_rn((float)v0, 255.f);
@@ -101,31 +102,45 @@ __global__ void scale_boxes_kernel(float* boxes, int n, int stride, float pad_w,
 
 }  // namespace
 
-extern "C" int yre_letterbox_geometry(yre_letterbox_desc* d, double* ratio, int32_t* pad_w, int32_t* pad_h) {
-    if (!d || d->h <= 0 || d->w <= 0 || d->new_shape <= 0) YRE_FAIL(YRE_EINVAL, "letterbox: bad size");
-    const double S = d->new_shape;
-    const double r = fmin(S / d->h, S / d->w);
+extern "C" int yre_letterbox_geometry_rect(yre_letterbox_desc* d, int32_t new_h, int32_t new_w, int32_t stride,
+                                           double* ratio, int32_t* pad_w, int32_t* pad_h) {
+    if (!d || d->h <= 0 || d->w <= 0 || new_h <= 0 || new_w <= 0 || stride < 0) YRE_FAIL(YRE_EINVAL, "letterbox: bad size");
+    const double r = fmin((double)new_h / d->h, (double)new_w / d->w);
     // Python round() and C nearbyint() under the default rounding mode both round half to even
     const int nw = (int)nearbyint(d->w * r), nh = (int)nearbyint(d->h * r);
-    const double dw = (S - nw) / 2.0, dh = (S - nh) / 2.0;
+    if (nw <= 0 || nh <= 0) YRE_FAIL(YRE_EINVAL, "letterbox: %dx%d resizes to nothing at %dx%d", d->w, d->h, new_w, new_h);
+    int pw = new_w - nw, ph = new_h - nh;                  // >= 0: r fits both axes
+    if (stride > 0) { pw %= stride; ph %= stride; }        // auto: the smallest stride-multiple rectangle
+    const double dw = pw / 2.0, dh = ph / 2.0;
     const int top = (int)nearbyint(dh - 0.1), bottom = (int)nearbyint(dh + 0.1);
     const int left = (int)nearbyint(dw - 0.1), right = (int)nearbyint(dw + 0.1);
-    if (nw <= 0 || nh <= 0 || nw + left + right != d->new_shape || nh + top + bottom != d->new_shape)
-        YRE_FAIL(YRE_EINVAL, "letterbox: %dx%d does not letterbox to %d (got %dx%d)", d->w, d->h, d->new_shape, nw + left + right, nh + top + bottom);
     d->new_w = nw; d->new_h = nh; d->top = top; d->left = left;
+    d->out_h = nh + top + bottom; d->out_w = nw + left + right;
     if (ratio) *ratio = r;
     if (pad_w) *pad_w = (int32_t)dw;          // int(dw): truncation, scripts/detect.py:71
     if (pad_h) *pad_h = (int32_t)dh;
     return YRE_OK;
 }
 
+extern "C" int yre_letterbox_geometry(yre_letterbox_desc* d, double* ratio, int32_t* pad_w, int32_t* pad_h) {
+    if (!d) YRE_FAIL(YRE_EINVAL, "letterbox: bad size");
+    return yre_letterbox_geometry_rect(d, d->new_shape, d->new_shape, 0, ratio, pad_w, pad_h);
+}
+
+static void lb_extent(const yre_letterbox_desc* d, int& oh, int& ow) {
+    oh = d->out_h; ow = d->out_w;
+    if (oh == 0 && ow == 0) oh = ow = d->new_shape;
+}
+
 static int lb_fill(const yre_letterbox_desc* d, LbParams& p) {
     if (!d || !d->src || !d->dst) YRE_FAIL(YRE_EINVAL, "letterbox: null pointer");
     if (d->h <= 0 || d->w <= 0 || d->row_pitch < 3ll * d->w) YRE_FAIL(YRE_EINVAL, "letterbox: bad source extent");
-    if (d->new_w <= 0 || d->new_h <= 0 || d->top < 0 || d->left < 0 || d->left + d->new_w > d->new_shape || d->top + d->new_h > d->new_shape)
-        YRE_FAIL(YRE_EINVAL, "letterbox: geometry does not fit %d", d->new_shape);
+    lb_extent(d, p.oh, p.ow);
+    if (p.oh <= 0 || p.ow <= 0 || d->new_w <= 0 || d->new_h <= 0 || d->top < 0 || d->left < 0 || d->left + d->new_w > p.ow ||
+        d->top + d->new_h > p.oh)
+        YRE_FAIL(YRE_EINVAL, "letterbox: geometry does not fit %dx%d", p.oh, p.ow);
     if (d->out_mode != YRE_LB_F32_CHW && d->out_mode != YRE_LB_U8_HWC) YRE_FAIL(YRE_EINVAL, "letterbox: bad out_mode");
-    p.src = d->src; p.h = d->h; p.w = d->w; p.pitch = d->row_pitch; p.S = d->new_shape;
+    p.src = d->src; p.h = d->h; p.w = d->w; p.pitch = d->row_pitch;
     p.nw = d->new_w; p.nh = d->new_h; p.top = d->top; p.left = d->left;
     p.c0 = d->color[0]; p.c1 = d->color[1]; p.c2 = d->color[2];
     p.mode = (d->w == d->new_w && d->h == d->new_h) ? 1 : ((d->w == 2 * d->new_w && d->h == 2 * d->new_h) ? 2 : 0);
@@ -134,21 +149,22 @@ static int lb_fill(const yre_letterbox_desc* d, LbParams& p) {
     return YRE_OK;
 }
 
-// n images with the same new_shape and out_mode, up to LB_BATCH per launch (grid.z = image)
+// n images with the same destination extent and out_mode, up to LB_BATCH per launch (grid.z = image)
 extern "C" int yre_letterbox_u8_batch(const yre_letterbox_desc* d, int32_t n, yre_stream_t s) {
     if (n < 0 || (n > 0 && !d)) YRE_FAIL(YRE_EINVAL, "letterbox: bad batch");
+    int oh = 0, ow = 0;
+    if (n > 0) lb_extent(d, oh, ow);
     for (int i0 = 0; i0 < n; i0 += LB_BATCH) {
         const int m = n - i0 < LB_BATCH ? n - i0 : LB_BATCH;
         LbBatch b;
         for (int i = 0; i < m; ++i) {
-            if (d[i0 + i].new_shape != d[0].new_shape || d[i0 + i].out_mode != d[0].out_mode)
-                YRE_FAIL(YRE_EINVAL, "letterbox: a batch must share new_shape and out_mode");
             const int rc = lb_fill(&d[i0 + i], b.p[i]);
             if (rc) return rc;
+            if (b.p[i].oh != oh || b.p[i].ow != ow || d[i0 + i].out_mode != d[0].out_mode)
+                YRE_FAIL(YRE_EINVAL, "letterbox: a batch must share the destination extent and out_mode");
         }
         for (int i = m; i < LB_BATCH; ++i) b.p[i] = b.p[0];
-        const int S = d[0].new_shape;
-        dim3 grid(yre_cdiv(S, 32), yre_cdiv(S, 8), (unsigned)m);
+        dim3 grid(yre_cdiv(ow, 32), yre_cdiv(oh, 8), (unsigned)m);
         if (d[0].out_mode == YRE_LB_U8_HWC) letterbox_kernel<1><<<grid, 256, 0, (cudaStream_t)s>>>(b);
         else letterbox_kernel<0><<<grid, 256, 0, (cudaStream_t)s>>>(b);
         YRE_LAUNCH_CHECK("letterbox");

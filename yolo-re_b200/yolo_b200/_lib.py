@@ -49,7 +49,8 @@ class NmsDesc(C.Structure):
 class LetterboxDesc(C.Structure):
     _fields_ = [("src", C.c_void_p), ("h", C.c_int32), ("w", C.c_int32), ("row_pitch", C.c_int64),
                 ("new_shape", C.c_int32), ("new_w", C.c_int32), ("new_h", C.c_int32), ("top", C.c_int32),
-                ("left", C.c_int32), ("color", C.c_uint8 * 4), ("out_mode", C.c_int32), ("dst", C.c_void_p)]
+                ("left", C.c_int32), ("color", C.c_uint8 * 4), ("out_mode", C.c_int32), ("dst", C.c_void_p),
+                ("out_h", C.c_int32), ("out_w", C.c_int32)]
 
 
 LB_F32_CHW, LB_U8_HWC = 0, 1
@@ -78,6 +79,8 @@ SYMBOLS = {
     "yre_nms_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int32]),
     "yre_nms_batched": (C.c_int, [C.POINTER(NmsDesc), C.c_void_p]),
     "yre_nms_filter_only": (C.c_int, [C.POINTER(NmsDesc), C.c_void_p]),
+    "yre_letterbox_geometry_rect": (C.c_int, [C.POINTER(LetterboxDesc), C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_double),
+                                    C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "yre_letterbox_geometry": (C.c_int, [C.POINTER(LetterboxDesc), C.POINTER(C.c_double), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "yre_letterbox_u8": (C.c_int, [C.POINTER(LetterboxDesc), C.c_void_p]),
     "yre_letterbox_u8_batch": (C.c_int, [C.POINTER(LetterboxDesc), C.c_int32, C.c_void_p]),
