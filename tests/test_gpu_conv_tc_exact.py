@@ -52,6 +52,7 @@ import torch.nn.functional as F
 pytestmark = pytest.mark.gpu
 
 from tests.conv_tc_cases import CASES, NUM_SMS, Case, desc, describe, row_key
+from tests.teacher_force import check_bound, conv_fp32_bound
 
 from yolo_b200 import _lib as L
 
@@ -151,23 +152,6 @@ def check_window(c: Case, y: torch.Tensor, what: str) -> torch.Tensor:
     return win
 
 
-def check_bound(got: torch.Tensor, ref, pre, A, silu: bool, what: str, tc: bool = True) -> float:
-    """asserts the per-element bound; returns the worst log2(err / A)"""
-    err = (got.double() - ref).abs()
-    if tc:
-        bound = 2.0 ** -14 * A + (2.0 ** -11 if silu else 0.0) * pre.abs() + 2.0 ** -22 * (pre.abs() + ref.abs())
-    else:
-        bound = 2.0 ** -19 * A + 2.0 ** -17 * ref.abs()
-    over = err > bound
-    if bool(over.any()):
-        i = tuple(int(v) for v in torch.unravel_index((err / bound).argmax(), err.shape))
-        raise AssertionError(f"{what}: {int(over.sum())} elements over the bound; worst at (b, y, x, c) = {i}: got "
-                             f"{got[i].item():.9g}, ref {ref[i].item():.9g}, pre {pre[i].item():.6g}, A {A[i].item():.6g}, "
-                             f"err / A = 2^{math.log2(err[i].item() / A[i].item()):.2f}")
-    ratio = (err / A.clamp_min(1e-300)).max().item()
-    return math.log2(ratio) if ratio > 0 else -math.inf
-
-
 def device_row(d: L.ConvDesc) -> int:
     return row_table().index(row_key(describe(d, torch.cuda.get_device_properties(0).multi_processor_count)))
 
@@ -258,7 +242,7 @@ def test_tcgen05_conv_waits_for_its_producer(case, f32, row):
         check_bound(got, ref, pre, A, c.silu, f"{c.name} after a producer")
     else:   # a bf16 output: the fp32 bound plus half an ulp of bf16
         err = (got.double() - ref).abs()
-        bound = 2.0 ** -14 * A + (2.0 ** -11 if c.silu else 0.0) * pre.abs() + 2.0 ** -22 * (pre.abs() + ref.abs()) + 2.0 ** -8 * ref.abs()
+        bound = conv_fp32_bound(ref, pre, A, c.silu) + 2.0 ** -8 * ref.abs()
         assert bool((err <= bound).all()), f"{c.name} after a producer: {int((err > bound).sum())} elements over the bound"
 
 

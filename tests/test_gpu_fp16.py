@@ -15,11 +15,12 @@ within 0.3 of the bf16 file's figures:
     row  7: -21.05   row  8: -21.17   row  9: -21.05   row 10: -19.78   row 11: -19.09   row 12: -19.58   row 13: -19.49
     row 14: -20.76   row 16: -20.70   row 17: -20.87   row 18: -21.13   row 19: -20.52   row 20: -20.38
 
-Full size, config 2, teacher-forced, measured on the same B200 as a fraction of max|ref| (gate = the bf16 gate / 8): conv
-4.4e-4 (1.25e-3), stem 1.24e-3 (2.5e-3), fp32-output convs 8.3e-7 (1.25e-4), ADown 7.0e-4 (1.25e-3), SPP / upsample exact.
-No stage needed more than the scaled bf16 tolerance.  Detections against tests/golden/gelan-c_640_dets.npz: the fp16 head
-teacher-forced with the fp32 engine's neck features recalls 0.999 of the reference's detections at precision 0.999; end
-to end fp16 recalls 0.681 at precision 0.682, where bf16 recalls 0.123 at precision 0.123 in the same test.
+Full size, config 2: every launch is checked per element by tests/teacher_force.py, with the bounds derived there for
+u = 2^-11, and one back-to-back run must reproduce every buffer bit for bit.
+
+Detections against tests/golden/gelan-c_640_dets.npz: the fp16 head teacher-forced with the fp32 engine's neck features
+recalls 0.999 of the reference's detections at precision 0.999; end to end fp16 recalls 0.681 at precision 0.682, where
+bf16 recalls 0.123 at precision 0.123 in the same test.
 
 Stem and ADown, derived from fp16 rounding (u = 2^-11, the unit roundoff of fp16):
   * stem (mma.sync on fp16 operands, fp32 accumulation, tanh.approx SiLU, one rounding of the output):
@@ -29,6 +30,7 @@ Stem and ADown, derived from fp16 rounding (u = 2^-11, the unit roundoff of fp16
 SPP, upsample, the NCHW <-> view conversions and CBFuse (fp32 sums in the kernel's order, one rounding) are exact."""
 import ctypes as C
 import math
+import time
 from collections import defaultdict
 
 import numpy as np
@@ -38,10 +40,10 @@ import torch.nn.functional as F
 
 from bench_data import make_inputs
 from oracle import gelan_ref as G
-from tests import cpu_plan_exec as X
+from tests import teacher_force as TF
 from tests.conftest import ROOT
 from tests.conv_tc_cases import CASES, NUM_SMS, Case, desc, describe, row_key
-from tests.test_gpu_conv_tc_exact import CHAINED, Operands, check_bound, nan_buffer, ptrs, row_table, stream
+from tests.test_gpu_conv_tc_exact import CHAINED, Operands, nan_buffer, ptrs, row_table, stream
 from tests.test_gpu_round2 import BF16_HEAD_AGREEMENT, match_fraction
 
 pytestmark = pytest.mark.gpu
@@ -126,7 +128,7 @@ def test_fp16_tcgen05_conv_matches_fp64(case):
         i = tuple((~same).nonzero()[0].tolist())
         raise AssertionError(f"{c.name}: fp16 output differs from the rounded fp32 output in {int((~same).sum())} elements, "
                              f"first at {i}: {yh[i].item()} vs {y32[i].item():.9g}")
-    worst = check_bound(y32, ref, pre, A, c.silu, c.name)
+    worst = TF.check_bound(y32, ref, pre, A, c.silu, c.name)
     WORST[row32] = max(WORST[row32], worst)
     WORST[rowh] = max(WORST[rowh], worst)
 
@@ -183,7 +185,7 @@ def test_fp16_ffma_conv_matches_fp64(case):
         L.check(L.lib().yre_conv(C.byref(d), stream()), f"yre_conv ffma {c.name}")
         torch.cuda.synchronize()
         outs.append(check_window(c, y, f"{c.name} ffma"))
-    check_bound(outs[0], ref, pre, A, c.silu, f"{c.name} ffma", tc=False)
+    TF.check_bound(outs[0], ref, pre, A, c.silu, f"{c.name} ffma", tc=False)
     assert bool(same_bits(outs[1], outs[0].to(torch.float16)).all()), f"{c.name} ffma: fp16 output != rounded fp32 output"
 
 
@@ -308,11 +310,6 @@ def test_fp16_spp_upsample_cbfuse_conversions_are_exact(Hs, Cn):
 
 
 # ---- full size -------------------------------------------------------------------------------------------------------------
-# tests/test_gpu_fullsize.py's bf16 tolerances divided by 8, the ratio of the unit roundoffs of bf16 (2^-8) and fp16 (2^-11)
-TOL_CONV = 1.0e-2 / 8
-TOL_STEM = 2.0e-2 / 8
-TOL_CONV_F32 = 1.0e-3 / 8
-TOL_POOL = 1.0e-2 / 8
 CONFIGS = {2: ("gelan-c", 640, 64), 5: ("gelan-c", 1280, 16), 4: ("yolov9-c", 640, 16)}
 
 
@@ -323,82 +320,20 @@ def _model(name, request, prec="fp16"):
     return m.to(DEV).eval().set_precision(prec)
 
 
-def _rel(got, ref):
-    return (got - ref).abs().max().item() / max(1e-6, ref.abs().max().item())
-
-
 def test_fp16_every_launch_of_the_config2_plan_teacher_forced(request):
     name, img, Bn = CONFIGS[2]
     model = _model(name, request)
     x = make_inputs(Bn, img, seed=7).to(DEV)
-    old = torch.backends.cudnn.allow_tf32
-    torch.backends.cudnn.allow_tf32 = False
-    try:
-        with torch.cuda.device(x.device):
-            p = E.compile_model(model, x)
-            names = [n for n, _ in p.op_table()]
-            assert "conv_ffma" not in names
-            worst = {}
-            for i, (kind, a) in enumerate(p.trace):
-                if kind == "conv":
-                    xin = X.nchw(X.read(a["x"]))
-                    if a.get("xu") is not None:
-                        xin = torch.cat((F.interpolate(X.nchw(X.read(a["xu"])), scale_factor=2.0, mode="nearest"), xin), 1)
-                    res = X.nchw(X.read(a["res"])) if a["res"] is not None else None
-                    p.run_op(i)
-                    ref = F.conv2d(xin, a["w"].float().permute(0, 3, 1, 2), a["b"].float(), a["stride"], a["k"] // 2)
-                    del xin
-                    if a["silu"]:
-                        ref = F.silu(ref)
-                    if res is not None:
-                        ref = ref + res
-                    f32 = a["y"].dtype == L.F32
-                    err, tol, key = _rel(X.nchw(X.read(a["y"])), ref), (TOL_CONV_F32 if f32 else TOL_CONV), ("conv f32out" if f32 else "conv")
-                elif kind == "stem":
-                    p.run_op(i)
-                    ref = F.conv2d(a["x"].float(), a["w"].float().permute(0, 3, 1, 2), a["b"].float(), a["stride"], 1)
-                    if a["silu"]:
-                        ref = F.silu(ref)
-                    err, tol, key = _rel(X.nchw(X.read(a["y"])), ref), TOL_STEM, "stem"
-                elif kind == "adown":
-                    xin = X.nchw(X.read(a["x"]))
-                    p.run_op(i)
-                    avg = F.avg_pool2d(xin, 2, 1, 0)
-                    half = xin.shape[1] // 2
-                    e1 = _rel(X.nchw(X.read(a["lo"])), avg[:, :half])
-                    e2 = _rel(X.nchw(X.read(a["hi"])), F.max_pool2d(avg[:, half:], 3, 2, 1))
-                    err, tol, key = max(e1, e2), TOL_POOL, "adown"
-                elif kind == "spp":
-                    xin = X.nchw(X.read(a["x"]))
-                    p.run_op(i)
-                    for k_, win in (("y5", 5), ("y9", 9), ("y13", 13)):
-                        assert torch.equal(X.nchw(X.read(a[k_])), F.max_pool2d(xin, win, 1, win // 2)), f"spp window {win}"
-                    err, tol, key = 0.0, 0.0, "spp"
-                elif kind == "upsample":
-                    xin = X.nchw(X.read(a["x"]))
-                    p.run_op(i)
-                    assert torch.equal(X.nchw(X.read(a["y"])), F.interpolate(xin, scale_factor=2.0, mode="nearest"))
-                    err, tol, key = 0.0, 0.0, "upsample"
-                elif kind == "cbfuse":
-                    tgt = X.nchw(X.read(a["target"]))
-                    acc = torch.zeros_like(tgt)
-                    for s_ in a["srcs"]:
-                        acc = acc + F.interpolate(X.nchw(X.read(s_)), size=tgt.shape[2:], mode="nearest")
-                    p.run_op(i)
-                    err, tol, key = _rel(X.nchw(X.read(a["y"])), acc + tgt), TOL_POOL, "cbfuse"
-                elif kind == "decode":
-                    p.run_op(i)
-                    assert bool(torch.isfinite(a["y"]).all())
-                    err, tol, key = 0.0, 0.0, "decode"
-                else:
-                    raise AssertionError(f"unexpected op {kind}")
-                torch.cuda.synchronize()
-                assert np.isfinite(err) and err <= tol, f"op {i} ({names[i]}: {p.op_descriptions()[i]}): error {err:.3e} > {tol:.1e}"
-                worst[key] = max(worst.get(key, 0.0), err)
-            print(f"fp16 config 2: {len(names)} launches checked, worst error per kernel family (fraction of max|ref|): "
-                  + ", ".join(f"{k} {v:.2e}" for k, v in worst.items()))
-    finally:
-        torch.backends.cudnn.allow_tf32 = old
+    with torch.cuda.device(x.device):
+        p = E.compile_model(model, x)
+        names = [n for n, _ in p.op_table()]
+        assert "conv_ffma" not in names
+        t0 = time.perf_counter()
+        worst = TF.teacher_force(p, label="fp16 config 2 ")
+        t1 = time.perf_counter()
+        TF.run_reproduces(p)
+        print(f"fp16 config 2: {len(names)} launches checked per element in {t1 - t0:.1f} s, worst err / bound per kernel "
+              f"family: {TF.report(worst)}; the back-to-back run reproduces every buffer")
 
 
 @pytest.mark.parametrize("config", [2, 4, 5])

@@ -1,15 +1,16 @@
 """Rectangular ("rect") inference on the GPU: the letterbox kernel writing an out_h x out_w destination, the whole path at
 non-square sizes against the oracle, every launch of non-square full-size plans teacher-forced, and the path identities
 (uint8 frames, fused box scaling, CUDA graphs, batch order) off the diagonal."""
+import time
+
 import numpy as np
 import pytest
 import torch
-import torch.nn.functional as F
 
 from oracle import gelan_ref as G
 from oracle import nms_ref as N
 from oracle import preproc_ref as P
-from tests import cpu_plan_exec as X
+from tests import teacher_force as TF
 from tests.conftest import ROOT
 from tests.test_cpu_conv_tc_select import tc_variant
 from tests.test_cpu_rect import letterbox_rect, rect_geometry
@@ -18,7 +19,6 @@ pytestmark = pytest.mark.gpu
 
 import yolo_b200
 from yolo_b200 import YOLO, letterbox, nms_raw, preprocess, scale_boxes, scale_rows
-from yolo_b200 import _lib as L
 from yolo_b200 import engine as E
 
 DEV = "cuda"
@@ -118,15 +118,7 @@ def test_fp32_end_to_end_vs_oracle_and_nms_non_square(gelan_c, H, W, batch):
         assert np.array_equal(a.cpu().numpy(), b)
 
 
-# ---- every launch of non-square full-size plans, teacher-forced ------------------------------------------------------------
-# tests/test_gpu_fullsize.py's per-kernel tolerances (fraction of max|ref|); fp16 divides them by 8 as tests/test_gpu_fp16.py
-TOL = {"conv": 1.0e-2, "stem": 2.0e-2, "conv f32out": 1.0e-3, "adown": 1.0e-2, "cbfuse": 1.0e-2, "decode": 1.0e-4}
-
-
-def _rel(got, ref):
-    return (got - ref).abs().max().item() / max(1e-6, ref.abs().max().item())
-
-
+# ---- every launch of non-square full-size plans, teacher-forced per element (tests/teacher_force.py) ------------------------
 def _rect_inputs(Bn, H, W, seed):
     """eight distinct multi-octave images repeated with a brightness ramp (bench_data.make_inputs, non-square)"""
     base = G.fractal(min(Bn, 8), H, torch.Generator().manual_seed(seed), w=W)
@@ -140,91 +132,20 @@ def test_every_launch_of_a_non_square_plan_teacher_forced(name, Bn, H, W, prec, 
     nodes, nc, sd = request.getfixturevalue("gelan_c" if name == "gelan-c" else "yolov9_c")
     model = _model(name, sd, prec)
     x = _rect_inputs(Bn, H, W, seed=7).to(DEV)
-    div = 8.0 if prec == "fp16" else 1.0
     sms = torch.cuda.get_device_properties(x.device).multi_processor_count
-    old = torch.backends.cudnn.allow_tf32
-    torch.backends.cudnn.allow_tf32 = False
-    try:
-        with torch.cuda.device(x.device):
-            p = E.compile_model(model, x)
-            names, variants = [n for n, _ in p.op_table()], p.op_variants()
-            assert "conv_ffma" not in names
-            worst = {}
-            for i, (kind, a) in enumerate(p.trace):
-                if kind == "conv":
-                    assert tc_variant(a, sms) == variants[i], (i, p.op_descriptions()[i])
-                    xin = X.nchw(X.read(a["x"]))
-                    if a.get("xu") is not None:
-                        xin = torch.cat((F.interpolate(X.nchw(X.read(a["xu"])), scale_factor=2.0, mode="nearest"), xin), 1)
-                    res = X.nchw(X.read(a["res"])) if a["res"] is not None else None
-                    p.run_op(i)
-                    ref = F.conv2d(xin, a["w"].float().permute(0, 3, 1, 2), a["b"].float(), a["stride"], a["k"] // 2)
-                    del xin
-                    if a["silu"]:
-                        ref = F.silu(ref)
-                    if res is not None:
-                        ref = ref + res
-                    key = "conv f32out" if a["y"].dtype == L.F32 else "conv"
-                    err = _rel(X.nchw(X.read(a["y"])), ref)
-                elif kind == "stem":
-                    p.run_op(i)
-                    ref = F.conv2d(a["x"].float(), a["w"].float().permute(0, 3, 1, 2), a["b"].float(), a["stride"], 1)
-                    if a["silu"]:
-                        ref = F.silu(ref)
-                    err, key = _rel(X.nchw(X.read(a["y"])), ref), "stem"
-                elif kind == "adown":
-                    xin = X.nchw(X.read(a["x"]))
-                    p.run_op(i)
-                    avg = F.avg_pool2d(xin, 2, 1, 0)
-                    half = xin.shape[1] // 2
-                    e1 = _rel(X.nchw(X.read(a["lo"])), avg[:, :half])
-                    e2 = _rel(X.nchw(X.read(a["hi"])), F.max_pool2d(avg[:, half:], 3, 2, 1))
-                    err, key = max(e1, e2), "adown"
-                elif kind == "spp":
-                    xin = X.nchw(X.read(a["x"]))
-                    p.run_op(i)
-                    for k_, win in (("y5", 5), ("y9", 9), ("y13", 13)):
-                        assert torch.equal(X.nchw(X.read(a[k_])), F.max_pool2d(xin, win, 1, win // 2)), f"spp window {win}"
-                    err, key = 0.0, "spp"
-                elif kind == "upsample":
-                    xin = X.nchw(X.read(a["x"]))
-                    p.run_op(i)
-                    assert torch.equal(X.nchw(X.read(a["y"])), F.interpolate(xin, scale_factor=2.0, mode="nearest"))
-                    err, key = 0.0, "upsample"
-                elif kind == "cbfuse":
-                    tgt = X.nchw(X.read(a["target"]))
-                    acc = torch.zeros_like(tgt)
-                    for s_ in a["srcs"]:
-                        acc = acc + F.interpolate(X.nchw(X.read(s_)), size=tgt.shape[2:], mode="nearest")
-                    p.run_op(i)
-                    err, key = _rel(X.nchw(X.read(a["y"])), acc + tgt), "cbfuse"
-                elif kind == "decode":
-                    p.run_op(i)
-                    outs = []
-                    for r, st in zip(a["raws"], a["strides"]):
-                        z = X.read(r)
-                        b_, Hl, Wl, _ = z.shape
-                        e = (z[..., :64].reshape(b_, Hl, Wl, 4, 16).softmax(-1) * torch.tensor(a["dfl_w"], device=z.device)).sum(-1)
-                        gy, gx = torch.meshgrid(torch.arange(Hl, device=z.device) + 0.5, torch.arange(Wl, device=z.device) + 0.5, indexing="ij")
-                        x1, y1, x2, y2 = gx - e[..., 0], gy - e[..., 1], gx + e[..., 2], gy + e[..., 3]
-                        box = torch.stack(((x1 + x2) / 2, (y1 + y2) / 2, x2 - x1, y2 - y1), -1) * st
-                        outs.append(torch.cat((box, z[..., 64:].sigmoid()), -1).reshape(b_, Hl * Wl, -1))
-                    ref = torch.cat(outs, 1)
-                    got = a["y"]
-                    eb = (got[..., :4] - ref[..., :4]).abs().max().item() / max(H, W)      # boxes: fraction of the image size
-                    es = (got[..., 4:] - ref[..., 4:]).abs().max().item()
-                    err, key = max(eb, es), "decode"
-                else:
-                    raise AssertionError(f"unexpected op {kind}")
-                torch.cuda.synchronize()
-                tol = TOL.get(key, 0.0) / (div if key != "decode" else 1.0)
-                assert np.isfinite(err) and err <= tol, f"{name} {prec} {Bn}x{H}x{W} op {i} ({names[i]}: {p.op_descriptions()[i]} " \
-                                                        f"{variants[i]}): error {err:.3e} > {tol:.1e}"
-                worst[key] = max(worst.get(key, 0.0), err)
-            print(f"{name} {prec} {Bn}x{H}x{W}: {len(names)} launches checked, worst error per kernel family (fraction of "
-                  "max|ref|): " + ", ".join(f"{k} {v:.2e}" for k, v in worst.items()))
-    finally:
-        torch.backends.cudnn.allow_tf32 = old
+    with torch.cuda.device(x.device):
+        p = E.compile_model(model, x)
+        names, variants = [n for n, _ in p.op_table()], p.op_variants()
+        assert "conv_ffma" not in names
+        for i, (kind, a) in enumerate(p.trace):
+            if kind == "conv":
+                assert tc_variant(a, sms) == variants[i], (i, p.op_descriptions()[i])
+        t0 = time.perf_counter()
+        worst = TF.teacher_force(p, label=f"{name} {prec} {Bn}x{H}x{W} ")
+        t1 = time.perf_counter()
+        TF.run_reproduces(p)
+        print(f"{name} {prec} {Bn}x{H}x{W}: {len(names)} launches checked per element in {t1 - t0:.1f} s, worst err / bound "
+              f"per kernel family: {TF.report(worst)}; the back-to-back run reproduces every buffer")
 
 
 # ---- path identities --------------------------------------------------------------------------------------------------------
