@@ -20,6 +20,8 @@ from __future__ import annotations
 
 import ctypes as C
 from contextlib import contextmanager
+from functools import cache
+from typing import NamedTuple
 
 import torch
 import torch.nn as nn
@@ -58,6 +60,20 @@ def precision(p: str):
         yield
     finally:
         _DEFAULT_PRECISION = old
+
+
+def _conv_out(n: int, k: int, stride: int) -> int:
+    """Output extent of a k x k conv with padding k // 2 over an extent of n."""
+    return (n + 2 * (k // 2) - k) // stride + 1
+
+
+class Fold(NamedTuple):
+    """A conv folded to one dense kernel: w[Cout,Cin,k,k] and b[Cout] in fp64."""
+    w: torch.Tensor
+    b: torch.Tensor
+    k: int
+    stride: int
+    silu: bool
 
 
 class V:
@@ -166,16 +182,15 @@ class Plan:
             d[g * cog:(g + 1) * cog, g * cig:(g + 1) * cig] = w[g * cog:(g + 1) * cog]
         return d
 
-    def fold(self, m) -> tuple[torch.Tensor, torch.Tensor, int, int, bool]:
-        """(w[Cout,Cin,k,k] fp64 dense, b[Cout] fp64, k, stride, silu) of a blocks.Conv / RepConv / nn.Conv2d.
+    def fold(self, m) -> Fold:
+        """The dense fp64 fold of a blocks.Conv / RepConv / nn.Conv2d.
         The folding arithmetic runs on the HOST in fp64 (the parameters are copied down once per compile): no torch
         element-wise kernels are launched on the device, only the folded weights are uploaded."""
         if isinstance(m, B.RepConv):
-            w3, b3, _, s, _ = self.fold(m.conv1)
-            w1, b1, _, _, _ = self.fold(m.conv2)
-            w = w3.clone()
-            w[:, :, 1:2, 1:2] += w1
-            return w, b3 + b1, 3, s, isinstance(m.act, nn.SiLU)
+            f3, f1 = self.fold(m.conv1), self.fold(m.conv2)
+            w = f3.w.clone()
+            w[:, :, 1:2, 1:2] += f1.w
+            return Fold(w, f3.b + f1.b, 3, f3.stride, isinstance(m.act, nn.SiLU))
         if isinstance(m, B.Conv):
             cv, bn = m.conv, m.bn
             k = cv.kernel_size[0]
@@ -187,12 +202,12 @@ class Plan:
             b = bn.bias.detach().cpu().double() - bn.running_mean.detach().cpu().double() * scale
             if not isinstance(m.act, (nn.SiLU, nn.Identity)):
                 raise L.YreError(f"unsupported activation {m.act}")
-            return w, b, k, cv.stride[0], isinstance(m.act, nn.SiLU)
+            return Fold(w, b, k, cv.stride[0], isinstance(m.act, nn.SiLU))
         if isinstance(m, nn.Conv2d):
             k = m.kernel_size[0]
             w = self._dense(m.weight.detach().cpu().double(), m.groups)
             b = m.bias.detach().cpu().double() if m.bias is not None else torch.zeros(w.shape[0], dtype=torch.float64, device=w.device)
-            return w, b, k, m.stride[0], False
+            return Fold(w, b, k, m.stride[0], False)
         raise L.YreError(f"cannot fold {type(m).__name__}")
 
     # -- op emission -------------------------------------------------------------------------------------
@@ -209,8 +224,7 @@ class Plan:
         if isinstance(x, VCat):
             assert k == 1 and stride == 1, "a virtual upsample+concat input needs a 1x1 stride-1 consumer"
             xu, x = x.up, x.rest
-        Ho = (x.H + 2 * (k // 2) - k) // stride + 1
-        Wo = (x.W + 2 * (k // 2) - k) // stride + 1
+        Ho, Wo = _conv_out(x.H, k, stride), _conv_out(x.W, k, stride)
         if out is None:
             out = self.alloc(Ho, Wo, cout, dtype=out_dtype)
         assert (out.H, out.W, out.C) == (Ho, Wo, cout), ((out.H, out.W, out.C), (Ho, Wo, cout))
@@ -229,8 +243,8 @@ class Plan:
     def conv_merged(self, ms, x: V, out: V | None = None) -> V:
         """Sibling convs on one input -> one GEMM with concatenated output channels."""
         fs = [self.fold(m) for m in ms]
-        assert len({(f[2], f[3], f[4]) for f in fs}) == 1
-        return self.conv(x, torch.cat([f[0] for f in fs]), torch.cat([f[1] for f in fs]), fs[0][2], fs[0][3], fs[0][4], out,
+        assert len({(f.k, f.stride, f.silu) for f in fs}) == 1
+        return self.conv(x, torch.cat([f.w for f in fs]), torch.cat([f.b for f in fs]), fs[0].k, fs[0].stride, fs[0].silu, out,
                          name=" + ".join(self.name_of(m) for m in ms))
 
     def stem(self, m: B.Conv, x: torch.Tensor, phase4: bool) -> V:
@@ -244,7 +258,7 @@ class Plan:
             Bn, H, W, Cin = x.shape
         else:
             Bn, Cin, H, W = x.shape
-        Ho, Wo = (H + 2 - 3) // s + 1, (W + 2 - 3) // s + 1
+        Ho, Wo = _conv_out(H, 3, s), _conv_out(W, 3, s)
         out = self.alloc(Ho, Wo, w.shape[0], layout=L.PHASE4 if phase4 else L.NHWC)
         wp = self.dev(w.permute(0, 2, 3, 1), torch.float32)
         bp = self.dev(b, torch.float32)
@@ -285,7 +299,7 @@ class Plan:
     def adown(self, m: B.ADown, x: V, out: V | None) -> V:
         half = x.C // 2
         co = m.conv_stride.conv.out_channels
-        Ho, Wo = (x.H - 1 + 2 - 3) // 2 + 1, (x.W - 1 + 2 - 3) // 2 + 1
+        Ho, Wo = _conv_out(x.H - 1, 3, 2), _conv_out(x.W - 1, 3, 2)      # 2x2 average pool, stride 1, then 3x3 / 2
         lo = self.alloc(x.H - 1, x.W - 1, half, layout=L.PHASE4)
         hi = self.alloc(Ho, Wo, half)
         L.check(self.lib.yre_plan_add_adown_prepool(self.h, C.byref(x.c()), C.byref(lo.c()), C.byref(hi.c())), "plan_add_adown")
@@ -365,11 +379,11 @@ class Plan:
             hb = self.conv_m(box[i][1], hb_in)
             self.conv_m(box[i][2], hb, out=raw.sl(0, 4 * REG_MAX))
             hc = self.conv_m(cls[i][1], hc_in)
-            wc, bc, kc, sc, silu_c = self.fold(cls[i][2])
+            fc = self.fold(cls[i][2])
             if ncp != nc:
-                wc = torch.cat([wc, wc.new_zeros((ncp - nc,) + tuple(wc.shape[1:]))])
-                bc = torch.cat([bc, bc.new_zeros(ncp - nc)])
-            self.conv(hc, wc, bc, kc, sc, silu_c, out=raw_full.sl(4 * REG_MAX, ncp), name=self.name_of(cls[i][2]))
+                fc = fc._replace(w=torch.cat([fc.w, fc.w.new_zeros((ncp - nc,) + tuple(fc.w.shape[1:]))]),
+                                 b=torch.cat([fc.b, fc.b.new_zeros(ncp - nc)]))
+            self.conv(hc, fc.w, fc.b, fc.k, fc.stride, fc.silu, out=raw_full.sl(4 * REG_MAX, ncp), name=self.name_of(cls[i][2]))
             raws.append(raw)
         A = sum(r.H * r.W for r in raws)
         y = torch.empty((self.batch, A, 4 + nc), dtype=torch.float32, device=self.device)
@@ -389,11 +403,11 @@ class Plan:
 
     def detect(self, m, feats: list[V], main_only: bool = False):
         strides = m.stride.tolist()
-        if main_only:                      # feats = the main half only; result looks like a single head's
-            y, raws = self.towers(m.main_box_convs, m.main_cls_convs, m.dfl2, feats, strides, m.num_classes)
-            return ("single", y, raws)
         if isinstance(m, DetectDFL):
             y, raws = self.towers(m.box_convs, m.cls_convs, m.dfl, feats, strides, m.num_classes)
+            return ("single", y, raws)
+        if main_only:                      # feats = the main half only; result looks like a single head's
+            y, raws = self.towers(m.main_box_convs, m.main_cls_convs, m.dfl2, feats, strides, m.num_classes)
             return ("single", y, raws)
         Ln = m.num_levels
         ya, ra = self.towers(m.aux_box_convs, m.aux_cls_convs, m.dfl, feats[:Ln], strides, m.num_classes)
@@ -408,11 +422,7 @@ class Plan:
             u = self.conv_m(m.conv1, x)
             return self.conv_m(m.conv2, u, out=out, res=x if m.add else None)
         if isinstance(m, B.RepNCSP):
-            v = self.csp(m, x)
-            if out is not None:
-                self.copy(v, out)
-                return out
-            return v
+            return self.csp(m, x)
         if isinstance(m, B.RepNCSPELAN4):
             return self.elan(m, x, out)
         if isinstance(m, B.ADown):
@@ -491,22 +501,93 @@ class Plan:
 
 
 # ------------------------------------------------------------------------------------------------------------
-def _out_channels(layer, cin: list[int]) -> int:
-    if isinstance(layer, B.Conv):
-        return layer.conv.out_channels
-    if isinstance(layer, (B.RepNCSPELAN4, B.SPPELAN)):
-        return layer.conv_out.conv.out_channels
-    if isinstance(layer, B.ADown):
-        return 2 * layer.conv_stride.conv.out_channels
-    if isinstance(layer, B.Concat):
-        return sum(cin)
-    if isinstance(layer, B.CBLinear):
-        return layer.out_channels_list[-1]
-    if isinstance(layer, B.CBFuse):
-        return cin[-1]
-    if isinstance(layer, (DetectDFL, DualDetectDFL)):
-        return 0
-    return cin[0]
+def _out_shape(m, ins: list[tuple[int, int, int]]) -> tuple[int, int, int]:
+    """(H, W, C) of a layer's output from the (H, W, C) of its inputs; a CBLinear's C is that of its last chunk."""
+    H, W, Cn = ins[-1] if isinstance(m, B.CBFuse) else ins[0]
+    if isinstance(m, B.Conv):
+        k, s = m.conv.kernel_size[0], m.conv.stride[0]
+        return _conv_out(H, k, s), _conv_out(W, k, s), m.conv.out_channels
+    if isinstance(m, B.ADown):
+        return _conv_out(H - 1, 3, 2), _conv_out(W - 1, 3, 2), 2 * m.conv_stride.conv.out_channels
+    if isinstance(m, B.Upsample):
+        return 2 * H, 2 * W, Cn
+    if isinstance(m, (B.RepNCSPELAN4, B.SPPELAN)):
+        return H, W, m.conv_out.conv.out_channels
+    if isinstance(m, B.Concat):
+        return H, W, sum(c for _, _, c in ins)
+    if isinstance(m, B.CBLinear):
+        return H, W, m.out_channels_list[-1]
+    return H, W, Cn
+
+
+class Wire(NamedTuple):
+    """How one layer sits in the plan, decided before anything is allocated."""
+    srcs: list[str]                  # layers it reads ("input": the image), past any Silence; a main_only head: its main half
+    H: int                           # output extent and channels
+    W: int
+    C: int
+    dest: tuple[str, int] | None     # (concat, channel offset) it writes its output into
+    lazy: bool                       # an Upsample its concat's consumers read in place (VCat): it emits nothing
+    needed: bool                     # False: main_only prunes it
+    phase4: bool                     # a stem that writes parity planes for the stride-2 3x3 conv reading it
+
+
+def wire_model(model, H: int, W: int, Cin: int) -> dict[str, Wire]:
+    """The wiring of model.layers / model.connections for an H x W x Cin image, by layer name; it touches no tensor."""
+    layers, names, conn = model.layers, list(model.layers.keys()), model.connections
+    srcs = {n: ([conn[n]] if isinstance(conn[n], str) else list(conn[n])) for n in names}
+    consumers: dict[str, list[str]] = {n: [] for n in ["input", *names]}
+    shape = {"input": (H, W, Cin)}
+    for n in names:
+        for s in srcs[n]:
+            consumers[s].append(n)
+        shape[n] = _out_shape(layers[n], [shape[s] for s in srcs[n]])
+    # Upsample -> Concat([up, skip]) -> RepNCSPELAN4: the ELAN's first op is a 1x1 conv over the whole concat, which can
+    # read the half-resolution tensor directly (VCat / yre_conv_desc.xu).  Such an Upsample emits no kernel and its half
+    # of the concat buffer is never allocated.
+    lazy: dict[str, str] = {}
+    if getattr(model, "fuse_upsample", True):
+        for n in names:
+            if not (isinstance(layers[n], B.Concat) and len(srcs[n]) >= 2):
+                continue
+            u = srcs[n][0]
+            if (u != "input" and isinstance(layers[u], B.Upsample) and consumers[u] == [n] and u not in srcs[n][1:]
+                    and consumers[n] and all(isinstance(layers[c], B.RepNCSPELAN4) and srcs[c] == [n] for c in consumers[n])
+                    and shape[u][2] % 64 == 0 and (shape[n][2] - shape[u][2]) % 64 == 0):
+                lazy[u] = n
+    # where should a layer write?  -> into the slice of the first Concat that consumes it, if its block takes a window
+    windowed = (B.Conv, B.RepNCSPELAN4, B.ADown, B.SPPELAN, B.Upsample, B.CBFuse)
+    dest: dict[str, tuple[str, int]] = {}
+    for n in names:
+        if isinstance(layers[n], B.Concat):
+            off = 0
+            for s in srcs[n]:
+                if lazy.get(s) == n:
+                    continue
+                if s not in dest and s != "input" and isinstance(layers[s], windowed):
+                    dest[s] = (n, off)
+                off += shape[s][2]
+    # main_only (opt-in, SURVEY.md 8f row 2): every caller of a dual-head model drops the auxiliary half
+    # (scripts/detect.py:239-241, eval/evaluator.py:107-109); compile only what the main towers need.
+    needed, head = set(names), names[-1]
+    if not isinstance(layers[head], (DetectDFL, DualDetectDFL)):
+        raise L.YreError("the last layer of the model must be a detection head")
+    if getattr(model, "main_only", False) and isinstance(layers[head], DualDetectDFL):
+        srcs[head] = srcs[head][layers[head].num_levels:]
+        needed = {head}
+        for n in reversed(names):                 # a layer comes after every layer it reads
+            if n in needed:
+                needed.update(srcs[n])
+    wire: dict[str, Wire] = {}
+    for n in names:
+        # a Silence passes its input on: it is nobody's source and emits nothing
+        srcs[n] = [srcs[s][0] if s != "input" and isinstance(layers[s], B.Silence) else s for s in srcs[n]]
+        c = consumers[n]
+        phase4 = ("input" in srcs[n] and len(c) == 1 and isinstance(layers[c[0]], B.Conv)
+                  and layers[c[0]].conv.stride[0] == 2 and layers[c[0]].conv.kernel_size[0] == 3 and n not in dest
+                  and model.precision in ("bf16", "fp16"))
+        wire[n] = Wire(srcs[n], *shape[n], dest.get(n), n in lazy, n in needed, phase4)
+    return wire
 
 
 def _weights_version(model: nn.Module) -> int:
@@ -529,128 +610,52 @@ def compile_model(model, x: torch.Tensor) -> Plan:
         Bn, H, W, Cin = x.shape
     else:
         Bn, Cin, H, W = x.shape
+    wire = wire_model(model, H, W, Cin)
     p = Plan(x.device, Bn, model.precision)
     p.names = {id(m): n for n, m in model.named_modules()}
-    names = list(model.layers.keys())
-    conn = model.connections
-    srcs = {n: ([conn[n]] if isinstance(conn[n], str) else list(conn[n])) for n in names}
-    consumers: dict[str, list[str]] = {"input": []}
-    for n in names:
-        consumers.setdefault(n, [])
-        for s in srcs[n]:
-            consumers.setdefault(s, []).append(n)
-    chan = {"input": Cin}
-    for n in names:
-        chan[n] = _out_channels(model.layers[n], [chan[s] for s in srcs[n]])
-    # Upsample -> Concat([up, skip]) -> RepNCSPELAN4: the ELAN's first op is a 1x1 conv over the whole concat, which can
-    # read the half-resolution tensor directly (VCat / yre_conv_desc.xu).  Such an Upsample emits no kernel and its half
-    # of the concat buffer is never allocated.
-    lazy_up: dict[str, str] = {}
-    if getattr(model, "fuse_upsample", True):
-        for n in names:
-            if not (isinstance(model.layers[n], B.Concat) and len(srcs[n]) >= 2):
-                continue
-            u = srcs[n][0]
-            if (u != "input" and isinstance(model.layers[u], B.Upsample) and consumers.get(u) == [n] and u not in srcs[n][1:]
-                    and consumers.get(n) and all(isinstance(model.layers[c], B.RepNCSPELAN4) and srcs[c] == [n] for c in consumers[n])
-                    and chan[u] % 64 == 0 and (chan[n] - chan[u]) % 64 == 0):
-                lazy_up[u] = n
-    cat_chan = {n: chan[n] - sum(chan[u] for u, k in lazy_up.items() if k == n) for n in names}
-    # where should a layer write?  -> into the slice of the first Concat that consumes it
-    dest: dict[str, tuple[str, int]] = {}
-    for n in names:
-        if isinstance(model.layers[n], B.Concat):
-            off = 0
-            for s in srcs[n]:
-                if lazy_up.get(s) == n:
-                    continue
-                if s not in dest and s != "input" and not isinstance(model.layers[s], (B.Silence, B.CBLinear, B.Concat)):
-                    dest[s] = (n, off)
-                off += chan[s]
-    cat_bufs: dict[str, V] = {}
-    # main_only (opt-in, SURVEY.md 8f row 2): every caller of a dual-head model drops the auxiliary half
-    # (scripts/detect.py:239-241, eval/evaluator.py:107-109); compile only what the main towers need.
-    needed, det_name, det_levels = None, names[-1], 0
-    if getattr(model, "main_only", False) and isinstance(model.layers[det_name], DualDetectDFL):
-        det_levels = model.layers[det_name].num_levels
-        needed, stack = {det_name}, list(srcs[det_name][det_levels:])
-        while stack:
-            s_ = stack.pop()
-            if s_ != "input" and s_ not in needed:
-                needed.add(s_)
-                stack.extend(srcs[s_])
 
-    def out_for(n: str, H_: int, W_: int) -> V | None:
-        if n not in dest:
-            return None
-        k, off = dest[n]
-        if k not in cat_bufs:
-            cat_bufs[k] = p.alloc(H_, W_, cat_chan[k])
-        return cat_bufs[k].sl(off, chan[n])
+    @cache
+    def cat_buf(n: str) -> V:
+        """the buffer of concat n, allocated at first use; it holds no channels of a lazy upsample"""
+        w = wire[n]
+        return p.alloc(w.H, w.W, w.C - sum(wire[s].C for s in w.srcs if wire[s].lazy))
 
     vals: dict[str, object] = {}
-    result = None
-    for n in names:
-        if needed is not None and n not in needed:
+    for n, m in model.layers.items():
+        w = wire[n]
+        if not w.needed or w.lazy or isinstance(m, B.Silence):
             continue
-        m = model.layers[n]
-        if needed is not None and n == det_name:
-            vals[n] = result = p.detect(m, [vals[s] for s in srcs[n][det_levels:]], main_only=True)
-            continue
-        ins = [("input" if s == "input" else vals[s]) for s in srcs[n]]
-        single = isinstance(conn[n], str)
-        if single and ins[0] == "input" or (not single and any(i == "input" for i in ins)):
-            if isinstance(m, B.Silence):
-                vals[n] = "input"
-                continue
+        if "input" in w.srcs:
             if not (isinstance(m, B.Conv) and m.conv.kernel_size[0] == 3 and Cin <= 4 and m.conv.groups == 1):
                 raise L.YreError(f"layer '{n}' reads the image but is not a 3x3 Conv (unsupported stem)")
-            cons = consumers.get(n, [])
-            ph = (len(cons) == 1 and isinstance(model.layers[cons[0]], B.Conv) and model.layers[cons[0]].conv.stride[0] == 2
-                  and model.layers[cons[0]].conv.kernel_size[0] == 3 and n not in dest and p.prec in ("bf16", "fp16"))
-            vals[n] = p.stem(m, x, ph)
+            vals[n] = p.stem(m, x, w.phase4)
             continue
-        a = ins[0] if single else ins
-        if n in lazy_up:                                   # Upsample folded into its consumer's first conv
-            vals[n] = ("lazy_upsample", a)
-            continue
-        if isinstance(m, B.Concat) and n in lazy_up.values():
-            if n not in cat_bufs:
-                cat_bufs[n] = p.alloc(ins[1].H, ins[1].W, cat_chan[n])
-            vals[n] = VCat(ins[0][1], p.concat(ins[1:], cat_bufs[n]))
-            result = vals[n]
-            continue
-        if isinstance(m, (B.Conv, B.RepNCSPELAN4, B.ADown, B.SPPELAN, B.Upsample, B.CBFuse)):
-            xin = a if isinstance(a, V) else (a[-1] if isinstance(m, B.CBFuse) else a)
-            if isinstance(m, B.Conv):
-                k, s_ = m.conv.kernel_size[0], m.conv.stride[0]
-                Ho, Wo = (xin.H + 2 * (k // 2) - k) // s_ + 1, (xin.W + 2 * (k // 2) - k) // s_ + 1
-            elif isinstance(m, B.ADown):
-                Ho, Wo = (xin.H - 2) // 2 + 1, (xin.W - 2) // 2 + 1
-            elif isinstance(m, B.Upsample):
-                Ho, Wo = 2 * xin.H, 2 * xin.W
-            else:
-                Ho, Wo = xin.H, xin.W
-            vals[n] = p.block(m, a, out_for(n, Ho, Wo))
+        ins = [vals[s] for s in w.srcs if not wire[s].lazy]
+        if isinstance(m, (DetectDFL, DualDetectDFL)):
+            p.result = p.detect(m, ins, main_only=getattr(model, "main_only", False))
         elif isinstance(m, B.Concat):
-            if n not in cat_bufs:
-                cat_bufs[n] = p.alloc(ins[0].H, ins[0].W, chan[n])
-            vals[n] = p.concat(ins, cat_bufs[n])
+            vals[n] = p.concat(ins, cat_buf(n))
+            up = wire[w.srcs[0]]
+            if up.lazy:                              # the Upsample is folded into the consumers' first conv
+                vals[n] = VCat(vals[up.srcs[0]], vals[n])
         else:
-            vals[n] = p.block(m, a)
-        result = vals[n]
-    if not (isinstance(result, tuple) and result and result[0] in ("single", "dual")):
-        raise L.YreError("the last layer of the model must be a detection head")
-    p.result = result
+            out = cat_buf(w.dest[0]).sl(w.dest[1], w.C) if w.dest else None
+            vals[n] = p.block(m, ins[0] if isinstance(model.connections[n], str) else ins, out)
     p.vals = vals                 # per-layer output windows (debugging / stage-wise tests)
     p.in_ptr = x.data_ptr()
     p.weight_version = _weights_version(model)
     return p
 
 
-def _fresh(p: Plan, t: torch.Tensor) -> torch.Tensor:
-    n = torch.empty_like(t)
-    p.rebind(t.data_ptr(), n.data_ptr())
+def _fresh(p: Plan, o):
+    """o (an output tensor, a raw-logit window or a list of them) re-pointed to new tensors that the plan writes"""
+    if isinstance(o, list):
+        return [_fresh(p, e) for e in o]
+    if isinstance(o, V):
+        o.t = _fresh(p, o.t)
+        return o
+    n = torch.empty_like(o)
+    p.rebind(o.data_ptr(), n.data_ptr())
     return n
 
 
@@ -705,24 +710,21 @@ def model_forward(model, x: torch.Tensor):
         elif p.in_ptr != x.data_ptr():
             p.rebind(p.in_ptr, x.data_ptr())
             p.in_ptr = x.data_ptr()
-        kind, y, raws = p.result
         if model.fresh_outputs:
             # the reference returns new tensors every call: re-point the plan's outputs
-            if kind == "single":
-                y = _fresh(p, y)
-                for r in raws:
-                    r.t = _fresh(p, r.t)
-            else:
-                y = [_fresh(p, t) for t in y]
-                for rs in raws:
-                    for r in rs:
-                        r.t = _fresh(p, r.t)
-            p.result = (kind, y, raws)
+            kind, y, raws = p.result
+            p.result = (kind, _fresh(p, y), _fresh(p, raws))
         if getattr(model, "use_cuda_graph", False) and not model.fresh_outputs:
             _replay_graph(p, x)
         else:
             p.run()
     p.x_keepalive = x
+    return _head_outputs(p.result)
+
+
+def _head_outputs(result):
+    """forward's value for a head result: (y[B,4+nc,A], [raw_i NCHW]), or ([y_aux, y_main], [raws_aux, raws_main])"""
+    kind, y, raws = result
     if kind == "single":
         return y.permute(0, 2, 1), [_raw_nchw(r) for r in raws]
     return [t.permute(0, 2, 1) for t in y], [[_raw_nchw(r) for r in rs] for rs in raws]
@@ -776,11 +778,8 @@ def compile_module(m: nn.Module, x, prec: str | None = None):
             return y
         return tuple(back(o) for o in v)
 
-    if isinstance(out, tuple) and out and out[0] in ("single", "dual"):
-        kind, y, raws = out
-        if kind == "single":
-            return p, (y.permute(0, 2, 1), [_raw_nchw(r) for r in raws])
-        return p, ([t.permute(0, 2, 1) for t in y], [[_raw_nchw(r) for r in rs] for rs in raws])
+    if isinstance(m, (DetectDFL, DualDetectDFL)):
+        return p, _head_outputs(out)
     return p, back(out)
 
 
