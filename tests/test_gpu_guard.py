@@ -213,16 +213,28 @@ def test_decode_writes_only_y(nc, levels):
     assert bool(torch.isfinite(y).all())
 
 
-@pytest.mark.parametrize("Bn,A,nc,conf,max_det", [(3, 8400, 80, 0.25, 300), (2, 33600, 80, 0.001, 300), (5, 777, 3, 0.05, 7), (1, 20000, 80, 0.0, 300)])
-def test_nms_writes_only_its_outputs(Bn, A, nc, conf, max_det):
-    """K7: out / counts / keep_anchor / workspace, incl. every anchor a candidate and more candidates than the shared-memory
-    sort holds (top-K selection and the full-sort fallback)."""
+@pytest.mark.parametrize("Bn,A,nc,conf,max_det,case", [
+    pytest.param(*a, None, id="-".join(map(str, a)))
+    for a in [(3, 8400, 80, 0.25, 300), (2, 33600, 80, 0.001, 300), (5, 777, 3, 0.05, 7), (1, 20000, 80, 0.0, 300)]] + [
+    pytest.param(None, None, None, None, None, name, id=name) for name in ("overflow", "redo_npow2_scale", "mixed4", "mixed3_npow2")])
+def test_nms_writes_only_its_outputs(Bn, A, nc, conf, max_det, case):
+    """K7: out / counts / keep_anchor / workspace, incl. every anchor a candidate, more candidates than the shared-memory
+    sort holds (sampled top-m selection), and the cases of tests/nms_path_cases.py that sort every candidate in global
+    memory (sort_global after an overflow of the sampled threshold or after a redo), alone and next to images that take
+    the other paths."""
     lib = L.lib()
-    g = torch.Generator().manual_seed(A)
-    pred = torch.rand((Bn, A, 4 + nc), generator=g)
-    pred[..., :2] *= 640
-    pred[..., 2:4] = pred[..., 2:4] * 80 + 4
-    pred[..., 4:] = pred[..., 4:] ** 6
+    if case is None:
+        g = torch.Generator().manual_seed(A)
+        pred = torch.rand((Bn, A, 4 + nc), generator=g)
+        pred[..., :2] *= 640
+        pred[..., 2:4] = pred[..., 2:4] * 80 + 4
+        pred[..., 4:] = pred[..., 4:] ** 6
+        iou = 0.45
+    else:
+        from tests import nms_path_cases as P
+        pred, kw = P.pred_of(case), P.CASES[case].kw
+        Bn, A, nc = pred.shape[0], pred.shape[1], pred.shape[2] - 4
+        conf, iou, max_det = kw["conf_thres"], kw["iou_thres"], kw.get("max_det", 300)
     pd = pred.to(DEV)
     wsb = lib.yre_nms_workspace_bytes(Bn, A)
     a = Arena()
@@ -231,7 +243,7 @@ def test_nms_writes_only_its_outputs(Bn, A, nc, conf, max_det):
     a.reserve((Bn, max_det), torch.int64)
     a.reserve((wsb,), torch.uint8)
     out, counts, keep, ws = a.build()
-    d = L.NmsDesc(pd.data_ptr(), Bn, A, nc, conf, 0.45, max_det, None, -1, 0, out.data_ptr(), counts.data_ptr(), keep.data_ptr(),
+    d = L.NmsDesc(pd.data_ptr(), Bn, A, nc, conf, iou, max_det, None, -1, 0, out.data_ptr(), counts.data_ptr(), keep.data_ptr(),
                   ws.data_ptr(), wsb, None)
     L.check(lib.yre_nms_batched(C.byref(d), torch.cuda.current_stream().cuda_stream), "nms")
     a.check_guards(f"nms B{Bn} A{A}")

@@ -31,6 +31,7 @@ constexpr int CHUNK = 512;            // candidates per greedy round
 constexpr int NT_SEL = 1024;          // threads of nms_select (two per candidate of a chunk)
 constexpr int MW = CHUNK / 32;        // 32-bit mask words per row
 constexpr int SMEM_KEYS = 8192;       // keys sorted in shared memory at a time (one segment)
+constexpr int NMS_MAX_DET = 4096;     // largest accepted max_det (sizes nms_select's shared-memory opt-in)
 
 typedef unsigned long long u64;
 
@@ -390,7 +391,8 @@ __global__ void __launch_bounds__(NT_SEL) nms_select_kernel(const SelectParams p
     // suppressed, skipped without evaluating it.
     IouThr ithr;
     ithr.thr = p.iou; ithr.lo = p.iou_lo; ithr.hi = p.iou_hi; ithr.quick = p.iou_hi > 0.f; ithr.nonneg = p.iou >= 0.0;
-    const bool prune = !p.agnostic && __fmul_rn(__int2float_rn(p.nc), scale) < 4194304.f;
+    // (a threshold < 0 suppresses pairs whose IoU is 0 as well, so the shortcut then does not apply)
+    const bool prune = !p.agnostic && ithr.nonneg && __fmul_rn(__int2float_rn(p.nc), scale) < 4194304.f;
     const int rowf = 4 + p.nc;
     int kept = 0;
     for (int pass = 0; pass < 2; ++pass) {
@@ -577,7 +579,7 @@ static int check_nms(const yre_nms_desc& d, bool outputs) {
     if (!d.pred || !d.workspace) YRE_FAIL(YRE_EINVAL, "nms: null pointer");
     if (outputs && (!d.out || !d.counts || !d.keep_anchor)) YRE_FAIL(YRE_EINVAL, "nms: null output pointer");
     if (d.B <= 0 || d.A <= 0 || d.nc <= 0) YRE_FAIL(YRE_EINVAL, "nms: bad extent B=%d A=%d nc=%d", d.B, d.A, d.nc);
-    if (d.max_det <= 0 || d.max_det > 4096) YRE_FAIL(YRE_EUNSUPPORTED, "nms: max_det=%d (supported 1..4096)", d.max_det);
+    if (d.max_det <= 0 || d.max_det > NMS_MAX_DET) YRE_FAIL(YRE_EUNSUPPORTED, "nms: max_det=%d (supported 1..%d)", d.max_det, NMS_MAX_DET);
     if (d.workspace_bytes < yre_nms_workspace_bytes(d.B, d.A)) YRE_FAIL(YRE_EINVAL, "nms: workspace too small");
     if (d.n_classes > 0 && !d.classes) YRE_FAIL(YRE_EINVAL, "nms: classes pointer missing");
     if ((reinterpret_cast<uintptr_t>(d.pred) & 15) || (reinterpret_cast<uintptr_t>(d.workspace) & 15))
@@ -623,14 +625,14 @@ int launch_nms(const yre_nms_desc& d, cudaStream_t s) {
         sp.iou_lo = (float)(d.iou_thres * (1.0 - 1.0 / 262144.0));
         sp.iou_hi = (float)(d.iou_thres * (1.0 + 1.0 / 262144.0));
     }
-    const size_t smem = select_smem_bytes(d.max_det);
+    // opt in to the shared memory of the largest max_det check_nms accepts (227 520 B; sm_100 allows 232 448 B a block)
     static YrePerDeviceOnce once;
     if (int e = once.run([]() -> int {
-            YRE_CUDA(cudaFuncSetAttribute(nms_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
+            YRE_CUDA(cudaFuncSetAttribute(nms_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                          (int)select_smem_bytes(NMS_MAX_DET)));
             return YRE_OK;
         })) return e;
-    if (smem > 200 * 1024) YRE_FAIL(YRE_EUNSUPPORTED, "nms: shared memory budget exceeded");
-    nms_select_kernel<<<d.B, NT_SEL, smem, s>>>(sp);
+    nms_select_kernel<<<d.B, NT_SEL, select_smem_bytes(d.max_det), s>>>(sp);
     YRE_LAUNCH_CHECK("nms_select");
     return YRE_OK;
 }
