@@ -102,6 +102,27 @@ int yre_conv(const yre_conv_desc* d, yre_stream_t s);
  * YRE_EUNSUPPORTED, with the reason in yre_last_error(), when the engine does not take the shape or its tile does not fit
  * shared memory. */
 int yre_conv_tc_describe(const yre_conv_desc* d, int32_t num_sms, char* out, int32_t cap);
+/* Host-only query, like yre_conv_tc_describe: the work schedule the tcgen05 kernel walks for the first n (1 <= n <= y.B)
+ * images of d on a device with num_sms SMs -- what a plan compiled for d.y.B images launches in yre_plan_run_batch(n).
+ * The tiling (tw x th x tb pixels x images by block_n channels) is the one chosen for all y.B images; n only shortens
+ * the walk to the first tiles_b = ceil(n / tb) image tiles and sizes the persistent grid for them.  Work item w of
+ * CTA (pair) c, for w = c, c + G, c + 2G ... (G = grid, or grid / 2 CTA pairs), decodes images outermost:
+ *   YRE_TC_GENERIC, YRE_TC_HALO_WS: tile w -> N tile w % tiles_n, M tile m = w / tiles_n;
+ *   YRE_TC_GENERIC_CTA2: unit w -> N tile w % tiles_n, M tiles 2 (w / tiles_n) + {0, 1} (one per CTA of the pair);
+ *   YRE_TC_HALO_STREAM: unit w -> N tile w / upn, M tiles npair (w % upn) + {0 .. npair-1};
+ * M tile m -> x tile m % tiles_x, y tile (m / tiles_x) % tiles_y, image tile m / (tiles_x tiles_y).  ybx = 1: the tile's
+ * pixel rows run (y, image, x) (8 x 8 pixels of two images). */
+enum { YRE_TC_GENERIC = 0, YRE_TC_GENERIC_CTA2 = 1, YRE_TC_HALO_WS = 2, YRE_TC_HALO_STREAM = 3 };
+typedef struct yre_tc_schedule {
+    int32_t kind, ybx;
+    int32_t tw, th, tb, block_n;
+    int32_t tiles_x, tiles_y, tiles_b, tiles_n;
+    int32_t mtiles;   /* tiles_x * tiles_y * tiles_b */
+    int32_t npair, upn;
+    int32_t work;     /* tiles (GENERIC, HALO_WS) or units (GENERIC_CTA2, HALO_STREAM) */
+    int32_t grid;     /* CTAs launched */
+} yre_tc_schedule;
+int yre_conv_tc_schedule(const yre_conv_desc* d, int32_t num_sms, int32_t n, yre_tc_schedule* out);
 
 /* ---- K2: first conv straight from the image ------------------------------------------------------
  * Replaces layers.stem1 (Conv 3x3 s2 on the input image; configs/models/gelan-c.yaml stem1,
@@ -294,6 +315,19 @@ int  yre_plan_add_nms(yre_plan* p, const yre_nms_desc* d);
  * of those fails with YRE_EUNSUPPORTED.  Returns the number of patched fields (>= 0). */
 int  yre_plan_rebind(yre_plan* p, const void* old_ptr, void* new_ptr);
 int  yre_plan_run(yre_plan* p, yre_stream_t s);
+/* Batch capacity: a plan whose ops were all recorded for the same B images (every plan the Python engine compiles) runs
+ * any n <= B of them.  yre_plan_batch_capacity returns that B, or YRE_EINVAL (with a message) for an empty plan or one
+ * whose ops disagree on B.
+ * yre_plan_run_batch(p, n, s) computes the first n images exactly as yre_plan_run computes them (bit-identical: every
+ * kernel keeps the tiling chosen for B images, each output element reads only its own image) and writes no row of an
+ * image >= n in any buffer -- so the caller's input and output tensors need only hold n images.  The launches are
+ * shorter: grids cover the first n images, the tcgen05 convs walk the first ceil(n / tb) image tiles of their tile
+ * schedule (yre_conv_tc_schedule) and store through output tensor maps that end at image n (encoded on the host at the
+ * first run of each n, and again when n or a re-bound output pointer changes; the encoding is host work only, so a
+ * run_batch is CUDA-graph capturable like yre_plan_run).  n == B launches exactly what yre_plan_run launches.
+ * YRE_EINVAL for n < 1, n > B or a plan without a capacity. */
+int  yre_plan_run_batch(yre_plan* p, int32_t n, yre_stream_t s);
+int  yre_plan_batch_capacity(const yre_plan* p);
 /* kernels launched by one yre_plan_run / ops recorded / of which tcgen05 convs */
 int  yre_plan_num_launches(const yre_plan* p);
 int  yre_plan_num_ops(const yre_plan* p);

@@ -122,7 +122,7 @@ double conv_flops(const yre_conv_desc& d) {
     return 2.0 * d.y.B * d.y.H * d.y.W * (double)d.y.C * (d.x.C + (d.xu.ptr ? d.xu.C : 0)) * d.k * d.k;
 }
 
-int launch_conv_ffma(const yre_conv_desc& d, cudaStream_t s) {
+int launch_conv_ffma(const yre_conv_desc& d, int nb, cudaStream_t s) {
     FfmaParams p;
     p.x = make_dview(d.x); p.y = make_dview(d.y);
     p.has_res = d.res.ptr != nullptr;
@@ -134,7 +134,7 @@ int launch_conv_ffma(const yre_conv_desc& d, cudaStream_t s) {
         if (d.xu.C % 4 || d.xu.c_off % 4 || d.xu.C_total % 4) YRE_FAIL(YRE_EUNSUPPORTED, "conv_ffma: channel counts/offsets must be multiples of 4");
         p.xu = make_dview(d.xu); p.Cu = d.xu.C; p.Cin += p.Cu;
     }
-    p.M = (long long)d.y.B * d.y.H * d.y.W;
+    p.M = (long long)nb * d.y.H * d.y.W;              // the first nb images: pixels are image-major
     if (p.Cin % 4 || p.Cout % 4 || d.x.c_off % 4 || d.y.c_off % 4 || d.x.C_total % 4 || d.y.C_total % 4 ||
         (p.has_res && (d.res.c_off % 4 || d.res.C_total % 4)))
         YRE_FAIL(YRE_EUNSUPPORTED, "conv_ffma: channel counts/offsets must be multiples of 4");

@@ -449,7 +449,7 @@ __device__ __forceinline__ void epilogue_role(const TcParams& p, const CUtensorM
             if (CTA2) {                           // CTA-pair schedule: cluster c takes units c, c + #clusters, ...
                 const int u = (int)(blockIdx.x >> 1) + j * (int)(gridDim.x >> 1);
                 if (u >= p.num_units) break;
-                int m = 2 * (u / p.tiles_n) + pair_rank;             // m >= mtiles (odd tile out): loads zero-fill, stores clip
+                int m = 2 * (u / p.tiles_n) + pair_rank;             // m >= mtiles (odd tile out): images >= B, stores clip
                 if (p.rev) m = ((p.mtiles + 1) & ~1) - 1 - m;
                 const int r = m / p.tiles_x;
                 x0 = (m % p.tiles_x) * p.tw; y0 = (r % p.tiles_y) * p.th; b0 = (r / p.tiles_y) * p.tb; n0 = (u % p.tiles_n) * p.block_n;
@@ -1040,7 +1040,7 @@ conv3_halo_stream_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
                         if (p.rev) m = (int)NPAIR * p.upn - 1 - m;
                         const int r = m / p.tiles_x;
                         const int x0 = (m % p.tiles_x) * p.tw - 1, y0 = (r % p.tiles_y) * p.th - 1;
-                        const int b0 = (r / p.tiles_y) * p.tb;            // b0 >= B for the odd patch out: zero-filled
+                        const int b0 = (r / p.tiles_y) * p.tb;            // b0 >= B for the odd patch out: its stores clip
                         const uint32_t dst = sA + (stage * NPAIR + h) * A_BYTES;
                         if (p.ybx) tma_load_4d(dst, &tmA, full, p.x_coff + kc * 64, x0, b0, y0);
                         else tma_load_4d(dst, &tmA, full, p.x_coff + kc * 64, x0, y0, b0);
@@ -1231,6 +1231,24 @@ int tc_shape_rules(const yre_conv_desc& d, char* why, size_t n) {
     return 1;
 }
 
+// The batch-dependent part of a schedule, for n images of a conv whose tiling was chosen for its whole batch.  Every kernel
+// walks images outermost (TileCur's bt digit; m / tiles_x / tiles_y of the CTA-pair and halo units), so the work of the first
+// n images is the prefix of ceil(n / tb) image tiles.  A tile of tb > 1 images, or the odd patch of a pair, may reach
+// images >= n: its loads read whatever those rows hold (no output element reads another image) and its stores are clipped
+// (B = n bounds the direct store, the output tensor map of a run of n images ends at image n).  The persistent grid is
+// sized for the prefix, so every CTA (pair) still has at least one work item.  conv_tc_select calls it with the whole
+// batch; a plan run of fewer images calls it on a copy of the parameters.
+void tc_batch(TcParams& p, int n, int sms, int* grid) {
+    p.B = n;
+    p.tiles_b = yre_cdiv(n, p.tb);
+    p.mtiles = p.tiles_x * p.tiles_y * p.tiles_b;
+    p.num_tiles = p.mtiles * p.tiles_n;
+    p.upn = yre_cdiv(p.mtiles, p.npair);
+    p.num_units = p.cta2 ? yre_cdiv(p.mtiles, 2) * p.tiles_n : p.upn * p.tiles_n;
+    // persistent grids: one CTA (pair) per work unit, at most one per SM
+    *grid = p.cta2 ? 2 * std::min(p.num_units, sms / 2) : std::min(p.halo == 2 ? p.num_units : p.num_tiles, sms);
+}
+
 // Kernel, tiling, pipeline depth, shared memory and grid of a conv that passes tc_shape_rules on a device with `sms` SMs.
 // A pure function: no CUDA call, no global state; pointers are copied into the parameters, never read.  The rules were
 // measured per layer (profiles/r02_notes.md).  Fails with YRE_EUNSUPPORTED when the tile does not fit shared memory.
@@ -1309,10 +1327,6 @@ int conv_tc_select(const yre_conv_desc& d, int sms, const TcKnobs& kn, TcParams*
     }
     p.block_n = bn;
     p.tiles_n = Cout / bn;
-    p.num_tiles = (int)(mtiles * p.tiles_n);
-    p.mtiles = (int)mtiles;
-    p.upn = (int)((mtiles + p.npair - 1) / p.npair);
-    p.num_units = p.upn * p.tiles_n;
     // CTA pairs for the wide N tiles of the generic kernel.  What they buy is operand traffic: per 128 x N x 64 k-iteration a
     // CTA pulls 16 KB of A + N * 128 B of B from L2 (and the MMAs read as much from shared memory); a pair halves the B half.
     // Rule from the per-layer sweep at batch 64 (scripts/gpu_sweep.sh, profiles/r02_notes.md): pairs win wherever the main
@@ -1323,7 +1337,6 @@ int conv_tc_select(const yre_conv_desc& d, int sms, const TcKnobs& kn, TcParams*
     const long long K_total = (long long)p.taps * Cin;
     const bool cta2_legal = !p.halo && bn >= 128 && mtiles >= 2;
     p.cta2 = kn.cta2 == 0 ? 0 : kn.cta2 == 1 ? cta2_legal : cta2_legal && (K_total >= 512 || (K_total >= 256 && bn >= 256));
-    if (p.cta2) p.num_units = (int)((mtiles + 1) / 2) * p.tiles_n;
     p.a_bytes = (uint32_t)(BLOCK_M * p.block_k * 2);
     if (p.halo) {
         p.halo_tx = (uint32_t)((p.ybx ? 10 * 2 * 10 : 10 * 18) * p.block_k * 2);
@@ -1406,8 +1419,7 @@ int conv_tc_select(const yre_conv_desc& d, int sms, const TcKnobs& kn, TcParams*
                        :               (size_t)stages * stage_bytes;
     *smem = rings + 8 * (2 * stages + 16 + (p.halo == 2 ? 2 * p.stages_b : p.halo ? 2 : 0)) + 32 + n_stage_bufs * p.stage_out_bytes +
             (size_t)Cout * 4 + align_slack;
-    // persistent grids: one CTA (pair) per work unit, at most one per SM
-    *grid = p.cta2 ? 2 * std::min(p.num_units, sms / 2) : std::min(p.halo == 2 ? p.num_units : p.num_tiles, sms);
+    tc_batch(p, B, sms, grid);
     // instruction descriptor: fp32 accumulator (bits 4-5), A and B bf16 (bits 7-9, 10-12; conv_tc_prepare clears them for
     // fp16 operands -- the tiling is the same for both 16-bit types), N >> 3, M >> 4
     p.idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(bn >> 3) << 17) | ((uint32_t)((p.cta2 ? 2 * BLOCK_M : BLOCK_M) >> 4) << 24);
@@ -1473,6 +1485,12 @@ struct ConvTcPlan {
     size_t smem;
     const TcKernel* kernel;
     int f16;                      // 1: fp16 activations and weights (kernel->fn[1]), 0: bf16
+    int sms;                      // SM count the grid was sized for
+    // output tensor map of the last run of fewer than p.B images (TMA stores clip at its image count), encoded on first use
+    // and again only when the image count or the output pointer changes
+    CUtensorMap tmYn;
+    int yn_b = 0;
+    void* yn_ptr = nullptr;
 };
 
 // ---- describe ----
@@ -1485,6 +1503,27 @@ static void tc_format(const TcParams& p, int grid, char* out, size_t n) {
 }
 
 void conv_tc_describe(const ConvTcPlan* pl, char* out, size_t n) { tc_format(pl->p, pl->grid, out, n); }
+
+extern "C" int yre_conv_tc_schedule(const yre_conv_desc* d, int32_t num_sms, int32_t n, yre_tc_schedule* out) {
+    if (!out || num_sms <= 0) YRE_FAIL(YRE_EINVAL, "conv_tc_schedule: null output or non-positive SM count");
+    if (int e = check_conv(d)) return e;
+    if (n < 1 || n > d->y.B) YRE_FAIL(YRE_EINVAL, "conv_tc_schedule: %d images outside 1..%d", n, d->y.B);
+    char why[256] = "";
+    if (!tc_shape_rules(*d, why, sizeof(why))) YRE_FAIL(YRE_EUNSUPPORTED, "conv_tc: %s", why);
+    TcParams p; int grid; size_t smem;
+    const TcKnobs kn = tc_knobs();
+    if (int e = conv_tc_select(*d, num_sms, kn, &p, &grid, &smem)) return e;
+    tc_batch(p, n, kn.sms > 0 ? kn.sms : num_sms, &grid);
+    *out = yre_tc_schedule{};
+    out->kind = p.halo == 1 ? YRE_TC_HALO_WS : p.halo == 2 ? YRE_TC_HALO_STREAM : p.cta2 ? YRE_TC_GENERIC_CTA2 : YRE_TC_GENERIC;
+    out->ybx = p.ybx;
+    out->tw = p.tw; out->th = p.th; out->tb = p.tb; out->block_n = p.block_n;
+    out->tiles_x = p.tiles_x; out->tiles_y = p.tiles_y; out->tiles_b = p.tiles_b; out->tiles_n = p.tiles_n;
+    out->mtiles = p.mtiles; out->npair = p.npair; out->upn = p.upn;
+    out->work = (p.cta2 || p.halo == 2) ? p.num_units : p.num_tiles;
+    out->grid = grid;
+    return YRE_OK;
+}
 
 extern "C" int yre_conv_tc_describe(const yre_conv_desc* d, int32_t num_sms, char* out, int32_t cap) {
     if (!out || cap <= 0 || num_sms <= 0) YRE_FAIL(YRE_EINVAL, "conv_tc_describe: null output or non-positive size / SM count");
@@ -1511,9 +1550,9 @@ int conv_tc_eligible(const yre_conv_desc& d, char* why, size_t n) {
 #undef NOPE
 
 // output tensor map of the staged TMA store: one box = the 32 pixels of a TMEM lane quarter x 32 (64 with stage64) channels;
-// fp32 outputs use 128-byte rows (32 channels) in a 128B-swizzled tile.  Also used when an output buffer is re-bound.
-static CUresult encode_y(ConvTcPlan* pl, void* ptr) {
-    const auto& p = pl->p;
+// fp32 outputs use 128-byte rows (32 channels) in a 128B-swizzled tile.  The map spans p.B images.  Also used when an output
+// buffer is re-bound and for runs of fewer images.
+static CUresult encode_y(const TcParams& p, int f16, void* ptr, CUtensorMap* out) {
     const cuuint64_t es = p.y_f32 ? 4 : 2, ct = (cuuint64_t)p.y_ctot;
     cuuint64_t gdim[4] = {ct, (cuuint64_t)p.Wo, (cuuint64_t)p.Ho, (cuuint64_t)p.B};
     cuuint64_t gstr[3] = {ct * es, (cuuint64_t)p.Wo * ct * es, (cuuint64_t)p.Ho * p.Wo * ct * es};
@@ -1525,8 +1564,8 @@ static CUresult encode_y(ConvTcPlan* pl, void* ptr) {
         box[2] = (cuuint32_t)p.stb; box[3] = (cuuint32_t)p.sth;
     }
     cuuint32_t est[4] = {1, 1, 1, 1};
-    const CUtensorMapDataType dt = p.y_f32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : pl->f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
-    return get_encode()(&pl->tmY, dt, 4, ptr, gdim, gstr, box, est,
+    const CUtensorMapDataType dt = p.y_f32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+    return get_encode()(out, dt, 4, ptr, gdim, gstr, box, est,
                         CU_TENSOR_MAP_INTERLEAVE_NONE, (p.stage64 || p.y_f32) ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
                         CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
 }
@@ -1541,6 +1580,7 @@ int conv_tc_prepare(const yre_conv_desc& d, ConvTcPlan** out) {
     std::unique_ptr<ConvTcPlan> pl(new ConvTcPlan());
     TcParams& p = pl->p;
     if (int e = conv_tc_select(d, sms, kn, &p, &pl->grid, &pl->smem)) return e;
+    pl->sms = kn.sms > 0 ? kn.sms : sms;
     pl->f16 = d.x.dtype == YRE_F16;
     if (pl->f16) p.idesc &= ~((7u << 7) | (7u << 10));      // A and B format 0 = F16
     const CUtensorMapDataType dt16 = pl->f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
@@ -1608,7 +1648,7 @@ int conv_tc_prepare(const yre_conv_desc& d, ConvTcPlan** out) {
     }
     if (r != CUDA_SUCCESS) YRE_FAIL(YRE_ECUDA, "conv_tc: cuTensorMapEncodeTiled(W) failed with %d", (int)r);
     if (p.tma_store) {
-        r = encode_y(pl.get(), d.y.ptr);
+        r = encode_y(p, pl->f16, d.y.ptr, &pl->tmY);
         if (r != CUDA_SUCCESS) YRE_FAIL(YRE_ECUDA, "conv_tc: cuTensorMapEncodeTiled(Y) failed with %d", (int)r);
     } else {
         pl->tmY = pl->tmB;   // unused
@@ -1618,7 +1658,8 @@ int conv_tc_prepare(const yre_conv_desc& d, ConvTcPlan** out) {
 }
 
 // ---- launch ----
-int conv_tc_launch(const ConvTcPlan* pl, cudaStream_t s) {
+// nb < p.B: the first nb images only (tc_batch on a copy of the parameters, an output map that ends at image nb)
+int conv_tc_launch(ConvTcPlan* pl, int nb, cudaStream_t s) {
     static YrePerDeviceOnce once;
     if (int e = once.run([]() -> int {
             for (const TcKernel& k : TC_KERNELS)
@@ -1626,9 +1667,28 @@ int conv_tc_launch(const ConvTcPlan* pl, cudaStream_t s) {
                     YRE_CUDA(cudaFuncSetAttribute(k.fn[t], cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
             return YRE_OK;
         })) return e;
+    const TcParams* p = &pl->p;
+    const CUtensorMap* tmY = &pl->tmY;
+    int grid = pl->grid;
+    TcParams q;
+    if (nb != pl->p.B) {
+        if (nb < 1 || nb > pl->p.B) YRE_FAIL(YRE_EINVAL, "conv_tc: %d images outside 1..%d", nb, pl->p.B);
+        q = pl->p;
+        tc_batch(q, nb, pl->sms, &grid);
+        p = &q;
+        if (q.tma_store) {
+            if (pl->yn_b != nb || pl->yn_ptr != q.y) {
+                pl->yn_b = 0;
+                const CUresult r = encode_y(q, pl->f16, q.y, &pl->tmYn);
+                if (r != CUDA_SUCCESS) YRE_FAIL(YRE_ECUDA, "conv_tc: cuTensorMapEncodeTiled(Y, %d images) failed with %d", nb, (int)r);
+                pl->yn_b = nb; pl->yn_ptr = q.y;
+            }
+            tmY = &pl->tmYn;
+        }
+    }
     static const int pdl = tc_knobs().pdl;
     cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)pl->grid); cfg.blockDim = dim3((unsigned)pl->p.nthreads); cfg.dynamicSmemBytes = pl->smem; cfg.stream = s;
+    cfg.gridDim = dim3((unsigned)grid); cfg.blockDim = dim3((unsigned)p->nthreads); cfg.dynamicSmemBytes = pl->smem; cfg.stream = s;
     cudaLaunchAttribute at[2];
     int n = 0;
     if (pdl) {
@@ -1636,13 +1696,13 @@ int conv_tc_launch(const ConvTcPlan* pl, cudaStream_t s) {
         at[n].val.programmaticStreamSerializationAllowed = 1;
         ++n;
     }
-    if (pl->p.cta2) {                     // CTA pairs: clusters of two (always on one TPC)
+    if (p->cta2) {                        // CTA pairs: clusters of two (always on one TPC)
         at[n].id = cudaLaunchAttributeClusterDimension;
         at[n].val.clusterDim.x = 2; at[n].val.clusterDim.y = 1; at[n].val.clusterDim.z = 1;
         ++n;
     }
     cfg.attrs = at; cfg.numAttrs = n;
-    YRE_CUDA(cudaLaunchKernelEx(&cfg, pl->kernel->fn[pl->f16], pl->tmA, pl->tmB, pl->tmY, pl->tmAu, pl->p));
+    YRE_CUDA(cudaLaunchKernelEx(&cfg, pl->kernel->fn[pl->f16], pl->tmA, pl->tmB, *tmY, pl->tmAu, *p));
     YRE_LAUNCH_CHECK(pl->kernel->name);
     return YRE_OK;
 }
@@ -1654,7 +1714,7 @@ void conv_tc_set_reverse(ConvTcPlan* pl, int rev) { pl->p.rev = rev ? 1 : 0; }
 int conv_tc_rebind(ConvTcPlan* pl, const void* old_ptr, void* new_ptr) {
     int n = 0;
     if (pl->p.y == old_ptr) {
-        if (pl->p.tma_store && encode_y(pl, new_ptr) != CUDA_SUCCESS) return -1;     // the output is baked into a TMA tensor map
+        if (pl->p.tma_store && encode_y(pl->p, pl->f16, new_ptr, &pl->tmY) != CUDA_SUCCESS) return -1;     // the output is baked into a TMA tensor map
         pl->p.y = new_ptr; ++n;
     }
     if (pl->p.res == old_ptr) { pl->p.res = new_ptr; ++n; }

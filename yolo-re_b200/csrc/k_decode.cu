@@ -171,7 +171,7 @@ __global__ void __launch_bounds__(WARPS * 32) decode_kernel(const DecodeParams p
 
 }  // namespace
 
-int launch_decode(const yre_decode_desc& d, cudaStream_t s) {
+int launch_decode(const yre_decode_desc& d, int nb, cudaStream_t s) {
     if (d.levels < 1 || d.levels > MAXL) YRE_FAIL(YRE_EINVAL, "decode: levels=%d", d.levels);
     if (!d.y) YRE_FAIL(YRE_EINVAL, "decode: null pointer");
     if (d.nc < 1) YRE_FAIL(YRE_EINVAL, "decode: nc=%d", d.nc);
@@ -193,7 +193,7 @@ int launch_decode(const yre_decode_desc& d, cudaStream_t s) {
         A += v.H * v.W;
     }
     p.a_start[d.levels] = A;
-    p.A = A; p.B = d.raw[0].B;
+    p.A = A; p.B = nb;                               // rows of y and raw pixels are image-major
     for (int k = 0; k < 16; ++k) p.dfl_w[k] = d.dfl_w[k];
     const int CH4 = (64 + d.nc + 3) / 4 * 4, OC = 4 + d.nc;
     const size_t smem = (size_t)WARPS * (TILE * (CH4 + 4) + TILE * OC) * sizeof(float);

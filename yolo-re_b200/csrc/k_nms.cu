@@ -587,18 +587,19 @@ static int check_nms(const yre_nms_desc& d, bool outputs) {
     return YRE_OK;
 }
 
-static int launch_nms_filter(const yre_nms_desc& d, const NmsWs& ws, cudaStream_t s) {
-    nms_init_kernel<<<yre_cdiv(d.B, 256), 256, 0, s>>>(ws.count, ws.maxc, d.B);
+// nb: the first nb images (the workspace keeps the layout of d.B images)
+static int launch_nms_filter(const yre_nms_desc& d, const NmsWs& ws, int nb, cudaStream_t s) {
+    nms_init_kernel<<<yre_cdiv(nb, 256), 256, 0, s>>>(ws.count, ws.maxc, nb);
     YRE_LAUNCH_CHECK("nms_init");
 
     FilterParams fp;
-    fp.pred = d.pred; fp.B = d.B; fp.A = d.A; fp.nc = d.nc; fp.conf = d.conf_thres;
+    fp.pred = d.pred; fp.B = nb; fp.A = d.A; fp.nc = d.nc; fp.conf = d.conf_thres;
     fp.classes = d.classes; fp.n_classes = d.n_classes; fp.ws = ws;
     const size_t per_warp = (d.nc % 4 == 0) ? (size_t)32 * ((d.nc / 4) | 1) * 8 : 16;
     int warps = 4;
     while (warps > 1 && per_warp * warps > 40 * 1024) warps >>= 1;
     if (per_warp * warps > 48 * 1024) YRE_FAIL(YRE_EUNSUPPORTED, "nms: nc=%d too large", d.nc);
-    const int tiles = yre_cdiv(d.A, 32) * d.B;
+    const int tiles = yre_cdiv(d.A, 32) * nb;
     nms_filter_kernel<<<yre_cdiv(tiles, warps), warps * 32, per_warp * warps, s>>>(fp);
     YRE_LAUNCH_CHECK("nms_filter");
     return YRE_OK;
@@ -607,16 +608,17 @@ static int launch_nms_filter(const yre_nms_desc& d, const NmsWs& ws, cudaStream_
 extern "C" int yre_nms_filter_only(const yre_nms_desc* d, yre_stream_t s) {
     if (!d) YRE_FAIL(YRE_EINVAL, "nms: null descriptor");
     if (int e = check_nms(*d, false)) return e;
-    return launch_nms_filter(*d, carve(d->workspace, d->B, d->A), (cudaStream_t)s);
+    return launch_nms_filter(*d, carve(d->workspace, d->B, d->A), d->B, (cudaStream_t)s);
 }
 
-int launch_nms(const yre_nms_desc& d, cudaStream_t s) {
+int launch_nms(const yre_nms_desc& d, int nb, cudaStream_t s) {
     if (int e = check_nms(d, true)) return e;
+    if (nb < 1 || nb > d.B) YRE_FAIL(YRE_EINVAL, "nms: %d images outside 1..%d", nb, d.B);
     NmsWs ws = carve(d.workspace, d.B, d.A);
-    if (int e = launch_nms_filter(d, ws, s)) return e;
+    if (int e = launch_nms_filter(d, ws, nb, s)) return e;
 
     SelectParams sp;
-    sp.pred = d.pred; sp.B = d.B; sp.A = d.A; sp.nc = d.nc; sp.iou = d.iou_thres; sp.max_det = d.max_det;
+    sp.pred = d.pred; sp.B = nb; sp.A = d.A; sp.nc = d.nc; sp.iou = d.iou_thres; sp.max_det = d.max_det;
     sp.agnostic = d.agnostic; sp.ws = ws; sp.out = d.out; sp.counts = d.counts;
     sp.keep_anchor = reinterpret_cast<long long*>(d.keep_anchor);
     sp.scale = d.scale;
@@ -632,7 +634,7 @@ int launch_nms(const yre_nms_desc& d, cudaStream_t s) {
                                           (int)select_smem_bytes(NMS_MAX_DET)));
             return YRE_OK;
         })) return e;
-    nms_select_kernel<<<d.B, NT_SEL, select_smem_bytes(d.max_det), s>>>(sp);
+    nms_select_kernel<<<nb, NT_SEL, select_smem_bytes(d.max_det), s>>>(sp);
     YRE_LAUNCH_CHECK("nms_select");
     return YRE_OK;
 }

@@ -13,11 +13,11 @@ namespace {
 // it emits the four average-map pixels (2oy+py, 2ox+px) -- i.e. one cell of each parity plane;
 // for the high half it emits max over average rows/cols 2o-1..2o+1.
 template <typename T>
-__global__ void __launch_bounds__(256, 2) adown_prepool_kernel(DView x, DView lo, DView hi, int Ho, int Wo, int half) {
+__global__ void __launch_bounds__(256, 2) adown_prepool_kernel(DView x, DView lo, DView hi, int Ho, int Wo, int half, int nb) {
     // blockIdx.y selects the channel half, so the (very different) low/high paths never share a warp
     const int hgroups = half / 8;
     const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const long long total = (long long)x.B * Ho * Wo * hgroups;
+    const long long total = (long long)nb * Ho * Wo * hgroups;     // the first nb images; lo.B stays the plane layout
     if (idx >= total) return;
     const int g = (int)(idx % hgroups);
     long long t = idx / hgroups;
@@ -410,10 +410,10 @@ __global__ void __launch_bounds__(256, sizeof(T) == 2 ? 4 : 3) adown_tiled_kerne
 // -------------------------------------------------------------------------------------------------
 // K4: windows 5/9/13 max (== three chained MaxPool2d(5,1,2); reference sppelan.py:44-47)
 template <typename T>
-__global__ void __launch_bounds__(256) spp_kernel(DView x, DView y5, DView y9, DView y13) {
+__global__ void __launch_bounds__(256) spp_kernel(DView x, DView y5, DView y9, DView y13, int nb) {
     const int groups = x.C / 8;
     const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const long long total = (long long)x.B * x.H * x.W * groups;
+    const long long total = (long long)nb * x.H * x.W * groups;
     if (idx >= total) return;
     const int c = (int)(idx % groups) * 8;
     long long t = idx / groups;
@@ -576,11 +576,11 @@ __global__ void __launch_bounds__(1024) spp_plane16_kernel(DView x, DView y5, DV
 // -------------------------------------------------------------------------------------------------
 // K5: nearest x2 (reference: nn.Upsample, parser.py:159-171) written into the consumer's slice
 template <typename T>
-__global__ void __launch_bounds__(256) upsample2x_kernel(DView x, DView y) {
-    // one thread per INPUT (pixel, 8-channel group): one 16-byte load feeds the four output pixels
+__global__ void __launch_bounds__(256) upsample2x_kernel(DView x, DView y, int nb) {
+    // one thread per INPUT (pixel, 8-channel group) of the first nb images: one 16-byte load feeds the four output pixels
     const int groups = x.C / 8;
     const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const long long total = (long long)x.B * x.H * x.W * groups;
+    const long long total = (long long)nb * x.H * x.W * groups;
     if (idx >= total) return;
     const int c = (int)(idx % groups) * 8;
     long long t = idx / groups;
@@ -605,10 +605,10 @@ __global__ void __launch_bounds__(256) upsample2x_kernel(DView x, DView y) {
 // stack with the target and sum in that order.
 struct FuseSrcs { DView v[8]; int n; };
 template <typename T>
-__global__ void __launch_bounds__(256) cbfuse_kernel(FuseSrcs srcs, DView tgt, DView y) {
+__global__ void __launch_bounds__(256) cbfuse_kernel(FuseSrcs srcs, DView tgt, DView y, int nb) {
     const int groups = y.C / 8;
     const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    const long long total = (long long)y.B * y.H * y.W * groups;
+    const long long total = (long long)nb * y.H * y.W * groups;
     if (idx >= total) return;
     const int c = (int)(idx % groups) * 8;
     long long t = idx / groups;
@@ -695,7 +695,7 @@ int check8(const yre_view& v, const char* what) {
 
 }  // namespace
 
-int launch_adown_prepool(const yre_view& x, const yre_view& lo, const yre_view& hi, cudaStream_t s) {
+int launch_adown_prepool(const yre_view& x, const yre_view& lo, const yre_view& hi, int nb, cudaStream_t s) {
     if (check8(x, "adown.x") || check8(lo, "adown.avg_lo") || check8(hi, "adown.max_hi")) return YRE_EINVAL;
     if (x.layout != YRE_NHWC || hi.layout != YRE_NHWC) YRE_FAIL(YRE_EUNSUPPORTED, "adown: x and max_hi must be NHWC");
     if (x.C % 16) YRE_FAIL(YRE_EUNSUPPORTED, "adown: C must be a multiple of 16");
@@ -707,7 +707,8 @@ int launch_adown_prepool(const yre_view& x, const yre_view& lo, const yre_view& 
     // the thread grid walks ceil((H-1)/2) x ceil((W-1)/2) cells, which covers both outputs
     const int Gy = (x.H - 1 + 1) / 2, Gx = (x.W - 1 + 1) / 2;
     if (Gy < Ho || Gx < Wo) YRE_FAIL(YRE_EINVAL, "adown: grid smaller than the pooled output");
-    const long long total = (long long)x.B * Gy * Gx * (half / 8);
+    if (nb < 1 || nb > x.B) YRE_FAIL(YRE_EINVAL, "adown: %d images outside 1..%d", nb, x.B);
+    const long long total = (long long)nb * Gy * Gx * (half / 8);
     dim3 grid(yre_cdiv(total, 256), 2);
     // NB: kernel indexes its cell grid with (Ho,Wo) = (Gy,Gx); cells beyond hi's extent never
     // occur because Gy==Ho, Gx==Wo for every H,W >= 2.
@@ -715,24 +716,25 @@ int launch_adown_prepool(const yre_view& x, const yre_view& lo, const yre_view& 
     const int chn = x.dtype == YRE_F32 ? 32 : 64;      // 128 bytes of channels per CTA
     if (half % chn == 0) {
         const int tiles_x = yre_cdiv(Gx, AD_TX), tiles_y = yre_cdiv(Gy, AD_TY);
-        dim3 tg((unsigned)(tiles_x * tiles_y * x.B), (unsigned)(x.C / chn));
+        dim3 tg((unsigned)(tiles_x * tiles_y * nb), (unsigned)(x.C / chn));
         if (x.dtype == YRE_F32) adown_tiled_kernel<float><<<tg, 256, 0, s>>>(make_dview(x), make_dview(lo), make_dview(hi), half, tiles_x, tiles_y);
         else if (x.dtype == YRE_F16) adown_tiled_kernel<__half><<<tg, 256, 0, s>>>(make_dview(x), make_dview(lo), make_dview(hi), half, tiles_x, tiles_y);
         else adown_tiled_kernel<__nv_bfloat16><<<tg, 256, 0, s>>>(make_dview(x), make_dview(lo), make_dview(hi), half, tiles_x, tiles_y);
-    } else if (x.dtype == YRE_F32) adown_prepool_kernel<float><<<grid, 256, 0, s>>>(make_dview(x), make_dview(lo), make_dview(hi), Gy, Gx, half);
-    else if (x.dtype == YRE_F16) adown_prepool_kernel<__half><<<grid, 256, 0, s>>>(make_dview(x), make_dview(lo), make_dview(hi), Gy, Gx, half);
-    else adown_prepool_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(make_dview(x), make_dview(lo), make_dview(hi), Gy, Gx, half);
+    } else if (x.dtype == YRE_F32) adown_prepool_kernel<float><<<grid, 256, 0, s>>>(make_dview(x), make_dview(lo), make_dview(hi), Gy, Gx, half, nb);
+    else if (x.dtype == YRE_F16) adown_prepool_kernel<__half><<<grid, 256, 0, s>>>(make_dview(x), make_dview(lo), make_dview(hi), Gy, Gx, half, nb);
+    else adown_prepool_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(make_dview(x), make_dview(lo), make_dview(hi), Gy, Gx, half, nb);
     YRE_LAUNCH_CHECK("adown_prepool");
     return YRE_OK;
 }
 
-int launch_spp_maxpool(const yre_view& x, const yre_view& y5, const yre_view& y9, const yre_view& y13, cudaStream_t s) {
+int launch_spp_maxpool(const yre_view& x, const yre_view& y5, const yre_view& y9, const yre_view& y13, int nb, cudaStream_t s) {
     if (check8(x, "spp.x") || check8(y5, "spp.y5") || check8(y9, "spp.y9") || check8(y13, "spp.y13")) return YRE_EINVAL;
     const yre_view* ys[3] = {&y5, &y9, &y13};
     for (auto* y : ys)
         if (y->B != x.B || y->H != x.H || y->W != x.W || y->C != x.C || y->dtype != x.dtype || y->layout != YRE_NHWC)
             YRE_FAIL(YRE_EINVAL, "spp: output views must match the input");
     if (x.layout != YRE_NHWC) YRE_FAIL(YRE_EUNSUPPORTED, "spp: NHWC only");
+    if (nb < 1 || nb > x.B) YRE_FAIL(YRE_EINVAL, "spp: %d images outside 1..%d", nb, x.B);
     // bf16 / fp16: plane-resident kernel on 16-byte words, 64 (or 32) channels per CTA when the two 16-bit planes fit in
     // shared memory
     if (x.dtype == YRE_BF16 || x.dtype == YRE_F16) {
@@ -751,7 +753,7 @@ int launch_spp_maxpool(const yre_view& x, const yre_view& y5, const yre_view& y9
                         for (SppFn f : row) YRE_CUDA(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, 112 * 1024));
                     return YRE_OK;
                 })) return e;
-            dim3 pg((unsigned)x.B, (unsigned)(x.C / chk));
+            dim3 pg((unsigned)nb, (unsigned)(x.C / chk));
             const SppFn f = fns[x.dtype == YRE_F16][chk == 64 ? 0 : chk == 32 ? 1 : chk == 16 ? 2 : 3];
             f<<<pg, 1024, smem, s>>>(make_dview(x), make_dview(y5), make_dview(y9), make_dview(y13));
             YRE_LAUNCH_CHECK("spp_plane16");
@@ -771,36 +773,37 @@ int launch_spp_maxpool(const yre_view& x, const yre_view& y5, const yre_view& y9
                 YRE_CUDA(cudaFuncSetAttribute(spp_plane_kernel<__half>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024));
                 return YRE_OK;
             })) return e;
-        dim3 pg((unsigned)x.B, (unsigned)(x.C / chk));
+        dim3 pg((unsigned)nb, (unsigned)(x.C / chk));
         if (x.dtype == YRE_F32) spp_plane_kernel<float><<<pg, 256, smem, s>>>(make_dview(x), make_dview(y5), make_dview(y9), make_dview(y13), chk);
         else if (x.dtype == YRE_F16) spp_plane_kernel<__half><<<pg, 256, smem, s>>>(make_dview(x), make_dview(y5), make_dview(y9), make_dview(y13), chk);
         else spp_plane_kernel<__nv_bfloat16><<<pg, 256, smem, s>>>(make_dview(x), make_dview(y5), make_dview(y9), make_dview(y13), chk);
         YRE_LAUNCH_CHECK("spp_plane");
         return YRE_OK;
     }
-    const long long total = (long long)x.B * x.H * x.W * (x.C / 8);
+    const long long total = (long long)nb * x.H * x.W * (x.C / 8);
     dim3 grid(yre_cdiv(total, 256));
-    if (x.dtype == YRE_F32) spp_kernel<float><<<grid, 256, 0, s>>>(make_dview(x), make_dview(y5), make_dview(y9), make_dview(y13));
-    else if (x.dtype == YRE_F16) spp_kernel<__half><<<grid, 256, 0, s>>>(make_dview(x), make_dview(y5), make_dview(y9), make_dview(y13));
-    else spp_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(make_dview(x), make_dview(y5), make_dview(y9), make_dview(y13));
+    if (x.dtype == YRE_F32) spp_kernel<float><<<grid, 256, 0, s>>>(make_dview(x), make_dview(y5), make_dview(y9), make_dview(y13), nb);
+    else if (x.dtype == YRE_F16) spp_kernel<__half><<<grid, 256, 0, s>>>(make_dview(x), make_dview(y5), make_dview(y9), make_dview(y13), nb);
+    else spp_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(make_dview(x), make_dview(y5), make_dview(y9), make_dview(y13), nb);
     YRE_LAUNCH_CHECK("spp_maxpool");
     return YRE_OK;
 }
 
-int launch_upsample2x(const yre_view& x, const yre_view& y, cudaStream_t s) {
+int launch_upsample2x(const yre_view& x, const yre_view& y, int nb, cudaStream_t s) {
     if (check8(x, "upsample.x") || check8(y, "upsample.y")) return YRE_EINVAL;
     if (y.B != x.B || y.H != 2 * x.H || y.W != 2 * x.W || y.C != x.C || y.dtype != x.dtype)
         YRE_FAIL(YRE_EINVAL, "upsample2x: output must be 2x the input");
-    const long long total = (long long)x.B * x.H * x.W * (x.C / 8);
+    if (nb < 1 || nb > x.B) YRE_FAIL(YRE_EINVAL, "upsample2x: %d images outside 1..%d", nb, x.B);
+    const long long total = (long long)nb * x.H * x.W * (x.C / 8);
     dim3 grid(yre_cdiv(total, 256));
-    if (x.dtype == YRE_F32) upsample2x_kernel<float><<<grid, 256, 0, s>>>(make_dview(x), make_dview(y));
-    else if (x.dtype == YRE_F16) upsample2x_kernel<__half><<<grid, 256, 0, s>>>(make_dview(x), make_dview(y));
-    else upsample2x_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(make_dview(x), make_dview(y));
+    if (x.dtype == YRE_F32) upsample2x_kernel<float><<<grid, 256, 0, s>>>(make_dview(x), make_dview(y), nb);
+    else if (x.dtype == YRE_F16) upsample2x_kernel<__half><<<grid, 256, 0, s>>>(make_dview(x), make_dview(y), nb);
+    else upsample2x_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(make_dview(x), make_dview(y), nb);
     YRE_LAUNCH_CHECK("upsample2x");
     return YRE_OK;
 }
 
-int launch_cbfuse_sum(const yre_view* srcs, int n, const yre_view& tgt, const yre_view& y, cudaStream_t s) {
+int launch_cbfuse_sum(const yre_view* srcs, int n, const yre_view& tgt, const yre_view& y, int nb, cudaStream_t s) {
     if (n < 0 || n > 8) YRE_FAIL(YRE_EUNSUPPORTED, "cbfuse: %d sources (max 8)", n);
     if (check8(tgt, "cbfuse.target") || check8(y, "cbfuse.y")) return YRE_EINVAL;
     FuseSrcs fs; fs.n = n;
@@ -810,19 +813,21 @@ int launch_cbfuse_sum(const yre_view* srcs, int n, const yre_view& tgt, const yr
         fs.v[i] = make_dview(srcs[i]);
     }
     if (tgt.B != y.B || tgt.H != y.H || tgt.W != y.W || tgt.C != y.C || tgt.dtype != y.dtype) YRE_FAIL(YRE_EINVAL, "cbfuse: target mismatch");
-    const long long total = (long long)y.B * y.H * y.W * (y.C / 8);
+    if (nb < 1 || nb > y.B) YRE_FAIL(YRE_EINVAL, "cbfuse: %d images outside 1..%d", nb, y.B);
+    const long long total = (long long)nb * y.H * y.W * (y.C / 8);
     dim3 grid(yre_cdiv(total, 256));
-    if (y.dtype == YRE_F32) cbfuse_kernel<float><<<grid, 256, 0, s>>>(fs, make_dview(tgt), make_dview(y));
-    else if (y.dtype == YRE_F16) cbfuse_kernel<__half><<<grid, 256, 0, s>>>(fs, make_dview(tgt), make_dview(y));
-    else cbfuse_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(fs, make_dview(tgt), make_dview(y));
+    if (y.dtype == YRE_F32) cbfuse_kernel<float><<<grid, 256, 0, s>>>(fs, make_dview(tgt), make_dview(y), nb);
+    else if (y.dtype == YRE_F16) cbfuse_kernel<__half><<<grid, 256, 0, s>>>(fs, make_dview(tgt), make_dview(y), nb);
+    else cbfuse_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(fs, make_dview(tgt), make_dview(y), nb);
     YRE_LAUNCH_CHECK("cbfuse_sum");
     return YRE_OK;
 }
 
-int launch_nchw_to_view(const float* x, const yre_view& y, cudaStream_t s) {
+int launch_nchw_to_view(const float* x, const yre_view& y, int nb, cudaStream_t s) {
     if (!x) YRE_FAIL(YRE_EINVAL, "nchw_to_view: null input");
     if (yre_check_view(&y, "nchw_to_view.y")) return YRE_EINVAL;
-    dim3 grid(yre_cdiv((long long)y.H * y.W, 32), yre_cdiv(y.C, 32), y.B);
+    if (nb < 1 || nb > y.B) YRE_FAIL(YRE_EINVAL, "nchw_to_view: %d images outside 1..%d", nb, y.B);
+    dim3 grid(yre_cdiv((long long)y.H * y.W, 32), yre_cdiv(y.C, 32), nb);
     if (y.dtype == YRE_F32) nchw_to_view_kernel<float><<<grid, 256, 0, s>>>(x, make_dview(y));
     else if (y.dtype == YRE_F16) nchw_to_view_kernel<__half><<<grid, 256, 0, s>>>(x, make_dview(y));
     else nchw_to_view_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(x, make_dview(y));
@@ -830,10 +835,11 @@ int launch_nchw_to_view(const float* x, const yre_view& y, cudaStream_t s) {
     return YRE_OK;
 }
 
-int launch_view_to_nchw(const yre_view& x, float* y, cudaStream_t s) {
+int launch_view_to_nchw(const yre_view& x, float* y, int nb, cudaStream_t s) {
     if (!y) YRE_FAIL(YRE_EINVAL, "view_to_nchw: null output");
     if (yre_check_view(&x, "view_to_nchw.x")) return YRE_EINVAL;
-    dim3 grid(yre_cdiv((long long)x.H * x.W, 32), yre_cdiv(x.C, 32), x.B);
+    if (nb < 1 || nb > x.B) YRE_FAIL(YRE_EINVAL, "view_to_nchw: %d images outside 1..%d", nb, x.B);
+    dim3 grid(yre_cdiv((long long)x.H * x.W, 32), yre_cdiv(x.C, 32), nb);
     if (x.dtype == YRE_F32) view_to_nchw_kernel<float><<<grid, 256, 0, s>>>(make_dview(x), y);
     else if (x.dtype == YRE_F16) view_to_nchw_kernel<__half><<<grid, 256, 0, s>>>(make_dview(x), y);
     else view_to_nchw_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(make_dview(x), y);

@@ -21,10 +21,10 @@ namespace {
 struct StemParams {
     const float* x;
     const uint8_t* xu8;  // non-null: uint8 [B][H][W][3] frames in BGR order (cv2 layout); value / 255 and BGR->RGB fused
-    DView y;
+    DView y;            // y.B is the layout (the parity-plane stride of YRE_PHASE4)
     const float* w;     // [Cout][3][3][Cin]
     const float* bias;
-    int B, Cin, H, W, Ho, Wo, Cout, stride, act;
+    int B, Cin, H, W, Ho, Wo, Cout, stride, act;     // B: the images computed (the first B of y's y.B)
 };
 
 constexpr int PX = 4;   // output pixels per thread (consecutive in x): weights are read once per 4 pixels
@@ -583,17 +583,17 @@ __global__ void __launch_bounds__(128, MINB) stem_mma_s2u8_kernel(const StemPara
 // The stem kernels write output pixels only.  A parity-plane output of an odd extent also has cells without a source
 // pixel (the last row of the planes of odd rows when Ho is odd, the last column of the planes of odd columns when Wo is
 // odd), which a stride-2 conv reads at its last output row and column: they must hold zeros (include/yre.h).  One thread
-// per 8 channels of a cell on the last row or column of a plane.
+// per 8 channels of a cell on the last row or column of a plane, for the first nb images (planes p * y.B + b, b < nb).
 template <typename T>
-__global__ void __launch_bounds__(256) phase4_zero_edges_kernel(const DView y) {
+__global__ void __launch_bounds__(256) phase4_zero_edges_kernel(const DView y, int nb) {
     const int groups = y.C / 8, cells = y.Hp + y.Wp;
-    const long long total = 4LL * y.B * cells * groups;
+    const long long total = 4LL * nb * cells * groups;
     const float z[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
         const int g = (int)(i % groups);
         long long r = i / groups;
         const int cell = (int)(r % cells); r /= cells;
-        const int b = (int)(r % y.B), p = (int)(r / y.B);
+        const int b = (int)(r % nb), p = (int)(r / nb);
         const int py = 2 * (cell < y.Wp ? y.Hp - 1 : cell - y.Wp) + (p >> 1), px = 2 * (cell < y.Wp ? cell : y.Wp - 1) + (p & 1);
         if (py >= y.H || px >= y.W) st8<T>(y.ptr, dview_pix(y, b, py, px) + g * 8, z);
     }
@@ -601,23 +601,23 @@ __global__ void __launch_bounds__(256) phase4_zero_edges_kernel(const DView y) {
 
 }  // namespace
 
-static int launch_stem_pixels(const yre_stem_desc& d, cudaStream_t s);
+static int launch_stem_pixels(const yre_stem_desc& d, int nb, cudaStream_t s);
 
-int launch_stem(const yre_stem_desc& d, cudaStream_t s) {
-    if (int e = launch_stem_pixels(d, s)) return e;
+int launch_stem(const yre_stem_desc& d, int nb, cudaStream_t s) {
+    if (int e = launch_stem_pixels(d, nb, s)) return e;
     if (d.y.layout == YRE_PHASE4 && ((d.y.H | d.y.W) & 1)) {
         const DView y = make_dview(d.y);
-        const long long total = 4LL * y.B * (y.Hp + y.Wp) * (y.C / 8);
+        const long long total = 4LL * nb * (y.Hp + y.Wp) * (y.C / 8);
         const unsigned grid = (unsigned)std::min<long long>(yre_cdiv(total, 256), 1024);
-        if (d.y.dtype == YRE_F32) phase4_zero_edges_kernel<float><<<grid, 256, 0, s>>>(y);
-        else if (d.y.dtype == YRE_F16) phase4_zero_edges_kernel<__half><<<grid, 256, 0, s>>>(y);
-        else phase4_zero_edges_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(y);
+        if (d.y.dtype == YRE_F32) phase4_zero_edges_kernel<float><<<grid, 256, 0, s>>>(y, nb);
+        else if (d.y.dtype == YRE_F16) phase4_zero_edges_kernel<__half><<<grid, 256, 0, s>>>(y, nb);
+        else phase4_zero_edges_kernel<__nv_bfloat16><<<grid, 256, 0, s>>>(y, nb);
         YRE_LAUNCH_CHECK("stem_phase4_edges");
     }
     return YRE_OK;
 }
 
-static int launch_stem_pixels(const yre_stem_desc& d, cudaStream_t s) {
+static int launch_stem_pixels(const yre_stem_desc& d, int nb, cudaStream_t s) {
     const bool u8 = d.x_u8_hwc != nullptr;
     if ((!d.x_nchw && !u8) || !d.w) YRE_FAIL(YRE_EINVAL, "stem: null pointer");
     if (u8 && d.Cin != 3) YRE_FAIL(YRE_EUNSUPPORTED, "stem: uint8 HWC frames need Cin == 3 (got %d)", d.Cin);
@@ -627,14 +627,15 @@ static int launch_stem_pixels(const yre_stem_desc& d, cudaStream_t s) {
     if (d.y.C % 16 || d.y.c_off % 8 || d.y.C_total % 8) YRE_FAIL(YRE_EUNSUPPORTED, "stem: Cout must be a multiple of 16");
     const int Ho = (d.H + 2 - 3) / d.stride + 1, Wo = (d.W + 2 - 3) / d.stride + 1;
     if (Ho != d.y.H || Wo != d.y.W || d.B != d.y.B) YRE_FAIL(YRE_EINVAL, "stem: output extent mismatch");
+    if (nb < 1 || nb > d.B) YRE_FAIL(YRE_EINVAL, "stem: %d images outside 1..%d", nb, d.B);
     StemParams p;
     p.x = d.x_nchw; p.xu8 = d.x_u8_hwc; p.y = make_dview(d.y); p.w = d.w; p.bias = d.bias;
-    p.B = d.B; p.Cin = d.Cin; p.H = d.H; p.W = d.W; p.Ho = Ho; p.Wo = Wo; p.Cout = d.y.C; p.stride = d.stride; p.act = d.act;
+    p.B = nb; p.Cin = d.Cin; p.H = d.H; p.W = d.W; p.Ho = Ho; p.Wo = Wo; p.Cout = d.y.C; p.stride = d.stride; p.act = d.act;
     const bool f16 = d.y.dtype == YRE_F16;
     if (u8 && d.y.dtype != YRE_F32 && d.y.C == 64 && d.stride == 2 && d.W % 16 == 0 &&
         (reinterpret_cast<uintptr_t>(d.y.ptr) & 15) == 0 && (reinterpret_cast<uintptr_t>(d.x_u8_hwc) & 15) == 0) {
         const int segs = yre_cdiv(Wo, SM_PX);
-        const long long tiles = (long long)d.B * Ho * segs;
+        const long long tiles = (long long)nb * Ho * segs;
         int dev = 0, sms = 148;
         cudaGetDevice(&dev);
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -647,7 +648,7 @@ static int launch_stem_pixels(const yre_stem_desc& d, cudaStream_t s) {
     }
     if (!u8 && d.y.dtype != YRE_F32 && d.Cin <= 3 && d.y.C == 64 && (reinterpret_cast<uintptr_t>(d.y.ptr) & 15) == 0) {
         const int segs = yre_cdiv(Wo, SM_PX);
-        const long long tiles = (long long)d.B * Ho * segs;
+        const long long tiles = (long long)nb * Ho * segs;
         int dev = 0, sms = 148;
         cudaGetDevice(&dev);
         cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -667,7 +668,7 @@ static int launch_stem_pixels(const yre_stem_desc& d, cudaStream_t s) {
         YRE_LAUNCH_CHECK("stem_mma");
         return YRE_OK;
     }
-    const long long total = (long long)d.B * Ho * ((Wo + PX - 1) / PX);
+    const long long total = (long long)nb * Ho * ((Wo + PX - 1) / PX);
     const size_t smem = (size_t)(9 * d.Cin + 1) * d.y.C * sizeof(float);
     if (smem > 48 * 1024) YRE_FAIL(YRE_EUNSUPPORTED, "stem: Cout too large for the weight cache");
     dim3 grid(yre_cdiv(total, 128));

@@ -32,19 +32,33 @@ struct Op {
     double flops = 0.0;
 };
 
-int run_op(const Op& o, cudaStream_t s) {
+// the batch an op was recorded for (the B of its views / descriptor)
+int op_batch(const Op& o) {
     switch (o.kind) {
-        case OP_CONV_FFMA: return launch_conv_ffma(o.conv, s);
-        case OP_CONV_TC:   return conv_tc_launch(o.tc, s);
-        case OP_STEM:      return launch_stem(o.stem, s);
-        case OP_ADOWN:     return launch_adown_prepool(o.v[0], o.v[1], o.v[2], s);
-        case OP_SPP:       return launch_spp_maxpool(o.v[0], o.v[1], o.v[2], o.v[3], s);
-        case OP_UP:        return launch_upsample2x(o.v[0], o.v[1], s);
-        case OP_FUSE:      return launch_cbfuse_sum(o.v + 2, o.n_v - 2, o.v[0], o.v[1], s);
-        case OP_TO_VIEW:   return launch_nchw_to_view(o.fin, o.v[0], s);
-        case OP_TO_NCHW:   return launch_view_to_nchw(o.v[0], o.fout, s);
-        case OP_DECODE:    return launch_decode(o.dec, s);
-        case OP_NMS:       return launch_nms(o.nms, s);
+        case OP_CONV_FFMA:
+        case OP_CONV_TC:   return o.conv.y.B;
+        case OP_STEM:      return o.stem.y.B;
+        case OP_DECODE:    return o.dec.raw[0].B;
+        case OP_NMS:       return o.nms.B;
+        case OP_FUSE:      return o.v[1].B;
+        default:           return o.v[0].B;
+    }
+}
+
+// launches op o for its first nb images (nb == op_batch(o): the whole batch)
+int run_op(Op& o, int nb, cudaStream_t s) {
+    switch (o.kind) {
+        case OP_CONV_FFMA: return launch_conv_ffma(o.conv, nb, s);
+        case OP_CONV_TC:   return conv_tc_launch(o.tc, nb, s);
+        case OP_STEM:      return launch_stem(o.stem, nb, s);
+        case OP_ADOWN:     return launch_adown_prepool(o.v[0], o.v[1], o.v[2], nb, s);
+        case OP_SPP:       return launch_spp_maxpool(o.v[0], o.v[1], o.v[2], o.v[3], nb, s);
+        case OP_UP:        return launch_upsample2x(o.v[0], o.v[1], nb, s);
+        case OP_FUSE:      return launch_cbfuse_sum(o.v + 2, o.n_v - 2, o.v[0], o.v[1], nb, s);
+        case OP_TO_VIEW:   return launch_nchw_to_view(o.fin, o.v[0], nb, s);
+        case OP_TO_NCHW:   return launch_view_to_nchw(o.v[0], o.fout, nb, s);
+        case OP_DECODE:    return launch_decode(o.dec, nb, s);
+        case OP_NMS:       return launch_nms(o.nms, nb, s);
     }
     return YRE_EINVAL;
 }
@@ -142,7 +156,7 @@ int yre_device_check(void) {
 int yre_conv(const yre_conv_desc* d, yre_stream_t s) {
     Op o;
     if (int e = make_conv_op(d, o)) return e;
-    const int r = run_op(o, (cudaStream_t)s);
+    const int r = run_op(o, d->y.B, (cudaStream_t)s);
     if (o.tc) {   // the tensor maps are kernel parameters (copied at launch), safe to free now
         conv_tc_free(o.tc);
     }
@@ -151,39 +165,39 @@ int yre_conv(const yre_conv_desc* d, yre_stream_t s) {
 
 int yre_stem_conv(const yre_stem_desc* d, yre_stream_t s) {
     if (!d) YRE_FAIL(YRE_EINVAL, "stem: null descriptor");
-    return launch_stem(*d, (cudaStream_t)s);
+    return launch_stem(*d, d->B, (cudaStream_t)s);
 }
 int yre_adown_prepool(const yre_view* x, const yre_view* lo, const yre_view* hi, yre_stream_t s) {
     if (!x || !lo || !hi) YRE_FAIL(YRE_EINVAL, "adown: null view");
-    return launch_adown_prepool(*x, *lo, *hi, (cudaStream_t)s);
+    return launch_adown_prepool(*x, *lo, *hi, x->B, (cudaStream_t)s);
 }
 int yre_spp_maxpool(const yre_view* x, const yre_view* y5, const yre_view* y9, const yre_view* y13, yre_stream_t s) {
     if (!x || !y5 || !y9 || !y13) YRE_FAIL(YRE_EINVAL, "spp: null view");
-    return launch_spp_maxpool(*x, *y5, *y9, *y13, (cudaStream_t)s);
+    return launch_spp_maxpool(*x, *y5, *y9, *y13, x->B, (cudaStream_t)s);
 }
 int yre_upsample2x(const yre_view* x, const yre_view* y, yre_stream_t s) {
     if (!x || !y) YRE_FAIL(YRE_EINVAL, "upsample2x: null view");
-    return launch_upsample2x(*x, *y, (cudaStream_t)s);
+    return launch_upsample2x(*x, *y, x->B, (cudaStream_t)s);
 }
 int yre_cbfuse_sum(const yre_view* srcs, int32_t n, const yre_view* t, const yre_view* y, yre_stream_t s) {
     if ((!srcs && n > 0) || !t || !y) YRE_FAIL(YRE_EINVAL, "cbfuse: null view");
-    return launch_cbfuse_sum(srcs, n, *t, *y, (cudaStream_t)s);
+    return launch_cbfuse_sum(srcs, n, *t, *y, y->B, (cudaStream_t)s);
 }
 int yre_nchw_to_view(const float* x, const yre_view* y, yre_stream_t s) {
     if (!y) YRE_FAIL(YRE_EINVAL, "nchw_to_view: null view");
-    return launch_nchw_to_view(x, *y, (cudaStream_t)s);
+    return launch_nchw_to_view(x, *y, y->B, (cudaStream_t)s);
 }
 int yre_view_to_nchw(const yre_view* x, float* y, yre_stream_t s) {
     if (!x) YRE_FAIL(YRE_EINVAL, "view_to_nchw: null view");
-    return launch_view_to_nchw(*x, y, (cudaStream_t)s);
+    return launch_view_to_nchw(*x, y, x->B, (cudaStream_t)s);
 }
 int yre_dfl_decode_score(const yre_decode_desc* d, yre_stream_t s) {
     if (!d) YRE_FAIL(YRE_EINVAL, "decode: null descriptor");
-    return launch_decode(*d, (cudaStream_t)s);
+    return launch_decode(*d, d->raw[0].B, (cudaStream_t)s);
 }
 int yre_nms_batched(const yre_nms_desc* d, yre_stream_t s) {
     if (!d) YRE_FAIL(YRE_EINVAL, "nms: null descriptor");
-    return launch_nms(*d, (cudaStream_t)s);
+    return launch_nms(*d, d->B, (cudaStream_t)s);
 }
 
 // ---- plan -----------------------------------------------------------------------------------------
@@ -333,14 +347,32 @@ int yre_plan_rebind(yre_plan* p, const void* old_ptr, void* new_ptr) {
 
 int yre_plan_run(yre_plan* p, yre_stream_t s) {
     PLAN_GUARD(p);
-    for (size_t i = 0; i < p->ops.size(); ++i)
-        if (int e = run_op(p->ops[i], (cudaStream_t)s)) return e;
+    for (auto& o : p->ops)
+        if (int e = run_op(o, op_batch(o), (cudaStream_t)s)) return e;
+    return YRE_OK;
+}
+int yre_plan_batch_capacity(const yre_plan* p) {
+    PLAN_GUARD(p);
+    if (p->ops.empty()) YRE_FAIL(YRE_EINVAL, "plan_batch_capacity: the plan has no ops");
+    const int b = op_batch(p->ops[0]);
+    for (size_t i = 1; i < p->ops.size(); ++i)
+        if (op_batch(p->ops[i]) != b)
+            YRE_FAIL(YRE_EINVAL, "plan_batch_capacity: op %zu (%s) was recorded for %d images, op 0 (%s) for %d", i,
+                     op_name(p->ops[i].kind), op_batch(p->ops[i]), op_name(p->ops[0].kind), b);
+    return b;
+}
+int yre_plan_run_batch(yre_plan* p, int32_t n, yre_stream_t s) {
+    const int cap = yre_plan_batch_capacity(p);
+    if (cap < 0) return cap;
+    if (n < 1 || n > cap) YRE_FAIL(YRE_EINVAL, "plan_run_batch: %d images, the plan holds 1..%d", n, cap);
+    for (auto& o : p->ops)
+        if (int e = run_op(o, n, (cudaStream_t)s)) return e;
     return YRE_OK;
 }
 int yre_plan_run_op(yre_plan* p, int32_t i, yre_stream_t s) {
     PLAN_GUARD(p);
     if (i < 0 || (size_t)i >= p->ops.size()) YRE_FAIL(YRE_EINVAL, "plan_run_op: index %d out of range", i);
-    return run_op(p->ops[i], (cudaStream_t)s);
+    return run_op(p->ops[i], op_batch(p->ops[i]), (cudaStream_t)s);
 }
 int yre_plan_num_ops(const yre_plan* p) { return p ? (int)p->ops.size() : 0; }
 int yre_plan_num_launches(const yre_plan* p) {

@@ -178,22 +178,23 @@ __device__ __forceinline__ float silu_tanh(float x) {
 struct ConvTcPlan;   // pre-encoded tensor maps + tile config of one tcgen05 conv (k_conv_tc.cu)
 
 int check_conv(const yre_conv_desc* d);                                     // descriptor validation shared by every conv entry point
-int launch_conv_ffma(const yre_conv_desc& d, cudaStream_t s);
+// Every launcher takes nb, the number of images to compute (1 <= nb <= the views' B): the first nb images of the batch the
+// views describe.  nb bounds grids and loops only; a view's B stays its layout (the parity-plane stride of YRE_PHASE4).
+int launch_conv_ffma(const yre_conv_desc& d, int nb, cudaStream_t s);
 int conv_tc_eligible(const yre_conv_desc& d, char* why, size_t why_len);
 int conv_tc_prepare(const yre_conv_desc& d, ConvTcPlan** out);
-int conv_tc_launch(const ConvTcPlan* p, cudaStream_t s);
+int conv_tc_launch(ConvTcPlan* p, int nb, cudaStream_t s);
 void conv_tc_free(ConvTcPlan* p);
-void conv_tc_set_reverse(ConvTcPlan* p, int rev);
+void conv_tc_set_reverse(ConvTcPlan* p, int rev);                          // walk the M tiles last-to-first
 void conv_tc_describe(const ConvTcPlan* p, char* out, size_t n);          // kernel variant + tile shape, for yre_plan_op_variant
-                        // walk the M tiles last-to-first
 int conv_tc_rebind(ConvTcPlan* p, const void* old_ptr, void* new_ptr);   // patches y/res only
-int launch_stem(const yre_stem_desc& d, cudaStream_t s);
-int launch_adown_prepool(const yre_view& x, const yre_view& avg_lo, const yre_view& max_hi, cudaStream_t s);
-int launch_spp_maxpool(const yre_view& x, const yre_view& y5, const yre_view& y9, const yre_view& y13, cudaStream_t s);
-int launch_upsample2x(const yre_view& x, const yre_view& y, cudaStream_t s);
-int launch_cbfuse_sum(const yre_view* srcs, int n, const yre_view& target, const yre_view& y, cudaStream_t s);
-int launch_nchw_to_view(const float* x, const yre_view& y, cudaStream_t s);
-int launch_view_to_nchw(const yre_view& x, float* y, cudaStream_t s);
-int launch_decode(const yre_decode_desc& d, cudaStream_t s);
-int launch_nms(const yre_nms_desc& d, cudaStream_t s);   // 3 launches (memset kernel, filter, sort+scan)
+int launch_stem(const yre_stem_desc& d, int nb, cudaStream_t s);
+int launch_adown_prepool(const yre_view& x, const yre_view& avg_lo, const yre_view& max_hi, int nb, cudaStream_t s);
+int launch_spp_maxpool(const yre_view& x, const yre_view& y5, const yre_view& y9, const yre_view& y13, int nb, cudaStream_t s);
+int launch_upsample2x(const yre_view& x, const yre_view& y, int nb, cudaStream_t s);
+int launch_cbfuse_sum(const yre_view* srcs, int n, const yre_view& target, const yre_view& y, int nb, cudaStream_t s);
+int launch_nchw_to_view(const float* x, const yre_view& y, int nb, cudaStream_t s);
+int launch_view_to_nchw(const yre_view& x, float* y, int nb, cudaStream_t s);
+int launch_decode(const yre_decode_desc& d, int nb, cudaStream_t s);
+int launch_nms(const yre_nms_desc& d, int nb, cudaStream_t s);   // 3 launches (memset kernel, filter, sort+scan)
 double conv_flops(const yre_conv_desc& d);

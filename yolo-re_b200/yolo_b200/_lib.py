@@ -27,6 +27,14 @@ class ConvDesc(C.Structure):
                 ("k", C.c_int32), ("stride", C.c_int32), ("act", C.c_int32), ("engine", C.c_int32), ("xu", View)]
 
 
+TC_GENERIC, TC_GENERIC_CTA2, TC_HALO_WS, TC_HALO_STREAM = 0, 1, 2, 3
+
+
+class TcSchedule(C.Structure):
+    _fields_ = [(n, C.c_int32) for n in ("kind", "ybx", "tw", "th", "tb", "block_n", "tiles_x", "tiles_y", "tiles_b", "tiles_n",
+                                         "mtiles", "npair", "upn", "work", "grid")]
+
+
 class StemDesc(C.Structure):
     _fields_ = [("x_nchw", C.c_void_p), ("B", C.c_int32), ("Cin", C.c_int32), ("H", C.c_int32), ("W", C.c_int32),
                 ("y", View), ("w", C.c_void_p), ("bias", C.c_void_p), ("stride", C.c_int32), ("act", C.c_int32),
@@ -68,6 +76,7 @@ SYMBOLS = {
     "yre_device_check": (C.c_int, []),
     "yre_conv": (C.c_int, [C.POINTER(ConvDesc), C.c_void_p]),
     "yre_conv_tc_describe": (C.c_int, [C.POINTER(ConvDesc), C.c_int32, C.c_char_p, C.c_int32]),
+    "yre_conv_tc_schedule": (C.c_int, [C.POINTER(ConvDesc), C.c_int32, C.c_int32, C.POINTER(TcSchedule)]),
     "yre_stem_conv": (C.c_int, [C.POINTER(StemDesc), C.c_void_p]),
     "yre_adown_prepool": (C.c_int, [C.POINTER(View)] * 3 + [C.c_void_p]),
     "yre_spp_maxpool": (C.c_int, [C.POINTER(View)] * 4 + [C.c_void_p]),
@@ -100,6 +109,8 @@ SYMBOLS = {
     "yre_plan_add_nms": (C.c_int, [C.c_void_p, C.POINTER(NmsDesc)]),
     "yre_plan_rebind": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "yre_plan_run": (C.c_int, [C.c_void_p, C.c_void_p]),
+    "yre_plan_run_batch": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p]),
+    "yre_plan_batch_capacity": (C.c_int, [C.c_void_p]),
     "yre_plan_run_op": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p]),
     "yre_plan_num_launches": (C.c_int, [C.c_void_p]),
     "yre_plan_num_ops": (C.c_int, [C.c_void_p]),

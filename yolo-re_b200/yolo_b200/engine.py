@@ -255,9 +255,10 @@ class Plan:
             _check_f16_range(w, self.name_of(m))
         u8 = x.dtype == torch.uint8
         if u8:
-            Bn, H, W, Cin = x.shape
+            _, H, W, Cin = x.shape
         else:
-            Bn, Cin, H, W = x.shape
+            _, Cin, H, W = x.shape
+        Bn = self.batch                          # x may hold fewer images: a plan compiled for a batch capacity
         Ho, Wo = _conv_out(H, 3, s), _conv_out(W, 3, s)
         out = self.alloc(Ho, Wo, w.shape[0], layout=L.PHASE4 if phase4 else L.NHWC)
         wp = self.dev(w.permute(0, 2, 3, 1), torch.float32)
@@ -449,9 +450,22 @@ class Plan:
         if r < 0:
             L.check(r, "plan_rebind")
 
-    def run(self) -> None:
+    def run(self, n: int | None = None) -> None:
+        """Runs the launch list for all ``batch`` images, or for the first n of them (yre_plan_run_batch: bit-identical
+        results for those n, no row of a later image is written, shorter launches)."""
         s = torch.cuda.current_stream(self.device).cuda_stream
-        L.check(self.lib.yre_plan_run(self.h, s), "plan_run")
+        if n is None:
+            L.check(self.lib.yre_plan_run(self.h, s), "plan_run")
+        else:
+            L.check(self.lib.yre_plan_run_batch(self.h, n, s), "plan_run_batch")
+
+    @property
+    def capacity(self) -> int:
+        """The most images one run computes (the batch every op was recorded for)."""
+        r = self.lib.yre_plan_batch_capacity(self.h)
+        if r < 0:
+            L.check(r, "plan_batch_capacity")
+        return r
 
     @property
     def num_launches(self) -> int:
@@ -604,12 +618,14 @@ def _weights_version(model: nn.Module) -> int:
     return hash(tuple([(t.data_ptr(), t._version) for t in ts[1]]))
 
 
-def compile_model(model, x: torch.Tensor) -> Plan:
-    """Compiles the whole YOLO graph for x's shape/device (x: fp32 [B,C,H,W] or uint8 [B,H,W,3] BGR frames)."""
+def compile_model(model, x: torch.Tensor, capacity: int | None = None) -> Plan:
+    """Compiles the whole YOLO graph for x's shape/device (x: fp32 [B,C,H,W] or uint8 [B,H,W,3] BGR frames).
+    capacity: compile for that many images instead of x's B (x may hold fewer; the plan runs any 1..capacity of them)."""
     if x.dtype == torch.uint8:
         Bn, H, W, Cin = x.shape
     else:
         Bn, Cin, H, W = x.shape
+    Bn = Bn if capacity is None else capacity
     wire = wire_model(model, H, W, Cin)
     p = Plan(x.device, Bn, model.precision)
     p.names = {id(m): n for n, m in model.named_modules()}
@@ -647,26 +663,33 @@ def compile_model(model, x: torch.Tensor) -> Plan:
     return p
 
 
-def _fresh(p: Plan, o):
-    """o (an output tensor, a raw-logit window or a list of them) re-pointed to new tensors that the plan writes"""
+def _fresh(p: Plan, o, rows: int | None = None):
+    """o (an output tensor, a raw-logit window or a list of them) re-pointed to new tensors that the plan writes, of
+    `rows` images (default: the plan's batch; a run of n images writes rows [:n] only)"""
     if isinstance(o, list):
-        return [_fresh(p, e) for e in o]
+        return [_fresh(p, e, rows) for e in o]
     if isinstance(o, V):
-        o.t = _fresh(p, o.t)
+        o.t = _fresh(p, o.t, rows)
         return o
-    n = torch.empty_like(o)
+    n = torch.empty((p.batch if rows is None else rows,) + tuple(o.shape[1:]), dtype=o.dtype, device=o.device)
     p.rebind(o.data_ptr(), n.data_ptr())
     return n
 
 
-def _replay_graph(p: Plan, x: torch.Tensor) -> None:
+def _rows(o) -> int:
+    """images held by the output tensors of a head result (y, or the first of a dual head's)"""
+    return _rows(o[0]) if isinstance(o, list) else o.shape[0]
+
+
+def _replay_graph(p: Plan, x: torch.Tensor, n: int | None = None) -> None:
     """Static-buffer mode: the whole launch list (incl. its programmatic-dependent-launch edges) is captured once per
-    input BUFFER into a CUDA graph and replayed -- no per-launch CPU work, ~1 us between kernels.  Meant for callers
-    that reuse a few input buffers (a double-buffered upload ring): every new buffer address costs a warm-up run and a
-    capture.  At most 8 (graph, buffer) pairs are held; the oldest pair is dropped together, so a caller that passes
-    a fresh tensor every time pays the capture each call but does not accumulate memory."""
+    input BUFFER (and image count n of a plan with a batch capacity, None: the whole batch) into a CUDA graph and
+    replayed -- no per-launch CPU work, ~1 us between kernels.  Meant for callers that reuse a few input buffers (a
+    double-buffered upload ring): every new buffer address costs a warm-up run and a capture.  At most 8 (graph, buffer)
+    pairs are held; the oldest pair is dropped together, so a caller that passes a fresh tensor every time pays the
+    capture each call but does not accumulate memory."""
     graphs = p.__dict__.setdefault("graphs", {})
-    key = x.data_ptr()
+    key = (x.data_ptr(), n)
     ent = graphs.get(key)
     g = ent[0] if ent is not None else None
     if g is None:
@@ -674,11 +697,11 @@ def _replay_graph(p: Plan, x: torch.Tensor) -> None:
         side = torch.cuda.Stream(p.device)
         side.wait_stream(cur)
         with torch.cuda.stream(side):
-            p.run()                                  # warm-up outside capture: one-time function attributes, lazy module load
+            p.run(n)                                 # warm-up outside capture: one-time function attributes, lazy module load
         cur.wait_stream(side)
         g = torch.cuda.CUDAGraph()
         with torch.cuda.graph(g):
-            p.run()
+            p.run(n)
         if len(graphs) >= 8:
             graphs.pop(next(iter(graphs)))           # drops the graph AND the input buffer it pinned
         graphs[key] = (g, x)                         # the captured graph reads this buffer: keep it alive with the graph
@@ -698,28 +721,63 @@ def model_forward(model, x: torch.Tensor):
         x = x.contiguous()
     else:
         x = x.contiguous().float()
-    key = (tuple(x.shape), x.dtype, x.device.index, model.precision, bool(getattr(model, "fuse_upsample", True)),
-           bool(getattr(model, "main_only", False)))
+    cap = _capacity(model, x)
+    key = plan_key(model, x)
     p = model._plans.get(key)
     if p is not None and model.check_weights and p.weight_version != _weights_version(model):
         p = None
+    n = None if cap is None else x.shape[0]          # None: the plan's whole batch, x's own
     with torch.cuda.device(x.device):
         if p is None:
-            p = compile_model(model, x)
+            p = compile_model(model, x, capacity=cap)
             model._plans[key] = p
         elif p.in_ptr != x.data_ptr():
             p.rebind(p.in_ptr, x.data_ptr())
             p.in_ptr = x.data_ptr()
+        kind, y, raws = p.result
         if model.fresh_outputs:
-            # the reference returns new tensors every call: re-point the plan's outputs
-            kind, y, raws = p.result
+            # the reference returns new tensors every call: re-point the plan's outputs (to n-image tensors for a run of
+            # n images -- nothing past row n is written)
+            p.result = (kind, _fresh(p, y, n), _fresh(p, raws, n))
+        elif _rows(y) != p.batch:
+            # static buffers after fresh outputs of fewer images: back to buffers that hold the whole batch
             p.result = (kind, _fresh(p, y), _fresh(p, raws))
         if getattr(model, "use_cuda_graph", False) and not model.fresh_outputs:
-            _replay_graph(p, x)
+            _replay_graph(p, x, n)
         else:
-            p.run()
+            p.run(n)
     p.x_keepalive = x
-    return _head_outputs(p.result)
+    out = _head_outputs(p.result)
+    return out if n is None or model.fresh_outputs else _first_rows(out, n)
+
+
+def _capacity(model, x: torch.Tensor) -> int | None:
+    """model.max_batch after checking x's batch against it (None: no capacity, plans are compiled per batch size)"""
+    cap = getattr(model, "max_batch", None)
+    if cap is None:
+        return None
+    if int(cap) < 1:
+        raise ValueError(f"model.max_batch must be a positive image count or None (got {cap})")
+    if not 1 <= x.shape[0] <= cap:
+        raise ValueError(f"a forward of {x.shape[0]} images: this model runs 1..{cap} images per forward "
+                         f"(model.max_batch = {cap})")
+    return int(cap)
+
+
+def plan_key(model, x: torch.Tensor) -> tuple:
+    """The key of the plan model_forward runs x on: x's shape (its batch replaced by model.max_batch when that is set),
+    dtype and device, and the engine settings that change what is compiled."""
+    cap = getattr(model, "max_batch", None)
+    shape = tuple(x.shape) if cap is None else (int(cap),) + tuple(x.shape[1:])
+    return (shape, x.dtype, x.device.index, model.precision, bool(getattr(model, "fuse_upsample", True)),
+            bool(getattr(model, "main_only", False)))
+
+
+def _first_rows(obj, n: int):
+    """rows [:n] of every tensor of a forward's value"""
+    if isinstance(obj, torch.Tensor):
+        return obj[:n]
+    return type(obj)(_first_rows(o, n) for o in obj)
 
 
 def _head_outputs(result):

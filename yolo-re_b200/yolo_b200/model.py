@@ -120,6 +120,10 @@ class YOLO(nn.Module):
         self.check_weights = True        # re-fold when a parameter was modified in place
         self.use_cuda_graph = False      # with fresh_outputs=False: capture the launch list once per input buffer and replay it
         self.main_only = False           # dual-head models: True compiles the main branch only -> (y, raws) like a single head
+        # None: one plan per input shape (batch size included).  N: one plan compiled for N images serves every forward of
+        # 1..N images (same results as the first n images of a full run, shorter launches, one set of buffers); a larger
+        # batch raises ValueError
+        self.max_batch: int | None = None
         self._plans: dict = {}
         self.register_load_state_dict_post_hook(lambda m, _k: m.invalidate())
 
