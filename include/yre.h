@@ -291,6 +291,63 @@ typedef struct yre_match_desc {
 } yre_match_desc;
 int yre_match_detections(const yre_match_desc* d, yre_stream_t s);
 
+/* ---- K12/K13: test-time augmentation (YOLOv5/v8/v9 `model(x, augment=True)`) -----------------------------
+ * Upstream's _forward_augment runs the batch at three branches (s, flip) = (1, none), (0.83, left-right), (0.67, none)
+ * and concatenates their decoded predictions before NMS:
+ *   scale_img       flip the width axis (branch 1), F.interpolate(bilinear, align_corners=False) to (int(h s), int(w s)),
+ *                   F.pad(value=0.447) right and bottom to (ceil(h s / 32) 32, ceil(w s / 32) 32)
+ *   _descale_pred   columns 0..3 / s (fp32), x = w - x for the flipped branch (w: the ORIGINAL width)
+ *   _clip_augmented g = 21 (1 + 4 + 16, three levels): branch 0 drops its last A0 / g anchors (P5), branch 2 its first
+ *                   16 (A2 / g) (P3); exact for every stride-32 rectangle.
+ * oracle/tta_ref.py restates the definition.
+ *
+ * Host-only: the branch geometry of an h x w input (positive multiples of 32, at most 65536).  YRE_EINVAL otherwise. */
+#define YRE_TTA_BRANCHES 3
+typedef struct yre_tta_geom {
+    int32_t h, w;                        /* the input */
+    float   scale[YRE_TTA_BRANCHES];     /* (float)s: 1, 0.83, 0.67 */
+    int32_t flip[YRE_TTA_BRANCHES];      /* 0, 1, 0 */
+    int32_t rh[YRE_TTA_BRANCHES], rw[YRE_TTA_BRANCHES];         /* resized extent int(h s) x int(w s) */
+    int32_t out_h[YRE_TTA_BRANCHES], out_w[YRE_TTA_BRANCHES];   /* padded branch input, multiples of 32 */
+    int32_t A[YRE_TTA_BRANCHES];         /* anchors of the branch's y (strides 8, 16, 32) */
+    int32_t a_begin[YRE_TTA_BRANCHES], a_end[YRE_TTA_BRANCHES];  /* anchor window kept by _clip_augmented */
+    int32_t A_tot;                       /* sum of the windows */
+} yre_tta_geom;
+int yre_tta_geometry(int32_t h, int32_t w, yre_tta_geom* out);
+/* K12: one branch's input.  x: fp32 NCHW RGB [B][3][H][W] (x_nchw) or uint8 BGR frames [B][H][W][3] (x_u8_hwc, the
+ * other NULL; the value is (float)v / 255 with channel c read from byte 2 - c, as K8's fp32 mode and the uint8 stem).
+ * y: fp32 NCHW [B][3][out_h][out_w]; the first n (1 <= n <= B) images are written.  Pixel (Y, X) with Y < rh, X < rw is
+ * the bilinear sample of the (flipped) source, in fp32 without contraction:
+ *   scale = (float)in / out;  src = max(scale (d + 0.5) - 0.5, 0);  i0 = (int)src;  i1 = i0 + (i0 < in - 1);
+ *   l1 = src - i0;  l0 = 1 - l1;  v = hl0 (wl0 v00 + wl1 v01) + hl1 (wl0 v10 + wl1 v11)
+ * every other pixel is 0.447f.  Pointers 4-byte aligned; 1 <= rh <= out_h, 1 <= rw <= out_w. */
+typedef struct yre_tta_scale_desc {
+    const float*   x_nchw;
+    const uint8_t* x_u8_hwc;
+    int32_t        B, n, H, W;
+    int32_t        flip;             /* 1: mirror the width axis before the resize */
+    int32_t        rh, rw;
+    int32_t        out_h, out_w;
+    float*         y;
+} yre_tta_scale_desc;
+int yre_tta_scale_img(const yre_tta_scale_desc* d, yre_stream_t s);
+/* K13: the merged predictions.  Branch i's y: fp32 [B][A_i][4+nc] (the K6 layout), rows [a_begin, a_end) of each of the
+ * first n images are written, in branch order, to out fp32 [B][A_tot][4+nc], A_tot = sum of the windows:
+ *   columns 0..3 / scale (fp32 division); then, when flip_w != 0, column 0 = (float)flip_w - column 0; classes copied.
+ * y and out 16-byte aligned, 1 <= nc <= 4096, 1 <= n <= B, 0 <= a_begin < a_end <= A_i, scale > 0, flip_w >= 0. */
+typedef struct yre_tta_merge_branch {
+    const float* y;
+    int32_t      A, a_begin, a_end;
+    float        scale;
+    int32_t      flip_w;
+} yre_tta_merge_branch;
+typedef struct yre_tta_merge_desc {
+    yre_tta_merge_branch br[YRE_TTA_BRANCHES];
+    int32_t              B, n, nc;
+    float*               out;
+} yre_tta_merge_desc;
+int yre_tta_merge(const yre_tta_merge_desc* d, yre_stream_t s);
+
 /* ---- flat launch plan -------------------------------------------------------------------------
  * Replaces the named-DAG interpreter loop of YOLO.forward  src/yolo/model/model.py:87-107
  * The host walks the module tree once, records every op (descriptors are copied, TMA tensor

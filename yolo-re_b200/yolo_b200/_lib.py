@@ -69,6 +69,28 @@ class MatchDesc(C.Structure):
                 ("gt_cls", C.c_void_p), ("gt_off", C.c_void_p), ("B", C.c_int32), ("n_thr", C.c_int32), ("thr", C.c_double * 16),
                 ("max_gt_per_image", C.c_int32), ("tp", C.c_void_p)]
 
+
+TTA_BRANCHES = 3
+
+
+class TtaGeom(C.Structure):
+    _fields_ = [("h", C.c_int32), ("w", C.c_int32), ("scale", C.c_float * TTA_BRANCHES), ("flip", C.c_int32 * TTA_BRANCHES)] + \
+               [(n, C.c_int32 * TTA_BRANCHES) for n in ("rh", "rw", "out_h", "out_w", "A", "a_begin", "a_end")] + [("A_tot", C.c_int32)]
+
+
+class TtaScaleDesc(C.Structure):
+    _fields_ = [("x_nchw", C.c_void_p), ("x_u8_hwc", C.c_void_p)] + \
+               [(n, C.c_int32) for n in ("B", "n", "H", "W", "flip", "rh", "rw", "out_h", "out_w")] + [("y", C.c_void_p)]
+
+
+class TtaMergeBranch(C.Structure):
+    _fields_ = [("y", C.c_void_p), ("A", C.c_int32), ("a_begin", C.c_int32), ("a_end", C.c_int32), ("scale", C.c_float),
+                ("flip_w", C.c_int32)]
+
+
+class TtaMergeDesc(C.Structure):
+    _fields_ = [("br", TtaMergeBranch * TTA_BRANCHES), ("B", C.c_int32), ("n", C.c_int32), ("nc", C.c_int32), ("out", C.c_void_p)]
+
 # name -> (restype, argtypes); every symbol include/yre.h declares
 SYMBOLS = {
     "yre_version": (C.c_int, []),
@@ -95,6 +117,9 @@ SYMBOLS = {
     "yre_letterbox_u8_batch": (C.c_int, [C.POINTER(LetterboxDesc), C.c_int32, C.c_void_p]),
     "yre_scale_boxes": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_void_p]),
     "yre_match_detections": (C.c_int, [C.POINTER(MatchDesc), C.c_void_p]),
+    "yre_tta_geometry": (C.c_int, [C.c_int32, C.c_int32, C.POINTER(TtaGeom)]),
+    "yre_tta_scale_img": (C.c_int, [C.POINTER(TtaScaleDesc), C.c_void_p]),
+    "yre_tta_merge": (C.c_int, [C.POINTER(TtaMergeDesc), C.c_void_p]),
     "yre_plan_create": (C.c_int, [C.POINTER(C.c_void_p)]),
     "yre_plan_destroy": (None, [C.c_void_p]),
     "yre_plan_add_conv": (C.c_int, [C.c_void_p, C.POINTER(ConvDesc)]),

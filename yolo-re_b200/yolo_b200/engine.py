@@ -546,8 +546,9 @@ class Wire(NamedTuple):
     phase4: bool                     # a stem that writes parity planes for the stride-2 3x3 conv reading it
 
 
-def wire_model(model, H: int, W: int, Cin: int) -> dict[str, Wire]:
-    """The wiring of model.layers / model.connections for an H x W x Cin image, by layer name; it touches no tensor."""
+def wire_model(model, H: int, W: int, Cin: int, main_only: bool | None = None) -> dict[str, Wire]:
+    """The wiring of model.layers / model.connections for an H x W x Cin image, by layer name; it touches no tensor.
+    main_only: None follows model.main_only."""
     layers, names, conn = model.layers, list(model.layers.keys()), model.connections
     srcs = {n: ([conn[n]] if isinstance(conn[n], str) else list(conn[n])) for n in names}
     consumers: dict[str, list[str]] = {n: [] for n in ["input", *names]}
@@ -586,7 +587,7 @@ def wire_model(model, H: int, W: int, Cin: int) -> dict[str, Wire]:
     needed, head = set(names), names[-1]
     if not isinstance(layers[head], (DetectDFL, DualDetectDFL)):
         raise L.YreError("the last layer of the model must be a detection head")
-    if getattr(model, "main_only", False) and isinstance(layers[head], DualDetectDFL):
+    if _main_only(model, main_only) and isinstance(layers[head], DualDetectDFL):
         srcs[head] = srcs[head][layers[head].num_levels:]
         needed = {head}
         for n in reversed(names):                 # a layer comes after every layer it reads
@@ -618,15 +619,21 @@ def _weights_version(model: nn.Module) -> int:
     return hash(tuple([(t.data_ptr(), t._version) for t in ts[1]]))
 
 
-def compile_model(model, x: torch.Tensor, capacity: int | None = None) -> Plan:
+def _main_only(model, main_only: bool | None = None) -> bool:
+    """main_only, or model.main_only when it is None"""
+    return bool(getattr(model, "main_only", False)) if main_only is None else bool(main_only)
+
+
+def compile_model(model, x: torch.Tensor, capacity: int | None = None, main_only: bool | None = None) -> Plan:
     """Compiles the whole YOLO graph for x's shape/device (x: fp32 [B,C,H,W] or uint8 [B,H,W,3] BGR frames).
-    capacity: compile for that many images instead of x's B (x may hold fewer; the plan runs any 1..capacity of them)."""
+    capacity: compile for that many images instead of x's B (x may hold fewer; the plan runs any 1..capacity of them).
+    main_only: None follows model.main_only."""
     if x.dtype == torch.uint8:
         Bn, H, W, Cin = x.shape
     else:
         Bn, Cin, H, W = x.shape
     Bn = Bn if capacity is None else capacity
-    wire = wire_model(model, H, W, Cin)
+    wire = wire_model(model, H, W, Cin, main_only)
     p = Plan(x.device, Bn, model.precision)
     p.names = {id(m): n for n, m in model.named_modules()}
 
@@ -648,7 +655,7 @@ def compile_model(model, x: torch.Tensor, capacity: int | None = None) -> Plan:
             continue
         ins = [vals[s] for s in w.srcs if not wire[s].lazy]
         if isinstance(m, (DetectDFL, DualDetectDFL)):
-            p.result = p.detect(m, ins, main_only=getattr(model, "main_only", False))
+            p.result = p.detect(m, ins, main_only=_main_only(model, main_only))
         elif isinstance(m, B.Concat):
             vals[n] = p.concat(ins, cat_buf(n))
             up = wire[w.srcs[0]]
@@ -708,7 +715,7 @@ def _replay_graph(p: Plan, x: torch.Tensor, n: int | None = None) -> None:
     g.replay()
 
 
-def model_forward(model, x: torch.Tensor):
+def model_forward(model, x: torch.Tensor, augment: bool = False):
     if not x.is_cuda:
         raise L.YreError("the yolo-re B200 path runs on CUDA tensors only (there is no CPU fallback)")
     if x.dim() != 4:
@@ -722,14 +729,25 @@ def model_forward(model, x: torch.Tensor):
     else:
         x = x.contiguous().float()
     cap = _capacity(model, x)
-    key = plan_key(model, x)
+    if augment:
+        from .tta import forward_augment
+        with torch.cuda.device(x.device):
+            return forward_augment(model, x, cap)
+    return run_forward(model, x, cap)
+
+
+def run_forward(model, x: torch.Tensor, cap: int | None, main_only: bool | None = None, tag=None):
+    """forward's value for x (checked and made contiguous by model_forward) on its plan, compiled at first use.
+    cap: model.max_batch (checked against x); main_only: None follows model.main_only; tag: extends the plan key, so
+    that a caller's plan is never shared with another input of the same shape (the branches of forward_augment)."""
+    key = plan_key(model, x, main_only) + ((tag,) if tag is not None else ())
     p = model._plans.get(key)
     if p is not None and model.check_weights and p.weight_version != _weights_version(model):
         p = None
     n = None if cap is None else x.shape[0]          # None: the plan's whole batch, x's own
     with torch.cuda.device(x.device):
         if p is None:
-            p = compile_model(model, x, capacity=cap)
+            p = compile_model(model, x, capacity=cap, main_only=main_only)
             model._plans[key] = p
         elif p.in_ptr != x.data_ptr():
             p.rebind(p.in_ptr, x.data_ptr())
@@ -764,13 +782,13 @@ def _capacity(model, x: torch.Tensor) -> int | None:
     return int(cap)
 
 
-def plan_key(model, x: torch.Tensor) -> tuple:
+def plan_key(model, x: torch.Tensor, main_only: bool | None = None) -> tuple:
     """The key of the plan model_forward runs x on: x's shape (its batch replaced by model.max_batch when that is set),
-    dtype and device, and the engine settings that change what is compiled."""
+    dtype and device, and the engine settings that change what is compiled (main_only: None follows model.main_only)."""
     cap = getattr(model, "max_batch", None)
     shape = tuple(x.shape) if cap is None else (int(cap),) + tuple(x.shape[1:])
     return (shape, x.dtype, x.device.index, model.precision, bool(getattr(model, "fuse_upsample", True)),
-            bool(getattr(model, "main_only", False)))
+            _main_only(model, main_only))
 
 
 def _first_rows(obj, n: int):

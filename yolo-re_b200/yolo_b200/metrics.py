@@ -160,14 +160,16 @@ class Evaluator:
     `evaluate()` result.  Every batch runs model -> NMS on the GPU and the detections never leave it until the final
     aggregation (the reference copies every image's detections to the CPU and loops over predictions in Python).
     The dataloader yields `(images [B,3,S,S] float in [0,1], targets [n,6] = (image index, class, cx, cy, w, h normalised),
-    _, orig_shapes)` exactly like the reference's (evaluator.py:96, 133-150).  Debug visualisation is out of scope."""
+    _, orig_shapes)` exactly like the reference's (evaluator.py:96, 133-150).  Debug visualisation is out of scope.
+    augment=True evaluates with test-time augmentation (``model(images, augment=True)``, like upstream's
+    ``val.py --augment``)."""
 
     def __init__(self, model, dataloader, num_classes: int = 80, conf_thres: float = 0.001, iou_thres: float = 0.6,
-                 device="cuda", debug_dir=None):
+                 device="cuda", debug_dir=None, augment: bool = False):
         if debug_dir is not None:
             raise NotImplementedError("debug visualisation is outside the B200 hot path (SURVEY.md section 2)")
         self.model, self.dataloader, self.num_classes = model, dataloader, num_classes
-        self.conf_thres, self.iou_thres = conf_thres, iou_thres
+        self.conf_thres, self.iou_thres, self.augment = conf_thres, iou_thres, augment
         self.device = torch.device("cuda" if device == "auto" else device)
         if self.device.type != "cuda":
             raise L.YreError("Evaluator: the B200 path needs a CUDA device (no CPU fallback)")
@@ -181,7 +183,7 @@ class Evaluator:
         for images, targets, _, _orig_shapes in self.dataloader:
             images = images.to(self.device, non_blocking=True)
             bsz, img_size = images.shape[0], images.shape[2]
-            outputs = self.model(images)
+            outputs = self.model(images, augment=True) if self.augment else self.model(images)
             if not isinstance(outputs, tuple):
                 raise NotImplementedError("Raw feature map decoding not implemented")     # evaluator.py:113-115
             preds = outputs[0]

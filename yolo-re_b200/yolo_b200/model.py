@@ -125,13 +125,16 @@ class YOLO(nn.Module):
         # batch raises ValueError
         self.max_batch: int | None = None
         self._plans: dict = {}
+        self._tta: dict = {}             # test-time augmentation: scaled-image buffers per (input shape, capacity)
         self.register_load_state_dict_post_hook(lambda m, _k: m.invalidate())
 
     # -- engine plumbing ------------------------------------------------------------------------
     def invalidate(self) -> None:
         """Drops the compiled launch plans (weights changed / moved).  Call it after edits the per-forward check cannot
-        see: writes through ``.data`` and re-assignment of a whole ``nn.Parameter`` object."""
+        see: writes through ``.data`` and re-assignment of a whole ``nn.Parameter`` object.  Frees the plans' buffers and
+        the test-time-augmentation image buffers with them."""
         self._plans.clear()
+        self._tta.clear()
         self.__dict__.pop("_wt_tensors", None)
 
     def set_precision(self, precision: str) -> "YOLO":
@@ -149,6 +152,7 @@ class YOLO(nn.Module):
 
     def _apply(self, fn, *a, **k):
         self._plans = {}
+        self._tta = {}
         self.__dict__.pop("_wt_tensors", None)
         return super()._apply(fn, *a, **k)
 
@@ -157,13 +161,15 @@ class YOLO(nn.Module):
             self._plans = {}
         return super().train(mode)
 
-    def forward(self, x: torch.Tensor):
+    def forward(self, x: torch.Tensor, augment: bool = False):
+        """Eval-mode forward (see the module docstring).  augment=True: upstream's test-time augmentation (yolo_b200.tta),
+        returning (y [B, 4+nc, A_tot], None) -- for a dual head the main head's merged y."""
         if self.training:
             raise NotImplementedError("train-mode forward is outside the B200 inference path (BatchNorm would need batch "
                                       "statistics; the launch plan folds the running ones): call .eval() -- YOLO.from_yaml "
                                       "returns the model in train mode, like the reference")
         from .engine import model_forward
-        return model_forward(self, x)
+        return model_forward(self, x, augment)
 
     # -- stride discovery ---------------------------------------------------------------------------
     def _detect_layer(self):
