@@ -224,6 +224,22 @@ int    yre_nms_batched(const yre_nms_desc* d, yre_stream_t s);
  * keep_anchor are not touched. */
 int    yre_nms_filter_only(const yre_nms_desc* d, yre_stream_t s);
 
+/* Multi-label NMS: upstream YOLOv9's non_max_suppression(..., multi_label=True) candidate set, which its val.py uses for
+ * every published mAP (val.py: `non_max_suppression(preds, conf_thres, iou_thres, labels=lb, multi_label=True, ...)`;
+ * utils/general.py: `i, j = (x[:, 5:mi] > conf_thres).nonzero(as_tuple=False).T`), on top of yolo-re's algorithm.
+ * Extends nms.py:54-59 (first-max class per anchor, strict >, class filter): every (anchor a, class c) with
+ * score[a][c] > conf_thres (and c in classes, when given) is a candidate, in the order (a ascending, then c).  Everything
+ * after that is nms.py:61-92 unchanged: xyxy boxes, the class offset c * (max_coord + 1) with max_coord over the candidate
+ * boxes, agnostic, a stable descending score sort (ties -> lower (a, c)), greedy IoU, keep[:max_det] with no pre-NMS cap.
+ * Not upstream's max_wh = 7680 offset, max_nms = 30000 cap or unstable argsort.
+ * Same descriptor and outputs as yre_nms_batched; keep_anchor is the anchor index, so several rows may share one anchor.
+ * The workspace holds pow2ceil(A * nc) keys per image.  A * nc above 2^30 fails with YRE_EUNSUPPORTED (the workspace
+ * size is then 0), as does an nc whose 32 rows do not fit the filter's 48 KB of shared memory (nc > 380). */
+size_t yre_nms_multi_label_workspace_bytes(int32_t B, int32_t A, int32_t nc);
+int    yre_nms_batched_multi_label(const yre_nms_desc* d, yre_stream_t s);
+/* the candidate pass of yre_nms_batched_multi_label on its own (stage timing, as yre_nms_filter_only) */
+int    yre_nms_multi_label_filter_only(const yre_nms_desc* d, yre_stream_t s);
+
 /* ---- K8/K9: the steps either side of the path (SURVEY.md 8f row 1) -----------------------------------
  * K8 replaces letterbox                                  scripts/detect.py:40-71
  *             cv2.resize(INTER_LINEAR) on uint8          (OpenCV; 8-bit fixed point, bit-exact restatement)

@@ -18,6 +18,8 @@
 //               exact), and warp 0 resolves the chunk by walking the set bits of the survivors.  The scan stops
 //               as soon as max_det boxes are kept, which is exactly `keep[:max_det]` of the reference -- there
 //               is no pre-NMS top-k cap.
+//   multi-label (upstream val.py's multi_label=True): nms_filter_ml keys every (anchor, class) pair above the
+//               threshold, nms_select_kernel<true> decodes the class from the key; the rest is the same code.
 //
 // Bit-exactness notes: every fp32 op is an explicitly rounded intrinsic (no FMA contraction);
 // the class offset is `float(cls) * (max_coord + 1)` then `box + offset` as two rounded ops
@@ -187,6 +189,111 @@ __global__ void __launch_bounds__(128) nms_filter_kernel(const FilterParams p) {
     }
 }
 
+// multi-label filter (upstream val.py's multi_label=True): every (anchor a, class c) with score > conf is a candidate, keyed
+// (~ordered(score) << 32) | (a * nc + c).  One warp per 32 consecutive anchors of one image: the warp's rows are staged in
+// shared memory (coalesced float4 loads; scalar ones when nc % 4 != 0), then walked twice in (anchor, class) order, one pair
+// per lane per step -- once to count, once to write after the warp's single atomicAdd.  A warp's keys therefore sit in its
+// slot range in (anchor, class) order: when every pair is a candidate and A % 32 == 0, every warp's range starts at a
+// multiple of 32 * nc.  The class is idx % nc, so no class map is written.
+__device__ __forceinline__ bool ml_cand(const FilterParams& p, float v, int c) {
+    if (!(v > p.conf)) return false;
+    if (p.n_classes < 0) return true;
+    bool ok = false;
+    for (int k = 0; k < p.n_classes; ++k) ok |= (p.classes[k] == c);
+    return ok;
+}
+
+__global__ void __launch_bounds__(128) nms_filter_ml_kernel(const FilterParams p) {
+    extern __shared__ __align__(16) unsigned char smraw[];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int rowf = 4 + p.nc;
+    float* rows = reinterpret_cast<float*>(smraw) + (size_t)warp * 32 * rowf;    // [32][4 + nc] this warp's rows
+
+    const int tiles = (p.A + 31) / 32;
+    const int wglobal = blockIdx.x * (blockDim.x >> 5) + warp;
+    if (wglobal >= tiles * p.B) return;
+    const int b = wglobal / tiles, a0 = (wglobal % tiles) * 32;
+    const int na = min(32, p.A - a0);
+    const float* src = p.pred + ((size_t)b * p.A + a0) * rowf;
+    if ((p.nc & 3) == 0) {                   // 16-byte aligned rows: float4, 8 loads in flight per lane
+        const int n4 = na * rowf / 4;
+        const float4* s4 = reinterpret_cast<const float4*>(src);
+        float4* r4 = reinterpret_cast<float4*>(rows);
+        for (int base0 = 0; base0 < n4; base0 += 8 * 32) {
+            float4 buf[8];
+#pragma unroll
+            for (int q = 0; q < 8; ++q) {
+                const int idx = base0 + q * 32 + lane;
+                if (idx < n4) buf[q] = s4[idx];
+            }
+#pragma unroll
+            for (int q = 0; q < 8; ++q) {
+                const int idx = base0 + q * 32 + lane;
+                if (idx < n4) r4[idx] = buf[q];
+            }
+        }
+    } else {
+        const int n1 = na * rowf;
+        for (int base0 = 0; base0 < n1; base0 += 8 * 32) {
+            float buf[8];
+#pragma unroll
+            for (int q = 0; q < 8; ++q) {
+                const int idx = base0 + q * 32 + lane;
+                if (idx < n1) buf[q] = src[idx];
+            }
+#pragma unroll
+            for (int q = 0; q < 8; ++q) {
+                const int idx = base0 + q * 32 + lane;
+                if (idx < n1) rows[idx] = buf[q];
+            }
+        }
+    }
+    __syncwarp();
+
+    // pass 1: count the candidates; the max coordinate over the boxes of anchors with at least one candidate
+    const int npairs = na * p.nc;
+    int al = lane / p.nc, c = lane - al * p.nc;     // pair t = al * nc + c, advanced by 32 per step
+    int total = 0, last = -1;
+    unsigned mo = 0u;
+    for (int t0 = 0; t0 < npairs; t0 += 32) {
+        const bool cand = t0 + lane < npairs && ml_cand(p, rows[al * rowf + 4 + c], c);
+        if (cand && al != last) {
+            last = al;
+            const float* r = rows + al * rowf;
+            const float hw = __fmul_rn(r[2], 0.5f), hh = __fmul_rn(r[3], 0.5f);
+            mo = max(mo, max(max(f2ord(__fsub_rn(r[0], hw)), f2ord(__fsub_rn(r[1], hh))),
+                             max(f2ord(__fadd_rn(r[0], hw)), f2ord(__fadd_rn(r[1], hh)))));
+        }
+        total += __popc(__ballot_sync(0xffffffffu, cand));
+        c += 32;
+        while (c >= p.nc) { c -= p.nc; ++al; }
+    }
+    if (total == 0) return;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) mo = max(mo, __shfl_xor_sync(0xffffffffu, mo, o));
+    int slot = 0;
+    if (lane == 0) {
+        atomicMax(p.ws.maxc + b, mo);
+        slot = atomicAdd(p.ws.count + b, total);
+    }
+    slot = __shfl_sync(0xffffffffu, slot, 0);
+
+    // pass 2: the keys, in (anchor, class) order from the warp's first slot
+    u64* keys = p.ws.keys + (size_t)b * p.ws.cap;
+    al = lane / p.nc; c = lane - al * p.nc;
+    for (int t0 = 0; t0 < npairs; t0 += 32) {
+        const float v = t0 + lane < npairs ? rows[al * rowf + 4 + c] : 0.f;
+        const bool cand = t0 + lane < npairs && ml_cand(p, v, c);
+        const unsigned ballot = __ballot_sync(0xffffffffu, cand);
+        if (cand)
+            keys[slot + __popc(ballot & ((1u << lane) - 1u))] =
+                ((u64)(~f2ord(v)) << 32) | (unsigned)((a0 + al) * p.nc + c);
+        slot += __popc(ballot);
+        c += 32;
+        while (c >= p.nc) { c -= p.nc; ++al; }
+    }
+}
+
 // ---------------------------------------------------------------------------------------------
 struct SelectParams {
     const float* pred; int B, A, nc; double iou; int max_det, agnostic;
@@ -341,6 +448,8 @@ __device__ __forceinline__ bool may_overlap(int ia, int ib) {
     return ((ca > cb ? ia : ib) >> 30) & 1;               // the box of the HIGHER class must reach below -0.5 in x and y
 }
 
+// ML: multi-label keys (index a * nc + c, the class decoded from it) instead of anchor keys and the class map
+template <bool ML>
 __global__ void __launch_bounds__(NT_SEL) nms_select_kernel(const SelectParams p) {
     extern __shared__ __align__(16) unsigned char smraw[];
     // carve shared memory.  Every array the inner loops touch sits at a COMPILE-TIME offset (fixed-size arrays first, the
@@ -369,7 +478,7 @@ __global__ void __launch_bounds__(NT_SEL) nms_select_kernel(const SelectParams p
     __shared__ bool s_partial;
 
     const int b = blockIdx.x, tid = threadIdx.x;
-    const int n = min(p.ws.count[b], p.A);
+    const int n = min(p.ws.count[b], ML ? p.A * p.nc : p.A);
     if (n == 0) { if (tid == 0) p.counts[b] = 0; return; }
     u64* gkeys = p.ws.keys + (size_t)b * p.ws.cap;
     NMS_STAMP(0);
@@ -403,9 +512,10 @@ __global__ void __launch_bounds__(NT_SEL) nms_select_kernel(const SelectParams p
         if (tid < CHUNK) dead[tid] = 0;
         if (tid < cnt) {
             const u64 key = keys[c0 + tid];
-            const int a = (int)(unsigned)(key & 0xffffffffu);
+            const unsigned idx = (unsigned)(key & 0xffffffffu);
+            const int a = ML ? (int)(idx / (unsigned)p.nc) : (int)idx;
             const float conf = ord2f(~(unsigned)(key >> 32));
-            const int cls = p.ws.cls[(size_t)b * p.A + a];
+            const int cls = ML ? (int)(idx - (unsigned)a * (unsigned)p.nc) : p.ws.cls[(size_t)b * p.A + a];
             const float* row = p.pred + ((size_t)b * p.A + a) * rowf;
             const float4 bx = (p.nc & 3) ? make_float4(row[0], row[1], row[2], row[3]) : *reinterpret_cast<const float4*>(row);
             const float hw = __fmul_rn(bx.z, 0.5f), hh = __fmul_rn(bx.w, 0.5f);
@@ -568,6 +678,19 @@ NmsWs carve(void* ws, int B, int A) {
     return w;
 }
 
+// multi-label: pow2ceil(A * nc) keys per image (sort_global pads in place), no class map
+constexpr long long NMS_ML_MAX_PAIRS = 1ll << 30;   // A * nc: the int counters and pow2ceil(A * nc) must not overflow
+NmsWs carve_ml(void* ws, int B, int A, int nc) {
+    NmsWs w;
+    w.cap = pow2ceil(A * nc);
+    unsigned char* p = reinterpret_cast<unsigned char*>(ws);
+    w.keys = reinterpret_cast<u64*>(p); p += sizeof(u64) * (size_t)B * w.cap;
+    w.cls = nullptr;
+    w.count = reinterpret_cast<int*>(p); p += sizeof(int) * (size_t)B;
+    w.maxc = reinterpret_cast<unsigned*>(p);
+    return w;
+}
+
 }  // namespace
 
 extern "C" size_t yre_nms_workspace_bytes(int32_t B, int32_t A) {
@@ -575,12 +698,20 @@ extern "C" size_t yre_nms_workspace_bytes(int32_t B, int32_t A) {
     return sizeof(u64) * (size_t)B * pow2ceil(A) + sizeof(int) * (size_t)B * A + 2 * sizeof(int) * (size_t)B + 256;
 }
 
-static int check_nms(const yre_nms_desc& d, bool outputs) {
+extern "C" size_t yre_nms_multi_label_workspace_bytes(int32_t B, int32_t A, int32_t nc) {
+    if (B <= 0 || A <= 0 || nc <= 0 || (long long)A * nc > NMS_ML_MAX_PAIRS) return 0;
+    return sizeof(u64) * (size_t)B * pow2ceil(A * nc) + 2 * sizeof(int) * (size_t)B + 256;
+}
+
+static int check_nms(const yre_nms_desc& d, bool outputs, bool ml = false) {
     if (!d.pred || !d.workspace) YRE_FAIL(YRE_EINVAL, "nms: null pointer");
     if (outputs && (!d.out || !d.counts || !d.keep_anchor)) YRE_FAIL(YRE_EINVAL, "nms: null output pointer");
     if (d.B <= 0 || d.A <= 0 || d.nc <= 0) YRE_FAIL(YRE_EINVAL, "nms: bad extent B=%d A=%d nc=%d", d.B, d.A, d.nc);
+    if (ml && (long long)d.A * d.nc > NMS_ML_MAX_PAIRS)
+        YRE_FAIL(YRE_EUNSUPPORTED, "nms: multi-label A*nc=%lld above %lld", (long long)d.A * d.nc, NMS_ML_MAX_PAIRS);
     if (d.max_det <= 0 || d.max_det > NMS_MAX_DET) YRE_FAIL(YRE_EUNSUPPORTED, "nms: max_det=%d (supported 1..%d)", d.max_det, NMS_MAX_DET);
-    if (d.workspace_bytes < yre_nms_workspace_bytes(d.B, d.A)) YRE_FAIL(YRE_EINVAL, "nms: workspace too small");
+    if (d.workspace_bytes < (ml ? yre_nms_multi_label_workspace_bytes(d.B, d.A, d.nc) : yre_nms_workspace_bytes(d.B, d.A)))
+        YRE_FAIL(YRE_EINVAL, "nms: workspace too small");
     if (d.n_classes > 0 && !d.classes) YRE_FAIL(YRE_EINVAL, "nms: classes pointer missing");
     if ((reinterpret_cast<uintptr_t>(d.pred) & 15) || (reinterpret_cast<uintptr_t>(d.workspace) & 15))
         YRE_FAIL(YRE_EINVAL, "nms: pred/workspace must be 16-byte aligned");
@@ -588,20 +719,26 @@ static int check_nms(const yre_nms_desc& d, bool outputs) {
 }
 
 // nb: the first nb images (the workspace keeps the layout of d.B images)
-static int launch_nms_filter(const yre_nms_desc& d, const NmsWs& ws, int nb, cudaStream_t s) {
+static int launch_nms_filter(const yre_nms_desc& d, const NmsWs& ws, int nb, cudaStream_t s, bool ml = false) {
     nms_init_kernel<<<yre_cdiv(nb, 256), 256, 0, s>>>(ws.count, ws.maxc, nb);
     YRE_LAUNCH_CHECK("nms_init");
 
     FilterParams fp;
     fp.pred = d.pred; fp.B = nb; fp.A = d.A; fp.nc = d.nc; fp.conf = d.conf_thres;
     fp.classes = d.classes; fp.n_classes = d.n_classes; fp.ws = ws;
-    const size_t per_warp = (d.nc % 4 == 0) ? (size_t)32 * ((d.nc / 4) | 1) * 8 : 16;
+    const size_t per_warp = ml ? (size_t)32 * (4 + d.nc) * 4                       // the warp's rows
+                               : (d.nc % 4 == 0) ? (size_t)32 * ((d.nc / 4) | 1) * 8 : 16;
     int warps = 4;
     while (warps > 1 && per_warp * warps > 40 * 1024) warps >>= 1;
     if (per_warp * warps > 48 * 1024) YRE_FAIL(YRE_EUNSUPPORTED, "nms: nc=%d too large", d.nc);
     const int tiles = yre_cdiv(d.A, 32) * nb;
-    nms_filter_kernel<<<yre_cdiv(tiles, warps), warps * 32, per_warp * warps, s>>>(fp);
-    YRE_LAUNCH_CHECK("nms_filter");
+    if (ml) {
+        nms_filter_ml_kernel<<<yre_cdiv(tiles, warps), warps * 32, per_warp * warps, s>>>(fp);
+        YRE_LAUNCH_CHECK("nms_filter_ml");
+    } else {
+        nms_filter_kernel<<<yre_cdiv(tiles, warps), warps * 32, per_warp * warps, s>>>(fp);
+        YRE_LAUNCH_CHECK("nms_filter");
+    }
     return YRE_OK;
 }
 
@@ -611,11 +748,18 @@ extern "C" int yre_nms_filter_only(const yre_nms_desc* d, yre_stream_t s) {
     return launch_nms_filter(*d, carve(d->workspace, d->B, d->A), d->B, (cudaStream_t)s);
 }
 
-int launch_nms(const yre_nms_desc& d, int nb, cudaStream_t s) {
-    if (int e = check_nms(d, true)) return e;
+extern "C" int yre_nms_multi_label_filter_only(const yre_nms_desc* d, yre_stream_t s) {
+    if (!d) YRE_FAIL(YRE_EINVAL, "nms: null descriptor");
+    if (int e = check_nms(*d, false, true)) return e;
+    return launch_nms_filter(*d, carve_ml(d->workspace, d->B, d->A, d->nc), d->B, (cudaStream_t)s, true);
+}
+
+template <bool ML>
+static int launch_nms_impl(const yre_nms_desc& d, int nb, cudaStream_t s) {
+    if (int e = check_nms(d, true, ML)) return e;
     if (nb < 1 || nb > d.B) YRE_FAIL(YRE_EINVAL, "nms: %d images outside 1..%d", nb, d.B);
-    NmsWs ws = carve(d.workspace, d.B, d.A);
-    if (int e = launch_nms_filter(d, ws, nb, s)) return e;
+    NmsWs ws = ML ? carve_ml(d.workspace, d.B, d.A, d.nc) : carve(d.workspace, d.B, d.A);
+    if (int e = launch_nms_filter(d, ws, nb, s, ML)) return e;
 
     SelectParams sp;
     sp.pred = d.pred; sp.B = nb; sp.A = d.A; sp.nc = d.nc; sp.iou = d.iou_thres; sp.max_det = d.max_det;
@@ -630,14 +774,17 @@ int launch_nms(const yre_nms_desc& d, int nb, cudaStream_t s) {
     // opt in to the shared memory of the largest max_det check_nms accepts (227 520 B; sm_100 allows 232 448 B a block)
     static YrePerDeviceOnce once;
     if (int e = once.run([]() -> int {
-            YRE_CUDA(cudaFuncSetAttribute(nms_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+            YRE_CUDA(cudaFuncSetAttribute(nms_select_kernel<ML>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                           (int)select_smem_bytes(NMS_MAX_DET)));
             return YRE_OK;
         })) return e;
-    nms_select_kernel<<<nb, NT_SEL, select_smem_bytes(d.max_det), s>>>(sp);
+    nms_select_kernel<ML><<<nb, NT_SEL, select_smem_bytes(d.max_det), s>>>(sp);
     YRE_LAUNCH_CHECK("nms_select");
     return YRE_OK;
 }
+
+int launch_nms(const yre_nms_desc& d, int nb, cudaStream_t s) { return launch_nms_impl<false>(d, nb, s); }
+int launch_nms_multi_label(const yre_nms_desc& d, int nb, cudaStream_t s) { return launch_nms_impl<true>(d, nb, s); }
 
 #ifdef YRE_TUNING
 extern "C" int yre_debug_nms_prof(long long* host16) {

@@ -199,6 +199,10 @@ int yre_nms_batched(const yre_nms_desc* d, yre_stream_t s) {
     if (!d) YRE_FAIL(YRE_EINVAL, "nms: null descriptor");
     return launch_nms(*d, d->B, (cudaStream_t)s);
 }
+int yre_nms_batched_multi_label(const yre_nms_desc* d, yre_stream_t s) {
+    if (!d) YRE_FAIL(YRE_EINVAL, "nms: null descriptor");
+    return launch_nms_multi_label(*d, d->B, (cudaStream_t)s);
+}
 
 // ---- plan -----------------------------------------------------------------------------------------
 int yre_plan_create(yre_plan** out) {

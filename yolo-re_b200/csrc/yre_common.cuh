@@ -197,4 +197,5 @@ int launch_nchw_to_view(const float* x, const yre_view& y, int nb, cudaStream_t 
 int launch_view_to_nchw(const yre_view& x, float* y, int nb, cudaStream_t s);
 int launch_decode(const yre_decode_desc& d, int nb, cudaStream_t s);
 int launch_nms(const yre_nms_desc& d, int nb, cudaStream_t s);   // 3 launches (memset kernel, filter, sort+scan)
+int launch_nms_multi_label(const yre_nms_desc& d, int nb, cudaStream_t s);   // same, every class above conf_thres
 double conv_flops(const yre_conv_desc& d);

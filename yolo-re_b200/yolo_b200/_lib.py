@@ -110,6 +110,9 @@ SYMBOLS = {
     "yre_nms_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int32]),
     "yre_nms_batched": (C.c_int, [C.POINTER(NmsDesc), C.c_void_p]),
     "yre_nms_filter_only": (C.c_int, [C.POINTER(NmsDesc), C.c_void_p]),
+    "yre_nms_multi_label_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int32, C.c_int32]),
+    "yre_nms_batched_multi_label": (C.c_int, [C.POINTER(NmsDesc), C.c_void_p]),
+    "yre_nms_multi_label_filter_only": (C.c_int, [C.POINTER(NmsDesc), C.c_void_p]),
     "yre_letterbox_geometry_rect": (C.c_int, [C.POINTER(LetterboxDesc), C.c_int32, C.c_int32, C.c_int32, C.POINTER(C.c_double),
                                     C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "yre_letterbox_geometry": (C.c_int, [C.POINTER(LetterboxDesc), C.POINTER(C.c_double), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),

@@ -162,14 +162,15 @@ class Evaluator:
     The dataloader yields `(images [B,3,S,S] float in [0,1], targets [n,6] = (image index, class, cx, cy, w, h normalised),
     _, orig_shapes)` exactly like the reference's (evaluator.py:96, 133-150).  Debug visualisation is out of scope.
     augment=True evaluates with test-time augmentation (``model(images, augment=True)``, like upstream's
-    ``val.py --augment``)."""
+    ``val.py --augment``).  multi_label=True runs multi-label NMS (every class above conf_thres of an anchor is a
+    candidate), as upstream's val.py does for its published mAPs; the default is the reference's single-label NMS."""
 
     def __init__(self, model, dataloader, num_classes: int = 80, conf_thres: float = 0.001, iou_thres: float = 0.6,
-                 device="cuda", debug_dir=None, augment: bool = False):
+                 device="cuda", debug_dir=None, augment: bool = False, multi_label: bool = False):
         if debug_dir is not None:
             raise NotImplementedError("debug visualisation is outside the B200 hot path (SURVEY.md section 2)")
         self.model, self.dataloader, self.num_classes = model, dataloader, num_classes
-        self.conf_thres, self.iou_thres, self.augment = conf_thres, iou_thres, augment
+        self.conf_thres, self.iou_thres, self.augment, self.multi_label = conf_thres, iou_thres, augment, multi_label
         self.device = torch.device("cuda" if device == "auto" else device)
         if self.device.type != "cuda":
             raise L.YreError("Evaluator: the B200 path needs a CUDA device (no CPU fallback)")
@@ -189,7 +190,8 @@ class Evaluator:
             preds = outputs[0]
             if isinstance(preds, list):
                 preds = preds[1]                                                           # main branch (evaluator.py:107-109)
-            dets = non_max_suppression(preds.permute(0, 2, 1).contiguous(), conf_thres=self.conf_thres, iou_thres=self.iou_thres)
+            dets = non_max_suppression(preds.permute(0, 2, 1).contiguous(), conf_thres=self.conf_thres, iou_thres=self.iou_thres,
+                                       multi_label=self.multi_label)
             targets = targets.to(self.device)
             gtb, gtc = [], []
             for i in range(bsz):
