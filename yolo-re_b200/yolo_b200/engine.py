@@ -19,6 +19,7 @@ PyTorch is used for device memory only (torch.empty / data_ptr / current stream)
 from __future__ import annotations
 
 import ctypes as C
+import math
 from contextlib import contextmanager
 from functools import cache
 from typing import NamedTuple
@@ -47,6 +48,16 @@ def _check_f16_range(w: torch.Tensor, name: str) -> None:
 # Plan.trace and in the C plan) but never run -- tests/ replays the trace with a CPU interpreter to
 # check the graph wiring without a GPU.  The product path never sets this.
 _ALLOW_CPU_DRY_RUN = False
+# Offsets of the buffers a plan sub-allocates from a shape arena (model.max_shape) are multiples of this: the caching
+# allocator's own alignment, which the TMA tensor maps (16 B base) and the 64-B channel windows of every view rely on.
+ARENA_ALIGN = 512
+
+
+class _LayoutOnly:
+    """Stands in for libyre in a plan that only lays out its buffers (sizing a shape arena): every call succeeds and
+    records nothing."""
+    def __getattr__(self, name):
+        return lambda *a: 0
 
 
 @contextmanager
@@ -119,11 +130,18 @@ def _null_view() -> L.View:
 class Plan:
     """A compiled launch list plus the tensors it owns."""
 
-    def __init__(self, device: torch.device, batch: int, prec: str):
+    def __init__(self, device: torch.device, batch: int, prec: str, arena: torch.Tensor | None = None,
+                 wcache: dict | None = None, layout_only: bool = False):
+        """arena: a uint8 device buffer the plan sub-allocates its activations and static outputs from, instead of
+        tensors of its own (model.max_shape); wcache: packed weights shared with the other plans of that arena, by the
+        modules they were folded from and their packing; layout_only: a plan that lays out its buffers (arena_end, trace)
+        and neither allocates device memory nor records launches."""
         self.dry = device.type != "cuda"
-        if self.dry and not _ALLOW_CPU_DRY_RUN:
+        if self.dry and not (_ALLOW_CPU_DRY_RUN or layout_only):
             raise L.YreError("the yolo-re B200 path runs on CUDA tensors only (there is no CPU fallback)")
-        self.lib = L.lib()
+        self.arena, self.wcache, self.layout_only = arena, wcache, layout_only
+        self.arena_end = 0            # bytes of the arena layout used so far (every plan counts them)
+        self.lib = _LayoutOnly() if layout_only else L.lib()
         if not self.dry:
             with torch.cuda.device(device):
                 L.check(self.lib.yre_device_check(), "device_check")
@@ -143,6 +161,7 @@ class Plan:
         self.in_ptr = None            # image pointer currently bound
         self.out_tensors: list[torch.Tensor] = []   # externally visible outputs (rebindable)
         self.result = None
+        self.shape_name = ""          # "B x H x W", for error messages
 
     def __del__(self):
         try:
@@ -153,22 +172,56 @@ class Plan:
             pass
 
     # -- memory ---------------------------------------------------------------------------------------
+    def empty(self, shape: tuple, tdt: torch.dtype, zero: bool = False) -> torch.Tensor:
+        """A buffer the plan owns.  With an arena: the next ARENA_ALIGN-aligned bytes of it, in call order, holding
+        whatever the last plan left there (zero is ignored: the kernels write every cell they read); without: a tensor
+        of its own, zeroed when asked."""
+        nbytes = math.prod(shape) * tdt.itemsize
+        off = self.arena_end
+        self.arena_end = off + -(-nbytes // ARENA_ALIGN) * ARENA_ALIGN
+        if self.layout_only:
+            t = torch.empty((), dtype=tdt).expand(shape)            # no storage: only the layout is wanted
+        elif self.arena is not None:
+            if off + nbytes > self.arena.numel():
+                raise L.YreError(f"a plan for a {self.shape_name} input does not fit the shape arena of "
+                                 f"{self.arena.numel()} bytes (it needs more than {off + nbytes})")
+            t = self.arena[off:off + nbytes].view(tdt).view(shape)
+        else:
+            t = (torch.zeros if zero else torch.empty)(shape, dtype=tdt, device=self.device)
+        self.keep.append(t)
+        return t
+
     def alloc(self, H: int, W: int, Cn: int, dtype=None, layout=L.NHWC) -> V:
         dtype = self.dt if dtype is None else dtype
         tdt = _TORCH_DT[dtype]
         if layout == L.PHASE4:
-            shape = (4, self.batch, (H + 1) // 2, (W + 1) // 2, Cn)
-            t = torch.zeros(shape, dtype=tdt, device=self.device)   # cells without a source pixel stay 0
+            # cells without a source pixel hold 0: the stem and ADown kernels write them, the zeroing of a buffer of
+            # the plan's own only repeats that
+            t = self.empty((4, self.batch, (H + 1) // 2, (W + 1) // 2, Cn), tdt, zero=True)
         else:
-            t = torch.empty((self.batch, H, W, Cn), dtype=tdt, device=self.device)
-        self.keep.append(t)
+            t = self.empty((self.batch, H, W, Cn), tdt)
         self.act_bytes += t.numel() * t.element_size()
         return V(t, self.batch, H, W, Cn, 0, Cn, dtype, layout)
 
     def dev(self, t: torch.Tensor, dtype) -> torch.Tensor:
+        if self.layout_only:
+            return t
         t = t.to(device=self.device, dtype=dtype).contiguous()
         self.keep.append(t)
         return t
+
+    def pack(self, key: tuple | None, w: torch.Tensor, b: torch.Tensor, wdt: torch.dtype) -> tuple[torch.Tensor, torch.Tensor]:
+        """Device weights [Cout][kh][kw][Cin] in wdt and fp32 bias of a fold.  key: the modules it was folded from and
+        its packing; plans that share a weight cache upload each key once."""
+        key = None if key is None or self.wcache is None else key + (wdt,)
+        wb = self.wcache.get(key) if key is not None else None
+        if wb is None:
+            wb = self.dev(w.permute(0, 2, 3, 1), wdt), self.dev(b, torch.float32)
+            if key is not None:
+                self.wcache[key] = wb
+        else:
+            self.keep.extend(wb)
+        return wb
 
     # -- weight folding ------------------------------------------------------------------------------------
     @staticmethod
@@ -215,7 +268,7 @@ class Plan:
         return self.names.get(id(m), type(m).__name__)
 
     def conv(self, x: V | VCat, w, b, k, stride, silu, out: V | None = None, res: V | None = None, out_dtype=None,
-             name: str = "conv") -> V:
+             name: str = "conv", key: tuple | None = None) -> V:
         cout, cin = w.shape[0], w.shape[1]
         if self.prec == "fp16":
             _check_f16_range(w, name)
@@ -228,8 +281,7 @@ class Plan:
         if out is None:
             out = self.alloc(Ho, Wo, cout, dtype=out_dtype)
         assert (out.H, out.W, out.C) == (Ho, Wo, cout), ((out.H, out.W, out.C), (Ho, Wo, cout))
-        wp = self.dev(w.permute(0, 2, 3, 1), self.tdt)           # [Cout][kh][kw][Cin]
-        bp = self.dev(b, torch.float32)
+        wp, bp = self.pack(key, w, b, self.tdt)                 # [Cout][kh][kw][Cin]
         d = L.ConvDesc(x.c(), out.c(), res.c() if res is not None else _null_view(), wp.data_ptr(), bp.data_ptr(),
                        k, stride, L.ACT_SILU if silu else L.ACT_NONE, self.engine, xu.c() if xu is not None else _null_view())
         L.check(self.lib.yre_plan_add_conv(self.h, C.byref(d)), "plan_add_conv")
@@ -238,14 +290,14 @@ class Plan:
 
     def conv_m(self, m, x: V, out: V | None = None, res: V | None = None, out_dtype=None) -> V:
         w, b, k, s, silu = self.fold(m)
-        return self.conv(x, w, b, k, s, silu, out, res, out_dtype, name=self.name_of(m))
+        return self.conv(x, w, b, k, s, silu, out, res, out_dtype, name=self.name_of(m), key=("conv", self.name_of(m)))
 
     def conv_merged(self, ms, x: V, out: V | None = None) -> V:
         """Sibling convs on one input -> one GEMM with concatenated output channels."""
         fs = [self.fold(m) for m in ms]
         assert len({(f.k, f.stride, f.silu) for f in fs}) == 1
         return self.conv(x, torch.cat([f.w for f in fs]), torch.cat([f.b for f in fs]), fs[0].k, fs[0].stride, fs[0].silu, out,
-                         name=" + ".join(self.name_of(m) for m in ms))
+                         name=" + ".join(self.name_of(m) for m in ms), key=("conv",) + tuple(self.name_of(m) for m in ms))
 
     def stem(self, m: B.Conv, x: torch.Tensor, phase4: bool) -> V:
         """x: the fp32 NCHW image batch, or uint8 [B,H,W,3] BGR frames (BGR->RGB, HWC->CHW and /255 of
@@ -261,8 +313,7 @@ class Plan:
         Bn = self.batch                          # x may hold fewer images: a plan compiled for a batch capacity
         Ho, Wo = _conv_out(H, 3, s), _conv_out(W, 3, s)
         out = self.alloc(Ho, Wo, w.shape[0], layout=L.PHASE4 if phase4 else L.NHWC)
-        wp = self.dev(w.permute(0, 2, 3, 1), torch.float32)
-        bp = self.dev(b, torch.float32)
+        wp, bp = self.pack(("stem", self.name_of(m)), w, b, torch.float32)
         d = L.StemDesc(None if u8 else x.data_ptr(), Bn, Cin, H, W, out.c(), wp.data_ptr(), bp.data_ptr(), s,
                        L.ACT_SILU if silu else L.ACT_NONE, x.data_ptr() if u8 else None)
         L.check(self.lib.yre_plan_add_stem(self.h, C.byref(d)), "plan_add_stem")
@@ -384,11 +435,11 @@ class Plan:
             if ncp != nc:
                 fc = fc._replace(w=torch.cat([fc.w, fc.w.new_zeros((ncp - nc,) + tuple(fc.w.shape[1:]))]),
                                  b=torch.cat([fc.b, fc.b.new_zeros(ncp - nc)]))
-            self.conv(hc, fc.w, fc.b, fc.k, fc.stride, fc.silu, out=raw_full.sl(4 * REG_MAX, ncp), name=self.name_of(cls[i][2]))
+            self.conv(hc, fc.w, fc.b, fc.k, fc.stride, fc.silu, out=raw_full.sl(4 * REG_MAX, ncp), name=self.name_of(cls[i][2]),
+                      key=("conv", self.name_of(cls[i][2]), "classes padded to", ncp))
             raws.append(raw)
         A = sum(r.H * r.W for r in raws)
-        y = torch.empty((self.batch, A, 4 + nc), dtype=torch.float32, device=self.device)
-        self.keep.append(y)
+        y = self.empty((self.batch, A, 4 + nc), torch.float32)
         d = L.DecodeDesc()
         for i, r in enumerate(raws):
             d.raw[i] = r.c()
@@ -624,18 +675,20 @@ def _main_only(model, main_only: bool | None = None) -> bool:
     return bool(getattr(model, "main_only", False)) if main_only is None else bool(main_only)
 
 
-def compile_model(model, x: torch.Tensor, capacity: int | None = None, main_only: bool | None = None) -> Plan:
+def compile_model(model, x: torch.Tensor, capacity: int | None = None, main_only: bool | None = None,
+                  arena: torch.Tensor | None = None, wcache: dict | None = None, layout_only: bool = False) -> Plan:
     """Compiles the whole YOLO graph for x's shape/device (x: fp32 [B,C,H,W] or uint8 [B,H,W,3] BGR frames).
     capacity: compile for that many images instead of x's B (x may hold fewer; the plan runs any 1..capacity of them).
-    main_only: None follows model.main_only."""
+    main_only: None follows model.main_only.  arena, wcache, layout_only: see Plan."""
     if x.dtype == torch.uint8:
         Bn, H, W, Cin = x.shape
     else:
         Bn, Cin, H, W = x.shape
     Bn = Bn if capacity is None else capacity
     wire = wire_model(model, H, W, Cin, main_only)
-    p = Plan(x.device, Bn, model.precision)
+    p = Plan(x.device, Bn, model.precision, arena, wcache, layout_only)
     p.names = {id(m): n for n, m in model.named_modules()}
+    p.shape_name = f"{Bn} x {H} x {W}"
 
     @cache
     def cat_buf(n: str) -> V:
@@ -729,17 +782,20 @@ def model_forward(model, x: torch.Tensor, augment: bool = False):
     else:
         x = x.contiguous().float()
     cap = _capacity(model, x)
+    max_hw = _max_shape(model, x)
     if augment:
         from .tta import forward_augment
         with torch.cuda.device(x.device):
-            return forward_augment(model, x, cap)
-    return run_forward(model, x, cap)
+            return forward_augment(model, x, cap, max_hw)
+    return run_forward(model, x, cap, max_hw=max_hw)
 
 
-def run_forward(model, x: torch.Tensor, cap: int | None, main_only: bool | None = None, tag=None):
+def run_forward(model, x: torch.Tensor, cap: int | None, main_only: bool | None = None, tag=None,
+                max_hw: tuple[int, int] | None = None):
     """forward's value for x (checked and made contiguous by model_forward) on its plan, compiled at first use.
     cap: model.max_batch (checked against x); main_only: None follows model.main_only; tag: extends the plan key, so
-    that a caller's plan is never shared with another input of the same shape (the branches of forward_augment)."""
+    that a caller's plan is never shared with another input of the same shape (the branches of forward_augment);
+    max_hw: the largest input of x's shape arena (model.max_shape, checked against x; None: the plan owns its buffers)."""
     key = plan_key(model, x, main_only) + ((tag,) if tag is not None else ())
     p = model._plans.get(key)
     if p is not None and model.check_weights and p.weight_version != _weights_version(model):
@@ -747,7 +803,8 @@ def run_forward(model, x: torch.Tensor, cap: int | None, main_only: bool | None 
     n = None if cap is None else x.shape[0]          # None: the plan's whole batch, x's own
     with torch.cuda.device(x.device):
         if p is None:
-            p = compile_model(model, x, capacity=cap, main_only=main_only)
+            arena, wcache = _arena(model, x, cap, main_only, tag, max_hw) if max_hw is not None else (None, None)
+            p = compile_model(model, x, capacity=cap, main_only=main_only, arena=arena, wcache=wcache)
             model._plans[key] = p
         elif p.in_ptr != x.data_ptr():
             p.rebind(p.in_ptr, x.data_ptr())
@@ -782,13 +839,60 @@ def _capacity(model, x: torch.Tensor) -> int | None:
     return int(cap)
 
 
+def _max_shape(model, x: torch.Tensor) -> tuple[int, int] | None:
+    """model.max_shape as (H, W) after checking it and x's height and width against it (None: every plan owns its
+    buffers)"""
+    ms = getattr(model, "max_shape", None)
+    if ms is None:
+        return None
+    if getattr(model, "max_batch", None) is None:
+        raise ValueError("model.max_shape needs model.max_batch: the shape arena is sized for model.max_batch images of "
+                         "model.max_shape, so set both (or model.max_shape = None)")
+    if len(ms) != 2 or min(int(v) for v in ms) < 1:
+        raise ValueError(f"model.max_shape must be a (height, width) pair of positive extents or None (got {ms})")
+    mh, mw = int(ms[0]), int(ms[1])
+    H, W = (x.shape[1], x.shape[2]) if x.dtype == torch.uint8 else (x.shape[2], x.shape[3])
+    if H > mh or W > mw:
+        raise ValueError(f"a {H} x {W} input: this model runs inputs of up to {mh} x {mw} (model.max_shape = {ms})")
+    return mh, mw
+
+
+def arena_bytes(model, Cin: int, H: int, W: int, capacity: int, main_only: bool | None = None) -> int:
+    """Bytes of a shape arena for plans of up to capacity images of at most H x W: the buffer layout of that largest
+    plan.  Every buffer of a plan grows with the input extents, and a smaller input never lays out more buffers."""
+    x = torch.empty((), dtype=torch.float32).expand(capacity, Cin, H, W)       # no storage: only its shape is read
+    return compile_model(model, x, capacity, main_only, layout_only=True).arena_end
+
+
+def _arena(model, x: torch.Tensor, cap: int, main_only: bool | None, tag, max_hw: tuple[int, int]):
+    """(arena, weight cache) of x's plan.  One arena per precision, main_only, fuse_upsample, plan tag and device (and
+    capacity and maximum shape), allocated at first use for cap images of max_hw and never reallocated, so CUDA graphs
+    captured on its plans stay valid; the input dtype is not part of the key (it changes no buffer).  The weight cache
+    of the device holds the packed weights of every plan with an arena, for the weights' current version."""
+    key = (model.precision, _main_only(model, main_only), bool(getattr(model, "fuse_upsample", True)), tag,
+           x.device.index, cap, max_hw)
+    arena = model._arenas.get(key)
+    if arena is None:
+        Cin = x.shape[3] if x.dtype == torch.uint8 else x.shape[1]
+        arena = torch.empty(arena_bytes(model, Cin, *max_hw, cap, main_only), dtype=torch.uint8, device=x.device)
+        model._arenas[key] = arena
+    ver = _weights_version(model)
+    wc = model._arena_weights.get(x.device.index)
+    if wc is None or wc[0] != ver:
+        wc = model._arena_weights[x.device.index] = (ver, {})
+    return arena, wc[1]
+
+
 def plan_key(model, x: torch.Tensor, main_only: bool | None = None) -> tuple:
     """The key of the plan model_forward runs x on: x's shape (its batch replaced by model.max_batch when that is set),
-    dtype and device, and the engine settings that change what is compiled (main_only: None follows model.main_only)."""
+    dtype and device, and the engine settings that change what is compiled (main_only: None follows model.main_only),
+    and model.max_shape when that is set (its plans take their buffers from a shape arena)."""
     cap = getattr(model, "max_batch", None)
     shape = tuple(x.shape) if cap is None else (int(cap),) + tuple(x.shape[1:])
-    return (shape, x.dtype, x.device.index, model.precision, bool(getattr(model, "fuse_upsample", True)),
-            _main_only(model, main_only))
+    key = (shape, x.dtype, x.device.index, model.precision, bool(getattr(model, "fuse_upsample", True)),
+           _main_only(model, main_only))
+    ms = getattr(model, "max_shape", None)
+    return key if ms is None else key + (("max_shape", tuple(int(v) for v in ms)),)
 
 
 def _first_rows(obj, n: int):

@@ -159,8 +159,9 @@ class Evaluator:
     """Device-side mirror of the reference's Evaluator (src/yolo/eval/evaluator.py:23-213): same constructor arguments and
     `evaluate()` result.  Every batch runs model -> NMS on the GPU and the detections never leave it until the final
     aggregation (the reference copies every image's detections to the CPU and loops over predictions in Python).
-    The dataloader yields `(images [B,3,S,S] float in [0,1], targets [n,6] = (image index, class, cx, cy, w, h normalised),
-    _, orig_shapes)` exactly like the reference's (evaluator.py:96, 133-150).  Debug visualisation is out of scope.
+    The dataloader yields `(images [B,3,H,W] float in [0,1], targets [n,6] = (image index, class, cx, cy, w, h normalised),
+    _, orig_shapes)` like the reference's (evaluator.py:96, 133-150), whose batches are square (H = W); a batch may also be
+    a rectangle, as upstream val.py's rect batches are: normalised x and w then scale by W, y and h by H.  Debug visualisation is out of scope.
     augment=True evaluates with test-time augmentation (``model(images, augment=True)``, like upstream's
     ``val.py --augment``).  multi_label=True runs multi-label NMS (every class above conf_thres of an anchor is a
     candidate), as upstream's val.py does for its published mAPs; the default is the reference's single-label NMS."""
@@ -183,7 +184,7 @@ class Evaluator:
         acc = DetectionAccumulator(self.num_classes)
         for images, targets, _, _orig_shapes in self.dataloader:
             images = images.to(self.device, non_blocking=True)
-            bsz, img_size = images.shape[0], images.shape[2]
+            bsz, H, W = images.shape[0], images.shape[2], images.shape[3]
             outputs = self.model(images, augment=True) if self.augment else self.model(images)
             if not isinstance(outputs, tuple):
                 raise NotImplementedError("Raw feature map decoding not implemented")     # evaluator.py:113-115
@@ -193,10 +194,12 @@ class Evaluator:
             dets = non_max_suppression(preds.permute(0, 2, 1).contiguous(), conf_thres=self.conf_thres, iou_thres=self.iou_thres,
                                        multi_label=self.multi_label)
             targets = targets.to(self.device)
+            # fp32 (x, y, w, h) * (W, H, W, H): for a square batch the same fp32 products as the reference's * img_size
+            size = torch.tensor([W, H, W, H], dtype=torch.float32, device=self.device)
             gtb, gtc = [], []
             for i in range(bsz):
                 t = targets[targets[:, 0] == i]
-                xywh = t[:, 2:6].float() * img_size                                       # evaluator.py:139-141 (same fp32 ops)
+                xywh = t[:, 2:6].float() * size                                           # evaluator.py:139-141
                 xyxy = torch.zeros_like(xywh)
                 xyxy[:, 0] = xywh[:, 0] - xywh[:, 2] / 2
                 xyxy[:, 1] = xywh[:, 1] - xywh[:, 3] / 2

@@ -124,16 +124,25 @@ class YOLO(nn.Module):
         # 1..N images (same results as the first n images of a full run, shorter launches, one set of buffers); a larger
         # batch raises ValueError
         self.max_batch: int | None = None
+        # None: every plan owns its buffers.  (H, W), with max_batch set: the plans of every input shape up to H x W take
+        # their activations and static outputs from one shape arena sized for max_batch images of H x W, and share one
+        # upload of the folded weights; a larger input raises ValueError.  Static outputs are then valid until the next
+        # forward of any shape, and forwards must be ordered on one stream
+        self.max_shape: tuple[int, int] | None = None
         self._plans: dict = {}
+        self._arenas: dict = {}          # shape arenas (engine._arena)
+        self._arena_weights: dict = {}   # per device: (weights version, packed weights shared by the arena plans)
         self._tta: dict = {}             # test-time augmentation: scaled-image buffers per (input shape, capacity)
         self.register_load_state_dict_post_hook(lambda m, _k: m.invalidate())
 
     # -- engine plumbing ------------------------------------------------------------------------
     def invalidate(self) -> None:
         """Drops the compiled launch plans (weights changed / moved).  Call it after edits the per-forward check cannot
-        see: writes through ``.data`` and re-assignment of a whole ``nn.Parameter`` object.  Frees the plans' buffers and
-        the test-time-augmentation image buffers with them."""
+        see: writes through ``.data`` and re-assignment of a whole ``nn.Parameter`` object.  Frees the plans' buffers, the
+        shape arenas and their shared weights, and the test-time-augmentation image buffers with them."""
         self._plans.clear()
+        self._arenas.clear()
+        self._arena_weights.clear()
         self._tta.clear()
         self.__dict__.pop("_wt_tensors", None)
 
@@ -152,6 +161,7 @@ class YOLO(nn.Module):
 
     def _apply(self, fn, *a, **k):
         self._plans = {}
+        self._arenas, self._arena_weights = {}, {}
         self._tta = {}
         self.__dict__.pop("_wt_tensors", None)
         return super()._apply(fn, *a, **k)
@@ -159,6 +169,7 @@ class YOLO(nn.Module):
     def train(self, mode: bool = True):
         if mode:
             self._plans = {}
+            self._arenas, self._arena_weights = {}, {}
         return super().train(mode)
 
     def forward(self, x: torch.Tensor, augment: bool = False):

@@ -11,7 +11,8 @@ like upstream; feed y to ``non_max_suppression`` as a plain forward's y.  oracle
   * K13 (yre_tta_merge) writes the merged y.
 A dual-head model (yolov9-c) runs all three branches on main-only plans: every caller keeps the main head's y.  Height
 and width must be multiples of 32 (ValueError otherwise).  fresh_outputs, use_cuda_graph, max_batch and the precision
-apply to every branch as they do to a plain forward.
+apply to every branch as they do to a plain forward.  With model.max_shape, the plans of each branch take their buffers
+from an arena of that branch's own (their plan tag differs), sized for the branch input of model.max_shape.
 """
 from __future__ import annotations
 
@@ -74,8 +75,8 @@ def merge(ys: list[torch.Tensor], g: L.TtaGeom, out: torch.Tensor | None = None)
     return out
 
 
-def forward_augment(model, x: torch.Tensor, cap: int | None):
-    """model(x, augment=True) for x as model_forward checked it; cap: model.max_batch."""
+def forward_augment(model, x: torch.Tensor, cap: int | None, max_hw: tuple[int, int] | None = None):
+    """model(x, augment=True) for x as model_forward checked it; cap: model.max_batch; max_hw: model.max_shape."""
     u8 = x.dtype == torch.uint8
     n = x.shape[0]
     g = geometry(*((x.shape[1], x.shape[2]) if u8 else (x.shape[2], x.shape[3])))
@@ -86,10 +87,13 @@ def forward_augment(model, x: torch.Tensor, cap: int | None):
     if st is None:
         st = {"imgs": [torch.empty((rows, 3, g.out_h[i], g.out_w[i]), dtype=torch.float32, device=x.device) for i in (1, 2)]}
         model._tta[(tuple(x.shape[1:]), x.dtype, x.device.index, rows)] = st
-    ys = [E.run_forward(model, x, cap, main_only)[0]]
+    # the largest branch inputs: those of the largest height and width TTA takes (multiples of 32) up to max_hw
+    gmax = None if max_hw is None else geometry(max_hw[0] // 32 * 32, max_hw[1] // 32 * 32)
+    ys = [E.run_forward(model, x, cap, main_only, max_hw=max_hw)[0]]
     for i, buf in zip((1, 2), st["imgs"]):
         scale_img(x, g, i, out=buf, n=n)
-        ys.append(E.run_forward(model, buf[:n], cap, main_only, tag=("tta", i))[0])
+        ys.append(E.run_forward(model, buf[:n], cap, main_only, tag=("tta", i),
+                                max_hw=None if gmax is None else (gmax.out_h[i], gmax.out_w[i]))[0])
     ys = [y.permute(0, 2, 1) for y in ys]                      # the plans' [n, A, 4+nc] rows
     out = None
     if not model.fresh_outputs:
