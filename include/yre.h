@@ -278,6 +278,27 @@ int yre_letterbox_u8(const yre_letterbox_desc* d, yre_stream_t s);
 /* n images sharing the destination extent and out_mode in as few launches as possible (32 images per launch); their
  * resized sizes and offsets inside the destination may differ */
 int yre_letterbox_u8_batch(const yre_letterbox_desc* d, int32_t n, yre_stream_t s);
+/* K14: K8 on 4:2:0 YUV frames, the output of hardware and software video decoders.  Output is defined as K8 applied to
+ * cv2.cvtColor(frame, COLOR_YUV2BGR_<format>), bit for bit: limited range, 20-bit fixed point, nearest chroma (one
+ * (U, V) sample per 2 x 2 luma block).  YRE_YUV_BT601 uses cv2's coefficients, YRE_YUV_BT709 the same scheme on
+ * the BT.709 ones (HD video).  Each plane has its own pointer and pitch (pitched decoder surfaces, chroma apart from
+ * luma); cv2's single (h*3/2) x w array is the case of one allocation. */
+enum { YRE_YUV_NV12 = 0, YRE_YUV_NV21 = 1, YRE_YUV_I420 = 2, YRE_YUV_YV12 = 3 };
+enum { YRE_YUV_BT601 = 0, YRE_YUV_BT709 = 1 };
+typedef struct yre_yuv420_planes {
+    const uint8_t* luma;              /* h rows of w bytes, luma_pitch bytes apart */
+    int64_t        luma_pitch;
+    const uint8_t* chroma[2];         /* NV12 / NV21: [0] = the interleaved UV / VU plane (h/2 rows of w bytes), [1] = NULL;
+                                         I420: [0] = U, [1] = V; YV12: [0] = V, [1] = U (h/2 rows of w/2 bytes each) */
+    int64_t        chroma_pitch;      /* of every chroma plane */
+    int32_t        format;            /* YRE_YUV_NV12 ... */
+    int32_t        matrix;            /* YRE_YUV_BT601 / YRE_YUV_BT709 */
+} yre_yuv420_planes;
+/* n frames, planes[i] the source of d[i]: d[i] gives the luma extent h x w, the geometry, out_mode and dst as for
+ * yre_letterbox_u8_batch (geometry from yre_letterbox_geometry_rect on h x w); its src and row_pitch must be 0.
+ * YRE_EINVAL before any launch for an odd h or w, a pitch shorter than its plane's row, an unknown format or matrix,
+ * or a null plane. */
+int yre_letterbox_yuv420_batch(const yre_letterbox_desc* d, const yre_yuv420_planes* planes, int32_t n, yre_stream_t s);
 /* K9 replaces scale_boxes                                scripts/detect.py:74-109
  * boxes: n rows of xyxy fp32, `row_stride` floats apart (6 for detection rows), updated in place:
  * x = clamp((x - pad_w) / gain, 0, orig_w), y likewise -- fp32, true division, as torch does on the CPU. */

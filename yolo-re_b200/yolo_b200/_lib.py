@@ -62,6 +62,13 @@ class LetterboxDesc(C.Structure):
 
 
 LB_F32_CHW, LB_U8_HWC = 0, 1
+YUV_NV12, YUV_NV21, YUV_I420, YUV_YV12 = 0, 1, 2, 3
+YUV_BT601, YUV_BT709 = 0, 1
+
+
+class Yuv420Planes(C.Structure):
+    _fields_ = [("luma", C.c_void_p), ("luma_pitch", C.c_int64), ("chroma", C.c_void_p * 2), ("chroma_pitch", C.c_int64),
+                ("format", C.c_int32), ("matrix", C.c_int32)]
 
 
 class MatchDesc(C.Structure):
@@ -118,6 +125,7 @@ SYMBOLS = {
     "yre_letterbox_geometry": (C.c_int, [C.POINTER(LetterboxDesc), C.POINTER(C.c_double), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "yre_letterbox_u8": (C.c_int, [C.POINTER(LetterboxDesc), C.c_void_p]),
     "yre_letterbox_u8_batch": (C.c_int, [C.POINTER(LetterboxDesc), C.c_int32, C.c_void_p]),
+    "yre_letterbox_yuv420_batch": (C.c_int, [C.POINTER(LetterboxDesc), C.POINTER(Yuv420Planes), C.c_int32, C.c_void_p]),
     "yre_scale_boxes": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_void_p]),
     "yre_match_detections": (C.c_int, [C.POINTER(MatchDesc), C.c_void_p]),
     "yre_tta_geometry": (C.c_int, [C.c_int32, C.c_int32, C.POINTER(TtaGeom)]),
