@@ -189,6 +189,18 @@ typedef struct yre_decode_desc {
     float*       y;
 } yre_decode_desc;
 int yre_dfl_decode_score(const yre_decode_desc* d, yre_stream_t s);
+/* K6 for segmentation heads (upstream YOLOv9's Segment on DetectDFL): dec is decoded exactly as yre_dfl_decode_score
+ * decodes it, and the same launch writes mc: fp32 [B][A][nm], row a = the nm mask coefficients of anchor a, read from
+ * mask[l] at the anchor's pixel.  mask[l]: fp32 NHWC view [B,Hl,Wl,nm] of level l's mask tower output, with raw[l]'s
+ * extent.  So the coefficients of a kept detection are mc[b][keep_anchor[b][j]].  nm must be 32; anything else, or a
+ * mask view of another dtype, layout or extent, fails with YRE_EINVAL before the launch. */
+typedef struct yre_decode_masks_desc {
+    yre_decode_desc dec;
+    yre_view        mask[8];
+    int32_t         nm;
+    float*          mc;
+} yre_decode_masks_desc;
+int yre_dfl_decode_score_masks(const yre_decode_masks_desc* d, yre_stream_t s);
 
 /* ---- K7: batched class-aware NMS --------------------------------------------------------------
  * Replaces non_max_suppression                           src/yolo/utils/nms.py:19-94
@@ -385,6 +397,46 @@ typedef struct yre_tta_merge_desc {
 } yre_tta_merge_desc;
 int yre_tta_merge(const yre_tta_merge_desc* d, yre_stream_t s);
 
+/* ---- K15: instance-segmentation masks of the kept detections ------------------------------------------------------
+ * Replaces process_mask / process_mask_native / crop_mask        upstream YOLOv9 utils/segment/general.py
+ * One launch for a batch, after yre_nms_batched (or its multi-label form): detection j < counts[b] of image b takes the
+ * mask coefficients mc[b][keep_anchor[b][j]] and its box det[b][j][0..3] (xyxy).  With p = 1 / (1 + expf(-x)) of the logit
+ * x = sum_k mc[k] proto[y][x][k] (fp32, k = 0..nm-1 in order, no contraction), masks[b][j] is, as uint8 0 / 1:
+ *   YRE_MASK_PROTO   process_mask(upsample=False): out_h x out_w = mh x mw.  p cropped to the box scaled to proto pixels
+ *                    (x * (float)(mw / in_w), y * (float)(mh / in_h)): pixel (r, c) kept when c >= x1, c < x2, r >= y1,
+ *                    r < y2, else 0.  Then > 0.5.
+ *   YRE_MASK_INPUT   process_mask(upsample=True): out_h x out_w = in_h x in_w.  The cropped map of YRE_MASK_PROTO, resized
+ *                    bilinearly (align_corners=False, K12's arithmetic) to the input, then > 0.5.
+ *   YRE_MASK_NATIVE  process_mask_native: p uncropped; gain = min(mh / h0, mw / w0), pad = ((mw - w0 gain) / 2,
+ *                    (mh - h0 gain) / 2) in double; rows (int)pad_h .. (int)(mh - pad_h), columns likewise, resized
+ *                    bilinearly to h0 x w0; cropped with the box in frame pixels; > 0.5.  (w0, h0) = (int) columns 3 and 4
+ *                    of scale[b] (the rows yre_nms_desc.scale takes); image b writes the [0, h0) x [0, w0) window of its
+ *                    out_h x out_w planes, clipped to them.
+ * Only what can reach the output is computed: the box's proto pixels and their bilinear border.  Rows j >= counts[b]
+ * (read on the device: no host sync, CUDA-graph capturable), images >= n and bytes outside a native window are not
+ * written.  proto: fp32 NHWC [B][mh][mw][nm], pixels proto_pitch floats apart (a multiple of 4, >= nm), 16-byte aligned;
+ * mc: fp32 [B][A][nm], 16-byte aligned; det: fp32 [B][max_det][6]; counts: int32 [B]; keep_anchor: int64 [B][max_det];
+ * masks: uint8 [B][max_det][out_h][out_w].  YRE_EINVAL before any launch for a null pointer, nm != 32, an unknown mode,
+ * a bad pitch or alignment, non-positive extents, 1 <= n <= B violated, or out_h x out_w other than the mode's. */
+enum { YRE_MASK_PROTO = 0, YRE_MASK_INPUT = 1, YRE_MASK_NATIVE = 2 };
+typedef struct yre_mask_desc {
+    const float*   proto;
+    int32_t        B, n, mh, mw, nm;
+    int32_t        proto_pitch;
+    const float*   mc;
+    int32_t        A;
+    const float*   det;
+    const int32_t* counts;
+    const int64_t* keep_anchor;
+    int32_t        max_det;
+    int32_t        mode;
+    int32_t        in_h, in_w;       /* the network input (PROTO and INPUT modes) */
+    const float*   scale;            /* NATIVE: fp32 [B][5] = (pad_w, pad_h, gain, orig_w, orig_h) */
+    uint8_t*       masks;
+    int32_t        out_h, out_w;
+} yre_mask_desc;
+int yre_seg_masks(const yre_mask_desc* d, yre_stream_t s);
+
 /* ---- flat launch plan -------------------------------------------------------------------------
  * Replaces the named-DAG interpreter loop of YOLO.forward  src/yolo/model/model.py:87-107
  * The host walks the module tree once, records every op (descriptors are copied, TMA tensor
@@ -402,6 +454,7 @@ int  yre_plan_add_cbfuse_sum(yre_plan* p, const yre_view* srcs, int32_t n_src, c
 int  yre_plan_add_nchw_to_view(yre_plan* p, const float* x_nchw, const yre_view* y);
 int  yre_plan_add_view_to_nchw(yre_plan* p, const yre_view* x, float* y_nchw);
 int  yre_plan_add_decode(yre_plan* p, const yre_decode_desc* d);
+int  yre_plan_add_decode_masks(yre_plan* p, const yre_decode_masks_desc* d);
 int  yre_plan_add_nms(yre_plan* p, const yre_nms_desc* d);
 /* Re-points every recorded pointer field equal to old_ptr (image input, raw-logit / decoded /
  * NCHW outputs, residuals) to new_ptr, so one plan serves fresh input and output tensors on

@@ -10,6 +10,11 @@
 // sigmoid runs over the class logits, and the [TILE][4+nc] result leaves as one contiguous,
 // coalesced block.  Anchor coordinates come from the anchor's linear index (no anchor tensor,
 // no host sync).
+// Segmentation heads (NM = 32, yre_dfl_decode_score_masks): the same launch also copies every anchor's NM mask coefficients
+// from its level's mask-tower output into mc [B][A][NM], one coalesced 128-byte row per anchor.  Without YRE_DECODE_MASKS
+// this file compiles the detection kernel, instruction for instruction.  The mask instantiations are compiled in their own
+// translation unit (k_decode_masks.cu defines YRE_DECODE_MASKS and includes this file): ptxas allocates registers per
+// module, and kernels added to this one would change the detection kernels' register assignment.
 #include "yre_common.cuh"
 
 namespace {
@@ -27,14 +32,28 @@ struct DecodeParams {
     float* y;
 };
 
+struct MaskParams {
+    DView mask[MAXL];        // fp32 NHWC [B,Hl,Wl,>=NM] mask-tower outputs, levels as in DecodeParams::raw
+    float* mc;               // [B][A][NM]
+};
+
 __device__ __forceinline__ float sigmoid_fast(float z) {      // ex2.approx + rcp.approx: ~3e-7 abs error
     return __fdividef(1.0f, 1.0f + __expf(-z));
 }
 
 // NC > 0: class count known at compile time (80 = COCO, the common case) so every index is a constant
-// division; NC == 0: runtime class count.
+// division; NC == 0: runtime class count.  With YRE_DECODE_MASKS the kernel also takes m and copies NM = 32
+// coefficients per anchor (one per lane).
+#ifdef YRE_DECODE_MASKS
+constexpr int NM = 32;
+#define DECODE_PARAMS const DecodeParams p, const MaskParams m
+#define DECODE_ARGS p, m
+#else
+#define DECODE_PARAMS const DecodeParams p
+#define DECODE_ARGS p
+#endif
 template <typename T, int NC>
-__global__ void __launch_bounds__(WARPS * 32) decode_kernel(const DecodeParams p) {
+__global__ void __launch_bounds__(WARPS * 32) decode_kernel(DECODE_PARAMS) {
     extern __shared__ __align__(16) float sm[];
     const int nc = NC > 0 ? NC : p.nc;
     const int CH = 64 + nc;                 // logits per raw row
@@ -54,6 +73,9 @@ __global__ void __launch_bounds__(WARPS * 32) decode_kernel(const DecodeParams p
 
     // ---- per-anchor geometry (lanes 0..TILE-1 own one anchor each) ----
     long long my_src = 0; int my_lvl = 0; float my_ax = 0.f, my_ay = 0.f, my_st = 0.f;
+#ifdef YRE_DECODE_MASKS
+    long long my_msrc = 0;                            // the anchor's pixel in its mask-tower view
+#endif
     if (lane < na) {
         const int a = a0 + lane;
         int l = 0;
@@ -62,6 +84,9 @@ __global__ void __launch_bounds__(WARPS * 32) decode_kernel(const DecodeParams p
         const int W = p.raw[l].W;
         const int py = r / W, px = r - py * W;
         my_src = dview_pix(p.raw[l], b, py, px); my_lvl = l;
+#ifdef YRE_DECODE_MASKS
+        my_msrc = dview_pix(m.mask[l], b, py, px);
+#endif
         my_ax = (float)px + 0.5f; my_ay = (float)py + 0.5f; my_st = p.stride[l];
     }
     const int total = na * chunks;
@@ -167,15 +192,32 @@ __global__ void __launch_bounds__(WARPS * 32) decode_kernel(const DecodeParams p
     } else {
         for (int i = lane; i < nfl; i += 32) dst[i] = s_out[i];
     }
+
+    // ---- mask coefficients: lane k copies coefficient k of each of the tile's anchors ----
+#ifdef YRE_DECODE_MASKS
+    {
+        float v[TILE];
+#pragma unroll
+        for (int al = 0; al < TILE; ++al) {
+            const long long src = __shfl_sync(0xffffffffu, my_msrc, al);
+            const int lvl = __shfl_sync(0xffffffffu, my_lvl, al);
+            if (al < na) v[al] = static_cast<const float*>(m.mask[lvl].ptr)[src + lane];
+        }
+        float* mdst = m.mc + ((long long)b * p.A + a0) * NM;
+#pragma unroll
+        for (int al = 0; al < TILE; ++al)
+            if (al < na) mdst[al * NM + lane] = v[al];
+    }
+#endif
 }
 
 }  // namespace
 
-int launch_decode(const yre_decode_desc& d, int nb, cudaStream_t s) {
+// validates d and fills the kernel parameters, shared memory and grid of a decode launch for nb images
+static int decode_setup(const yre_decode_desc& d, int nb, DecodeParams& p, size_t& smem, dim3& grid) {
     if (d.levels < 1 || d.levels > MAXL) YRE_FAIL(YRE_EINVAL, "decode: levels=%d", d.levels);
     if (!d.y) YRE_FAIL(YRE_EINVAL, "decode: null pointer");
     if (d.nc < 1) YRE_FAIL(YRE_EINVAL, "decode: nc=%d", d.nc);
-    DecodeParams p;
     p.levels = d.levels; p.nc = d.nc; p.y = d.y;
     int A = 0;
     for (int l = 0; l < d.levels; ++l) {
@@ -196,22 +238,62 @@ int launch_decode(const yre_decode_desc& d, int nb, cudaStream_t s) {
     p.A = A; p.B = nb;                               // rows of y and raw pixels are image-major
     for (int k = 0; k < 16; ++k) p.dfl_w[k] = d.dfl_w[k];
     const int CH4 = (64 + d.nc + 3) / 4 * 4, OC = 4 + d.nc;
-    const size_t smem = (size_t)WARPS * (TILE * (CH4 + 4) + TILE * OC) * sizeof(float);
+    smem = (size_t)WARPS * (TILE * (CH4 + 4) + TILE * OC) * sizeof(float);
     const long long tiles = (long long)((A + TILE - 1) / TILE) * p.B;
-    dim3 grid((unsigned)((tiles + WARPS - 1) / WARPS));
+    grid = dim3((unsigned)((tiles + WARPS - 1) / WARPS));
     if (smem > 200 * 1024) YRE_FAIL(YRE_EUNSUPPORTED, "decode: nc=%d too large for the staging tile", d.nc);
+    return YRE_OK;
+}
+
+static int decode_launch(const yre_decode_desc& d, DECODE_PARAMS, size_t smem, dim3 grid, cudaStream_t s) {
     if (smem > 48 * 1024) {
         YRE_CUDA(cudaFuncSetAttribute(decode_kernel<float, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         YRE_CUDA(cudaFuncSetAttribute(decode_kernel<__nv_bfloat16, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     }
     const bool f32 = d.raw[0].dtype == YRE_F32;
     if (d.nc == 80) {
-        if (f32) decode_kernel<float, 80><<<grid, WARPS * 32, smem, s>>>(p);
-        else decode_kernel<__nv_bfloat16, 80><<<grid, WARPS * 32, smem, s>>>(p);
+        if (f32) decode_kernel<float, 80><<<grid, WARPS * 32, smem, s>>>(DECODE_ARGS);
+        else decode_kernel<__nv_bfloat16, 80><<<grid, WARPS * 32, smem, s>>>(DECODE_ARGS);
     } else {
-        if (f32) decode_kernel<float, 0><<<grid, WARPS * 32, smem, s>>>(p);
-        else decode_kernel<__nv_bfloat16, 0><<<grid, WARPS * 32, smem, s>>>(p);
+        if (f32) decode_kernel<float, 0><<<grid, WARPS * 32, smem, s>>>(DECODE_ARGS);
+        else decode_kernel<__nv_bfloat16, 0><<<grid, WARPS * 32, smem, s>>>(DECODE_ARGS);
     }
+    #ifdef YRE_DECODE_MASKS
+    YRE_LAUNCH_CHECK("dfl_decode_masks");
+#else
     YRE_LAUNCH_CHECK("dfl_decode_score");
+#endif
     return YRE_OK;
 }
+
+#ifndef YRE_DECODE_MASKS
+int launch_decode(const yre_decode_desc& d, int nb, cudaStream_t s) {
+    DecodeParams p;
+    size_t smem;
+    dim3 grid;
+    if (int e = decode_setup(d, nb, p, smem, grid)) return e;
+    return decode_launch(d, p, smem, grid, s);
+}
+#else
+
+int launch_decode_masks(const yre_decode_masks_desc& d, int nb, cudaStream_t s) {
+    DecodeParams p;
+    size_t smem;
+    dim3 grid;
+    if (int e = decode_setup(d.dec, nb, p, smem, grid)) return e;
+    if (d.nm != 32) YRE_FAIL(YRE_EINVAL, "decode_masks: nm=%d (32 mask coefficients only)", d.nm);
+    if (!d.mc) YRE_FAIL(YRE_EINVAL, "decode_masks: null mc");
+    MaskParams m;
+    m.mc = d.mc;
+    for (int l = 0; l < d.dec.levels; ++l) {
+        const yre_view& v = d.mask[l];
+        if (yre_check_view(&v, "decode_masks.mask")) return YRE_EINVAL;
+        if (v.layout != YRE_NHWC || v.dtype != YRE_F32 || v.C != d.nm || v.B != d.dec.raw[l].B || v.H != d.dec.raw[l].H ||
+            v.W != d.dec.raw[l].W)
+            YRE_FAIL(YRE_EINVAL, "decode_masks: mask level %d must be an fp32 NHWC [B,H,W,%d] view of raw level %d's extent", l,
+                     d.nm, l);
+        m.mask[l] = make_dview(v);
+    }
+    return decode_launch(d.dec, p, m, smem, grid, s);
+}
+#endif

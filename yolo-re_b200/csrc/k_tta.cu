@@ -23,16 +23,6 @@ struct TtaScaleParams {
     float* y;
 };
 
-// one axis of torch's bilinear source index (align_corners=False): (i0, i1, l0, l1) for destination index d
-__device__ __forceinline__ void tta_coeff(int d, float scale, int in, int& i0, int& i1, float& l0, float& l1) {
-    float src = __fsub_rn(__fmul_rn(scale, __fadd_rn((float)d, 0.5f)), 0.5f);
-    src = src < 0.f ? 0.f : src;
-    i0 = (int)src;
-    i1 = i0 + (i0 < in - 1 ? 1 : 0);
-    l1 = __fsub_rn(src, (float)i0);
-    l0 = __fsub_rn(1.f, l1);
-}
-
 template <int U8>
 __device__ __forceinline__ float tta_ld(const TtaScaleParams& p, int b, int c, int y, int x) {
     if (U8) return __fdiv_rn((float)p.xu[(((long long)b * p.H + y) * p.W + x) * 3 + (2 - c)], 255.f);   // BGR -> RGB, /255
@@ -51,8 +41,8 @@ __global__ void __launch_bounds__(256) tta_scale_kernel(const __grid_constant__ 
     }
     int y0, y1, x0, x1;
     float h0, h1, w0, w1;
-    tta_coeff(Y, p.sh, p.H, y0, y1, h0, h1);
-    tta_coeff(X, p.sw, p.W, x0, x1, w0, w1);
+    bilinear_coeff(Y, p.sh, p.H, y0, y1, h0, h1);
+    bilinear_coeff(X, p.sw, p.W, x0, x1, w0, w1);
     if (p.flip) { x0 = p.W - 1 - x0; x1 = p.W - 1 - x1; }      // column i of the mirrored image is column W-1-i
 #pragma unroll
     for (int c = 0; c < 3; ++c) {

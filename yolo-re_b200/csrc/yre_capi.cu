@@ -16,7 +16,7 @@ void yre_set_error(const char* fmt, ...) {
 
 namespace {
 
-enum OpKind { OP_CONV_FFMA, OP_CONV_TC, OP_STEM, OP_ADOWN, OP_SPP, OP_UP, OP_FUSE, OP_TO_VIEW, OP_TO_NCHW, OP_DECODE, OP_NMS };
+enum OpKind { OP_CONV_FFMA, OP_CONV_TC, OP_STEM, OP_ADOWN, OP_SPP, OP_UP, OP_FUSE, OP_TO_VIEW, OP_TO_NCHW, OP_DECODE, OP_NMS, OP_DECODE_MASKS };
 
 struct Op {
     OpKind kind;
@@ -28,6 +28,8 @@ struct Op {
     const float* fin = nullptr;
     float* fout = nullptr;
     yre_decode_desc dec;
+    yre_view mask[8];            // OP_DECODE_MASKS: the mask-tower views and mc (dec holds the rest)
+    float* mc = nullptr;
     yre_nms_desc nms;
     double flops = 0.0;
 };
@@ -38,7 +40,8 @@ int op_batch(const Op& o) {
         case OP_CONV_FFMA:
         case OP_CONV_TC:   return o.conv.y.B;
         case OP_STEM:      return o.stem.y.B;
-        case OP_DECODE:    return o.dec.raw[0].B;
+        case OP_DECODE:
+        case OP_DECODE_MASKS: return o.dec.raw[0].B;
         case OP_NMS:       return o.nms.B;
         case OP_FUSE:      return o.v[1].B;
         default:           return o.v[0].B;
@@ -59,6 +62,12 @@ int run_op(Op& o, int nb, cudaStream_t s) {
         case OP_TO_NCHW:   return launch_view_to_nchw(o.v[0], o.fout, nb, s);
         case OP_DECODE:    return launch_decode(o.dec, nb, s);
         case OP_NMS:       return launch_nms(o.nms, nb, s);
+        case OP_DECODE_MASKS: {
+            yre_decode_masks_desc d;
+            d.dec = o.dec; d.nm = 32; d.mc = o.mc;
+            for (int l = 0; l < 8; ++l) d.mask[l] = o.mask[l];
+            return launch_decode_masks(d, nb, s);
+        }
     }
     return YRE_EINVAL;
 }
@@ -76,6 +85,7 @@ const char* op_name(OpKind k) {
         case OP_TO_NCHW:   return "view_to_nchw";
         case OP_DECODE:    return "dfl_decode_score";
         case OP_NMS:       return "nms";
+        case OP_DECODE_MASKS: return "dfl_decode_masks";
     }
     return "?";
 }
@@ -195,6 +205,10 @@ int yre_dfl_decode_score(const yre_decode_desc* d, yre_stream_t s) {
     if (!d) YRE_FAIL(YRE_EINVAL, "decode: null descriptor");
     return launch_decode(*d, d->raw[0].B, (cudaStream_t)s);
 }
+int yre_dfl_decode_score_masks(const yre_decode_masks_desc* d, yre_stream_t s) {
+    if (!d) YRE_FAIL(YRE_EINVAL, "decode_masks: null descriptor");
+    return launch_decode_masks(*d, d->dec.raw[0].B, (cudaStream_t)s);
+}
 int yre_nms_batched(const yre_nms_desc* d, yre_stream_t s) {
     if (!d) YRE_FAIL(YRE_EINVAL, "nms: null descriptor");
     return launch_nms(*d, d->B, (cudaStream_t)s);
@@ -296,6 +310,15 @@ int yre_plan_add_decode(yre_plan* p, const yre_decode_desc* d) {
     p->ops.push_back(o);
     return YRE_OK;
 }
+int yre_plan_add_decode_masks(yre_plan* p, const yre_decode_masks_desc* d) {
+    PLAN_GUARD(p);
+    if (!d) YRE_FAIL(YRE_EINVAL, "decode_masks: null descriptor");
+    if (d->nm != 32) YRE_FAIL(YRE_EINVAL, "decode_masks: nm=%d (32 mask coefficients only)", d->nm);
+    Op o; o.kind = OP_DECODE_MASKS; o.dec = d->dec; o.mc = d->mc;
+    for (int l = 0; l < 8; ++l) o.mask[l] = d->mask[l];
+    p->ops.push_back(o);
+    return YRE_OK;
+}
 int yre_plan_add_nms(yre_plan* p, const yre_nms_desc* d) {
     PLAN_GUARD(p);
     if (!d) YRE_FAIL(YRE_EINVAL, "nms: null descriptor");
@@ -332,8 +355,13 @@ int yre_plan_rebind(yre_plan* p, const void* old_ptr, void* new_ptr) {
                 fix(o.stem.y.ptr);
                 break;
             case OP_DECODE:
+            case OP_DECODE_MASKS:
                 for (int l = 0; l < o.dec.levels; ++l) fix(o.dec.raw[l].ptr);
                 if (o.dec.y == old_ptr) { o.dec.y = (float*)new_ptr; ++n; }
+                if (o.kind == OP_DECODE_MASKS) {
+                    for (int l = 0; l < o.dec.levels; ++l) fix(o.mask[l].ptr);
+                    if (o.mc == old_ptr) { o.mc = (float*)new_ptr; ++n; }
+                }
                 break;
             case OP_NMS:
                 if (o.nms.pred == old_ptr) { o.nms.pred = (const float*)new_ptr; ++n; }

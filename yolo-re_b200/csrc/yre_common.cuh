@@ -164,6 +164,18 @@ template <> __device__ __forceinline__ void st8<__half>(void* p, long long i, co
     *reinterpret_cast<uint4*>((__half*)p + i) = u;
 }
 
+// One axis of torch's bilinear source index (F.interpolate(mode="bilinear", align_corners=False), size given): scale is
+// (float)in / out; returns (i0, i1, l0, l1) for destination index d, fp32 with every rounding explicit (no contraction).
+// Shared by K12 (TTA resize) and K15 (mask upsampling).
+__device__ __forceinline__ void bilinear_coeff(int d, float scale, int in, int& i0, int& i1, float& l0, float& l1) {
+    float src = __fsub_rn(__fmul_rn(scale, __fadd_rn((float)d, 0.5f)), 0.5f);
+    src = src < 0.f ? 0.f : src;
+    i0 = (int)src;
+    i1 = i0 + (i0 < in - 1 ? 1 : 0);
+    l1 = __fsub_rn(src, (float)i0);
+    l0 = __fsub_rn(1.f, l1);
+}
+
 __device__ __forceinline__ float silu_f(float v) { return v / (1.0f + __expf(-v)); }
 // SiLU with ONE MUFU op: x*sigmoid(x) = 0.5x*(1 + tanh(0.5x)); tanh.approx is good to ~2^-11 relative,
 // far inside bf16's 2^-8 -- used wherever the result is rounded to bf16 anyway.
@@ -196,6 +208,7 @@ int launch_cbfuse_sum(const yre_view* srcs, int n, const yre_view& target, const
 int launch_nchw_to_view(const float* x, const yre_view& y, int nb, cudaStream_t s);
 int launch_view_to_nchw(const yre_view& x, float* y, int nb, cudaStream_t s);
 int launch_decode(const yre_decode_desc& d, int nb, cudaStream_t s);
+int launch_decode_masks(const yre_decode_masks_desc& d, int nb, cudaStream_t s);   // K6 that also gathers mask coefficients
 int launch_nms(const yre_nms_desc& d, int nb, cudaStream_t s);   // 3 launches (memset kernel, filter, sort+scan)
 int launch_nms_multi_label(const yre_nms_desc& d, int nb, cudaStream_t s);   // same, every class above conf_thres
 double conv_flops(const yre_conv_desc& d);

@@ -10,7 +10,9 @@ from .nms import PendingDetections, nms_raw, non_max_suppression, non_max_suppre
 from .preprocess import letterbox, preprocess, scale_boxes, scale_rows
 from .checkpoint import convert_upstream_state_dict, load_checkpoint
 from .metrics import DetectionAccumulator, Evaluator, compute_map, match_detections
+from .seg import masks_raw, process_mask, process_mask_native
 
 __version__ = "0.2.0"
 __all__ = ["YOLO", "non_max_suppression", "non_max_suppression_async", "PendingDetections", "scale_rows", "nms_raw", "precision", "YreError", "lib", "ModelConfig", "parse_yaml",
-           "build_layers", "BLOCKS", "letterbox", "preprocess", "scale_boxes", "convert_upstream_state_dict", "load_checkpoint", "compute_map", "match_detections", "DetectionAccumulator", "Evaluator"]
+           "build_layers", "BLOCKS", "letterbox", "preprocess", "scale_boxes", "convert_upstream_state_dict", "load_checkpoint", "compute_map", "match_detections", "DetectionAccumulator", "Evaluator",
+           "masks_raw", "process_mask", "process_mask_native"]

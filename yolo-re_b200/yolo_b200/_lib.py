@@ -46,6 +46,10 @@ class DecodeDesc(C.Structure):
                 ("dfl_w", C.c_float * 16), ("y", C.c_void_p)]
 
 
+class DecodeMasksDesc(C.Structure):
+    _fields_ = [("dec", DecodeDesc), ("mask", View * 8), ("nm", C.c_int32), ("mc", C.c_void_p)]
+
+
 class NmsDesc(C.Structure):
     _fields_ = [("pred", C.c_void_p), ("B", C.c_int32), ("A", C.c_int32), ("nc", C.c_int32),
                 ("conf_thres", C.c_float), ("iou_thres", C.c_double), ("max_det", C.c_int32),
@@ -98,6 +102,16 @@ class TtaMergeBranch(C.Structure):
 class TtaMergeDesc(C.Structure):
     _fields_ = [("br", TtaMergeBranch * TTA_BRANCHES), ("B", C.c_int32), ("n", C.c_int32), ("nc", C.c_int32), ("out", C.c_void_p)]
 
+MASK_PROTO, MASK_INPUT, MASK_NATIVE = 0, 1, 2
+
+
+class MaskDesc(C.Structure):
+    _fields_ = [("proto", C.c_void_p)] + [(n, C.c_int32) for n in ("B", "n", "mh", "mw", "nm", "proto_pitch")] + \
+               [("mc", C.c_void_p), ("A", C.c_int32), ("det", C.c_void_p), ("counts", C.c_void_p), ("keep_anchor", C.c_void_p),
+                ("max_det", C.c_int32), ("mode", C.c_int32), ("in_h", C.c_int32), ("in_w", C.c_int32), ("scale", C.c_void_p),
+                ("masks", C.c_void_p), ("out_h", C.c_int32), ("out_w", C.c_int32)]
+
+
 # name -> (restype, argtypes); every symbol include/yre.h declares
 SYMBOLS = {
     "yre_version": (C.c_int, []),
@@ -114,6 +128,7 @@ SYMBOLS = {
     "yre_nchw_to_view": (C.c_int, [C.c_void_p, C.POINTER(View), C.c_void_p]),
     "yre_view_to_nchw": (C.c_int, [C.POINTER(View), C.c_void_p, C.c_void_p]),
     "yre_dfl_decode_score": (C.c_int, [C.POINTER(DecodeDesc), C.c_void_p]),
+    "yre_dfl_decode_score_masks": (C.c_int, [C.POINTER(DecodeMasksDesc), C.c_void_p]),
     "yre_nms_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int32]),
     "yre_nms_batched": (C.c_int, [C.POINTER(NmsDesc), C.c_void_p]),
     "yre_nms_filter_only": (C.c_int, [C.POINTER(NmsDesc), C.c_void_p]),
@@ -131,6 +146,7 @@ SYMBOLS = {
     "yre_tta_geometry": (C.c_int, [C.c_int32, C.c_int32, C.POINTER(TtaGeom)]),
     "yre_tta_scale_img": (C.c_int, [C.POINTER(TtaScaleDesc), C.c_void_p]),
     "yre_tta_merge": (C.c_int, [C.POINTER(TtaMergeDesc), C.c_void_p]),
+    "yre_seg_masks": (C.c_int, [C.POINTER(MaskDesc), C.c_void_p]),
     "yre_plan_create": (C.c_int, [C.POINTER(C.c_void_p)]),
     "yre_plan_destroy": (None, [C.c_void_p]),
     "yre_plan_add_conv": (C.c_int, [C.c_void_p, C.POINTER(ConvDesc)]),
@@ -142,6 +158,7 @@ SYMBOLS = {
     "yre_plan_add_nchw_to_view": (C.c_int, [C.c_void_p, C.c_void_p, C.POINTER(View)]),
     "yre_plan_add_view_to_nchw": (C.c_int, [C.c_void_p, C.POINTER(View), C.c_void_p]),
     "yre_plan_add_decode": (C.c_int, [C.c_void_p, C.POINTER(DecodeDesc)]),
+    "yre_plan_add_decode_masks": (C.c_int, [C.c_void_p, C.POINTER(DecodeMasksDesc)]),
     "yre_plan_add_nms": (C.c_int, [C.c_void_p, C.POINTER(NmsDesc)]),
     "yre_plan_rebind": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p]),
     "yre_plan_run": (C.c_int, [C.c_void_p, C.c_void_p]),

@@ -29,7 +29,7 @@ import torch.nn as nn
 
 from . import _lib as L
 from . import blocks as B
-from .heads import REG_MAX, DetectDFL, DualDetectDFL
+from .heads import REG_MAX, DetectDFL, DualDetectDFL, SegmentDFL
 
 _DEFAULT_PRECISION = "bf16"
 # per precision: (libyre activation dtype, torch dtype)
@@ -410,6 +410,14 @@ class Plan:
     def towers(self, box, cls, dfl, feats: list[V], strides: list[float], nc: int):
         """One head: per level first 3x3 of box and cls (merged into one GEMM on the small levels), the two
         towers, fp32 raw logits; then K6."""
+        raws = self.tower_convs(box, cls, feats, nc)
+        y, d = self.decode_desc(raws, strides, nc, dfl)
+        L.check(self.lib.yre_plan_add_decode(self.h, C.byref(d)), "plan_add_decode")
+        self.trace.append(("decode", dict(raws=raws, strides=list(strides), nc=nc, dfl_w=list(d.dfl_w), y=y)))
+        return y, raws
+
+    def tower_convs(self, box, cls, feats: list[V], nc: int) -> list[V]:
+        """The box and class towers of every level: the fp32 raw-logit windows [B,H,W,64+nc]."""
         raws = []
         for i, f in enumerate(feats):
             c2 = box[i][0].conv.out_channels
@@ -438,6 +446,10 @@ class Plan:
             self.conv(hc, fc.w, fc.b, fc.k, fc.stride, fc.silu, out=raw_full.sl(4 * REG_MAX, ncp), name=self.name_of(cls[i][2]),
                       key=("conv", self.name_of(cls[i][2]), "classes padded to", ncp))
             raws.append(raw)
+        return raws
+
+    def decode_desc(self, raws: list[V], strides: list[float], nc: int, dfl) -> tuple[torch.Tensor, L.DecodeDesc]:
+        """y [B,A,4+nc] (allocated here) and the K6 descriptor that fills it from the raw logits"""
         A = sum(r.H * r.W for r in raws)
         y = self.empty((self.batch, A, 4 + nc), torch.float32)
         d = L.DecodeDesc()
@@ -449,12 +461,35 @@ class Plan:
         for k in range(REG_MAX):
             d.dfl_w[k] = wd[k]
         d.y = y.data_ptr()
-        L.check(self.lib.yre_plan_add_decode(self.h, C.byref(d)), "plan_add_decode")
-        self.trace.append(("decode", dict(raws=raws, strides=list(strides), nc=nc, dfl_w=wd, y=y)))
-        return y, raws
+        return y, d
+
+    def segment(self, m: SegmentDFL, feats: list[V], strides: list[float]):
+        """A segmentation head: the detection towers exactly as DetectDFL's, then the prototype branch on the first level
+        (K1 convs around a K5 nearest upsample: its consumer is a 3x3 conv, which cannot read it through a tensor map;
+        the last conv writes fp32 NHWC [B,H/4,W/4,nm]), then the mask-coefficient towers (fp32 [B,Hl,Wl,nm]), then K6
+        writing y and mc [B,A,nm] in one launch."""
+        if m.num_masks != 32:
+            raise L.YreError(f"segmentation head with {m.num_masks} masks: the kernels take 32 mask coefficients only")
+        nc = m.num_classes
+        raws = self.tower_convs(m.box_convs, m.cls_convs, feats, nc)
+        pr = m.proto
+        proto = self.conv_m(pr.cv3, self.conv_m(pr.cv2, self.upsample(self.conv_m(pr.cv1, feats[0]), None)), out_dtype=L.F32)
+        masks = []
+        for i, f in enumerate(feats):
+            t = m.mask_convs[i]
+            masks.append(self.conv_m(t[2], self.conv_m(t[1], self.conv_m(t[0], f)), out_dtype=L.F32))
+        y, d = self.decode_desc(raws, strides, nc, m.dfl)
+        mc = self.empty((self.batch, y.shape[1], m.num_masks), torch.float32)
+        dm = L.DecodeMasksDesc(d, (L.View * 8)(*[v.c() for v in masks]), m.num_masks, mc.data_ptr())
+        L.check(self.lib.yre_plan_add_decode_masks(self.h, C.byref(dm)), "plan_add_decode_masks")
+        # recorded as a decode (what the detection path checks) with the mask views and mc alongside
+        self.trace.append(("decode", dict(raws=raws, strides=list(strides), nc=nc, dfl_w=list(d.dfl_w), y=y, masks=masks, mc=mc)))
+        return ("segment", y, [raws, mc, proto])
 
     def detect(self, m, feats: list[V], main_only: bool = False):
         strides = m.stride.tolist()
+        if isinstance(m, SegmentDFL):
+            return self.segment(m, feats, strides)
         if isinstance(m, DetectDFL):
             y, raws = self.towers(m.box_convs, m.cls_convs, m.dfl, feats, strides, m.num_classes)
             return ("single", y, raws)
@@ -784,6 +819,10 @@ def model_forward(model, x: torch.Tensor, augment: bool = False):
     cap = _capacity(model, x)
     max_hw = _max_shape(model, x)
     if augment:
+        _, head = model._detect_layer()
+        if isinstance(head, SegmentDFL):
+            raise ValueError("augment=True: test-time augmentation is defined for detection heads only (upstream has no "
+                             "segmentation TTA)")
         from .tta import forward_augment
         with torch.cuda.device(x.device):
             return forward_augment(model, x, cap, max_hw)
@@ -903,15 +942,20 @@ def _first_rows(obj, n: int):
 
 
 def _head_outputs(result):
-    """forward's value for a head result: (y[B,4+nc,A], [raw_i NCHW]), or ([y_aux, y_main], [raws_aux, raws_main])"""
+    """forward's value for a head result: (y[B,4+nc,A], [raw_i NCHW]), or ([y_aux, y_main], [raws_aux, raws_main]), or
+    for a segmentation head (y[B,4+nc,A], ([raw_i NCHW], mc[B,nm,A], proto[B,nm,H/4,W/4])), mc and proto views of
+    their A x nm and NHWC buffers"""
     kind, y, raws = result
     if kind == "single":
         return y.permute(0, 2, 1), [_raw_nchw(r) for r in raws]
+    if kind == "segment":
+        rs, mc, proto = raws
+        return y.permute(0, 2, 1), ([_raw_nchw(r) for r in rs], mc.permute(0, 2, 1), _raw_nchw(proto))
     return [t.permute(0, 2, 1) for t in y], [[_raw_nchw(r) for r in rs] for rs in raws]
 
 
 def _raw_nchw(r: "V") -> torch.Tensor:
-    """[B,64+nc,H,W] view of a raw-logit buffer (its channel count may be padded, towers())."""
+    """[B,C,H,W] view of a raw-logit or prototype buffer (a raw buffer's channel count may be padded, towers())."""
     t = r.t if r.C == r.C_total else r.t[..., r.c_off:r.c_off + r.C]
     return t.permute(0, 3, 1, 2)
 

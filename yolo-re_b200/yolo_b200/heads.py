@@ -1,6 +1,7 @@
 """Detection heads (parameter containers; see blocks.py for why they look the way they do).
 
-Reference: src/yolo/heads/detect.py:22-295, src/yolo/heads/dfl.py:14-50."""
+Reference: src/yolo/heads/detect.py:22-295, src/yolo/heads/dfl.py:14-50.  SegmentDFL: upstream YOLOv9's Proto
+(models/common.py) and Segment (models/yolo.py) on top of DetectDFL."""
 from __future__ import annotations
 
 import math
@@ -82,3 +83,27 @@ class DualDetectDFL(_EngineModule):
     def init_bias(self) -> None:
         _init_tower_bias(self.aux_box_convs, self.aux_cls_convs, self.stride, self.num_classes)
         _init_tower_bias(self.main_box_convs, self.main_cls_convs, self.stride, self.num_classes)
+
+
+class Proto(nn.Module):
+    """Mask prototypes (upstream models/common.py Proto): Conv 3x3 -> nearest x2 upsample -> Conv 3x3 -> Conv 1x1."""
+
+    def __init__(self, in_channels: int, num_protos: int = 256, num_masks: int = 32):
+        super().__init__()
+        self.cv1 = Conv(in_channels, num_protos, 3)
+        self.cv2 = Conv(num_protos, num_protos, 3)
+        self.cv3 = Conv(num_protos, num_masks, 1)
+
+
+class SegmentDFL(DetectDFL):
+    """DetectDFL plus upstream's instance-segmentation parts: the prototype branch on the first (stride-8) input and one
+    mask-coefficient tower per level, Conv 3x3 -> Conv 3x3 -> Conv2d 1x1 (bias, no activation) with
+    c4 = max(ch0 // 4, num_masks) channels (upstream models/yolo.py Segment)."""
+
+    def __init__(self, num_classes: int, in_channels: tuple[int, ...], num_masks: int = 32, num_protos: int = 256):
+        super().__init__(num_classes, in_channels)
+        self.num_masks, self.num_protos = num_masks, num_protos
+        self.proto = Proto(in_channels[0], num_protos, num_masks)
+        c4 = max(in_channels[0] // 4, num_masks)
+        self.mask_convs = nn.ModuleList(nn.Sequential(Conv(ch, c4, 3), Conv(c4, c4, 3), nn.Conv2d(c4, num_masks, 1))
+                                        for ch in in_channels)

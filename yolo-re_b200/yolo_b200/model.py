@@ -3,7 +3,8 @@
 Same public surface as the reference's ``yolo.model.model.YOLO`` (src/yolo/model/model.py:20-238):
 ``YOLO.from_yaml / from_config``, ``.layers`` (nn.ModuleDict), ``.connections``, ``.detect_inputs``,
 ``forward(x[B,C,H,W])`` returning ``(y[B,4+nc,A], [raw_i[B,64+nc,Hi,Wi]])`` in eval mode (dual
-head: ``([y_aux, y_main], [raws_aux, raws_main])``), ``state_dict``-compatible weights, model
+head: ``([y_aux, y_main], [raws_aux, raws_main])``; segmentation head, upstream YOLOv9's gelan-c-seg:
+``(y, (raws, mc[B,32,A], proto[B,32,H/4,W/4]))``), ``state_dict``-compatible weights, model
 returned in TRAIN mode (model.py:163), ``detect.stride`` a plain tensor attribute.
 
 Differences by design: eval-mode forward is one replay of a pre-compiled libyre launch plan on the
@@ -26,7 +27,7 @@ import torch.nn as nn
 import yaml
 
 from . import blocks as B
-from .heads import DetectDFL, DualDetectDFL
+from .heads import DetectDFL, DualDetectDFL, SegmentDFL
 
 
 @dataclass
@@ -59,7 +60,7 @@ _STANDARD = {"Conv": B.Conv, "ADown": B.ADown, "RepNCSPELAN4": B.RepNCSPELAN4, "
 # exported like the reference's registry (src/yolo/model/registry.py:14-26)
 BLOCKS: dict[str, type[nn.Module]] = {**_STANDARD, "Concat": B.Concat, "Silence": B.Silence, "CBLinear": B.CBLinear,
                                       "CBFuse": B.CBFuse, "DetectDFL": DetectDFL, "DualDetectDFL": DualDetectDFL,
-                                      "Upsample": B.Upsample}
+                                      "SegmentDFL": SegmentDFL, "Upsample": B.Upsample}
 
 
 def build_layers(config: ModelConfig, input_channels: int = 3):
@@ -78,8 +79,8 @@ def build_layers(config: ModelConfig, input_channels: int = 3):
             raise TypeError(f"from must be str or list[str], got {type(frm)}")
         connections[name] = frm
         cin = [chan[n] for n in frm] if isinstance(frm, list) else [chan[frm]]
-        if kind in ("DetectDFL", "DualDetectDFL"):
-            block, cout = BLOCKS[kind](config.num_classes, tuple(cin)), 0
+        if kind in ("DetectDFL", "DualDetectDFL", "SegmentDFL"):
+            block, cout = BLOCKS[kind](config.num_classes, tuple(cin), **p), 0
             detect_inputs = frm if isinstance(frm, list) else [frm]
         elif kind == "Concat":
             block, cout = B.Concat(p.get("dimension", 1)), sum(cin)
